@@ -8,11 +8,11 @@ travels to the GPU box with the repo snapshot (`/root/reference` does not exist 
    offline wheelhouse carries (the outcome is recorded in baseline/_ref/INSTALL.json).
 2. Fallback, equivalent to what the install would have produced for a pure-Python distribution: the package directory
    `pytorch_bayesian/` copied file by file.  Nothing is edited.
-Also copied, for the reference arm of bench.py and the alias tests: the three ELBO example model definitions
-(examples/{MNIST,FashionMNIST,CIFAR10}/model.py) and the reference's own tests/ + conftest.py.
+Also copied, for the reference arm of bench.py: the three ELBO example model definitions
+(examples/{MNIST,FashionMNIST,CIFAR10}/model.py).
 
-Nothing under baseline/_ref is imported by the product package; users are bench.py --impl reference, the
-"reference classes on CUDA" comparator and tests that run the reference's own test-suite against the drop-in.
+Nothing under baseline/_ref is imported by the product package or the tests; users are bench.py --impl reference and
+the "reference classes on CUDA" comparator.
 """
 import argparse
 import json
@@ -51,9 +51,6 @@ def install(reference="/root/reference", quiet=False):
         dst = os.path.join(TARGET, "examples", name)
         os.makedirs(dst, exist_ok=True)
         shutil.copy(os.path.join(reference, "examples", name, "model.py"), os.path.join(dst, "model.py"))
-    shutil.copytree(os.path.join(reference, "tests"), os.path.join(TARGET, "tests"),
-                    ignore=shutil.ignore_patterns("__pycache__"))
-    shutil.copy(os.path.join(reference, "conftest.py"), os.path.join(TARGET, "conftest.py"))
     with open(os.path.join(TARGET, "INSTALL.json"), "w") as fh:
         json.dump(record, fh, indent=1)
     if not quiet:

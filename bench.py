@@ -2,6 +2,7 @@
 """bench.py — ELBO training throughput of the variational hot path on B200 (driver contract).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload c3|c2|c4]
+                    [--dump-outputs DIR]
 
 Metric (BASELINE.json): ELBO train samples*MC/sec = (rows x Monte-Carlo samples evaluated by all ranks) / step time, where
 one step is the body of the reference's training loop, examples/MNIST/train.py:55-65: zero_grad -> model(x) (S
@@ -37,6 +38,7 @@ import sys
 import threading
 import time
 
+import numpy as np
 import torch
 import torch.nn.functional as F
 
@@ -252,10 +254,51 @@ class Env:
         return float(t)
 
 
+def dump_outputs(out_dir, arrays, budget_bytes=64 << 20, seed=0):
+    """Writes each tensor of `arrays` as out_dir/<name>.npy (float64 stays float64, other floating point types become
+    float32, integers float64), at most `budget_bytes` in all.  When the arrays do not fit, every array larger than an
+    even share of the budget is replaced by a fixed, seeded sample of its flattened elements: the same indices in every
+    run, in ascending order."""
+    os.makedirs(out_dir, exist_ok=True)
+    cap = budget_bytes // (8 * len(arrays))
+    sample = sum(t.numel() for t in arrays.values()) * 8 > budget_bytes
+    for name, t in arrays.items():
+        t = t.detach()
+        if sample and t.numel() > cap:
+            idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(seed))[:cap].sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        dtype = torch.float64 if t.dtype == torch.float64 or not t.is_floating_point() else torch.float32
+        np.save(os.path.join(out_dir, name + ".npy"), t.to("cpu", dtype).contiguous().numpy())
+
+
+def reset_training_state(model, trainer, initial):
+    """Puts the model and its trainer back, in place, into the state before their first training step: parameters and
+    buffers from `initial`, the optimizer's moments and step counts and the library's device-side Philox step counter to
+    zero.  In-place copies keep the addresses a captured CUDA graph holds.
+
+    Every timed step starts from this state, so what a step computes depends on its batch alone, not on the rounding of
+    the steps before it: the weight and bias gradients sum their per-sample partials with atomic adds, whose order (and
+    last bits) changes from run to run, and over a trajectory Adam turns such differences into whole learning-rate
+    steps on gradient components that are mostly rounding.  The work of a step does not depend on these values."""
+    from bayesianneuralnetworks_b200 import runtime
+    opt = trainer.opt
+    zeros = [t for o in (opt, getattr(opt, "_torch_adam", None)) if o is not None
+             for st in o.state.values() for t in st.values() if torch.is_tensor(t)]
+    zeros += list(getattr(opt, "_step_dev", {}).values())
+    counter = runtime.step_counter(trainer.device)
+    if counter is not None:
+        zeros.append(counter)
+    with torch.no_grad():
+        state = model.state_dict()
+        torch._foreach_copy_(list(state.values()), [initial[name] for name in state])
+        torch._foreach_zero_(zeros)
+
+
 def measure_step(env, workload, steps, warmup, precision, parallel_mode, with_e2e=True, with_roofline=True,
-                 channels_last=True, exchange="auto"):
+                 channels_last=True, exchange="auto", dump_dir=None):
     """Builds the workload's ElboTrainer, times `steps` device-resident steps (and, with_e2e, as many host-fed ones) and
-    returns the measurements of this workload as a dict (rank 0: complete; other ranks: timing only)."""
+    returns the measurements of this workload as a dict (rank 0: complete; other ranks: timing only).  With `dump_dir`,
+    rank 0 writes the loss and the model state of the last device-resident step there (dump_outputs)."""
     import bayesianneuralnetworks_b200 as bnn
     from bayesianneuralnetworks_b200 import _C, parallel
     from bayesianneuralnetworks_b200.training import ElboTrainer
@@ -286,6 +329,7 @@ def measure_step(env, workload, steps, warmup, precision, parallel_mode, with_e2
         for m in model.modules():        # layout conversions around each call; (mu, rho) stay row-major OIHW
             if isinstance(m, (torch.nn.Conv2d, torch.nn.BatchNorm2d)):
                 m.to(memory_format=torch.channels_last)
+    initial = {name: t.detach().clone() for name, t in model.state_dict().items()}
     trainer = ElboTrainer(model, N_BATCHES, lr=1e-3, graph=not args.no_graph, optimizer=args.optimizer,
                           loss_tail=args.loss_tail, exchange=exchange, sample_groups=sample_groups)
     gen = torch.Generator().manual_seed(1 + trainer.data_index)      # a data group shares its batch slice
@@ -294,7 +338,8 @@ def measure_step(env, workload, steps, warmup, precision, parallel_mode, with_e2
     dev = [(x.to(device), y.to(device)) for x, y in host]
 
     def timed(n_steps, feed_from_host):
-        """K steps, each bracketed by CUDA events on the current stream; L2 flushed (untimed) between steps."""
+        """K steps, each bracketed by CUDA events on the current stream; before each step (untimed) the training state
+        is reset (reset_training_state) and L2 is flushed."""
         starts = [torch.cuda.Event(enable_timing=True) for _ in range(n_steps)]
         stops = [torch.cuda.Event(enable_timing=True) for _ in range(n_steps)]
         env.barrier()
@@ -303,6 +348,7 @@ def measure_step(env, workload, steps, warmup, precision, parallel_mode, with_e2
         if feed_from_host:
             trainer.prefetch(*host[0])    # as a DataLoader does: the first batch is in flight before the loop starts
         for i in range(n_steps):
+            reset_training_state(model, trainer, initial)
             env.flush.zero_()
             starts[i].record()
             x, y = host[i % n_host] if feed_from_host else dev[i % n_host]
@@ -315,7 +361,7 @@ def measure_step(env, workload, steps, warmup, precision, parallel_mode, with_e2
         wall = time.perf_counter() - w0
         env.clocks.mark(t0, time.time())
         ms = sum(a.elapsed_time(b) for a, b in zip(starts, stops))
-        return ms / 1e3, wall, last, (t0, time.time())
+        return ms / 1e3, wall, last, (t0, time.time()), loss
 
     graph_note = "eager launches"
     if trainer.use_graph:
@@ -333,15 +379,18 @@ def measure_step(env, workload, steps, warmup, precision, parallel_mode, with_e2
     for i in range(max(warmup, 3)):
         trainer.step(*dev[i % n_host])
     launches0 = _C.launch_count
-    dev_s, dev_wall, _, window = timed(steps, False)
+    dev_s, dev_wall, _, window, step_loss = timed(steps, False)
     launches = _C.launch_count - launches0
+    if dump_dir is not None and env.rank == 0:
+        # what a caller of the last timed step holds: its loss and the model state it left behind
+        dump_outputs(dump_dir, {"loss": step_loss, **{"model." + k: v for k, v in model.state_dict().items()}})
     if trainer.graph is not None:
         launches = trainer.launches_per_step * steps      # replays launch the captured kernels
     res = {"ms_per_step": None}
     e2e_s = e2e_wall = last_loss = None
     if with_e2e:
         timed(2, True)                                    # untimed: first touch of the staging path
-        e2e_s, e2e_wall, last_loss, _ = timed(steps, True)
+        e2e_s, e2e_wall, last_loss, _, _ = timed(steps, True)
         e2e_s = env.max_over_ranks(e2e_s)
     dev_s = env.max_over_ranks(dev_s)
     units = B * data_groups * S_global * steps
@@ -380,6 +429,8 @@ def measure_step(env, workload, steps, warmup, precision, parallel_mode, with_e2
                    else "contiguous (NCHW, the examples' layout)",
                    "launch": graph_note,
                    "l2": "flushed between steps (256 MiB write, untimed); each step timed with its own CUDA event pair",
+                   "training_state": "every timed step starts from the state before the first training step (parameters, "
+                                     "buffers, optimizer moments, RNG step counters; restored in place, untimed)",
                    "step": "zero_grad+forward(S)+KL+CE+backward+" + ("exchange+" if world > 1 else "") + "Adam"},
         "dtype": "tf32" if tf32 else "fp32 (3xTF32 split on tcgen05)",
         "gpu_launches": launches, "wall_s": dev_wall, "clocks": env.clocks.summary([window]),
@@ -820,7 +871,7 @@ def run_b200(args):
     env.pk.update(tf32_burst=tf32_peak["burst_tflops"], tf32_sustained=tf32_peak["sustained_tflops"])
     main_mode = {"c4": "sample"}.get(args.workload, "grid") if args.parallel == "auto" else args.parallel
     main = measure_step(env, args.workload, args.steps, args.warmup, args.precision, main_mode,
-                        channels_last=not args.nchw_trunk, exchange=args.exchange)
+                        channels_last=not args.nchw_trunk, exchange=args.exchange, dump_dir=args.dump_outputs)
     out = {
         "metric": "ELBO train samples*MC/sec", "value": main["value"], "unit": "samples*MC/s", "n_gpus": world,
         "steps": args.steps, "warmup": max(args.warmup, 3), "ms_per_step": main["ms_per_step"],
@@ -900,7 +951,15 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="only the main workload (profiling runs)")
     ap.add_argument("--tf32-peak", type=float, default=0.0,
                     help="skip the in-run cuBLAS TF32 peak measurement and use this TFLOP/s figure (runs under a profiler)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps of the main workload, write the loss and the model state of its last step "
+                         "as DIR/<name>.npy (at most 64 MiB; larger arrays as a fixed, seeded sample), for comparing two "
+                         "builds output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     if args.impl == "reference":
         run_reference(args)
     else:

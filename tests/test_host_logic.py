@@ -334,47 +334,6 @@ def test_fused_cross_entropy_eligibility_and_gradient_buffers():
         _C.mc_cross_entropy_fwd(torch.zeros(4, 3), torch.zeros(2, dtype=torch.int64))
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/examples"), reason="the reference checkout is only mounted in the build container")
-def test_reference_example_models_construct_unchanged_on_the_drop_in():
-    """INTEGRATION.md option A: with `pytorch_bayesian` aliased to this package the reference's own example model files
-    (examples/{MNIST,FashionMNIST,CIFAR10}/model.py, executed unmodified from the read-only checkout) import, build their
-    networks, expose the reference's state_dict layout and load the shipped checkpoints.  (Forward needs the B200.)"""
-    import importlib.util
-    import sys
-    saved = {k: sys.modules.get(k) for k in ("pytorch_bayesian", "pytorch_bayesian.nn", "pytorch_bayesian.prune",
-                                             "pytorch_bayesian.utils")}
-    sys.modules.update({"pytorch_bayesian": bnn, "pytorch_bayesian.nn": bnn.nn, "pytorch_bayesian.prune": bnn.prune,
-                        "pytorch_bayesian.utils": bnn.utils})
-    try:
-        for example, cls, in_ch, ckpt in (("MNIST", "BCNN", 1, "mnist_pretrained.pth"),
-                                          ("FashionMNIST", "BCNN", 1, "fmnist_pretrained.pth"),
-                                          ("CIFAR10", "BCNN", 3, None)):
-            path = f"/root/reference/examples/{example}/model.py"
-            spec = importlib.util.spec_from_file_location(f"_ref_example_{example}", path)
-            mod = importlib.util.module_from_spec(spec)
-            spec.loader.exec_module(mod)
-            model = getattr(mod, cls)(in_ch, 10)
-            assert isinstance(model, bnn.nn.BayesianNetworkModule)
-            keys = model.state_dict().keys()
-            assert any(k.endswith("weight.mean") for k in keys) and any(k.endswith("weight.scale") for k in keys)
-            n_bayes = sum(isinstance(m, bnn.nn.BayesianModule) for m in model.modules())
-            assert n_bayes == 2
-            if ckpt and os.path.exists(f"/root/reference/examples/{example}/{ckpt}"):
-                sd = torch.load(f"/root/reference/examples/{example}/{ckpt}", map_location="cpu")
-                model.load_state_dict(sd)                      # same keys, same shapes
-            # their own Flatten is user code without state: eligible for the batched forward, probed at run time.
-            # MNIST (NormalConv2d + NormalLinear) runs on the fused kernels; the Flipout layers of FashionMNIST (f-1)
-            # and the full-covariance head of CIFAR10 (f-4) are torch composites that join the batched pass
-            plan = model._mc_plan()
-            assert plan.ok and [type(m) for m in plan.probes] == [mod.Flatten]
-    finally:
-        for k, v in saved.items():
-            if v is None:
-                sys.modules.pop(k, None)
-            else:
-                sys.modules[k] = v
-
-
 def test_elbo_adam_plans_the_same_tensors_and_coefficients_as_kl_divergence():
     """bnn.optim.ELBOAdam folds the gradient of KLDivergence(n_batches)(model) into its step: it must see the tensors the
     reference's traverse sees (weights and biases as separate entries, loss.py:30-38), give each the coefficient

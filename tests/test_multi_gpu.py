@@ -98,7 +98,7 @@ def _worker(rank, world, port, results):
 
 def test_peer_memory_gradient_exchange_matches_nccl_on_two_gpus():
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs two GPUs (gpurun --gpus 2)")
+        pytest.skip("needs two GPUs")
     import torch.multiprocessing as mp
     world, port = 2, _free_port()
     with mp.Manager() as m:
