@@ -124,6 +124,18 @@ _SIGNATURES = {
     "bnn_sampled_conv2d_wgrad": (ctypes.c_int, [_c_f32p, _c_f32p, ctypes.c_int64, _c_f32p, _c_f32p, _c_f32p, _c_f32p,
                                                 ctypes.POINTER(bnn_conv2d_nhwc), ctypes.c_int32, ctypes.c_uint32,
                                                 ctypes.POINTER(bnn_rng), ctypes.c_void_p]),
+    "bnn_sampled_conv_transpose2d_fwd": (ctypes.c_int, [_c_f32p, ctypes.c_int64, _c_f32p, _c_f32p, _c_f32p, _c_f32p, _c_f32p,
+                                                        _c_f32p, _c_f32p, ctypes.POINTER(bnn_conv2d_nhwc), ctypes.c_int32,
+                                                        ctypes.c_uint32, ctypes.POINTER(bnn_rng), ctypes.POINTER(bnn_rng),
+                                                        ctypes.c_void_p]),
+    "bnn_sampled_conv_transpose2d_dgrad": (ctypes.c_int, [_c_f32p, _c_f32p, _c_f32p, _c_f32p, _c_f32p, ctypes.c_int64,
+                                                          ctypes.POINTER(bnn_conv2d_nhwc), ctypes.c_int32, ctypes.c_uint32,
+                                                          ctypes.POINTER(bnn_rng), ctypes.c_void_p]),
+    "bnn_sampled_conv_transpose2d_wgrad": (ctypes.c_int, [_c_f32p, _c_f32p, ctypes.c_int64, _c_f32p, _c_f32p, _c_f32p,
+                                                          _c_f32p, ctypes.POINTER(bnn_conv2d_nhwc), ctypes.c_int32,
+                                                          ctypes.c_uint32, ctypes.POINTER(bnn_rng), ctypes.c_void_p]),
+    "bnn_debug_conv_transpose_phases": (ctypes.c_int, [ctypes.POINTER(bnn_conv2d_nhwc), ctypes.POINTER(ctypes.c_int32),
+                                                       ctypes.c_int32]),
     "bnn_conv2d_weight_layout": (ctypes.c_int, [_c_f32p, _c_f32p, _c_f32p, _c_f32p, _c_f32p, ctypes.c_int32, ctypes.c_int32,
                                                 ctypes.c_int32, ctypes.c_void_p]),
     "bnn_conv2d_weight_unlayout": (ctypes.c_int, [_c_f32p, _c_f32p, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32,
@@ -790,3 +802,48 @@ def selftest_umma(device="cuda", mn_major=False):
         _call("bnn_selftest_umma_mn" if mn_major else "bnn_selftest_umma", _ptr(out), _stream())
     _count()
     return float(out.item())
+
+
+# ---- transposed convolution (geometry = the conv view, see bnn_b200.h) ----------------------------------------------
+def try_sampled_conv_transpose2d_fwd(x, x_sample_stride, mu_w, sigma_w, mu_b, sigma_b, eps_w, eps_b, y, geom, S,
+                                     sample_begin, rng_w, rng_b):
+    """The phase-decomposed gather; False (nothing launched) when the kernels do not take the request."""
+    return _try_call("bnn_sampled_conv_transpose2d_fwd", y.device, _ptr(x), x_sample_stride, _ptr(mu_w), _ptr(sigma_w),
+                     _ptr(mu_b), _ptr(sigma_b), _ptr(eps_w), _ptr(eps_b), _ptr(y), ctypes.byref(geom), S, sample_begin,
+                     ctypes.byref(rng_w), ctypes.byref(rng_b) if rng_b is not None else None, _stream())
+
+
+def try_sampled_conv_transpose2d_dgrad(dy, mu_w, sigma_w, eps_w, dx, x_sample_stride, geom, S, sample_begin, rng_w):
+    return _try_call("bnn_sampled_conv_transpose2d_dgrad", dx.device, _ptr(dy), _ptr(mu_w), _ptr(sigma_w), _ptr(eps_w),
+                     _ptr(dx), x_sample_stride, ctypes.byref(geom), S, sample_begin, ctypes.byref(rng_w), _stream())
+
+
+def try_sampled_conv_transpose2d_wgrad(dy, x, x_sample_stride, rho_w, eps_w, dmu_w, drho_w, geom, S, sample_begin, rng_w):
+    return _try_call("bnn_sampled_conv_transpose2d_wgrad", x.device, _ptr(dy), _ptr(x), x_sample_stride, _ptr(rho_w),
+                     _ptr(eps_w), _ptr(dmu_w), _ptr(drho_w), ctypes.byref(geom), S, sample_begin, ctypes.byref(rng_w),
+                     _stream())
+
+
+def _try_call(name, device, *args):
+    """Like _call, but BNN_ERR_UNSUPPORTED (a request outside the kernels' stated limits) returns False."""
+    with torch.cuda.device(device):
+        fn = getattr(lib(), name)
+        rc = fn(*args)
+    if rc == 6:                                   # BNN_ERR_UNSUPPORTED
+        return False
+    _check(rc, name)
+    _count()
+    return True
+
+
+def conv_transpose_phases(geom):
+    """Host-side phase plan of bnn_sampled_conv_transpose2d_fwd: one dict per output phase (no device needed)."""
+    cap = 64
+    buf = (ctypes.c_int32 * (14 * cap))()
+    n = lib().bnn_debug_conv_transpose_phases(ctypes.byref(geom), buf, cap)
+    if n < 0:
+        _check(-n, "bnn_debug_conv_transpose_phases")
+    keys = ("rh", "rw", "rows_h", "rows_w", "taps_h", "taps_w", "last_h", "last_w", "tap_step_h", "tap_step_w",
+            "first_h", "first_w", "in_step_h", "in_step_w")
+    return [dict(zip(keys, buf[14 * i:14 * i + 14])) for i in range(min(n, cap))]
+

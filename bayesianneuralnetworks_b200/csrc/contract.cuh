@@ -27,7 +27,15 @@ struct View {
   float* base;
   int64_t bs;
   int P;
+  // phase view (TMA kernels' staged row-major drain only; pw == 0: off): row m = (img, i, j) of an img x (pimg / pw) x pw
+  // grid lands at base + img * s_img + i * s_i + j * bs — one output phase of a strided transposed convolution
+  int pw = 0, pimg = 0;
+  int64_t s_i = 0, s_img = 0;
 };
+__device__ __forceinline__ float* phase_row(const View& v, int m) {
+  const int img = m / v.pimg, r = m - img * v.pimg, i = r / v.pw, j = r - i * v.pw;
+  return v.base + static_cast<int64_t>(img) * v.s_img + static_cast<int64_t>(i) * v.s_i + static_cast<int64_t>(j) * v.bs;
+}
 __device__ __forceinline__ int64_t view_off(const View& v, int m, int n) {
   if (v.P == 1) return static_cast<int64_t>(m) * v.bs + n;
   const int b = m / v.P, p = m - b * v.P;
@@ -144,6 +152,19 @@ int tma_conv_dgrad(const float* dy, const float* mu_w, const float* sigma_w, con
 int tma_conv_wgrad(const float* dy, const float* x, int64_t x_sample_stride, const float* rho_w, const float* eps_w,
                    float* dmu_w, float* drho_w, const bnn_conv2d_nhwc* g, int S, uint32_t sample_begin,
                    const bnn_rng* rng_w, cudaStream_t st);
+// transposed convolution, geometry of its conv view (see bnn_b200.h): forward as the strided transposed-filter gather
+// (one launch per output phase), input gradient as the conv view's forward, weight gradient as the conv view's
+int tma_conv_transpose_fwd(const float* x, int64_t x_sample_stride, const float* mu_w, const float* sigma_w,
+                           const float* mu_b, const float* sigma_b, const float* eps_w, const float* eps_b, float* y,
+                           const bnn_conv2d_nhwc* g, int S, uint32_t sample_begin, const bnn_rng* rng_w,
+                           const bnn_rng* rng_b, cudaStream_t st);
+int tma_conv_transpose_dgrad(const float* dy, const float* mu_w, const float* sigma_w, const float* eps_w, float* dx,
+                             int64_t x_sample_stride, const bnn_conv2d_nhwc* g, int S, uint32_t sample_begin,
+                             const bnn_rng* rng_w, cudaStream_t st);
+int tma_conv_transpose_wgrad(const float* dy, const float* x, int64_t x_sample_stride, const float* rho_w,
+                             const float* eps_w, float* dmu_w, float* drho_w, const bnn_conv2d_nhwc* g, int S,
+                             uint32_t sample_begin, const bnn_rng* rng_w, cudaStream_t st);
+int conv_transpose_phases(const bnn_conv2d_nhwc* g, int32_t* out, int max_phases);   // host: the phase plan, 8 ints each
 int tma_selftest(float* max_err_dev, cudaStream_t st);
 int tma_pair_tile_plan(int m_blocks, int S, int slots, int32_t* out7);   // test aid: TilePlan fields {on, n_a, s1, a1, b1, a2, b2}
 int tma_force_variant(int variant);   // test aid: 0 = CTA pair, 8 = its balanced schedule, 1 / 2 / 4 = row blocks per CTA, -1 = cost model (default)

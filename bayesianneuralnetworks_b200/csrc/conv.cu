@@ -514,4 +514,68 @@ int bnn_sampled_conv2d_wgrad(const float* dy, const float* x, int64_t x_sample_s
   return rc;
 }
 
+
+int bnn_sampled_conv_transpose2d_fwd(const float* x, int64_t x_sample_stride, const float* mu_w, const float* sigma_w,
+                                     const float* mu_b, const float* sigma_b, const float* eps_w, const float* eps_b, float* y,
+                                     const bnn_conv2d_nhwc* g, int32_t S, uint32_t sample_begin, const bnn_rng* rng_w,
+                                     const bnn_rng* rng_b, void* stream) {
+  int rc = check_geom(g, "bnn_sampled_conv_transpose2d_fwd");
+  if (rc != BNN_OK) return rc;
+  BNN_REQUIRE(x && mu_w && sigma_w && y && rng_w && S > 0 && S <= 65535, BNN_ERR_BAD_ARGUMENT,
+              "bnn_sampled_conv_transpose2d_fwd: NULL pointer or bad sample count");
+  BNN_REQUIRE((mu_b == nullptr) == (sigma_b == nullptr) && (mu_b == nullptr || rng_b != nullptr), BNN_ERR_BAD_ARGUMENT,
+              "bnn_sampled_conv_transpose2d_fwd: bias needs mu_b, sigma_b and rng_b");
+  rc = check_device();
+  if (rc != BNN_OK) return rc;
+  rc = contract::tma_conv_transpose_fwd(x, x_sample_stride, mu_w, sigma_w, mu_b, sigma_b, eps_w, eps_b, y, g, S,
+                                        sample_begin, rng_w, rng_b, static_cast<cudaStream_t>(stream));
+  if (rc == contract::kNotEligible)
+    return fail(BNN_ERR_UNSUPPORTED, "bnn_sampled_conv_transpose2d_fwd: needs Cout %% 32 == 0, C %% 4 == 0, stride <= 8, "
+                                     "16-byte aligned tensors and phase corners within the im2col descriptor's limits "
+                                     "(use bnn_sampled_gemm_dgrad + bnn_col2im_nhwc)");
+  return rc;
+}
+
+int bnn_sampled_conv_transpose2d_dgrad(const float* dy, const float* mu_w, const float* sigma_w, const float* eps_w,
+                                       float* dx, int64_t x_sample_stride, const bnn_conv2d_nhwc* g, int32_t S,
+                                       uint32_t sample_begin, const bnn_rng* rng_w, void* stream) {
+  int rc = check_geom(g, "bnn_sampled_conv_transpose2d_dgrad");
+  if (rc != BNN_OK) return rc;
+  BNN_REQUIRE(dy && mu_w && sigma_w && dx && rng_w && S > 0 && S <= 65535, BNN_ERR_BAD_ARGUMENT,
+              "bnn_sampled_conv_transpose2d_dgrad: NULL pointer or bad sample count");
+  rc = check_device();
+  if (rc != BNN_OK) return rc;
+  rc = contract::tma_conv_transpose_dgrad(dy, mu_w, sigma_w, eps_w, dx, x_sample_stride, g, S, sample_begin, rng_w,
+                                          static_cast<cudaStream_t>(stream));
+  if (rc == contract::kNotEligible)
+    return fail(BNN_ERR_UNSUPPORTED, "bnn_sampled_conv_transpose2d_dgrad: needs C %% 32 == 0, Cout %% 4 == 0, 16-byte "
+                                     "aligned tensors and a filter window within the im2col descriptor's limits (use "
+                                     "bnn_im2col_nhwc + bnn_sampled_gemm_fwd)");
+  return rc;
+}
+
+int bnn_sampled_conv_transpose2d_wgrad(const float* dy, const float* x, int64_t x_sample_stride, const float* rho_w,
+                                       const float* eps_w, float* dmu_w, float* drho_w, const bnn_conv2d_nhwc* g, int32_t S,
+                                       uint32_t sample_begin, const bnn_rng* rng_w, void* stream) {
+  int rc = check_geom(g, "bnn_sampled_conv_transpose2d_wgrad");
+  if (rc != BNN_OK) return rc;
+  BNN_REQUIRE(dy && x && rho_w && dmu_w && drho_w && rng_w && S > 0 && S <= 65535, BNN_ERR_BAD_ARGUMENT,
+              "bnn_sampled_conv_transpose2d_wgrad: NULL pointer or bad sample count");
+  rc = check_device();
+  if (rc != BNN_OK) return rc;
+  rc = contract::tma_conv_transpose_wgrad(dy, x, x_sample_stride, rho_w, eps_w, dmu_w, drho_w, g, S, sample_begin, rng_w,
+                                          static_cast<cudaStream_t>(stream));
+  if (rc == contract::kNotEligible)
+    return fail(BNN_ERR_UNSUPPORTED, "bnn_sampled_conv_transpose2d_wgrad: needs C %% 32 == 0, Cout %% 4 == 0 and 16-byte "
+                                     "aligned tensors (use bnn_im2col_nhwc + bnn_sampled_gemm_wgrad)");
+  return rc;
+}
+
+int bnn_debug_conv_transpose_phases(const bnn_conv2d_nhwc* g, int32_t* out, int32_t max_phases) {
+  const int rc = check_geom(g, "bnn_debug_conv_transpose_phases");
+  if (rc != BNN_OK) return -rc;
+  if (out == nullptr && max_phases > 0) return -fail(BNN_ERR_BAD_ARGUMENT, "bnn_debug_conv_transpose_phases: NULL output");
+  return contract::conv_transpose_phases(g, out, max_phases);
+}
+
 }  // extern "C"

@@ -163,9 +163,17 @@ struct ConvCoords {
   int dh, dw;               // dilation
   int KW, taps;             // filter width, KH * KW
   int cblocks;              // 32-channel k-blocks per tap (channels of the LOADED tensor / 32)
-  int w_rows;               // data gradient: rows of the weight matrix (Cout); its row pitch is taps * K floats
+  int w_rows;               // data gradient: rows of the weight matrix (Cout); its row pitch is wtaps * K floats
   int chans;                // channels of the loaded tensor (weight gradient: groups beyond K load channel `chans` = zeros)
+  // data gradient: flipped tap t = (jh, jw) of the walk (jh = t / KW) is the weight's tap (tkh - jh tdh, tkw - jw tdw) of a
+  // wtaps = KH x wKW filter.  Stride 1: every tap (tkh = KH - 1, tdh = 1, ...); one phase of a strided transposed
+  // convolution: the taps of that phase only, tdh = sh / gcd(sh, dh) apart
+  int wtaps, wKW, tkh, tkw, tdh, tdw;
 };
+__device__ __forceinline__ int64_t conv_dgrad_tap(const ConvCoords& c, int tapf) {
+  const int jh = tapf / c.KW, jw = tapf - jh * c.KW;
+  return static_cast<int64_t>((c.tkh - jh * c.tdh) * c.wKW + c.tkw - jw * c.tdw);
+}
 __device__ __forceinline__ void conv_pixel(const ConvCoords& c, int m, int smp, int* w, int* h, int* n) {
   const int img = m / c.P, rem = m - img * c.P;
   const int ph = rem / c.OW, q = rem - ph * c.OW;
@@ -314,7 +322,9 @@ __device__ __forceinline__ bool stage_eligible(const View& out, bool vec_out, in
 // Halves [h_begin, h_end) (64 columns each) of one 128-row block, drained by one warp (TMEM lanes [32 quad, +32), rows
 // m0 .. m0 + 31 of the output, columns col0 .. col0 + cols_here): two tcgen05.ld per round trip, then (+ bias) ->
 // staging -> coalesced stores / adds.
-template <bool kBias>
+// kPhase: the output may be a phase view (View::pw; conv data-gradient instantiations only — the others keep the plain
+// row addressing)
+template <bool kBias, bool kPhase = false>
 __device__ __forceinline__ void drain_block_staged(uint32_t taddr, uint32_t stage, const float* aux, const View& out,
                                                    int m0, int M, int col0, int cols_here, int lane, bool add,
                                                    int h_begin = 0, int h_end = 2) {
@@ -373,7 +383,8 @@ __device__ __forceinline__ void drain_block_staged(uint32_t taddr, uint32_t stag
         const int row = 2 * i + (lane >> 4);
         if (c4 * 4 < cols_half && m0 + row < M) {
           const float4 q = lds128(stage + row * 272 + c4 * 16);
-          float* d = dst + static_cast<int64_t>(2 * i) * out.bs + h * 64;
+          float* d = (!kPhase || out.pw == 0) ? dst + static_cast<int64_t>(2 * i) * out.bs + h * 64
+                                              : phase_row(out, m0 + row) + col0 + (c4 << 2) + h * 64;
           if (add) red_add4(d, q.x, q.y, q.z, q.w);
           else *reinterpret_cast<float4*>(d) = q;
         }
@@ -400,7 +411,7 @@ __device__ __forceinline__ void drain_block_staged(uint32_t taddr, uint32_t stag
 constexpr int kDrainPerQuad = 4;
 constexpr int kDrainThreads = 4 * kDrainPerQuad * 32;
 constexpr int kDrainBarrier = 2;
-template <bool kBias>
+template <bool kBias, bool kPhase = false>
 __device__ __forceinline__ void drain_tile_shared(uint32_t tmem, uint32_t stage_base, const float* aux, const View& out,
                                                   int row0, int M, int mb_count, int col0, int cols_here, int quad,
                                                   int idx, int lane, bool add) {
@@ -409,7 +420,7 @@ __device__ __forceinline__ void drain_tile_shared(uint32_t tmem, uint32_t stage_
   for (int item = idx; item < mb_count * halves; item += kDrainPerQuad) {
     const int mb = item / halves, h = item - mb * halves;
     if (row0 + mb * 128 >= M) break;
-    drain_block_staged<kBias>(tmem + (static_cast<uint32_t>(quad * 32) << 16) + mb * 128, stage, aux, out,
+    drain_block_staged<kBias, kPhase>(tmem + (static_cast<uint32_t>(quad * 32) << 16) + mb * 128, stage, aux, out,
                               row0 + mb * 128 + quad * 32, M, col0, cols_here, lane, add, h, h + 1);
   }
 }
@@ -459,6 +470,8 @@ __global__ void __launch_bounds__(kThreadsTma, 1) contract_tma_kernel(const __gr
   out_tile.base += (p.sum_samples ? 0 : static_cast<int64_t>(blockIdx.z) * p.out_sample_stride);
   const int cols_tile = n_cols - col0 < 128 ? n_cols - col0 : 128;
   const bool staged = stage_eligible(out_tile, p.vec_out != 0, cols_tile) && (out_tile.P == 1 || (p.M & 3) == 0);
+  // sampled bias row in the epilogue: the forward pass, and the conv data gradient of a transposed convolution's forward
+  const bool bias = !kDgrad || (kConv && p.mu_b != nullptr);
 
   if (warp < kGenWarps) {
     // ------------------------------------------------------------------ weight generators (four groups, slot = group)
@@ -483,18 +496,22 @@ __global__ void __launch_bounds__(kThreadsTma, 1) contract_tma_kernel(const __gr
       else {          // conv data gradient: k-block = (flipped tap, 32 output channels o0 ..)
         const int tapf = rb / p.conv.cblocks, o0 = (rb - tapf * p.conv.cblocks) * kBK;
         gen_w_tile<128, true, kSigns>(tile, p.mu_w, p.sigma_w, eps, o0, p.conv.w_rows, col0, p.K, tid,
-                              static_cast<int64_t>(p.conv.taps) * p.K, static_cast<int64_t>(p.conv.taps - 1 - tapf) * p.K);
+                              static_cast<int64_t>(p.conv.wtaps) * p.K, conv_dgrad_tap(p.conv, tapf) * p.K);
       }
       fence_proxy_async_smem();
       __syncwarp();
       if (lane == 0) mbar_arrive(pipe.full_w + group);
     }
     if (staged && (warp >> 2) < kDrainPerQuad - 1) {     // join the drain (TMEM lane quarter = warp % 4)
-      if (!kDgrad) named_bar_sync(kDrainBarrier, kDrainThreads);          // the bias row is in shared memory
+      if (bias) named_bar_sync(kDrainBarrier, kDrainThreads);             // the bias row is in shared memory
       mbar_wait(pipe.accum_full, 0);
       tc_fence_after_sync();
-      drain_tile_shared<!kDgrad>(tmem, pipe.ring_a, pipe.aux, out_tile, row0, p.M, mb_used, col0, cols_tile, warp & 3,
-                                 1 + (warp >> 2), lane, kDgrad && p.atomic_out);
+      if (bias)
+        drain_tile_shared<true, kDgrad && kConv>(tmem, pipe.ring_a, pipe.aux, out_tile, row0, p.M, mb_used, col0, cols_tile, warp & 3,
+                                1 + (warp >> 2), lane, p.atomic_out != 0);
+      else
+        drain_tile_shared<false, kDgrad && kConv>(tmem, pipe.ring_a, pipe.aux, out_tile, row0, p.M, mb_used, col0, cols_tile, warp & 3,
+                                 1 + (warp >> 2), lane, p.atomic_out != 0);
     }
   } else if (warp == kTmaWarp) {
     // ------------------------------------------------------------------ TMA issuer
@@ -565,12 +582,12 @@ __global__ void __launch_bounds__(kThreadsTma, 1) contract_tma_kernel(const __gr
     // ------------------------------------------------------------------ epilogue
     const int et = threadIdx.x - kEpiWarp0T * 32;   // 0..127
     const int quad = warp & 3;
-    if (!kDgrad) {
+    if (bias) {
       float b = 0.f;
       const int n = col0 + et;
-      if (p.mu_b != nullptr && n < p.N) {
+      if (p.mu_b != nullptr && n < n_cols) {
         const int s = blockIdx.z;
-        const float e = p.eps_b ? __ldg(p.eps_b + static_cast<int64_t>(s) * p.N + n)
+        const float e = p.eps_b ? __ldg(p.eps_b + static_cast<int64_t>(s) * n_cols + n)
                                 : eps1(resolve_rng(p.rng_b), p.sample_begin + s, static_cast<uint64_t>(n));
         b = fmaf(__ldg(p.sigma_b + n), e, __ldg(p.mu_b + n));
       }
@@ -581,8 +598,12 @@ __global__ void __launch_bounds__(kThreadsTma, 1) contract_tma_kernel(const __gr
     mbar_wait(pipe.accum_full, 0);
     tc_fence_after_sync();
     if (staged) {
-      drain_tile_shared<!kDgrad>(tmem, pipe.ring_a, pipe.aux, out_tile, row0, p.M, mb_used, col0, cols_tile, quad, 0, lane,
-                                 kDgrad && p.atomic_out);
+      if (bias)
+        drain_tile_shared<true, kDgrad && kConv>(tmem, pipe.ring_a, pipe.aux, out_tile, row0, p.M, mb_used, col0, cols_tile, quad, 0, lane,
+                                p.atomic_out != 0);
+      else
+        drain_tile_shared<false, kDgrad && kConv>(tmem, pipe.ring_a, pipe.aux, out_tile, row0, p.M, mb_used, col0, cols_tile, quad, 0, lane,
+                                 p.atomic_out != 0);
     } else {
       const View& out = out_tile;
       const int cols_here = cols_tile;
@@ -591,12 +612,12 @@ __global__ void __launch_bounds__(kThreadsTma, 1) contract_tma_kernel(const __gr
         for (int c = 0; c * 16 < cols_here; ++c) {
           float v[16];
           tmem_ld16(tmem + (static_cast<uint32_t>(quad * 32) << 16) + mb * 128 + c * 16, v);
-          if (!kDgrad) {
+          if (bias) {
 #pragma unroll
             for (int j = 0; j < 16; ++j) v[j] += pipe.aux[c * 16 + j];
           }
           if (m < p.M) {
-            if (kDgrad && p.atomic_out) add_chunk(out, m, col0 + c * 16, n_cols, v, p.vec_out != 0);
+            if (p.atomic_out) add_chunk(out, m, col0 + c * 16, n_cols, v, p.vec_out != 0);
             else store_chunk(out, m, col0 + c * 16, n_cols, v, p.vec_out != 0);
           }
         }
@@ -759,6 +780,8 @@ contract_pair_kernel(const __grid_constant__ TmaContractParams p) {
   out_tile.base += (p.sum_samples ? 0 : static_cast<int64_t>(tile_s) * p.out_sample_stride);
   const int cols_tile = n_cols - col0 < 128 ? n_cols - col0 : 128;
   const bool staged = stage_eligible(out_tile, p.vec_out != 0, cols_tile) && (out_tile.P == 1 || (p.M & 3) == 0);
+  // sampled bias row in the epilogue: the forward pass, and the conv data gradient of a transposed convolution's forward
+  const bool bias = !kDgrad || (kConv && p.mu_b != nullptr);
 
   if (warp < kGenWarps) {
     // ------------------------------------------------------------------ weight generators (half tile per CTA, four groups)
@@ -787,18 +810,22 @@ contract_pair_kernel(const __grid_constant__ TmaContractParams p) {
       else {
         const int tapf = rb / p.conv.cblocks, o0 = (rb - tapf * p.conv.cblocks) * kBK;
         gen_w_tile<64, true, kSigns>(tile, p.mu_w, p.sigma_w, eps, o0, p.conv.w_rows, half0, p.K, tid,
-                             static_cast<int64_t>(p.conv.taps) * p.K, static_cast<int64_t>(p.conv.taps - 1 - tapf) * p.K);
+                             static_cast<int64_t>(p.conv.wtaps) * p.K, conv_dgrad_tap(p.conv, tapf) * p.K);
       }
       fence_proxy_async_smem();
       __syncwarp();
       if (lane == 0) mbar_arrive_cluster(lead_full_w0 + wslot * 8);
     }
     if (staged && (warp >> 2) < kDrainPerQuad - 1) {     // join the drain (TMEM lane quarter = warp % 4)
-      if (!kDgrad) named_bar_sync(kDrainBarrier, kDrainThreads);          // the bias row is in shared memory
+      if (bias) named_bar_sync(kDrainBarrier, kDrainThreads);             // the bias row is in shared memory
       mbar_wait(pipe.accum_full, 0);
       tc_fence_after_sync();
-      drain_tile_shared<!kDgrad>(tmem, pipe.ring_a, pipe.aux, out_tile, row0, p.M, mb_pair, col0, cols_tile, warp & 3,
-                                 1 + (warp >> 2), lane, kDgrad && p.atomic_out);
+      if (bias)
+        drain_tile_shared<true, kDgrad && kConv>(tmem, pipe.ring_a, pipe.aux, out_tile, row0, p.M, mb_pair, col0, cols_tile, warp & 3,
+                                1 + (warp >> 2), lane, p.atomic_out != 0);
+      else
+        drain_tile_shared<false, kDgrad && kConv>(tmem, pipe.ring_a, pipe.aux, out_tile, row0, p.M, mb_pair, col0, cols_tile, warp & 3,
+                                 1 + (warp >> 2), lane, p.atomic_out != 0);
     }
   } else if (warp == kTmaWarp) {
     // ------------------------------------------------------------------ TMA issuer (own rows; bytes counted by the leader)
@@ -871,12 +898,12 @@ contract_pair_kernel(const __grid_constant__ TmaContractParams p) {
     // ------------------------------------------------------------------ epilogue (own TMEM, own rows)
     const int et = threadIdx.x - kEpiWarp0T * 32;   // 0..127
     const int quad = warp & 3;
-    if (!kDgrad) {
+    if (bias) {
       float b = 0.f;
       const int n = col0 + et;
-      if (p.mu_b != nullptr && n < p.N) {
+      if (p.mu_b != nullptr && n < n_cols) {
         const int s = tile_s;
-        const float e = p.eps_b ? __ldg(p.eps_b + static_cast<int64_t>(s) * p.N + n)
+        const float e = p.eps_b ? __ldg(p.eps_b + static_cast<int64_t>(s) * n_cols + n)
                                 : eps1(resolve_rng(p.rng_b), p.sample_begin + s, static_cast<uint64_t>(n));
         b = fmaf(__ldg(p.sigma_b + n), e, __ldg(p.mu_b + n));
       }
@@ -890,8 +917,12 @@ contract_pair_kernel(const __grid_constant__ TmaContractParams p) {
     if (threadIdx.x == kEpiWarp0T * 32) BNN_STAGE(2, t_kernel0);
 #endif
     if (staged) {
-      drain_tile_shared<!kDgrad>(tmem, pipe.ring_a, pipe.aux, out_tile, row0, p.M, mb_pair, col0, cols_tile, quad, 0, lane,
-                                 kDgrad && p.atomic_out);
+      if (bias)
+        drain_tile_shared<true, kDgrad && kConv>(tmem, pipe.ring_a, pipe.aux, out_tile, row0, p.M, mb_pair, col0, cols_tile, quad, 0, lane,
+                                p.atomic_out != 0);
+      else
+        drain_tile_shared<false, kDgrad && kConv>(tmem, pipe.ring_a, pipe.aux, out_tile, row0, p.M, mb_pair, col0, cols_tile, quad, 0, lane,
+                                 p.atomic_out != 0);
     } else {
       const View& out = out_tile;
       const int cols_here = cols_tile;
@@ -901,12 +932,12 @@ contract_pair_kernel(const __grid_constant__ TmaContractParams p) {
         for (int c = 0; c * 16 < cols_here; ++c) {
           float v[16];
           tmem_ld16(tmem + (static_cast<uint32_t>(quad * 32) << 16) + mb * 128 + c * 16, v);
-          if (!kDgrad) {
+          if (bias) {
 #pragma unroll
             for (int j = 0; j < 16; ++j) v[j] += pipe.aux[c * 16 + j];
           }
           if (m < p.M) {
-            if (kDgrad && p.atomic_out) add_chunk(out, m, col0 + c * 16, n_cols, v, p.vec_out != 0);
+            if (p.atomic_out) add_chunk(out, m, col0 + c * 16, n_cols, v, p.vec_out != 0);
             else store_chunk(out, m, col0 + c * 16, n_cols, v, p.vec_out != 0);
           }
         }
@@ -1109,7 +1140,7 @@ contract_pair_sk_kernel(const __grid_constant__ TmaContractParams p) {
         else {
           const int tapf = rb / p.conv.cblocks, o0 = (rb - tapf * p.conv.cblocks) * kBK;
           gen_w_tile<64, true, kSigns>(tile, p.mu_w, p.sigma_w, eps, o0, p.conv.w_rows, half0, p.K, tid,
-                               static_cast<int64_t>(p.conv.taps) * p.K, static_cast<int64_t>(p.conv.taps - 1 - tapf) * p.K);
+                               static_cast<int64_t>(p.conv.wtaps) * p.K, conv_dgrad_tap(p.conv, tapf) * p.K);
         }
         fence_proxy_async_smem();
         __syncwarp();
@@ -1452,6 +1483,8 @@ template <bool kDgrad>
 bool plan_sk(TmaContractParams& p, int gx, int m_blocks, int uniform_pairs, bool forced) {
   p.sk_slots = 0;
   if (!forced && !sk_enabled()) return false;
+  // the balanced kernel has no phase view, no data-gradient bias and no summed forward
+  if (p.out.pw != 0 || (kDgrad && p.mu_b != nullptr) || (!kDgrad && p.sum_samples)) return false;
   if (p.sum_samples && p.out.P != 1) return false;
   const int slots = sk_max_slots();
   if (slots < 2) return false;
@@ -1614,6 +1647,7 @@ struct TmaWgradParams {
   uint32_t sample_begin;
   bnn_rng rng_w;
   int shared_a;
+  int shared_dy;            // all samples read sample 0 of dY (the weight gradient of a transposed conv with shared input)
   int n_chunks;             // the M reduction of every sample is cut into n_chunks pieces of chunk_blocks k-blocks:
   int chunk_blocks;         // a work unit = (sample, chunk); (sum_chunks G) o eps = sum_chunks (G o eps), so units are independent
 };
@@ -1685,7 +1719,7 @@ __global__ void __launch_bounds__(kWgThreads, 1) wgrad_tma_kernel(const __grid_c
         }
         for (int u = s_begin; u < s_end; ++u) {
           const int s = u / p.n_chunks;
-          const int sa = p.shared_a ? 0 : s;
+          const int sa = p.shared_a ? 0 : s, sd = p.shared_dy ? 0 : s;
           int mb0;
           const int m_blocks = unit_blocks(u, &mb0);
           for (int mb = mb0; mb < mb0 + m_blocks; ++mb, ++it) {
@@ -1698,7 +1732,7 @@ __global__ void __launch_bounds__(kWgThreads, 1) wgrad_tma_kernel(const __grid_c
               mbar_arrive_expect_tx(full + stage, 2 * kWgOperandBytes);
 #pragma unroll
               for (int g = 0; g < 4; ++g) {
-                tma_load_3d(base + g * kWgLbo, &p.map_dy, n0 + g * 32, mb * kWgRows, s, full + stage);
+                tma_load_3d(base + g * kWgLbo, &p.map_dy, n0 + g * 32, mb * kWgRows, sd, full + stage);
                 if (!p.conv.on) {
                   tma_load_3d(base + kWgOperandBytes + g * kWgLbo, &p.map_a, k0 + g * 32, mb * kWgRows, sa, full + stage);
                 } else {
@@ -1711,7 +1745,7 @@ __global__ void __launch_bounds__(kWgThreads, 1) wgrad_tma_kernel(const __grid_c
               if (rank == 0) mbar_arrive_expect_tx(full + stage, 2 * (kWgOperandBytes + kWgOperandBytes / 2));
 #pragma unroll
               for (int g = 0; g < 4; ++g)
-                tma_load_3d_pair(base + g * kWgLbo, &p.map_dy, n0 + g * 32, mb * kWgRows, s, lead_full);
+                tma_load_3d_pair(base + g * kWgLbo, &p.map_dy, n0 + g * 32, mb * kWgRows, sd, lead_full);
 #pragma unroll
               for (int g = 0; g < 2; ++g) {     // this CTA's half (64 columns) of the shared A^T tile
                 const int kc = k0 + static_cast<int>(rank) * 64 + g * 32;
@@ -2057,11 +2091,14 @@ bool conv_ok(const bnn_conv2d_nhwc& g) {
 }
 }  // namespace
 
-int tma_conv_fwd(const float* x, int64_t x_sample_stride, const float* mu_w, const float* sigma_w, const float* mu_b,
-                 const float* sigma_b, const float* eps_w, const float* eps_b, bnn_view y, int64_t y_sample_stride,
-                 const bnn_conv2d_nhwc* g, int S, uint32_t sample_begin, const bnn_rng* rng_w, const bnn_rng* rng_b,
-                 cudaStream_t st) {
-  const bool shared = x_sample_stride == 0;
+namespace {
+// sum_samples: every sample reads its own x and the S results are summed into one y (the input gradient of a transposed
+// convolution with shared input); else x_sample_stride == 0 means all samples share x
+int conv_fwd_launch(const float* x, int64_t x_sample_stride, const float* mu_w, const float* sigma_w, const float* mu_b,
+                    const float* sigma_b, const float* eps_w, const float* eps_b, bnn_view y, int64_t y_sample_stride,
+                    const bnn_conv2d_nhwc* g, int S, uint32_t sample_begin, const bnn_rng* rng_w, const bnn_rng* rng_b,
+                    bool sum_samples, cudaStream_t st) {
+  const bool shared = x_sample_stride == 0 && !sum_samples;
   if (!conv_ok(*g) || !aligned16(x) || rng_w->elem_offset % 4 != 0 || !aligned16(mu_w) || !aligned16(sigma_w) ||
       (eps_w != nullptr && !aligned16(eps_w)))
     return kNotEligible;
@@ -2076,12 +2113,21 @@ int tma_conv_fwd(const float* x, int64_t x_sample_stride, const float* mu_w, con
   p.w_numel = static_cast<int64_t>(p.N) * p.K;
   p.rng_w = *rng_w; p.rng_b = rng_b ? *rng_b : *rng_w;
   p.shared_l = shared ? 1 : 0;
-  p.sum_samples = 0;
+  p.sum_samples = sum_samples ? 1 : 0;
 #ifdef BNN_PROFILE_WAITS
   { const char* e = getenv("BNN_EXP_FLAGS"); p.exp_flags = e ? atoi(e) : 0; }
 #endif
   p.vec_out = (y.P == 1) && (y.batch_stride % 4 == 0) && (y_sample_stride % 4 == 0) && aligned16(y.base);
   return dispatch_tma_contract<false>(p, p.N, st);
+}
+}  // namespace
+
+int tma_conv_fwd(const float* x, int64_t x_sample_stride, const float* mu_w, const float* sigma_w, const float* mu_b,
+                 const float* sigma_b, const float* eps_w, const float* eps_b, bnn_view y, int64_t y_sample_stride,
+                 const bnn_conv2d_nhwc* g, int S, uint32_t sample_begin, const bnn_rng* rng_w, const bnn_rng* rng_b,
+                 cudaStream_t st) {
+  return conv_fwd_launch(x, x_sample_stride, mu_w, sigma_w, mu_b, sigma_b, eps_w, eps_b, y, y_sample_stride, g, S,
+                         sample_begin, rng_w, rng_b, false, st);
 }
 
 // dX[n][h][w][c] = sum_{kh, kw, o} dY[n][h + ph - kh dh][w + pw - kw dw][o] W[o][kh][kw][c]   (stride 1): the transposed-
@@ -2106,6 +2152,7 @@ int tma_conv_dgrad(const float* dy, const float* mu_w, const float* sigma_w, con
   c.on = 1; c.P = g->H * g->W; c.OW = g->W; c.imgs = g->B; c.sh = 1; c.sw = 1; c.lh = lo_h; c.lw = lo_w;
   c.dh = g->dh; c.dw = g->dw; c.KW = g->KW; c.taps = g->KH * g->KW; c.cblocks = g->Cout / kBK; c.w_rows = g->Cout;
   c.chans = g->Cout;
+  c.wtaps = c.taps; c.wKW = g->KW; c.tkh = g->KH - 1; c.tkw = g->KW - 1; c.tdh = 1; c.tdw = 1;
   p.conv = c;
   p.out.base = dx; p.out.bs = g->C; p.out.P = 1; p.out_sample_stride = x_sample_stride;
   p.mu_w = mu_w; p.sigma_w = sigma_w; p.eps_w = eps_w;
@@ -2137,6 +2184,175 @@ int tma_conv_wgrad(const float* dy, const float* x, int64_t x_sample_stride, con
   p.M = M; p.N = N; p.K = K; p.S = S; p.sample_begin = sample_begin;
   p.rng_w = *rng_w;
   p.shared_a = shared ? 1 : 0;
+  return wgrad_plan_and_launch(p, M, N, K, S, st);
+}
+
+// ---------------------------------------------------------------------------------------------- transposed convolution
+// A transposed convolution with weight W [Cin][Cout][KH][KW] is the adjoint of its CONV VIEW, the convolution from the
+// transposed output (C = Cout channels, H x W) to the transposed input (Cout_view = Cin channels, OH x OW) with the same W
+// read as OIHW.  Its forward is therefore the conv view's data gradient plus a bias:
+//   y[n][h][w][c] = b[c] + sum_{kh, kw, o : (h + ph - kh dh) % sh == 0, ...} x[n][(h + ph - kh dh) / sh][..][o] W[o][kh][kw][c]
+// Split the outputs into sh x sw phases (h % sh, w % sw).  In phase r a tap contributes iff (r + ph - kh dh) % sh == 0,
+// and then from input row i + (r + ph - kh dh) / sh for output row r + sh i: every phase is a STRIDE-1 gather over x with
+// its own taps (tdh = sh / gcd(sh, dh) apart, dh / gcd(sh, dh) input rows apart) and its own im2col corner.  One launch of
+// the data-gradient kernel per phase walks exactly that phase's taps x 32-channel blocks (no MMA on inserted zeros) and
+// writes its rows through a phase view; phases without a tap get the bias alone.
+namespace {
+struct PhaseDim {
+  int r, rows;              // phase offset, output rows of the phase
+  int taps, tlast, tstep;   // taps of the phase, the last one, their spacing
+  int lo, dstep;            // input row of (phase row 0, last tap) and input-row distance of consecutive walked taps
+};
+int gcd_int(int a, int b) { while (b != 0) { const int t = a % b; a = b; b = t; } return a; }
+// one dimension of output size n_out (the conv view's input size)
+PhaseDim phase_dim(int r, int n_out, int s, int pad, int d, int k) {
+  PhaseDim pd{};
+  pd.r = r;
+  pd.rows = (n_out - r + s - 1) / s;
+  const int gd = gcd_int(s, d);
+  pd.tstep = s / gd;
+  pd.dstep = d / gd;
+  pd.taps = 0;
+  pd.tlast = -1;
+  for (int kk = 0; kk < k; ++kk)
+    if ((((r + pad - kk * d) % s) + s) % s == 0) { ++pd.taps; pd.tlast = kk; }
+  pd.lo = pd.taps > 0 ? (r + pad - pd.tlast * d) / s : 0;     // exact division
+  return pd;
+}
+
+__global__ void phase_bias_kernel(float* y, int64_t ss, int64_t s_img, int64_t s_i, int64_t s_j, int S, int B, int rows,
+                                  int cols, int C, const float* mu_b, const float* sigma_b, const float* eps_b,
+                                  uint32_t sample_begin, bnn_rng rng_b) {
+  const int64_t total = static_cast<int64_t>(S) * B * rows * cols * C;
+  for (int64_t t = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; t < total;
+       t += static_cast<int64_t>(gridDim.x) * blockDim.x) {
+    int64_t q = t;
+    const int c = static_cast<int>(q % C); q /= C;
+    const int j = static_cast<int>(q % cols); q /= cols;
+    const int i = static_cast<int>(q % rows); q /= rows;
+    const int img = static_cast<int>(q % B);
+    const int s = static_cast<int>(q / B);
+    float b = 0.f;
+    if (mu_b != nullptr) {
+      const float e = eps_b ? __ldg(eps_b + static_cast<int64_t>(s) * C + c)
+                            : eps1(resolve_rng(rng_b), sample_begin + s, static_cast<uint64_t>(c));
+      b = fmaf(__ldg(sigma_b + c), e, __ldg(mu_b + c));
+    }
+    y[s * ss + img * s_img + i * s_i + j * s_j + c] = b;
+  }
+}
+}  // namespace
+
+int conv_transpose_phases(const bnn_conv2d_nhwc* g, int32_t* out, int max_phases) {
+  const int ph_h = g->sh < g->H ? g->sh : g->H, ph_w = g->sw < g->W ? g->sw : g->W;
+  int n = 0;
+  for (int rh = 0; rh < ph_h; ++rh)
+    for (int rw = 0; rw < ph_w; ++rw, ++n) {
+      if (n >= max_phases) continue;
+      const PhaseDim a = phase_dim(rh, g->H, g->sh, g->ph, g->dh, g->KH);
+      const PhaseDim b = phase_dim(rw, g->W, g->sw, g->pw, g->dw, g->KW);
+      const int32_t v[14] = {a.r, b.r, a.rows, b.rows, a.taps, b.taps, a.tlast, b.tlast, a.tstep, b.tstep, a.lo, b.lo,
+                             a.dstep, b.dstep};
+      for (int i = 0; i < 14; ++i) out[14 * n + i] = v[i];
+    }
+  return n;
+}
+
+int tma_conv_transpose_fwd(const float* x, int64_t x_sample_stride, const float* mu_w, const float* sigma_w,
+                           const float* mu_b, const float* sigma_b, const float* eps_w, const float* eps_b, float* y,
+                           const bnn_conv2d_nhwc* g, int S, uint32_t sample_begin, const bnn_rng* rng_w,
+                           const bnn_rng* rng_b, cudaStream_t st) {
+  // conv view: C = transposed output channels (the drained columns), Cout = transposed input channels (reduction)
+  const bool shared = x_sample_stride == 0;
+  if (g->Cout % kBK != 0 || g->C % 4 != 0 || g->sh > 8 || g->sw > 8 || !aligned16(x) || !aligned16(y) ||
+      rng_w->elem_offset % 4 != 0 || !aligned16(mu_w) || !aligned16(sigma_w) || (eps_w != nullptr && !aligned16(eps_w)))
+    return kNotEligible;
+  const int ph_h = g->sh < g->H ? g->sh : g->H, ph_w = g->sw < g->W ? g->sw : g->W;
+  // every phase's corners and tap offsets within the im2col descriptor's range, checked before anything is launched
+  for (int rh = 0; rh < ph_h; ++rh)
+    for (int rw = 0; rw < ph_w; ++rw) {
+      const PhaseDim a = phase_dim(rh, g->H, g->sh, g->ph, g->dh, g->KH);
+      const PhaseDim b = phase_dim(rw, g->W, g->sw, g->pw, g->dw, g->KW);
+      if (a.taps == 0 || b.taps == 0) continue;
+      const int up_h = a.lo + a.rows - g->OH, up_w = b.lo + b.rows - g->OW;
+      if (a.lo < -128 || a.lo > 127 || b.lo < -128 || b.lo > 127 || up_h < -128 || up_h > 127 || up_w < -128 ||
+          up_w > 127 || (a.taps - 1) * a.dstep >= 256 || (b.taps - 1) * b.dstep >= 256)
+        return kNotEligible;
+    }
+  const int64_t C = g->C, img_y = static_cast<int64_t>(g->H) * g->W * C, y_ss = g->B * img_y;
+  for (int rh = 0; rh < ph_h; ++rh)
+    for (int rw = 0; rw < ph_w; ++rw) {
+      const PhaseDim a = phase_dim(rh, g->H, g->sh, g->ph, g->dh, g->KH);
+      const PhaseDim b = phase_dim(rw, g->W, g->sw, g->pw, g->dw, g->KW);
+      float* base = y + (static_cast<int64_t>(rh) * g->W + rw) * C;
+      if (a.taps == 0 || b.taps == 0) {
+        const int64_t total = static_cast<int64_t>(S) * g->B * a.rows * b.rows * C;
+        const int blocks = static_cast<int>(std::min<int64_t>((total + 255) / 256, 4 * sm_count()));
+        phase_bias_kernel<<<blocks, 256, 0, st>>>(base, y_ss, img_y, g->sh * g->W * C, g->sw * C, S, g->B, a.rows, b.rows,
+                                                  g->C, mu_b, sigma_b, eps_b, sample_begin, rng_b ? *rng_b : *rng_w);
+        BNN_CUDA_OK(cudaGetLastError());
+        continue;
+      }
+      TmaContractParams p{};
+      const int up_h = a.lo + a.rows - g->OH, up_w = b.lo + b.rows - g->OW;
+      int rc = make_im2col_map(&p.map_l, x, g->Cout, g->OW, g->OH, static_cast<int64_t>(shared ? 1 : S) * g->B, b.lo, a.lo,
+                               up_w, up_h, 1, 1, 128, false);
+      if (rc != BNN_OK) return rc;
+      ConvCoords c{};
+      c.on = 1; c.P = a.rows * b.rows; c.OW = b.rows; c.imgs = g->B; c.sh = 1; c.sw = 1; c.lh = a.lo; c.lw = b.lo;
+      c.dh = a.dstep; c.dw = b.dstep; c.KW = b.taps; c.taps = a.taps * b.taps; c.cblocks = g->Cout / kBK;
+      c.w_rows = g->Cout; c.chans = g->Cout;
+      c.wtaps = g->KH * g->KW; c.wKW = g->KW; c.tkh = a.tlast; c.tkw = b.tlast; c.tdh = a.tstep; c.tdw = b.tstep;
+      p.conv = c;
+      p.out.base = base; p.out.bs = g->sw * C; p.out.P = 1;
+      p.out.pw = b.rows; p.out.pimg = a.rows * b.rows; p.out.s_i = g->sh * g->W * C; p.out.s_img = img_y;
+      p.out_sample_stride = y_ss;
+      p.mu_w = mu_w; p.sigma_w = sigma_w; p.eps_w = eps_w; p.mu_b = mu_b; p.sigma_b = sigma_b; p.eps_b = eps_b;
+      p.M = g->B * a.rows * b.rows; p.N = c.taps * g->Cout; p.K = g->C; p.S = S; p.sample_begin = sample_begin;
+      p.w_numel = static_cast<int64_t>(g->Cout) * c.wtaps * g->C;
+      p.rng_w = *rng_w; p.rng_b = rng_b ? *rng_b : *rng_w;
+      p.shared_l = shared ? 1 : 0;
+      p.sum_samples = 0;
+      p.vec_out = 1;            // C % 4 == 0: every CTA takes the staged drain, the only one with the phase view
+      rc = dispatch_tma_contract<true>(p, p.K, st);
+      if (rc != BNN_OK) return rc;
+    }
+  return BNN_OK;
+}
+
+int tma_conv_transpose_dgrad(const float* dy, const float* mu_w, const float* sigma_w, const float* eps_w, float* dx,
+                             int64_t x_sample_stride, const bnn_conv2d_nhwc* g, int S, uint32_t sample_begin,
+                             const bnn_rng* rng_w, cudaStream_t st) {
+  if (!conv_ok(*g) || g->Cout % 4 != 0 || !aligned16(dy) || !aligned16(dx) || rng_w->elem_offset % 4 != 0 ||
+      !aligned16(mu_w) || !aligned16(sigma_w) || (eps_w != nullptr && !aligned16(eps_w)))
+    return kNotEligible;
+  bnn_view v{};
+  v.base = dx; v.batch_stride = g->Cout; v.P = 1;
+  return conv_fwd_launch(dy, static_cast<int64_t>(g->B) * g->H * g->W * g->C, mu_w, sigma_w, nullptr, nullptr, eps_w,
+                         nullptr, v, x_sample_stride, g, S, sample_begin, rng_w, nullptr, x_sample_stride == 0, st);
+}
+
+int tma_conv_transpose_wgrad(const float* dy, const float* x, int64_t x_sample_stride, const float* rho_w,
+                             const float* eps_w, float* dmu_w, float* drho_w, const bnn_conv2d_nhwc* g, int S,
+                             uint32_t sample_begin, const bnn_rng* rng_w, cudaStream_t st) {
+  // conv view: "dY" operand = the transposed input x [S or 1][B*OH*OW][Cout], A = im2col(dy) over [S][B][H][W][C]
+  const int M = g->B * g->OH * g->OW, N = g->Cout, K = g->KH * g->KW * g->C;
+  if (!conv_ok(*g) || N % 4 != 0 || !aligned16(dy) || !aligned16(x) || rng_w->elem_offset % 4 != 0 || !aligned16(rho_w) ||
+      !aligned16(dmu_w) || !aligned16(drho_w) || (eps_w != nullptr && !aligned16(eps_w)))
+    return kNotEligible;
+  const bool shared = x_sample_stride == 0;
+  TmaWgradParams p{};
+  int rc = make_map(&p.map_dy, x, N, M, shared ? 1 : S, N, static_cast<int64_t>(M) * N, kWgRows, true);
+  if (rc != BNN_OK) return rc;
+  rc = make_im2col_map(&p.map_a, dy, g->C, g->W, g->H, static_cast<int64_t>(S) * g->B, -g->pw, -g->ph,
+                       g->pw - (g->KW - 1) * g->dw, g->ph - (g->KH - 1) * g->dh, g->sw, g->sh, kWgRows, true);
+  if (rc != BNN_OK) return rc;
+  p.conv = conv_coords_fwd(*g);
+  p.rho_w = rho_w; p.eps_w = eps_w; p.dmu_w = dmu_w; p.drho_w = drho_w;
+  p.M = M; p.N = N; p.K = K; p.S = S; p.sample_begin = sample_begin;
+  p.rng_w = *rng_w;
+  p.shared_a = 0;
+  p.shared_dy = shared ? 1 : 0;
   return wgrad_plan_and_launch(p, M, N, K, S, st);
 }
 

@@ -394,6 +394,236 @@ class SampledConv2dImplicit(torch.autograd.Function):
         return (dx, dmu, drho, bg[0] if need_b else None, bg[1] if need_b else None) + (None,) * 8
 
 
+# ------------------------------------------------------------------------------------------------ transposed convolution
+def conv_transpose_out(size, k, s, p, op, d):
+    return (size - 1) * s - 2 * p + d * (k - 1) + op + 1
+
+
+def _per_sample(x, S, shared):
+    """The S-sample batch a kernel without a shared-operand mode reads: a shared [B, ...] input is repeated S times."""
+    if not shared or S == 1:
+        return x
+    return x.unsqueeze(0).expand((S,) + tuple(x.shape)).reshape((S * x.shape[0],) + tuple(x.shape[1:]))
+
+
+def _add_sampled_bias(y, mu_b, rho_b, S, spec_b):
+    """y [S*B, C, H, W] += b_s (explicit lowering: the sampled bias materialised by the library, [S, C])."""
+    b = _C.materialize(mu_b.contiguous(), _C.stddev(rho_b.contiguous()), S, spec_b.sample_begin, spec_b.rng(),
+                       eps_in=_eps_slice(spec_b, S, mu_b.numel()))
+    y.view((S, y.shape[0] // S) + tuple(y.shape[1:])).add_(b[:, None, :, None, None])
+
+
+class SampledConvTranspose2dImplicit(torch.autograd.Function):
+    """y[s] = conv_transpose2d(x[s], W_s, b_s) for S samples, W [Cin, Cout, KH, KW], for layers whose CONV VIEW (the
+    convolution from y back to x with the same W read as OIHW) is implicit-eligible: groups == 1, Cout % 32 == 0.  The roles
+    of SampledConv2dImplicit swap: the forward is the conv view's input gradient, computed in TF32 by the phase-decomposed
+    gather (bnn_sampled_conv_transpose2d_fwd: one stride-1 gather per output phase over that phase's taps, the bias in its
+    epilogue); the input gradient is the conv view's forward and the weight gradient its weight gradient.  fp32 (3xTF32)
+    mode, or a request the kernels refuse (e.g. Cin % 32 != 0), lowers explicitly in the same (o, kh, kw, c) column order:
+    bnn_sampled_gemm_dgrad + bnn_col2im_nhwc forward, bnn_im2col_nhwc + bnn_sampled_gemm_fwd / _wgrad backward.
+
+    x: logical [S*B, Cin, H, W] (sample-major) or, when `shared`, [B, Cin, H, W].  The kernels write channels-last; the
+    result is converted once to NCHW-contiguous unless set_conv_output_format('preserve') and x is channels_last."""
+
+    @staticmethod
+    def forward(ctx, x, mu_w, rho_w, mu_b, rho_b, S, shared, spec_w, spec_b, precision, stride, padding, output_padding,
+                dilation):
+        for n, t in (("input", x), ("weight.mean", mu_w), ("weight.scale", rho_w), ("bias.mean", mu_b),
+                     ("bias.scale", rho_b)):
+            _check_f32_cuda(n, t)
+        Cin, Cout, KH, KW = mu_w.shape
+        if x.dim() != 4 or x.shape[1] != Cin:
+            raise RuntimeError(f"sampled conv_transpose2d: input {tuple(x.shape)} does not match weight {tuple(mu_w.shape)}")
+        rows, _, H, W = x.shape
+        B = rows if shared else rows // S
+        if not shared and B * S != rows:
+            raise RuntimeError(f"sampled conv_transpose2d: batch {rows} is not divisible by {S} Monte-Carlo samples")
+        OH = conv_transpose_out(H, KH, stride[0], padding[0], output_padding[0], dilation[0])
+        OW = conv_transpose_out(W, KW, stride[1], padding[1], output_padding[1], dilation[1])
+        if OH <= 0 or OW <= 0:
+            raise RuntimeError("sampled conv_transpose2d: empty output")
+        nchw_out = _CONV_OUTPUT["format"] == "contiguous" or x.is_contiguous()
+        x_cl = _nhwc(x)
+        geom = _C.conv_geom(B, OH, OW, Cout, H, W, Cin, KH, KW, stride, padding, dilation)        # the conv view
+        wl = _C.conv_weight_layout(mu_w.contiguous(), rho_w.contiguous())      # (o = Cin, kh, kw, c = Cout) order
+        has_bias = mu_b is not None
+        mu_b_c = mu_b.contiguous() if has_bias else None
+        sigma_b = _C.stddev(rho_b.contiguous()) if has_bias else None
+        eps_w = _eps_slice(spec_w, S, mu_w.numel())
+        y = torch.empty((S * B, Cout, OH, OW), device=x.device, dtype=torch.float32, memory_format=torch.channels_last)
+        done = precision == _C.PREC_TF32 and _C.try_sampled_conv_transpose2d_fwd(
+            x_cl, 0 if shared else B * H * W * Cin, wl[0], wl[1], mu_b_c, sigma_b, eps_w,
+            _eps_slice(spec_b, S, Cout) if has_bias else None, y, geom, S, spec_w.sample_begin, spec_w.rng(),
+            spec_b.rng() if has_bias else None)
+        if not done:
+            M, K = B * H * W, KH * KW * Cout
+            x_rows = _per_sample(x_cl, S, shared).permute(0, 2, 3, 1).reshape(S * M, Cin)
+            dcol = torch.empty((S * M, K), device=x.device, dtype=torch.float32)
+            _C.sampled_gemm_dgrad(_C.make_view(x_rows.data_ptr(), Cin, 1), M * Cin, wl[0], wl[1], eps_w, dcol, K, M * K, M,
+                                  Cin, K, S, spec_w.sample_begin, spec_w.rng(), precision)
+            _C.col2im_nhwc(dcol, y, geom, S * B)
+            if has_bias:
+                _add_sampled_bias(y, mu_b, rho_b, S, spec_b)
+        ctx.save_for_backward(x_cl, wl, rho_b)
+        ctx.meta = (S, shared, spec_w, spec_b, precision, geom, tuple(mu_w.shape), rows)
+        return y.contiguous() if nchw_out else y
+
+    @staticmethod
+    def backward(ctx, dy):
+        x_cl, wl, rho_b = ctx.saved_tensors
+        S, shared, spec_w, spec_b, precision, geom, w_shape, rows = ctx.meta
+        Cin, Cout, KH, KW = w_shape
+        B, H, W, OH, OW = geom.B, geom.OH, geom.OW, geom.H, geom.W          # transposed input H x W, output OH x OW
+        M, K = B * H * W, KH * KW * Cout
+        eps_w = _eps_slice(spec_w, S, Cin * K)
+        x_ss = 0 if shared else M * Cin
+        tf32 = precision == _C.PREC_TF32
+        need_x = ctx.needs_input_grad[0]
+        need_w = ctx.needs_input_grad[1] or ctx.needs_input_grad[2]
+        need_b = rho_b is not None and (ctx.needs_input_grad[3] or ctx.needs_input_grad[4])
+        bias_done, bg_fused = False, None
+        if dy.permute(0, 2, 3, 1).is_contiguous():
+            dy_cl = dy
+        else:
+            dy_cl = None
+            if dy.is_contiguous():
+                if need_b:
+                    bg_fused = torch.zeros((2, Cout), device=dy.device, dtype=torch.float32)
+                dy_cl = _C.nchw_to_nhwc_bias_grad(dy, B, rho_b.contiguous() if need_b else None,
+                                                  _eps_slice(spec_b, S, Cout) if need_b else None,
+                                                  bg_fused[0] if need_b else None, bg_fused[1] if need_b else None,
+                                                  spec_b.sample_begin if need_b else 0, spec_b.rng() if need_b else None)
+                bias_done = dy_cl is not None and need_b
+            if dy_cl is None:
+                dy_cl = dy.contiguous(memory_format=torch.channels_last)
+        col = None
+        if (need_x or need_w) and not tf32:
+            col = _C.im2col_nhwc(dy_cl, geom, S * B)
+        dx = None
+        if need_x:
+            dx = torch.empty(x_cl.shape, device=dy.device, dtype=torch.float32, memory_format=torch.channels_last)
+            done = tf32 and _C.try_sampled_conv_transpose2d_dgrad(dy_cl, wl[0], wl[1], eps_w, dx, x_ss, geom, S,
+                                                                  spec_w.sample_begin, spec_w.rng())
+            if not done:
+                if col is None:
+                    col = _C.im2col_nhwc(dy_cl, geom, S * B)
+                out = dx if not shared or S == 1 else torch.empty((S * M, Cin), device=dy.device, dtype=torch.float32)
+                _C.sampled_gemm_fwd(col, K, M * K, wl[0], wl[1], None, None, eps_w, None,
+                                    _C.make_view(out.data_ptr(), Cin, 1), M * Cin, M, Cin, K, S, spec_w.sample_begin,
+                                    spec_w.rng(), None, precision)
+                if out is not dx:               # shared input: the per-sample contributions summed
+                    dx.permute(0, 2, 3, 1).copy_(out.view(S, B, H, W, Cin).sum(0))
+        grads_p, bg = _zero_grads((Cin * K,) if need_w else None, Cout if (need_b and not bias_done) else None, dy.device)
+        if bias_done:
+            bg = bg_fused
+        dmu = drho = None
+        if need_w:
+            done = tf32 and _C.try_sampled_conv_transpose2d_wgrad(dy_cl, x_cl, x_ss, wl[2], eps_w, grads_p[0], grads_p[1],
+                                                                  geom, S, spec_w.sample_begin, spec_w.rng())
+            if not done:
+                if col is None:
+                    col = _C.im2col_nhwc(dy_cl, geom, S * B)
+                x_rows = _per_sample(x_cl, S, shared).permute(0, 2, 3, 1).reshape(S * M, Cin)
+                _C.sampled_gemm_wgrad(_C.make_view(x_rows.data_ptr(), Cin, 1), M * Cin, col, K, M * K, wl[2], eps_w,
+                                      grads_p[0], grads_p[1], M, Cin, K, S, spec_w.sample_begin, spec_w.rng(), precision)
+            g = _C.conv_weight_unlayout(grads_p, w_shape)
+            dmu, drho = g[0], g[1]
+        if need_b and not bias_done:
+            _C.bias_grad(_C.make_view(dy_cl.data_ptr(), Cout, 1), B * OH * OW * Cout, rho_b.contiguous(),
+                         _eps_slice(spec_b, S, Cout), bg[0], bg[1], B * OH * OW, Cout, S, spec_b.sample_begin, spec_b.rng())
+        return (dx, dmu, drho, bg[0] if need_b else None, bg[1] if need_b else None) + (None,) * 9
+
+
+class SampledConvTranspose2d(torch.autograd.Function):
+    """y[s] = conv_transpose2d(x[s], W_s, b_s, groups=groups) for S samples, for layers whose conv view is not
+    implicit-eligible (groups > 1, or Cout % 32 != 0 such as a 3-channel image): the NCHW lowering of SampledConv2d with the
+    roles swapped — per group the column gradients of the conv view (bnn_sampled_gemm_dgrad, x in the role of dY) gathered
+    by bnn_col2im; backward bnn_im2col of dy + bnn_sampled_gemm_fwd / _wgrad.  Weights keyed in storage (OIHW) order."""
+
+    @staticmethod
+    def forward(ctx, x, mu_w, rho_w, mu_b, rho_b, S, shared, spec_w, spec_b, precision, stride, padding, output_padding,
+                dilation, groups):
+        for n, t in (("input", x), ("weight.mean", mu_w), ("weight.scale", rho_w), ("bias.mean", mu_b),
+                     ("bias.scale", rho_b)):
+            _check_f32_cuda(n, t)
+        Cin, Cout_g, KH, KW = mu_w.shape
+        Cout = Cout_g * groups
+        if x.dim() != 4 or x.shape[1] != Cin:
+            raise RuntimeError(f"sampled conv_transpose2d: input {tuple(x.shape)} does not match weight {tuple(mu_w.shape)}")
+        rows, _, H, W = x.shape
+        B = rows if shared else rows // S
+        if not shared and B * S != rows:
+            raise RuntimeError(f"sampled conv_transpose2d: batch {rows} is not divisible by {S} Monte-Carlo samples")
+        OH = conv_transpose_out(H, KH, stride[0], padding[0], output_padding[0], dilation[0])
+        OW = conv_transpose_out(W, KW, stride[1], padding[1], output_padding[1], dilation[1])
+        if OH <= 0 or OW <= 0:
+            raise RuntimeError("sampled conv_transpose2d: empty output")
+        geo = (B, Cin, H, W, Cout, KH, KW, OH, OW, tuple(stride), tuple(padding), tuple(dilation), groups)
+        xs = _per_sample(x.contiguous(), S, shared)
+        mu_w_c, rho_w_c = mu_w.contiguous(), rho_w.contiguous()
+        sigma_w = _C.stddev(rho_w_c)
+        Cin_g, Kg, P = Cin // groups, Cout_g * KH * KW, H * W
+        M = B * P
+        y = torch.empty((S * B, Cout, OH, OW), device=x.device, dtype=torch.float32)
+        dcol = torch.empty((S * M, Kg), device=x.device, dtype=torch.float32)
+        for g in range(groups):
+            lo, hi = g * Cin_g * Kg, (g + 1) * Cin_g * Kg
+            _C.sampled_gemm_dgrad(_C.make_view(xs.data_ptr() + 4 * g * Cin_g * P, Cin * P, P), B * Cin * P,
+                                  mu_w_c.view(-1)[lo:hi], sigma_w.view(-1)[lo:hi], _eps_slice(spec_w, S, mu_w.numel(), lo, hi),
+                                  dcol, Kg, M * Kg, M, Cin_g, Kg, S, spec_w.sample_begin, spec_w.rng(lo), precision)
+            _C.col2im(dcol, y, SampledConvTranspose2d._geom(S * B, geo, g), False)
+        if mu_b is not None:
+            _add_sampled_bias(y, mu_b, rho_b, S, spec_b)
+        ctx.save_for_backward(xs, mu_w_c, rho_w_c, sigma_w, rho_b)
+        ctx.meta = (S, shared, spec_w, spec_b, precision, geo)
+        return y
+
+    @staticmethod
+    def _geom(batch, geo, g):
+        """bnn_conv2d_geom of group g of the conv view (input = the transposed output)."""
+        B, Cin, H, W, Cout, KH, KW, OH, OW, stride, padding, dilation, groups = geo
+        Cout_g = Cout // groups
+        return _C.bnn_conv2d_geom(batch, Cout, OH, OW, g * Cout_g, Cout_g, KH, KW, H, W, stride[0], stride[1],
+                                  padding[0], padding[1], dilation[0], dilation[1])
+
+    @staticmethod
+    def backward(ctx, dy):
+        xs, mu_w, rho_w, sigma_w, rho_b = ctx.saved_tensors
+        S, shared, spec_w, spec_b, precision, geo = ctx.meta
+        B, Cin, H, W, Cout, KH, KW, OH, OW, stride, padding, dilation, groups = geo
+        dy = dy.contiguous()
+        Cin_g, Kg, P, Q = Cin // groups, (Cout // groups) * KH * KW, H * W, OH * OW
+        M = B * P
+        need_x = ctx.needs_input_grad[0]
+        need_w = ctx.needs_input_grad[1] or ctx.needs_input_grad[2]
+        need_b = rho_b is not None and (ctx.needs_input_grad[3] or ctx.needs_input_grad[4])
+        dxs = torch.empty(xs.shape, device=dy.device, dtype=torch.float32) if need_x else None
+        grads, bg = _zero_grads(tuple(mu_w.shape) if need_w else None, Cout if need_b else None, dy.device)
+        col = torch.empty((S * M, Kg), device=dy.device, dtype=torch.float32) if (need_x or need_w) else None
+        for g in range(groups):
+            lo, hi = g * Cin_g * Kg, (g + 1) * Cin_g * Kg
+            eps_w = _eps_slice(spec_w, S, mu_w.numel(), lo, hi)
+            if need_x or need_w:
+                _C.im2col(dy, col, SampledConvTranspose2d._geom(S * B, geo, g))
+            if need_x:
+                _C.sampled_gemm_fwd(col, Kg, M * Kg, mu_w.view(-1)[lo:hi], sigma_w.view(-1)[lo:hi], None, None, eps_w, None,
+                                    _C.make_view(dxs.data_ptr() + 4 * g * Cin_g * P, Cin * P, P), B * Cin * P, M, Cin_g,
+                                    Kg, S, spec_w.sample_begin, spec_w.rng(lo), None, precision)
+            if need_w:
+                _C.sampled_gemm_wgrad(_C.make_view(xs.data_ptr() + 4 * g * Cin_g * P, Cin * P, P), B * Cin * P, col, Kg,
+                                      M * Kg, rho_w.view(-1)[lo:hi], eps_w, grads[0].view(-1)[lo:hi],
+                                      grads[1].view(-1)[lo:hi], M, Cin_g, Kg, S, spec_w.sample_begin, spec_w.rng(lo),
+                                      precision)
+        if need_b:
+            _C.bias_grad(_C.make_view(dy.data_ptr(), Cout * Q, Q), B * Cout * Q, rho_b.contiguous(),
+                         _eps_slice(spec_b, S, Cout), bg[0], bg[1], B * Q, Cout, S, spec_b.sample_begin, spec_b.rng())
+        dx = None
+        if need_x:
+            dx = dxs.view(S, B, Cin, H, W).sum(0) if shared and S > 1 else dxs
+        return (dx, grads[0] if need_w else None, grads[1] if need_w else None,
+                bg[0] if need_b else None, bg[1] if need_b else None) + (None,) * 10
+
+
 # ------------------------------------------------------------------------------------------------
 class Materialize(torch.autograd.Function):
     """W_s = mean + stddev * eps_s for s in [0, S) as a tensor [S, *shape] (core.py:44-45); used by

@@ -2,8 +2,8 @@
 
 Constructor signatures, attributes (`weight`, `bias`, `sampled`, `sample()`, priors, conv geometry)
 and `forward(x, sample=True)` follow the reference; the arithmetic runs in libbnn_b200.so:
-NormalLinear and NormalConv1d/2d call the fused sample-and-contract kernels (no sampled weight in
-memory), NormalConv3d contracts materialised samples with torch's conv3d.
+NormalLinear, NormalConv1d/2d and NormalConvTranspose1d/2d call the fused sample-and-contract kernels (no sampled
+weight in memory), NormalConv3d contracts materialised samples with torch's conv3d.
 """
 import math
 
@@ -12,7 +12,8 @@ from torch.distributions.normal import Normal
 from torch.nn import init
 
 from .. import runtime
-from ..functional import SampledConv2d, SampledConv2dImplicit, SampledLinear, conv_implicit_eligible
+from ..functional import (SampledConv2d, SampledConv2dImplicit, SampledConvTranspose2d, SampledConvTranspose2dImplicit,
+                          SampledLinear, conv_implicit_eligible)
 from ..utils.traversal import _pair, _single, _triple
 from .container import BayesianModule
 from .variational import WeightNormal
@@ -172,9 +173,10 @@ class NormalConvNd(BayesianConvNd):
 
 def _mark_implicit(layer):
     """Layers with groups == 1 and in_channels % 32 == 0 run the implicit-GEMM path; their weight's eps stream is keyed in
-    (o, kh, kw, c) order (variational.WeightNormal._eps_layout)."""
+    (o, kh, kw, c) order (variational.WeightNormal._eps_layout).  A transposed layer is judged by its conv view (the
+    convolution from its output back to its input, whose in_channels are the layer's out_channels)."""
     w = layer.weight.mean
-    layer._implicit = conv_implicit_eligible(layer.in_channels, layer.groups) and not layer.transposed
+    layer._implicit = conv_implicit_eligible(layer.out_channels if layer.transposed else layer.in_channels, layer.groups)
     if layer._implicit:
         layer.weight._eps_layout = (w.shape[0], w.shape[1], w.numel() // (w.shape[0] * w.shape[1]))
 
@@ -225,6 +227,79 @@ class NormalConv1d(_FusedBayesianLayer, NormalConvNd):
         w_shape = (self.weight.mean.shape[0], self.weight.mean.shape[1], 1, self.weight.mean.shape[2])
         y = _sampled_conv2d(self, x.unsqueeze(2), w_shape, S, shared, spec_w, spec_b, (1, tuple(self.stride)[0]),
                             (0, tuple(self.padding)[0]), (1, tuple(self.dilation)[0]))
+        if ctx is not None:
+            ctx.expanded = True
+        return y.squeeze(2)
+
+
+class NormalConvTransposeNd(NormalConvNd):
+    """Bayesian transposed convolution: weight [in_channels, out_channels // groups, *kernel_size] as the reference's
+    BayesianConvNd(transposed=True) stores it (conv.py:26-28), plus `output_padding`.  The reference never wrote its forward;
+    this one computes F.conv_transposeNd(x, W_s, b_s, stride, padding, output_padding, groups, dilation) for all
+    Monte-Carlo samples in one fused call."""
+
+    def __init__(self, in_channels, out_channels, kernel_size, stride, padding, output_padding, groups, bias, dilation,
+                 prior):
+        super(NormalConvTransposeNd, self).__init__(in_channels, out_channels, kernel_size, stride, padding, dilation,
+                                                    True, groups, bias, prior)
+        for op, s, d in zip(output_padding, self.stride, self.dilation):
+            if not 0 <= op < max(s, d):
+                raise ValueError(f"output_padding {tuple(output_padding)} must be smaller than either stride "
+                                 f"{tuple(self.stride)} or dilation {tuple(self.dilation)} in every dimension")
+        self.output_padding = output_padding
+        _mark_implicit(self)
+
+    def _conv_transpose2d(self, x, w_shape, S, shared, spec_w, spec_b, stride, padding, output_padding, dilation):
+        # output_padding >= stride (possible when dilation > stride): the rows beyond the conv view are reached by
+        # appending zero input rows, which leaves output_padding % stride
+        extra = [op // s for op, s in zip(output_padding, stride)]
+        if any(extra):
+            x = torch.nn.functional.pad(x, (0, extra[1], 0, extra[0]))
+            output_padding = tuple(op % s for op, s in zip(output_padding, stride))
+        bias = self.bias
+        mean, scale = self.weight.mean.view(w_shape), self.weight.scale.view(w_shape)
+        args = (x, mean, scale, bias.mean if bias is not None else None, bias.scale if bias is not None else None, S,
+                shared, spec_w, spec_b, runtime.precision(), stride, padding, output_padding, dilation)
+        if self._implicit:
+            return SampledConvTranspose2dImplicit.apply(*args)
+        return SampledConvTranspose2d.apply(*args, self.groups)
+
+
+class NormalConvTranspose2d(_FusedBayesianLayer, NormalConvTransposeNd):
+    """torch.nn.ConvTranspose2d's constructor order with a Normal variational posterior on weight and bias."""
+
+    def __init__(self, in_channels, out_channels, kernel_size, stride=1, padding=0, output_padding=0, groups=1,
+                 bias=True, dilation=1, prior=Normal(0, .1)):
+        super(NormalConvTranspose2d, self).__init__(in_channels, out_channels, _pair(kernel_size), _pair(stride),
+                                                    _pair(padding), _pair(output_padding), groups, bias,
+                                                    _pair(dilation), prior)
+
+    def forward(self, x, sample=True):
+        S, shared, offset, total, ctx = self._mc_shape(x)
+        spec_w, spec_b = self._draws(sample, S, offset, total)
+        y = self._conv_transpose2d(x, tuple(self.weight.mean.shape), S, shared, spec_w, spec_b, tuple(self.stride),
+                                   tuple(self.padding), tuple(self.output_padding), tuple(self.dilation))
+        if ctx is not None:
+            ctx.expanded = True
+        return y
+
+
+class NormalConvTranspose1d(_FusedBayesianLayer, NormalConvTransposeNd):
+    """torch.nn.ConvTranspose1d's constructor order — evaluated as a 2-d transposed convolution with a height of one."""
+
+    def __init__(self, in_channels, out_channels, kernel_size, stride=1, padding=0, output_padding=0, groups=1,
+                 bias=True, dilation=1, prior=Normal(0, .1)):
+        super(NormalConvTranspose1d, self).__init__(in_channels, out_channels, _single(kernel_size), _single(stride),
+                                                    _single(padding), _single(output_padding), groups, bias,
+                                                    _single(dilation), prior)
+
+    def forward(self, x, sample=True):
+        S, shared, offset, total, ctx = self._mc_shape(x)
+        spec_w, spec_b = self._draws(sample, S, offset, total)
+        w = self.weight.mean.shape
+        y = self._conv_transpose2d(x.unsqueeze(2), (w[0], w[1], 1, w[2]), S, shared, spec_w, spec_b,
+                                   (1, tuple(self.stride)[0]), (0, tuple(self.padding)[0]),
+                                   (0, tuple(self.output_padding)[0]), (1, tuple(self.dilation)[0]))
         if ctx is not None:
             ctx.expanded = True
         return y.squeeze(2)

@@ -204,6 +204,39 @@ int bnn_sampled_conv2d_dgrad(const float* dy, const float* mu_w, const float* si
 int bnn_sampled_conv2d_wgrad(const float* dy, const float* x, int64_t x_sample_stride, const float* rho_w,
                              const float* eps_w, float* dmu_w, float* drho_w, const bnn_conv2d_nhwc* g, int32_t S,
                              uint32_t sample_begin, const bnn_rng* rng_w, void* stream);
+/* ---- transposed convolution on the same kernels ----
+ * NormalConvTranspose2d.forward (F.conv_transpose2d(x, W_s, b_s, stride, padding, output_padding, 1, dilation) for S
+ * Monte-Carlo samples) and its autograd.  W [Cin][Cout][KH][KW]; `g` describes the CONV VIEW of the layer, the convolution
+ * from the transposed output to the transposed input with the same W read as OIHW: g->C = Cout and g->H, g->W = output
+ * size; g->Cout = Cin and g->OH, g->OW = input size; KH, KW, stride, padding, dilation as given (output_padding is the
+ * part of g->H, g->W the conv view rounds away, so it must be below the stride).  Weights, sigma, rho, eps and gradients
+ * in the conv view's (o, kh, kw, c) order = [Cin][KH][KW][Cout] (bnn_conv2d_weight_layout with Cout = Cin).
+ *   fwd    y[s] = conv_transpose2d(x[s], W_s) + b_s: x NHWC [S or 1][B][OH][OW][Cin] (x_sample_stride = 0: shared), y NHWC
+ *          [S][B][H][W][Cout] contiguous.  The outputs are cut into sh x sw phases (h % sh, w % sw); each phase is a
+ *          stride-1 transposed-filter gather over its own taps (one launch per phase), phases without a tap get b_s.
+ *          Needs Cin % 32 == 0, Cout % 4 == 0, stride <= 8.
+ *   dgrad  dx[s] = conv2d(dy[s], W_s) (the conv view's forward, no bias); dy NHWC [S][B][H][W][Cout], dx NHWC;
+ *          x_sample_stride = 0 sums the S contributions into one dx.  Needs Cout % 32 == 0, Cin % 4 == 0.
+ *   wgrad  G_s = x[s]^T im2col(dy[s]) accumulated as bnn_sampled_conv2d_wgrad; x_sample_stride = 0: all samples read x.
+ *          Needs Cout % 32 == 0, Cin % 4 == 0.
+ * No allocation, no stream synchronisation.  BNN_ERR_UNSUPPORTED when a requirement is not met (callers then lower
+ * explicitly: bnn_sampled_gemm_dgrad + bnn_col2im_nhwc for the forward, bnn_im2col_nhwc + bnn_sampled_gemm_fwd / _wgrad
+ * for the gradients). */
+int bnn_sampled_conv_transpose2d_fwd(const float* x, int64_t x_sample_stride, const float* mu_w, const float* sigma_w,
+                                     const float* mu_b, const float* sigma_b, const float* eps_w, const float* eps_b, float* y,
+                                     const bnn_conv2d_nhwc* g, int32_t S, uint32_t sample_begin, const bnn_rng* rng_w,
+                                     const bnn_rng* rng_b, void* stream);
+int bnn_sampled_conv_transpose2d_dgrad(const float* dy, const float* mu_w, const float* sigma_w, const float* eps_w,
+                                       float* dx, int64_t x_sample_stride, const bnn_conv2d_nhwc* g, int32_t S,
+                                       uint32_t sample_begin, const bnn_rng* rng_w, void* stream);
+int bnn_sampled_conv_transpose2d_wgrad(const float* dy, const float* x, int64_t x_sample_stride, const float* rho_w,
+                                       const float* eps_w, float* dmu_w, float* drho_w, const bnn_conv2d_nhwc* g, int32_t S,
+                                       uint32_t sample_begin, const bnn_rng* rng_w, void* stream);
+/* Host only (test aid): the phase plan of bnn_sampled_conv_transpose2d_fwd, 14 ints per phase {rh, rw, rows_h, rows_w,
+ * taps_h, taps_w, last tap h, last tap w, tap step h, tap step w, first input row h, w, input step h, w}: walked tap j of
+ * the phase is kh = last - j * tap step, read at input row i + first + j * input step for output row rh + sh * i.  Returns
+ * the number of phases (may exceed max_phases; only max_phases are written) or a negative bnn_status. */
+int bnn_debug_conv_transpose_phases(const bnn_conv2d_nhwc* g, int32_t* out, int32_t max_phases);
 /* OIHW parameters [Cout][Cg][taps] -> (o, kh, kw, c) order: mu_p, and optionally sigma_p = 1e-10 + softplus(rho) and
  * rho_p (NULL to skip); the inverse for `n_arrays` arrays stored back to back (gradients of mean and scale). */
 int bnn_conv2d_weight_layout(const float* mu, const float* rho, float* mu_p, float* sigma_p, float* rho_p, int32_t Cout,
