@@ -237,17 +237,26 @@ def kernel_timing_summary(steps=1):
     return out
 
 
-def _call(name, *args):
+_ERR_UNSUPPORTED = 6      # BNN_ERR_UNSUPPORTED: a request outside the kernels' stated limits, refused before any launch
+
+
+def _invoke(name, *args):
+    """Status of one library call, bracketed with CUDA events while kernel timing is on (a refused request is not
+    recorded: it launched nothing)."""
     fn = getattr(lib(), name)
     if _timing is None:
-        rc = fn(*args)
-    else:
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record()
-        rc = fn(*args)
-        e1.record()
+        return fn(*args)
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    e0.record()
+    rc = fn(*args)
+    e1.record()
+    if rc != _ERR_UNSUPPORTED:
         _timing.append((name, e0, e1))
-    _check(rc, name)
+    return rc
+
+
+def _call(name, *args):
+    _check(_invoke(name, *args), name)
 
 
 def _count(n=1):
@@ -508,6 +517,26 @@ def sampled_conv2d_wgrad(dy, x, x_sample_stride, rho_w, eps_w, dmu_w, drho_w, ge
         _call("bnn_sampled_conv2d_wgrad", _ptr(dy), _ptr(x), x_sample_stride, _ptr(rho_w), _ptr(eps_w), _ptr(dmu_w),
               _ptr(drho_w), ctypes.byref(geom), S, sample_begin, ctypes.byref(rng_w), _stream())
     _count()
+
+
+# The same three calls for callers with an explicit lowering to fall back on: False (nothing launched) when the kernels
+# refuse the request (stride > 8, a filter window outside the im2col descriptor's range, Cout not a multiple of 32 for
+# the input gradient or of 4 for the weight gradient, ...).  The C entry points are the one place that decides.
+def try_sampled_conv2d_fwd(x, x_sample_stride, mu_w, sigma_w, mu_b, sigma_b, eps_w, eps_b, y_view, y_sample_stride, geom,
+                           S, sample_begin, rng_w, rng_b):
+    return _try_call("bnn_sampled_conv2d_fwd", x.device, _ptr(x), x_sample_stride, _ptr(mu_w), _ptr(sigma_w), _ptr(mu_b),
+                     _ptr(sigma_b), _ptr(eps_w), _ptr(eps_b), y_view, y_sample_stride, ctypes.byref(geom), S, sample_begin,
+                     ctypes.byref(rng_w), ctypes.byref(rng_b) if rng_b is not None else None, _stream())
+
+
+def try_sampled_conv2d_dgrad(dy, mu_w, sigma_w, eps_w, dx, x_sample_stride, geom, S, sample_begin, rng_w):
+    return _try_call("bnn_sampled_conv2d_dgrad", dx.device, _ptr(dy), _ptr(mu_w), _ptr(sigma_w), _ptr(eps_w), _ptr(dx),
+                     x_sample_stride, ctypes.byref(geom), S, sample_begin, ctypes.byref(rng_w), _stream())
+
+
+def try_sampled_conv2d_wgrad(dy, x, x_sample_stride, rho_w, eps_w, dmu_w, drho_w, geom, S, sample_begin, rng_w):
+    return _try_call("bnn_sampled_conv2d_wgrad", x.device, _ptr(dy), _ptr(x), x_sample_stride, _ptr(rho_w), _ptr(eps_w),
+                     _ptr(dmu_w), _ptr(drho_w), ctypes.byref(geom), S, sample_begin, ctypes.byref(rng_w), _stream())
 
 
 _kl_ws = {}
@@ -827,9 +856,8 @@ def try_sampled_conv_transpose2d_wgrad(dy, x, x_sample_stride, rho_w, eps_w, dmu
 def _try_call(name, device, *args):
     """Like _call, but BNN_ERR_UNSUPPORTED (a request outside the kernels' stated limits) returns False."""
     with torch.cuda.device(device):
-        fn = getattr(lib(), name)
-        rc = fn(*args)
-    if rc == 6:                                   # BNN_ERR_UNSUPPORTED
+        rc = _invoke(name, *args)
+    if rc == _ERR_UNSUPPORTED:
         return False
     _check(rc, name)
     _count()

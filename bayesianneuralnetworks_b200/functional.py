@@ -278,8 +278,10 @@ class SampledConv2dImplicit(torch.autograd.Function):
     activations reach the tensor cores through a TMA im2col tensor map, the weights are presented in (o, kh, kw, c) order
     (one small layout kernel per step, which also produces sigma), the input gradient of stride-1 layers is the
     transposed-filter gather, the weight gradient reads dY and x through tensor maps and is returned in OIHW order.
-    TF32 mode; fp32 (3xTF32) mode and the input gradient of strided layers lower explicitly in the same column order
-    (bnn_im2col_nhwc / bnn_col2im_nhwc + the register-staged / TMA GEMM kernels).
+    TF32 mode; fp32 (3xTF32) mode, the input gradient of strided layers and every request the kernels refuse (stride > 8,
+    a filter window outside the im2col descriptor's range, Cout % 32 != 0 for the input gradient or Cout % 4 != 0 for the
+    weight gradient: the C entry point returns BNN_ERR_UNSUPPORTED before launching anything) lower explicitly in the
+    same column order (bnn_im2col_nhwc / bnn_col2im_nhwc + the register-staged / TMA GEMM kernels).
 
     x: logical [S*B, C, H, W] (sample-major) or, when `shared`, [B, C, H, W]; any memory format — channels_last input gives
     a channels_last result under set_conv_output_format('preserve'); by default the result is NCHW-contiguous (written
@@ -319,10 +321,10 @@ class SampledConv2dImplicit(torch.autograd.Function):
         eps_w = _eps_slice(spec_w, S, Cout * K)
         eps_b = _eps_slice(spec_b, S, Cout) if has_bias else None
         x_ss = 0 if shared else B * H * W * C
-        if precision == _C.PREC_TF32:
-            _C.sampled_conv2d_fwd(x_cl, x_ss, wl[0], wl[1], mu_b_c, sigma_b, eps_w, eps_b, y_view, y_ss, geom, S,
-                                  spec_w.sample_begin, spec_w.rng(), spec_b.rng() if has_bias else None)
-        else:
+        done = precision == _C.PREC_TF32 and _C.try_sampled_conv2d_fwd(
+            x_cl, x_ss, wl[0], wl[1], mu_b_c, sigma_b, eps_w, eps_b, y_view, y_ss, geom, S, spec_w.sample_begin,
+            spec_w.rng(), spec_b.rng() if has_bias else None)
+        if not done:
             col = _C.im2col_nhwc(x_cl, geom, rows)
             _C.sampled_gemm_fwd(col, K, 0 if shared else M * K, wl[0], wl[1], mu_b_c, sigma_b, eps_w, eps_b, y_view, y_ss,
                                 M, Cout, K, S, spec_w.sample_begin, spec_w.rng(), spec_b.rng() if has_bias else None,
@@ -367,9 +369,9 @@ class SampledConv2dImplicit(torch.autograd.Function):
         dx = None
         if need_x:
             dx = torch.empty(x_cl.shape, device=dy.device, dtype=torch.float32, memory_format=torch.channels_last)
-            if tf32 and geom.sh == 1 and geom.sw == 1 and Cout % 32 == 0:
-                _C.sampled_conv2d_dgrad(dy_cl, wl[0], wl[1], eps_w, dx, x_ss, geom, S, spec_w.sample_begin, spec_w.rng())
-            else:                                       # strided layers / fp32 mode: column gradients + gather
+            done = tf32 and _C.try_sampled_conv2d_dgrad(dy_cl, wl[0], wl[1], eps_w, dx, x_ss, geom, S,
+                                                        spec_w.sample_begin, spec_w.rng())
+            if not done:                                # strided / refused layers, fp32 mode: column gradients + gather
                 dcol = torch.empty((rows * P, K), device=dy.device, dtype=torch.float32)
                 _C.sampled_gemm_dgrad(dy_view, dy_ss, wl[0], wl[1], eps_w, dcol, K, 0 if shared else M * K, M, Cout, K, S,
                                       spec_w.sample_begin, spec_w.rng(), precision)
@@ -379,10 +381,9 @@ class SampledConv2dImplicit(torch.autograd.Function):
             bg = bg_fused
         dmu = drho = None
         if need_w:
-            if tf32 and Cout % 4 == 0:
-                _C.sampled_conv2d_wgrad(dy_cl, x_cl, x_ss, wl[2], eps_w, grads_p[0], grads_p[1], geom, S,
-                                        spec_w.sample_begin, spec_w.rng())
-            else:
+            done = tf32 and _C.try_sampled_conv2d_wgrad(dy_cl, x_cl, x_ss, wl[2], eps_w, grads_p[0], grads_p[1], geom, S,
+                                                        spec_w.sample_begin, spec_w.rng())
+            if not done:
                 col = _C.im2col_nhwc(x_cl, geom, rows)
                 _C.sampled_gemm_wgrad(dy_view, dy_ss, col, K, 0 if shared else M * K, wl[2], eps_w, grads_p[0], grads_p[1],
                                       M, Cout, K, S, spec_w.sample_begin, spec_w.rng(), precision)
