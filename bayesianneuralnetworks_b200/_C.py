@@ -175,10 +175,6 @@ _SIGNATURES = {
     "bnn_debug_force_contract_variant": (ctypes.c_int, [ctypes.c_int32]),
     "bnn_debug_pair_tile_plan": (ctypes.c_int, [ctypes.c_int32, ctypes.c_int32, ctypes.c_int32,
                                                 ctypes.POINTER(ctypes.c_int32)]),
-    "bnn_contract_set_balanced": (ctypes.c_int, [ctypes.c_int32]),
-    "bnn_debug_balanced_plan": (ctypes.c_int, [ctypes.c_int32] * 7 + [ctypes.POINTER(ctypes.c_int32), ctypes.c_int32]),
-    "bnn_debug_balanced_schedule": (ctypes.c_int, [ctypes.c_int32, ctypes.POINTER(ctypes.c_int32),
-                                                   ctypes.POINTER(ctypes.c_int32)]),
     "bnn_selftest_umma": (ctypes.c_int, [_c_f32p, ctypes.c_void_p]),
     "bnn_selftest_umma_mn": (ctypes.c_int, [_c_f32p, ctypes.c_void_p]),
 }
@@ -352,38 +348,6 @@ def materialize(mu, sigma, S, sample_begin, rng, eps_in=None, want_eps=False):
                                      mu.numel(), S, sample_begin, ctypes.byref(rng), _stream())
     _count()
     return (out, eps_out) if want_eps else out
-
-
-def set_balanced_schedule(flag=True):
-    """True: the CTA-pair contraction kernels may take their balanced (persistent) schedule where the launcher's cost
-    model prefers it (bnn_contract_set_balanced).  Off by default — measured slower on B200, DESIGN §4; BNN_BALANCED=1 in
-    the environment starts the process with it on."""
-    _check(lib().bnn_contract_set_balanced(1 if flag else 0), "bnn_contract_set_balanced")
-
-
-def balanced_plan(m_blocks, samples, column_tiles, red_blocks, sum_samples, slots, slot):
-    """Host-side test aid: [(leader's first row, row blocks per CTA, column tile, sample, first k-block, k-blocks)] that
-    `slot` walks in the balanced schedule (no device needed)."""
-    cap = 64
-    while True:
-        buf = (ctypes.c_int32 * (6 * cap))()
-        n = lib().bnn_debug_balanced_plan(m_blocks, samples, column_tiles, red_blocks, 1 if sum_samples else 0, slots, slot,
-                                          buf, cap)
-        if n < 0:
-            _check(-n, "bnn_debug_balanced_plan")
-        if n <= cap:
-            return [tuple(buf[6 * i:6 * i + 6]) for i in range(n)]
-        cap = n
-
-
-def balanced_schedule_state(slot_cap=-1, device=None):
-    """(launches that took the balanced schedule so far, co-resident CTA pairs of the device); slot_cap >= 0 caps the
-    clusters of the schedule (test aid; 0 removes the cap)."""
-    launches, slots = ctypes.c_int32(0), ctypes.c_int32(0)
-    with torch.cuda.device(device if device is not None else torch.cuda.current_device()):
-        _check(lib().bnn_debug_balanced_schedule(int(slot_cap), ctypes.byref(launches), ctypes.byref(slots)),
-               "bnn_debug_balanced_schedule")
-    return launches.value, slots.value
 
 
 def sampled_gemm_fwd(a, lda, a_sample_stride, mu_w, sigma_w, mu_b, sigma_b, eps_w, eps_b, y_view,
@@ -819,9 +783,8 @@ def selftest_prune_interval(mu, rho, variant=1):
 
 
 def force_contract_variant(variant):
-    """Test aid: 'pair' | 'balanced' (the pair kernel's balanced schedule) | 'mb4' | 'mb2' | 'mb1' | None (cost model) for
-    the TMA-fed forward / data-gradient kernels."""
-    code = {None: -1, "pair": 0, "mb1": 1, "mb2": 2, "mb4": 4, "balanced": 8}[variant]
+    """Test aid: 'pair' | 'mb4' | 'mb2' | 'mb1' | None (cost model) for the TMA-fed forward / data-gradient kernels."""
+    code = {None: -1, "pair": 0, "mb1": 1, "mb2": 2, "mb4": 4}[variant]
     _check(lib().bnn_debug_force_contract_variant(code), "bnn_debug_force_contract_variant")
 
 

@@ -167,11 +167,7 @@ int tma_conv_transpose_wgrad(const float* dy, const float* x, int64_t x_sample_s
 int conv_transpose_phases(const bnn_conv2d_nhwc* g, int32_t* out, int max_phases);   // host: the phase plan, 8 ints each
 int tma_selftest(float* max_err_dev, cudaStream_t st);
 int tma_pair_tile_plan(int m_blocks, int S, int slots, int32_t* out7);   // test aid: TilePlan fields {on, n_a, s1, a1, b1, a2, b2}
-int tma_force_variant(int variant);   // test aid: 0 = CTA pair, 8 = its balanced schedule, 1 / 2 / 4 = row blocks per CTA, -1 = cost model (default)
-int tma_balanced_plan(int m_blocks, int S, int gx, int red_blocks, int sum_samples, int slots, int slot, int32_t* out,
-                      int max_segments);                // test aid (host arithmetic): segments of one slot, returns their number
-int contract_set_balanced(int on);                      // process-wide switch of the balanced schedule (default on)
-int contract_balanced_state(int slot_cap, int* launches_out, int* slots_out);   // test aid / bench counter
+int tma_force_variant(int variant);   // test aid: 0 = CTA pair, 1 / 2 / 4 = row blocks per CTA, -1 = cost model (default)
 int tma_stage_counters(unsigned long long* out8, int reset);  // profiling builds only: CTA timeline of the pair kernels
 int tma_wait_counters(unsigned long long* out8, int reset);   // profiling builds (-DBNN_PROFILE_WAITS) only
 

@@ -214,14 +214,6 @@ struct TmaContractParams {
   int atomic_out;           //   sums are ADDED to the (zeroed) output
   int vec_out;
   int exp_flags;            // profiling builds: 1 = skip weight generation, 2 = skip TMA loads, 4 = skip MMA issue
-  // balanced schedule (contract_pair_sk_kernel): a line of sk_total items cut into sk_slots equal ranges, one per
-  // resident CTA pair.  sk_msplit: items = 256-row units of the (sample, column tile) columns, sk_mtiles units each;
-  // else items = k-block iterations of the 1024-row tiles (sk_its each; sk_mtiles tiles per column)
-  int sk_slots;             // > 0: pair slots (clusters) of the launch
-  int sk_msplit;
-  int sk_mtiles, sk_gx;     // column = z * sk_gx + y  (y: 128-column tile, z: sample)
-  int sk_its;               // k-block iterations per tile (reduction blocks x samples summed into the tile)
-  int sk_total;
 };
 
 struct TmaPipe {
@@ -307,8 +299,7 @@ __device__ __forceinline__ void gen_w_tile(uint32_t tile, const float* __restric
 //   NCHW output (P = OH*OW, P % 4 == 0): staging [column][32 rows + 4]; four rows of a lane's group are four consecutive
 //     pixels of one image, i.e. one aligned float4 of out[img][n][p..p+3]; a store instruction covers 4 columns x 8 row
 //     groups: for P = 16 two runs of 256 contiguous bytes (was: two runs of 64 bytes per scalar store).
-// kStageWarpBytes per warp; the uniform-grid kernels alias the operand ring (dead once the accumulator is complete), the
-// balanced schedule keeps its own region because its producers run ahead into the next segment.
+// kStageWarpBytes per warp; the kernels alias the operand ring (dead once the accumulator is complete).
 constexpr int kStageWarpBytes = 64 * 36 * 4;     // 9216: [64 columns][32 + 4] floats; the row-major form needs 32 x 68 x 4 = 8704
 __device__ __forceinline__ float4 lds128(uint32_t addr) {
   float4 v;
@@ -675,7 +666,6 @@ constexpr int kPairWShift = 2;               // the four generator groups).  Eig
                                              // less (19 k instead of 26 k cycles per C3 tile), the MMA thread's 8.8 k cycles of
                                              // waiting for weights do not move — they are the cold start of a tile (first
                                              // mu / sigma loads, instruction cache), not a lack of slack in the ring
-constexpr int kSkWSlots = 4;                 // balanced schedule: four slots (its epilogue staging needs the space)
 constexpr int kHalfTileBytes = kTileBytes / 2;
 constexpr size_t kPairSmem = kSmemAux + 1024 + static_cast<size_t>(kASlots) * kTileBytes + kPairWSlots * kHalfTileBytes;
 
@@ -988,398 +978,18 @@ int launch_pair_contract(const TmaContractParams& p, dim3 grid, cudaStream_t st)
   return launch_pair_contract_v<MB, kDgrad, 0>(p, grid, st);
 }
 
-// ---------------------------------------------------------------------------------------------- balanced schedule
-// contract_pair_sk_kernel: the CTA-pair kernel as a PERSISTENT grid of `sk_slots` clusters (one per resident SM pair).
-// The uniform grid runs whole 1024-row tiles, so a layer with 128 tiles on 74 pair slots (the example conv layers)
-// pays two full waves for 1.73 waves of work, and the shared-input data gradient (64 sample-group tiles) leaves 10 of
-// 74 slots idle.  Here all work forms one line of items that is cut into sk_slots equal ranges; a slot walks its
-// range segment by segment, keeping barriers, TMEM and the producer pipelines alive across segments — generators and
-// the TMA thread run ahead into the next segment while the epilogue warps drain the accumulator of the previous one
-// (the MMA thread waits on `tmem_empty`).  Two ways to cut, neither needs scratch memory or a hand-over between slots:
-//   sk_msplit == 1 (forward, per-sample data gradient): items are UNITS of 256 rows (one 128-row block per CTA) of the
-//     (sample, column tile) columns of the output; a segment is a tile of 1..4 consecutive units over the whole
-//     reduction, stored like a uniform tile (C3 conv forward: 512 units on 74 slots = 7 or 6 units per slot, run as
-//     4 + 3 / 3 + 3 instead of two waves of 4);
-//   sk_msplit == 0 (summed data gradient: one output for all samples, zeroed first): items are the k-block
-//     iterations (reduction blocks x samples) of the 1024-row tiles; every segment ADDS its partial sums
-//     (red.global.add), as the uniform grid does when it splits the samples over grid.z.
-struct SkPipe {
-  uint64_t* full_a;      // [2]  as PairPipe
-  uint64_t* full_w;      // [4]
-  uint64_t* empty_w;     // [4]
-  uint64_t* accum_full;  // both CTAs: one phase per segment
-  uint64_t* tmem_empty;  // leader: one arrival per epilogue warp of both CTAs, one phase per segment
-  uint32_t* tmem_slot;
-  float* aux;            // [2][128]: sampled bias rows, double buffered by segment parity
-  uint32_t ring_a, ring_w;
-  uint32_t stage;        // four staging buffers of the epilogue warps (the rings stay live across segments)
-};
-constexpr size_t kPairSkSmem = kSmemAux + 1024 + static_cast<size_t>(kASlots) * kTileBytes + kSkWSlots * kHalfTileBytes +
-                               4 * static_cast<size_t>(kStageWarpBytes);
-__device__ __forceinline__ SkPipe carve_sk(uint8_t* smem_raw) {
-  SkPipe p;
-  p.full_a = reinterpret_cast<uint64_t*>(smem_raw);
-  p.full_w = p.full_a + 2;
-  p.empty_w = p.full_w + kSkWSlots;
-  p.accum_full = p.empty_w + kSkWSlots;
-  p.tmem_empty = p.accum_full + 1;
-  p.tmem_slot = reinterpret_cast<uint32_t*>(p.tmem_empty + 1);
-  p.aux = reinterpret_cast<float*>(smem_raw + 512);
-  const uint32_t base = smem_u32(smem_raw) + kSmemAux;
-  p.ring_a = (base + 1023u) & ~1023u;
-  p.ring_w = p.ring_a + kASlots * kTileBytes;
-  p.stage = p.ring_w + kSkWSlots * kHalfTileBytes;
-  return p;
-}
-struct SkSeg {
-  int lead_row0;         // first output row of the leader CTA
-  int mb_cap;            // row blocks per CTA of this tile (1..4); the peer's rows start mb_cap * 128 further
-  int y, z;              // column tile, sample (0 for a summed tile)
-  int i0, n;             // first k-block iteration inside the tile, iterations of this segment
-};
-// units of a tile that starts a run of `run` units: never a lone unit after a full tile (5 -> 3 + 2, 6 -> 3 + 3, 7 -> 4 + 3)
-__host__ __device__ __forceinline__ int sk_tile_units(int run) {
-  return (run >= 8 || run <= 4) ? (run < 4 ? run : 4) : (run + 1) / 2;
-}
-// next segment of the range [pos, end); advances pos
-__host__ __device__ __forceinline__ bool sk_next(const TmaContractParams& p, int& pos, int end, SkSeg* s) {
-  if (pos >= end) return false;
-  if (p.sk_msplit) {
-    const int col = pos / p.sk_mtiles, u0 = pos - col * p.sk_mtiles;        // sk_mtiles: units per column
-    int run = p.sk_mtiles - u0;
-    if (run > end - pos) run = end - pos;
-    const int u = sk_tile_units(run);
-    s->lead_row0 = u0 * 256;
-    s->mb_cap = u;
-    s->z = col / p.sk_gx;
-    s->y = col - s->z * p.sk_gx;
-    s->i0 = 0;
-    s->n = p.sk_its;
-    pos += u;
-    return true;
-  }
-  const int t = pos / p.sk_its;
-  s->i0 = pos - t * p.sk_its;
-  const int left = end - pos, room = p.sk_its - s->i0;
-  s->n = left < room ? left : room;
-  const int r = t / p.sk_mtiles;                                            // sk_mtiles: 1024-row tiles per column
-  s->lead_row0 = (t - r * p.sk_mtiles) * 1024;
-  s->mb_cap = 4;
-  s->z = r / p.sk_gx;
-  s->y = r - s->z * p.sk_gx;
-  pos += s->n;
-  return true;
-}
-
-template <bool kDgrad, int kMode>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreadsTma, 1)
-contract_pair_sk_kernel(const __grid_constant__ TmaContractParams p) {
-  constexpr bool kConv = kMode == 1;
-  constexpr int kSigns = kMode == 2 ? 1 : 0;
-  constexpr int MB = 4;
-  extern __shared__ __align__(16) uint8_t smem_raw[];
-  long long w_mma_w = 0, w_mma_a = 0, w_mma_t = 0, w_gen = 0, w_tma = 0, w_epi = 0;
-  (void)w_mma_w; (void)w_mma_a; (void)w_mma_t; (void)w_gen; (void)w_tma; (void)w_epi;
-#ifdef BNN_PROFILE_WAITS
-  const long long t_kernel0 = clock64();
-  if (threadIdx.x == 0) {
-    unsigned long long g;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(g));
-    atomicMin(&g_stage_cycles[6], g);
-  }
-#endif
-  const SkPipe pipe = carve_sk(smem_raw);
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const uint32_t rank = cluster_ctarank();          // 0 = leader
-  if (threadIdx.x == 0) {
-    for (int i = 0; i < 2; ++i) mbar_init(pipe.full_a + i, 1);
-    for (int i = 0; i < 4; ++i) { mbar_init(pipe.full_w + i, 2 * kGroupWarps); mbar_init(pipe.empty_w + i, 1); }
-    mbar_init(pipe.accum_full, 1);
-    mbar_init(pipe.tmem_empty, 2 * (kEpiThreads / 32));
-    fence_mbar_init();
-  }
-  if (warp == kTmaWarp && lane == 0) tma_prefetch_desc(&p.map_l);
-  if (warp == kMmaWarpT) tmem_alloc_pair(pipe.tmem_slot, 512);
-  tc_fence_before_sync();
-  cluster_sync_all();
-  tc_fence_after_sync();
-  const uint32_t tmem = *reinterpret_cast<volatile uint32_t*>(pipe.tmem_slot);
-#ifdef BNN_PROFILE_WAITS
-  if (threadIdx.x == 0) { BNN_STAGE(0, t_kernel0); atomicAdd(&g_stage_cycles[5], 1ull); }
-#endif
-
-  const int slot = static_cast<int>(blockIdx.x >> 1);
-  const int range_a = static_cast<int>(static_cast<long long>(p.sk_total) * slot / p.sk_slots);
-  const int range_b = static_cast<int>(static_cast<long long>(p.sk_total) * (slot + 1) / p.sk_slots);
-  const int n_cols = kDgrad ? p.K : p.N;
-  const int n_red = kDgrad ? p.N : p.K;
-  const int red_blocks = (n_red + kBK - 1) / kBK;
-
-  if (warp < kGenWarps) {
-    // ------------------------------------------------------------------ weight generators (half tile per CTA, four groups)
-    const int group = warp / kGroupWarps, tid = threadIdx.x - group * kGroupThreads;
-    const RngKey key = resolve_rng(p.rng_w);
-    const uint32_t lead_full_w = mapa_u32(smem_u32(pipe.full_w + group), 0);
-    const uint32_t tile = pipe.ring_w + group * kHalfTileBytes;
-    int pos = range_a, gi0 = 0;
-    SkSeg sg;
-    while (sk_next(p, pos, range_b, &sg)) {
-      const int half0 = sg.y * 128 + static_cast<int>(rank) * 64;
-      for (int j = (group - gi0) & 3; j < sg.n; j += kGenGroups) {       // iterations gi = gi0 + j with gi % 4 == group
-        const int gi = gi0 + j, it = sg.i0 + j;
-        const int ds = it / red_blocks, rb = it - ds * red_blocks;
-        EpsSrc eps;
-        eps.inj = p.eps_w ? p.eps_w + static_cast<int64_t>(sg.z + ds) * p.w_numel : nullptr;
-        eps.key = key;
-        eps.sample = p.sample_begin + sg.z + ds;
-        { BNN_T0(); mbar_wait(pipe.empty_w + group, ((gi >> 2) & 1) ^ 1); BNN_ACC(w_gen); }
-        if (!kDgrad)
-          gen_w_tile<64, false, kSigns>(tile, p.mu_w, p.sigma_w, eps, half0, p.N, rb * kBK, p.K, tid, p.K, 0);
-        else if (!kConv)
-          gen_w_tile<64, true, kSigns>(tile, p.mu_w, p.sigma_w, eps, rb * kBK, p.N, half0, p.K, tid, p.K, 0);
-        else {
-          const int tapf = rb / p.conv.cblocks, o0 = (rb - tapf * p.conv.cblocks) * kBK;
-          gen_w_tile<64, true, kSigns>(tile, p.mu_w, p.sigma_w, eps, o0, p.conv.w_rows, half0, p.K, tid,
-                               static_cast<int64_t>(p.conv.wtaps) * p.K, conv_dgrad_tap(p.conv, tapf) * p.K);
-        }
-        fence_proxy_async_smem();
-        __syncwarp();
-        if (lane == 0) mbar_arrive_cluster(lead_full_w);
-      }
-      gi0 += sg.n;
-    }
-  } else if (warp == kTmaWarp) {
-    // ------------------------------------------------------------------ TMA issuer (own rows; bytes counted by the leader)
-    if (lane == 0) {
-      const uint32_t lead_full_a = mapa_u32(smem_u32(pipe.full_a), 0);
-      int pos = range_a, gi = 0;
-      SkSeg sg;
-      while (sk_next(p, pos, range_b, &sg)) {
-        const int row0 = sg.lead_row0 + static_cast<int>(rank) * (sg.mb_cap * 128);
-        int mb_pair = (p.M - sg.lead_row0 + 127) / 128;
-        if (mb_pair > sg.mb_cap) mb_pair = sg.mb_cap;
-        int ds = sg.i0 / red_blocks, rb = sg.i0 - ds * red_blocks;
-        int smp = p.shared_l ? 0 : sg.z + ds;
-        int cw[MB], ch[MB], cn[MB];
-        int tap = 0, cb = 0;
-        if (kConv) {
-#pragma unroll
-          for (int mb = 0; mb < MB; ++mb) conv_pixel(p.conv, row0 + mb * 128, smp, &cw[mb], &ch[mb], &cn[mb]);
-          tap = rb / p.conv.cblocks;
-          cb = rb - tap * p.conv.cblocks;
-        }
-        for (int j = 0; j < sg.n; ++j, ++gi) {
-          const int g = gi & 1;
-          if (gi >= 2) { BNN_T0(); mbar_wait(pipe.empty_w + ((gi - 2) & 3), ((gi - 2) >> 2) & 1); BNN_ACC(w_tma); }
-          if (rank == 0) mbar_arrive_expect_tx(pipe.full_a + g, 2 * mb_pair * kTileBytes);
-          if (!kConv) {
-            for (int mb = 0; mb < mb_pair; ++mb)
-              tma_load_3d_pair(pipe.ring_a + (g * MB + mb) * kTileBytes, &p.map_l, rb * kBK, row0 + mb * 128, smp,
-                               lead_full_a + g * 8);
-          } else {
-            const int kh = tap / p.conv.KW, kw = tap - kh * p.conv.KW;
-#pragma unroll
-            for (int mb = 0; mb < MB; ++mb)
-              if (mb < mb_pair)
-                tma_load_im2col_4d_pair(pipe.ring_a + (g * MB + mb) * kTileBytes, &p.map_l, cb * kBK, cw[mb], ch[mb], cn[mb],
-                                        static_cast<uint16_t>(kw * p.conv.dw), static_cast<uint16_t>(kh * p.conv.dh),
-                                        lead_full_a + g * 8);
-            if (++cb == p.conv.cblocks) { cb = 0; ++tap; }
-          }
-          if (++rb == red_blocks) {                  // next sample of a summed tile
-            rb = 0; ++ds; tap = 0; cb = 0;
-            if (!p.shared_l) {
-              smp = sg.z + ds;
-              if (kConv) {
-#pragma unroll
-                for (int mb = 0; mb < MB; ++mb) cn[mb] += p.conv.imgs;
-              }
-            }
-          }
-        }
-      }
-    }
-    __syncwarp();
-  } else if (warp == kMmaWarpT) {
-    // ------------------------------------------------------------------ MMA issuer (leader only)
-    if (rank == 0 && lane == 0) {
-      const uint32_t idesc = make_idesc_tf32(256, 128, false, kDgrad);
-      const uint64_t desc_a0 = make_smem_desc(pipe.ring_a);
-      const uint64_t desc_w0 = kDgrad ? make_smem_desc_mn(pipe.ring_w, kMnLbo, kMnSbo) : make_smem_desc(pipe.ring_w);
-      int pos = range_a, gi = 0, seg = 0;
-      SkSeg sg;
-      while (sk_next(p, pos, range_b, &sg)) {
-        int mb_pair = (p.M - sg.lead_row0 + 127) / 128;
-        if (mb_pair > sg.mb_cap) mb_pair = sg.mb_cap;
-        if (seg > 0) {                                 // the epilogue warps of both CTAs have drained the last segment
-          { BNN_T0(); mbar_wait_cluster(pipe.tmem_empty, (seg - 1) & 1); BNN_ACC(w_mma_t); }
-          tc_fence_after_sync();
-        }
-        for (int j = 0; j < sg.n; ++j, ++gi) {
-          const int wslot = gi & 3, g = gi & 1;
-          { BNN_T0(); mbar_wait_cluster(pipe.full_w + wslot, (gi >> 2) & 1); BNN_ACC(w_mma_w); }
-          { BNN_T0(); mbar_wait_cluster(pipe.full_a + g, (gi >> 1) & 1); BNN_ACC(w_mma_a); }
-          tc_fence_after_sync();
-          const uint64_t da0 = desc_advance(desc_a0, static_cast<uint32_t>(g * MB) * (kTileBytes >> 4));
-          const uint64_t db0 = desc_advance(desc_w0, static_cast<uint32_t>(wslot) * (kHalfTileBytes >> 4));
-          for (int mb = 0; mb < mb_pair; ++mb) {
-#pragma unroll
-            for (int ks = 0; ks < kBK / 8; ++ks)
-              mma_tf32_pair(tmem + mb * 128, desc_advance(da0, mb * (kTileBytes >> 4) + ks * 2),
-                            desc_advance(db0, ks * ((kDgrad ? kMnKStep : 32u) >> 4)), idesc, j > 0 || ks > 0);
-          }
-          mma_commit_pair(pipe.empty_w + wslot, 3);
-        }
-        mma_commit_pair(pipe.accum_full, 3);
-        ++seg;
-      }
-    }
-    __syncwarp();
-  } else {
-    // ------------------------------------------------------------------ epilogue (own TMEM, own rows)
-    const int et = threadIdx.x - kEpiWarp0T * 32;   // 0..127
-    const int quad = warp & 3;
-    const uint32_t lead_tmem_empty = mapa_u32(smem_u32(pipe.tmem_empty), 0);
-    int pos = range_a, seg = 0;
-    SkSeg sg;
-    while (sk_next(p, pos, range_b, &sg)) {
-      const int col0 = sg.y * 128;
-      const int row0 = sg.lead_row0 + static_cast<int>(rank) * (sg.mb_cap * 128);
-      int mb_pair = (p.M - sg.lead_row0 + 127) / 128;
-      if (mb_pair > sg.mb_cap) mb_pair = sg.mb_cap;
-      const bool add = p.atomic_out != 0;              // summed tiles: every segment adds into the zeroed output
-      float* aux = pipe.aux + (seg & 1) * 128;
-      if (!kDgrad) {
-        float b = 0.f;
-        const int n = col0 + et;
-        if (p.mu_b != nullptr && n < p.N) {
-          const float e = p.eps_b ? __ldg(p.eps_b + static_cast<int64_t>(sg.z) * p.N + n)
-                                  : eps1(resolve_rng(p.rng_b), p.sample_begin + sg.z, static_cast<uint64_t>(n));
-          b = fmaf(__ldg(p.sigma_b + n), e, __ldg(p.mu_b + n));
-        }
-        aux[et] = b;
-        named_bar_sync(kEpiBarrier, kEpiThreads);
-      }
-      mbar_wait(pipe.accum_full, seg & 1);
-      tc_fence_after_sync();
-#ifdef BNN_PROFILE_WAITS
-      const long long t_epi0 = clock64();
-#endif
-      View out = p.out;
-      out.base += (p.sum_samples ? 0 : static_cast<int64_t>(sg.z) * p.out_sample_stride);
-      const int cols_here = n_cols - col0 < 128 ? n_cols - col0 : 128;
-      const bool staged = stage_eligible(out, p.vec_out != 0, cols_here) && (out.P == 1 || (p.M & 3) == 0);
-      for (int mb = 0; mb < mb_pair; ++mb) {
-        const int m = row0 + mb * 128 + quad * 32 + lane;
-        if (row0 + mb * 128 >= p.M) break;               // uniform per CTA
-        if (staged) {
-          drain_block_staged<!kDgrad>(tmem + (static_cast<uint32_t>(quad * 32) << 16) + mb * 128,
-                                      pipe.stage + quad * kStageWarpBytes, aux, out, row0 + mb * 128 + quad * 32,
-                                      p.M, col0, cols_here, lane, add);
-          continue;
-        }
-        for (int c = 0; c * 16 < cols_here; ++c) {
-          float v[16];
-          tmem_ld16(tmem + (static_cast<uint32_t>(quad * 32) << 16) + mb * 128 + c * 16, v);
-          if (!kDgrad) {
-#pragma unroll
-            for (int j = 0; j < 16; ++j) v[j] += aux[c * 16 + j];
-          }
-          if (m < p.M) {
-            if (add) add_chunk(out, m, col0 + c * 16, n_cols, v, p.vec_out != 0);
-            else store_chunk(out, m, col0 + c * 16, n_cols, v, p.vec_out != 0);
-          }
-        }
-      }
-      tc_fence_before_sync();                            // all tcgen05.ld of this segment have completed (wait::ld)
-      __syncwarp();
-      if (lane == 0) mbar_arrive_cluster(lead_tmem_empty);
-#ifdef BNN_PROFILE_WAITS
-      w_epi += clock64() - t_epi0;
-#endif
-      ++seg;
-    }
-  }
-#ifdef BNN_PROFILE_WAITS
-  if (threadIdx.x == kEpiWarp0T * 32) BNN_STAGE(3, t_kernel0);
-  if (threadIdx.x == 0) BNN_STAGE(1, t_kernel0);
-  if (lane == 0) {      // [0] kernel [1] MMA: weights [2] MMA: activations [3] generator warp 0 [4] TMA [5] CTAs [6] MMA: TMEM drain [7] epilogue busy
-    if (warp == 0) { atomicAdd(&g_wait_cycles[3], (unsigned long long)w_gen); atomicAdd(&g_wait_cycles[0], (unsigned long long)(clock64() - t_kernel0)); atomicAdd(&g_wait_cycles[5], 1ull); }
-    if (w_mma_w | w_mma_a | w_mma_t) { atomicAdd(&g_wait_cycles[1], (unsigned long long)w_mma_w); atomicAdd(&g_wait_cycles[2], (unsigned long long)w_mma_a); atomicAdd(&g_wait_cycles[6], (unsigned long long)w_mma_t); }
-    if (w_tma) atomicAdd(&g_wait_cycles[4], (unsigned long long)w_tma);
-    if (warp == kEpiWarp0T) atomicAdd(&g_wait_cycles[7], (unsigned long long)w_epi);
-  }
-#endif
-  tc_fence_before_sync();
-  cluster_sync_all();                                // nobody leaves while the partner may still signal or read
-  if (warp == kMmaWarpT) {
-    tc_fence_after_sync();
-    tmem_dealloc_pair(tmem, 512);
-  }
-#ifdef BNN_PROFILE_WAITS
-  if (threadIdx.x == 0) {
-    BNN_STAGE(4, t_kernel0);
-    unsigned long long g;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(g));
-    atomicMax(&g_stage_cycles[7], g);
-  }
-#endif
-}
-
-template <bool kDgrad, int kMode>
-int launch_pair_sk_v(const TmaContractParams& p, cudaStream_t st) {
-  static SmemOptIn opt_in;
-  const int rc = allow_dynamic_smem(contract_pair_sk_kernel<kDgrad, kMode>, kPairSkSmem, &opt_in);
-  if (rc != BNN_OK) return rc;
-  contract_pair_sk_kernel<kDgrad, kMode><<<dim3(2 * p.sk_slots, 1, 1), kThreadsTma, kPairSkSmem, st>>>(p);
-  BNN_CUDA_OK(cudaGetLastError());
-  return BNN_OK;
-}
-template <bool kDgrad>
-int launch_pair_sk(const TmaContractParams& p, cudaStream_t st) {
-  if (p.conv.on) return launch_pair_sk_v<kDgrad, 1>(p, st);
-  if (p.rng_w.row_sign != nullptr) return launch_pair_sk_v<kDgrad, 2>(p, st);
-  return launch_pair_sk_v<kDgrad, 0>(p, st);
-}
-
-bool pair_enabled() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("BNN_DISABLE_CTA_PAIRS");
-    v = (e != nullptr && e[0] == '1') ? 0 : 1;
-  }
-  return v == 1;
-}
-
 // Test aid: force one kernel variant (0 = pair, 1 / 2 / 4 = rows blocks per CTA, -1 = cost model) so that small test
-// shapes reach every variant.  Set through bnn_debug_force_contract_variant (tests) — the environment variable
-// BNN_CONTRACT_VARIANT = pair | balanced | mb4 | mb2 | mb1 only provides the initial value, read once.  8 = the CTA-pair
-// kernel's balanced schedule (contract_pair_sk_kernel) whenever the pair kernel is eligible.
-std::atomic<int> g_forced_variant{-2};
-int forced_variant() {
-  int v = g_forced_variant.load(std::memory_order_relaxed);
-  if (v != -2) return v;
-  v = -1;
-  const char* e = getenv("BNN_CONTRACT_VARIANT");
-  if (e != nullptr && e[0] == 'p') v = 0;
-  else if (e != nullptr && e[0] == 'b') v = 8;                  // "balanced"
-  else if (e != nullptr && e[0] == 'm' && e[1] == 'b') v = e[2] == '4' ? 4 : (e[2] == '2' ? 2 : (e[2] == '1' ? 1 : -1));
-  g_forced_variant.store(v, std::memory_order_relaxed);
-  return v;
-}
+// shapes reach every variant.  Set through bnn_debug_force_contract_variant.
+std::atomic<int> g_forced_variant{-1};
 
 // Tile plan of the CTA-pair kernel (TilePlan): when the uniform grid needs a fraction of a wave more than a whole
 // number (1 < tiles / slots < 2 is the case that matters: the example conv layers), look for a cut of every sample into
 // 8- and 6-row-block tiles — at most two kinds of samples — whose list schedule (all 8-block tiles first) finishes
 // earlier.  Cost unit: one row block of MMAs per k-block; the fixed cost per tile is ignored, so a plan must win by 8 %.
-bool tile_plan_enabled() {                                     // BNN_TILE_PLAN=0 (read once) keeps the uniform grid: A/B runs
-  static const bool on = [] { const char* e = getenv("BNN_TILE_PLAN"); return !(e != nullptr && e[0] == '0'); }();
-  return on;
-}
 bool solve_pair_tiles(TilePlan* plan, int m_blocks, int S, int slots);
 bool plan_pair_tiles(TilePlan* plan, int m_blocks, int S, int gx, int gz, bool sum_samples, int slots) {
   plan->on = 0;
-  if (!tile_plan_enabled() || sum_samples || gx != 1 || gz != S || S < 1 || slots < 1) return false;
+  if (sum_samples || gx != 1 || gz != S || S < 1 || slots < 1) return false;
   // the search costs milliseconds: one result per (rows, samples, machine) for the life of the process
   static std::mutex mu;
   static std::vector<std::pair<std::array<int, 3>, TilePlan>> cache;
@@ -1425,127 +1035,6 @@ bool solve_pair_tiles(TilePlan* plan, int m_blocks, int S, int slots) {
       }
   if (best * 100 > base * 92) return false;
   *plan = found;
-  return true;
-}
-
-// ---- balanced schedule, host side
-std::atomic<int> g_sk_slot_cap{0};              // test aid: fewer slots than the machine has (0 = no cap)
-std::atomic<int> g_sk_launches{0};              // launches that took the balanced schedule (tests, bench)
-std::atomic<int> g_sk_on{-1};                   // -1: not decided yet (off unless BNN_BALANCED=1 is in the environment)
-bool sk_enabled() {                             // opt-in (bnn_contract_set_balanced / BNN_BALANCED=1): measured slower on B200, DESIGN §4
-  int v = g_sk_on.load(std::memory_order_relaxed);
-  if (v < 0) {
-    const char* e = getenv("BNN_BALANCED");
-    v = (e != nullptr && e[0] == '1') ? 1 : 0;
-    g_sk_on.store(v, std::memory_order_relaxed);
-  }
-  return v == 1;
-}
-// clusters of contract_pair_sk_kernel that are resident at the same time on the current device (cached per device);
-// the schedule does not depend on co-residency (slots never wait for each other), it only sizes the grid
-int sk_max_slots() {
-  static std::mutex mu;
-  static int cached[64];
-  static bool known[64];
-  int dev = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return 0;
-  std::lock_guard<std::mutex> lock(mu);
-  if (!known[dev]) {
-    known[dev] = true;
-    cached[dev] = 0;
-    static SmemOptIn opt_in;
-    if (allow_dynamic_smem(contract_pair_sk_kernel<false, 0>, kPairSkSmem, &opt_in) == BNN_OK) {
-      cudaLaunchConfig_t cfg{};
-      cfg.gridDim = dim3(static_cast<unsigned>(sm_count() & ~1), 1, 1);
-      cfg.blockDim = dim3(kThreadsTma, 1, 1);
-      cfg.dynamicSmemBytes = kPairSkSmem;
-      cudaLaunchAttribute attr{};
-      attr.id = cudaLaunchAttributeClusterDimension;
-      attr.val.clusterDim.x = 2; attr.val.clusterDim.y = 1; attr.val.clusterDim.z = 1;
-      cfg.attrs = &attr;
-      cfg.numAttrs = 1;
-      int n = 0;
-      if (cudaOccupancyMaxActiveClusters(&n, contract_pair_sk_kernel<false, 0>, &cfg) == cudaSuccess) cached[dev] = n;
-      else (void)cudaGetLastError();
-    }
-  }
-  return cached[dev];
-}
-
-// k-block cost of a tile of u units (one row block per CTA each), in cycles (CTA timeline of a profiling build at the C3
-// conv shape: the leader issues a 256 x 128 x 8 MMA per ~117 cycles, a CTA generates its half tile in ~1200)
-inline double sk_kblock_cycles(int u) {
-  const double mma = 117.0 * 4 * u + 130.0;
-  return mma > 1250.0 ? mma : 1250.0;
-}
-
-template <bool kDgrad>
-bool plan_sk(TmaContractParams& p, int gx, int m_blocks, int uniform_pairs, bool forced) {
-  p.sk_slots = 0;
-  if (!forced && !sk_enabled()) return false;
-  // the balanced kernel has no phase view, no data-gradient bias and no summed forward
-  if (p.out.pw != 0 || (kDgrad && p.mu_b != nullptr) || (!kDgrad && p.sum_samples)) return false;
-  if (p.sum_samples && p.out.P != 1) return false;
-  const int slots = sk_max_slots();
-  if (slots < 2) return false;
-  const int red_blocks = ((kDgrad ? p.N : p.K) + kBK - 1) / kBK;
-  const int cap = g_sk_slot_cap.load(std::memory_order_relaxed);
-  const double fixed = 6000.0, epilogue = 3500.0;         // launch + prologue + pipeline fill; per row block of a tile
-  const double waves = static_cast<double>((uniform_pairs + slots - 1) / slots);
-  if (p.sum_samples) {
-    // items = k-block iterations of the 1024-row tiles over ALL samples; every segment adds
-    const int m_tiles = (m_blocks + 7) / 8;
-    const int64_t n_tiles = static_cast<int64_t>(gx) * m_tiles;
-    const int64_t its = static_cast<int64_t>(red_blocks) * p.S;
-    const int64_t total = n_tiles * its;
-    if (total <= 0 || total > (int64_t(1) << 30)) return false;
-    int64_t q = slots;
-    if (q > total / 8) q = total / 8;           // at least eight k-blocks per slot
-    if (cap > 0 && q > cap) q = cap;
-    if (q < 1) return false;
-    if (!forced) {
-      const double per_slot = static_cast<double>((total + q - 1) / q);
-      const double segs = per_slot / static_cast<double>(its) + 1.0;
-      const double sk_cost = fixed + per_slot * sk_kblock_cycles(4) + segs * 4 * epilogue * 1.4;
-      const double uniform_cost = waves * (fixed + static_cast<double>(red_blocks) * p.z_per * sk_kblock_cycles(4) + 4 * epilogue * 1.4);
-      if (sk_cost > 0.95 * uniform_cost) return false;
-    }
-    p.sk_msplit = 0;
-    p.sk_slots = static_cast<int>(q);
-    p.sk_mtiles = m_tiles;
-    p.sk_gx = gx;
-    p.sk_its = static_cast<int>(its);
-    p.sk_total = static_cast<int>(total);
-  } else {
-    // items = 256-row units of the (sample, column tile) columns; a segment = a tile of 1..4 units, whole reduction
-    const int m_units = (m_blocks + 1) / 2;
-    const int64_t total = static_cast<int64_t>(gx) * p.S * m_units;
-    if (total <= 0 || total > (int64_t(1) << 30)) return false;
-    int64_t q = slots;
-    if (q > total) q = total;
-    if (cap > 0 && q > cap) q = cap;
-    if (q < 1) return false;
-    if (!forced) {
-      // the busiest slot: ceil(total / q) units cut by sk_tile_units (ranges that straddle a column cost one more cut)
-      int left = static_cast<int>((total + q - 1) / q);
-      double sk_cost = fixed;
-      while (left > 0) {
-        const int u = sk_tile_units(left < m_units ? left : m_units);
-        sk_cost += red_blocks * sk_kblock_cycles(u) + u * epilogue;
-        left -= u;
-      }
-      const int u_uniform = m_units < 4 ? m_units : 4;
-      const double uniform_cost = waves * (fixed + red_blocks * sk_kblock_cycles(u_uniform) + u_uniform * epilogue);
-      if (sk_cost > 0.95 * uniform_cost) return false;
-    }
-    p.sk_msplit = 1;
-    p.sk_slots = static_cast<int>(q);
-    p.sk_mtiles = m_units;
-    p.sk_gx = gx;
-    p.sk_its = red_blocks;
-    p.sk_total = static_cast<int>(total);
-  }
-  p.plan.on = 0;
   return true;
 }
 
@@ -1598,22 +1087,11 @@ int dispatch_tma_contract(TmaContractParams& p, int n_cols, cudaStream_t st) {
     const double c = cost_single(mb);
     if (c < best_cost) { best_cost = c; best = mb; }
   }
-  if (m_blocks > 4 && pair_enabled() && cost_pair() < 0.9 * best_cost) best = 0;       // a clear win only: the model is coarse
-  const int forced = forced_variant();
-  const bool force_sk = forced == 8 && m_blocks > 4;
-  if (force_sk) best = 0;
-  else if ((forced > 0 && forced != 8) || (forced == 0 && m_blocks > 4)) best = forced;
+  if (m_blocks > 4 && cost_pair() < 0.9 * best_cost) best = 0;       // a clear win only: the model is coarse
+  const int forced = g_forced_variant.load(std::memory_order_relaxed);
+  if (forced > 0 || (forced == 0 && m_blocks > 4)) best = forced;
   if (best == 0) {                                                // two CTAs (one cluster) per 1024 rows
     const int pairs = (m_blocks + 7) / 8;
-    if ((forced < 0 || force_sk) && plan_sk<kDgrad>(p, gx, m_blocks, pairs * gx * gz, force_sk)) {
-      if (p.sum_samples && !p.atomic_out) {                       // every segment adds: the output starts from zero
-        p.atomic_out = 1;
-        BNN_CUDA_OK(cudaMemset2DAsync(p.out.base, static_cast<size_t>(p.out.bs) * 4, 0, static_cast<size_t>(n_cols) * 4,
-                                      static_cast<size_t>(p.M), st));
-      }
-      g_sk_launches.fetch_add(1, std::memory_order_relaxed);
-      return launch_pair_sk<kDgrad>(p, st);
-    }
     if (plan_pair_tiles(&p.plan, m_blocks, p.S, gx, gz, p.sum_samples != 0, sms / 2))
       return launch_pair_contract<4, kDgrad>(p, dim3(2 * (p.plan.n_a + p.plan.s1 * p.plan.b1 + (p.S - p.plan.s1) * p.plan.b2), 1, 1), st);
     return launch_pair_contract<4, kDgrad>(p, dim3(2 * pairs, gx, gz), st);
@@ -2029,7 +1507,7 @@ int wgrad_plan_and_launch(TmaWgradParams& p, int M, int N, int K, int S, cudaStr
   if (rc == BNN_OK) rc = allow_dynamic_smem(wgrad_tma_kernel<true, true>, kWgradSmem, &opt_in[3]);
   if (rc != BNN_OK) return rc;
   const int n_tiles = (N + 127) / 128, k_tiles = (K + 127) / 128;
-  if (n_tiles >= 2 && pair_enabled() && static_cast<int64_t>(tiles) * groups >= 2 * sm_count()) {
+  if (n_tiles >= 2 && static_cast<int64_t>(tiles) * groups >= 2 * sm_count()) {
     // CTA pairs over adjacent n-tiles (large problems: the kernel is paced by operand delivery, a pair halves the A^T traffic)
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((n_tiles + 1) / 2 * 2, k_tiles, groups);
@@ -2384,33 +1862,6 @@ int tma_stage_counters(unsigned long long* out8, int reset) {
 #endif
 }
 
-// host only: the segments contract_pair_sk_kernel's slot `slot` of `slots` would walk (the kernel's own sk_next), six ints
-// each: {first row of the leader, row blocks per CTA, column tile, sample, first k-block iteration, iterations}
-int tma_balanced_plan(int m_blocks, int S, int gx, int red_blocks, int sum_samples, int slots, int slot, int32_t* out,
-                      int max_segments) {
-  TmaContractParams p{};
-  if (sum_samples) {
-    p.sk_msplit = 0; p.sk_mtiles = (m_blocks + 7) / 8; p.sk_its = red_blocks * S;
-    p.sk_total = gx * p.sk_mtiles * p.sk_its;
-  } else {
-    p.sk_msplit = 1; p.sk_mtiles = (m_blocks + 1) / 2; p.sk_its = red_blocks;
-    p.sk_total = gx * S * p.sk_mtiles;
-  }
-  p.sk_gx = gx; p.sk_slots = slots;
-  int pos = static_cast<int>(static_cast<long long>(p.sk_total) * slot / slots);
-  const int end = static_cast<int>(static_cast<long long>(p.sk_total) * (slot + 1) / slots);
-  SkSeg sg;
-  int n = 0;
-  while (sk_next(p, pos, end, &sg)) {
-    if (n < max_segments) {
-      int32_t* o = out + 6 * n;
-      o[0] = sg.lead_row0; o[1] = sg.mb_cap; o[2] = sg.y; o[3] = sg.z; o[4] = sg.i0; o[5] = sg.n;
-    }
-    ++n;
-  }
-  return n;
-}
-
 int tma_pair_tile_plan(int m_blocks, int S, int slots, int32_t* out7) {      // host only: the plan the launcher would use
   TilePlan plan{};
   solve_pair_tiles(&plan, m_blocks, S, slots);
@@ -2419,19 +1870,8 @@ int tma_pair_tile_plan(int m_blocks, int S, int slots, int32_t* out7) {      // 
 }
 
 int tma_force_variant(int variant) {
-  const bool ok = variant == -1 || variant == 0 || variant == 1 || variant == 2 || variant == 4 || variant == 8;
+  const bool ok = variant == -1 || variant == 0 || variant == 1 || variant == 2 || variant == 4;
   g_forced_variant.store(ok ? variant : -1, std::memory_order_relaxed);
-  return BNN_OK;
-}
-
-int contract_set_balanced(int on) {
-  g_sk_on.store(on ? 1 : 0, std::memory_order_relaxed);
-  return BNN_OK;
-}
-int contract_balanced_state(int slot_cap, int* launches_out, int* slots_out) {
-  if (slot_cap >= 0) g_sk_slot_cap.store(slot_cap, std::memory_order_relaxed);
-  if (launches_out) *launches_out = g_sk_launches.load(std::memory_order_relaxed);
-  if (slots_out) *slots_out = sk_max_slots();
   return BNN_OK;
 }
 

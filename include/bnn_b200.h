@@ -146,17 +146,6 @@ int bnn_bias_grad(bnn_view dy, int64_t dy_sample_stride, const float* rho_b, con
                   float* dmu_b, float* drho_b, int32_t M, int32_t N, int32_t S,
                   uint32_t sample_begin, const bnn_rng* rng_b, void* stream);
 
-/* ---- balanced schedule of the CTA-pair contraction kernels (opt-in) ----
- * The CTA-pair forward / data-gradient kernels (more than 512 rows per sample, TF32) run one cluster per 1024-row tile.
- * Where that grid wastes part of a wave (the example conv layers: 128 tiles on 74 SM pairs = two waves for 1.73 waves of
- * work; their summed data gradient: 64 tiles on 74 pairs) an alternative launcher runs a persistent grid of one cluster
- * per SM pair in which every cluster gets an equal share of the work: tiles of 1..4 row-block pairs for the forward pass
- * and the per-sample data gradient, k-block ranges added into the zeroed output for the summed data gradient.  No
- * scratch memory, no hand-over between clusters; forward results are bit-identical to the uniform grid.  OFF by
- * default: on B200 it needs 4-7 % fewer SM cycles but the board lowers the SM clock when all 148 SMs run tensor work, and
- * the launch ends up 3-20 % slower (DESIGN §4).  Process-wide switch (BNN_BALANCED=1 in the environment starts it on). */
-int bnn_contract_set_balanced(int32_t on);
-
 /* ---- conv2d lowering helpers (NCHW, fp32) ----
  * col[(b*OH*OW + oh*OW + ow)][(c*KH + kh)*KW + kw] = x[b][c0 + c][oh*sh - ph + kh*dh][...] (0 outside).
  * c runs over `Cg` channels starting at c0 (one conv group). */
@@ -442,22 +431,9 @@ int bnn_selftest_umma(float* max_err_dev, void* stream);
 int bnn_selftest_umma_mn(float* max_err_dev, void* stream);
 
 /* ---- test aid: force the TMA-fed forward / data-gradient contraction onto one kernel variant so that small test
- * shapes reach all of them: 0 = CTA pair (needs more than four 128-row blocks), 8 = CTA pair with the balanced schedule,
- * 1 / 2 / 4 = row blocks per CTA,
+ * shapes reach all of them: 0 = CTA pair (needs more than four 128-row blocks), 1 / 2 / 4 = row blocks per CTA,
  * -1 = the launcher's cost model (default).  Process-wide; not for production use. */
 int bnn_debug_force_contract_variant(int32_t variant);
-/* test aid / counter: slot_cap >= 0 caps the clusters of the balanced schedule (0 = no cap; small test shapes then cut
- * several slots share a column of the output), slot_cap < 0 leaves the cap; *launches_out = launches that took the balanced schedule so far,
- * *slots_out = co-resident clusters on the current device (either may be NULL).  Variant 8 of
- * bnn_debug_force_contract_variant forces the schedule wherever the CTA-pair kernel is eligible. */
-int bnn_debug_balanced_schedule(int32_t slot_cap, int32_t* launches_out, int32_t* slots_out);
-/* test aid, host arithmetic only: the segments that slot `slot` of `slots` walks in the balanced schedule for `samples`
- * samples of `m_blocks` 128-row blocks x `column_tiles` 128-column tiles with `red_blocks` 32-wide k-blocks (sum_samples:
- * the summed data gradient).  Six ints per segment: {first row of the leader CTA, row blocks per CTA, column tile, sample,
- * first k-block iteration of the tile, iterations}.  Returns the number of segments (may exceed max_segments; only
- * max_segments are written) or a negative bnn_status. */
-int bnn_debug_balanced_plan(int32_t m_blocks, int32_t samples, int32_t column_tiles, int32_t red_blocks, int32_t sum_samples,
-                            int32_t slots, int32_t slot, int32_t* out, int32_t max_segments);
 /* test aid, host arithmetic only: the heterogeneous tile list of the CTA-pair kernel for `samples` samples of `m_blocks`
  * 128-row blocks on `pair_slots` SM pairs (narrow layers: one column tile).  out7 = {on, n_a, s1, a1, b1, a2, b2}: samples
  * [0, s1) are cut into a1 tiles of 8 row blocks followed by b1 tiles of 6, the others into a2 / b2; n_a = number of

@@ -47,8 +47,6 @@ def wgrad():
 
 
 import os  # noqa: E402
-if os.environ.get("BNN_SK_CAP"):          # cap the pair slots of the balanced schedule (scaling experiments)
-    C.balanced_schedule_state(slot_cap=int(os.environ["BNN_SK_CAP"]))
 if os.environ.get("BNN_FORCE_VARIANT"):
     C.force_contract_variant(os.environ["BNN_FORCE_VARIANT"])
 for _ in range(3):
@@ -62,8 +60,7 @@ for name, fn in (("fwd", fwd), ("dgrad", dgrad), ("wgrad", wgrad)):
         a.record(); fn(); b.record()
         torch.cuda.synchronize()
         best = min(best, a.elapsed_time(b))
-    print(f"{which} {'shared' if shared else 'per-sample'} {name}: {best * 1e3:.1f} us  {flops / best / 1e9:.1f} TFLOP/s"
-          f"  (balanced launches so far: {C.balanced_schedule_state()[0]})")
+    print(f"{which} {'shared' if shared else 'per-sample'} {name}: {best * 1e3:.1f} us  {flops / best / 1e9:.1f} TFLOP/s")
 
 # profiling builds only (BNN_EXTRA_NVCC_FLAGS=-DBNN_PROFILE_WAITS): wait cycles of the contraction kernels' roles
 import ctypes  # noqa: E402
@@ -91,7 +88,6 @@ try:
             n = buf[5]
             print(f"{name}: CTAs {n}  kernel {buf[0] / n:.0f} cycles/CTA | MMA thread waits: weights {buf[1] / n * 2:.0f} (leader only) "
                   f"activations {buf[2] / n * 2:.0f} | generators wait for a free slot {buf[3] / n:.0f} | TMA thread waits {buf[4] / n:.0f}"
-                  f" | uniform grid: first weight tile ready at {buf[6] / n * 2:.0f}, weight waits of k-blocks 0..4 {buf[7] / n * 2:.0f}"
-                  f" (balanced schedule: MMA waits for the TMEM drain / epilogue busy)")
+                  f" | uniform grid: first weight tile ready at {buf[6] / n * 2:.0f}, weight waits of k-blocks 0..4 {buf[7] / n * 2:.0f}")
 except AttributeError:
     pass

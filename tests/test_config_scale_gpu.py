@@ -94,45 +94,6 @@ def test_conv_layer_at_configuration_scale_matches_torch_conv2d(shape, shared, p
     assert rel_err(layer.bias.scale.grad, rb.grad) < 1e-4
 
 
-def test_c3_conv_layer_takes_the_balanced_schedule_and_agrees_with_the_uniform_grid():
-    """At the C3 shape (128 pair tiles on 74 SM pairs; shared-input input gradient: 64 sample-group tiles) the launcher's
-    cost model, once the opt-in schedule is enabled, picks contract_pair_sk_kernel for the forward pass and the input
-    gradient (launch counter), and the
-    forward pass must be bit-identical to the uniform grid (bnn.set_balanced_schedule(False): same products, same
-    accumulation order), the input gradients equal up to the order of the atomic adds — in-kernel Philox, same counters."""
-    import bayesianneuralnetworks_b200 as bnn
-    from bayesianneuralnetworks_b200 import _C, runtime
-    from bayesianneuralnetworks_b200.nn import NormalConv2d
-    B, S, C, HW = 512, 16, 128, 4
-    bnn.set_precision("tf32")
-    torch.manual_seed(5)
-    layer = NormalConv2d(C, C, 3, padding=1).cuda()
-    g = torch.Generator(device="cuda").manual_seed(6)
-    results = {}
-    try:
-        for shared in (True, False):
-            x0 = torch.randn(B if shared else S * B, C, HW, HW, device="cuda", generator=g)
-            dy = torch.randn(S * B, C, HW, HW, device="cuda", generator=g)
-            for balanced in (True, False):
-                bnn.set_balanced_schedule(balanced)
-                bnn.manual_seed(11)
-                layer.weight._draw = layer.bias._draw = 0          # the same Philox draws in both runs
-                x = x0.clone().requires_grad_(True)
-                ctx = runtime.MCContext(S, B)
-                ctx.expanded = not shared
-                before = _C.balanced_schedule_state()[0]
-                with runtime.mc_batch(ctx):
-                    y = layer(x)
-                y.backward(dy)
-                took = _C.balanced_schedule_state()[0] - before
-                assert took == (2 if balanced else 0), (shared, balanced, took)
-                results[(shared, balanced)] = (y.detach(), x.grad.detach())
-            assert bool(torch.equal(results[(shared, True)][0], results[(shared, False)][0]))
-            assert rel_err(results[(shared, True)][1], results[(shared, False)][1]) < 2e-5     # atomic adds: any order
-    finally:
-        bnn.set_balanced_schedule(False)
-
-
 # ------------------------------------------------------------------------------------------------ (b) the bench step
 def _oracle_stages(model):
     """oracle.ElboStepOracle stages from a (CPU) copy of a bench model: Bayesian layers become plain leaf tensors."""

@@ -429,62 +429,3 @@ def test_pair_kernel_tile_plans_cover_every_row_block_exactly_once():
     out = (ctypes.c_int32 * 7)()
     lib.bnn_debug_pair_tile_plan(64, 16, 74, out)           # C3 conv forward: 74 + 72 tiles on 74 pair slots
     assert out[0] == 1 and out[1] + out[2] * out[4] + (16 - out[2]) * out[6] <= 148
-
-
-def test_balanced_schedule_covers_every_work_item_exactly_once():
-    """sampled_gemm_tma.cu: contract_pair_sk_kernel.  The segments every slot walks (bnn_debug_balanced_plan: the kernel's
-    own sk_next evaluated on the host) must partition the work: forward / per-sample input gradient — every 256-row unit of
-    every (sample, column tile) column in exactly one tile of 1..4 units over the whole reduction, tiles inside one column,
-    never a lone unit after a full tile of the same run; summed input gradient — every k-block iteration of every
-    1024-row tile in exactly one segment; the slots' loads differ by at most one item (tile cuts aside)."""
-    n_cases = 0
-    for m_blocks, S, gx, red_blocks, slots in [(64, 16, 1, 36, 74), (17, 5, 1, 3, 4), (11, 3, 2, 5, 7), (24, 6, 1, 9, 5),
-                                               (9, 9, 1, 2, 2), (8, 32, 32, 128, 74), (5, 1, 1, 1, 3), (64, 16, 1, 36, 1)]:
-        # ---- tiles of units (sum_samples = 0)
-        m_units = (m_blocks + 1) // 2
-        seen = {}
-        loads = []
-        for slot in range(slots):
-            segs = _C.balanced_plan(m_blocks, S, gx, red_blocks, False, slots, slot)
-            load = 0
-            for lead_row0, mb_cap, y, z, i0, n in segs:
-                assert 1 <= mb_cap <= 4 and i0 == 0 and n == red_blocks
-                assert lead_row0 % 256 == 0 and 0 <= y < gx and 0 <= z < S
-                u0 = lead_row0 // 256
-                assert u0 + mb_cap <= m_units, "a tile stays inside its column"
-                for u in range(u0, u0 + mb_cap):
-                    key = (z, y, u)
-                    assert key not in seen, f"unit {key} assigned twice"
-                    seen[key] = slot
-                load += mb_cap
-            loads.append(load)
-        assert len(seen) == S * gx * m_units
-        assert max(loads) - min(loads) <= 1
-        # ---- k-block ranges (sum_samples = 1): tiles of 1024 rows, all S samples in one tile
-        m_tiles = (m_blocks + 7) // 8
-        its = red_blocks * S
-        cover = {}
-        loads = []
-        for slot in range(slots):
-            segs = _C.balanced_plan(m_blocks, S, gx, red_blocks, True, slots, slot)
-            load = 0
-            for lead_row0, mb_cap, y, z, i0, n in segs:
-                assert mb_cap == 4 and z == 0 and lead_row0 % 1024 == 0 and 0 <= y < gx and lead_row0 // 1024 < m_tiles
-                assert 0 <= i0 and n >= 1 and i0 + n <= its
-                for it in range(i0, i0 + n):
-                    key = (y, lead_row0 // 1024, it)
-                    assert key not in cover
-                    cover[key] = slot
-                load += n
-            loads.append(load)
-        assert len(cover) == gx * m_tiles * its
-        assert max(loads) - min(loads) <= 1
-        n_cases += 1
-    assert n_cases == 8
-    # the tile-size rule: runs of 5 / 6 / 7 units are cut 3 + 2 / 3 + 3 / 4 + 3, never 4 + 1
-    segs = _C.balanced_plan(10, 1, 1, 4, False, 1, 0)               # one column of 5 units on one slot
-    assert [s[1] for s in segs] == [3, 2]
-    segs = _C.balanced_plan(14, 1, 1, 4, False, 1, 0)               # 7 units
-    assert [s[1] for s in segs] == [4, 3]
-    with pytest.raises(_C.BnnError):
-        _C.balanced_plan(4, 1, 1, 1, False, 2, 2)                   # slot out of range

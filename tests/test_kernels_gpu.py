@@ -592,67 +592,6 @@ def test_pair_kernel_tile_plan_covers_every_row_once(C, request, M, N, K, S):
     assert rel_err(da, torch.bmm(dy.double(), w)) < TOL[0]
 
 
-@pytest.mark.parametrize("M,N,K,S,cap", [(2100, 128, 96, 5, 4), (1300, 200, 160, 3, 7), (3000, 64, 288, 6, 5),
-                                         (1030, 128, 64, 9, 2), (8192, 128, 128, 4, 0)])
-def test_balanced_schedule_of_the_pair_kernel(C, request, M, N, K, S, cap):
-    """contract_pair_sk_kernel: a persistent grid in which every CTA pair takes an equal share of the work — tiles of 1..4
-    row-block pairs for the forward pass and the per-sample input gradient, k-block ranges added into the zeroed output
-    for the shared-input input gradient.  bnn_debug_balanced_schedule caps the number of pair slots so that small shapes
-    cut the work in every way: ranges that straddle samples and column tiles, ragged last tiles, tiles of 1, 2, 3 and 4
-    units, several segments per slot (the TMEM hand-over between the MMA thread and the epilogue warps).  Against torch
-    fp64 on the injected eps; NaN-filled outputs prove that every element is written, a second pass that nothing is left
-    behind in the pipeline state."""
-    C.force_contract_variant("balanced")
-    C.balanced_schedule_state(slot_cap=cap)
-    request.addfinalizer(lambda: (C.force_contract_variant(None), C.balanced_schedule_state(slot_cap=0)))
-    g = torch.Generator().manual_seed(41)
-    a, mu_w, rho_w, mu_b, rho_b, eps_w, eps_b = gemm_inputs(M, N, K, S, False, g)
-    sig = orc.stddev(rho_w.double())
-    w = mu_w.double().unsqueeze(0) + sig.unsqueeze(0) * eps_w.double()                     # [S, N, K]
-    b = mu_b.double().unsqueeze(0) + orc.stddev(rho_b.double()).unsqueeze(0) * eps_b.double()
-    ref = torch.bmm(a.double(), w.transpose(1, 2)) + b.unsqueeze(1)
-    before = C.balanced_schedule_state()[0]
-    for _ in range(2):
-        y = run_fwd(C, a, mu_w, rho_w, mu_b, rho_b, eps_w, eps_b, S, 0)
-        assert bool(torch.isfinite(y).all())
-        assert rel_err(y, ref) < TOL[0]
-    # shared activations: every sample reads sample 0
-    y0 = run_fwd(C, a[:1], mu_w, rho_w, mu_b, rho_b, eps_w, eps_b, S, 0)
-    ref0 = torch.matmul(a[0].double().unsqueeze(0), w.transpose(1, 2)) + b.unsqueeze(1)
-    assert rel_err(y0, ref0) < TOL[0]
-    dy = torch.randn(S, M, N, generator=g)
-    ddy = dy.cuda()
-    sig_dev = C.stddev(rho_w.cuda())
-    for _ in range(2):
-        da = torch.full(tuple(a.shape), float("nan"), device="cuda")
-        C.sampled_gemm_dgrad(C.make_view(ddy.data_ptr(), N, 1), M * N, mu_w.cuda(), sig_dev, eps_w.cuda(), da,
-                             K, M * K, M, N, K, S, 0, C.make_rng(0, 0, 0), 0)
-        assert bool(torch.isfinite(da).all())
-        assert rel_err(da, torch.bmm(dy.double(), w)) < TOL[0]
-    da0 = torch.full((1, M, K), float("nan"), device="cuda")
-    C.sampled_gemm_dgrad(C.make_view(ddy.data_ptr(), N, 1), M * N, mu_w.cuda(), sig_dev, eps_w.cuda(), da0,
-                         K, 0, M, N, K, S, 0, C.make_rng(0, 0, 0), 0)
-    assert bool(torch.isfinite(da0).all())
-    assert rel_err(da0[0], torch.bmm(dy.double(), w).sum(0)) < TOL[0]
-    assert C.balanced_schedule_state()[0] >= before + 6          # every launch above took the balanced schedule
-
-
-def test_balanced_schedule_philox_equals_the_uniform_grid(C, request):
-    """Same Philox counters, same TF32 products, same accumulation order per output element: the forward pass of the
-    balanced schedule is bit-identical to the uniform CTA-pair grid."""
-    M, N, K, S = 2500, 128, 160, 7
-    g = torch.Generator().manual_seed(43)
-    a, mu_w, rho_w, mu_b, rho_b, _, _ = gemm_inputs(M, N, K, S, False, g)
-    rw, rb = C.make_rng(77, 3, 5), C.make_rng(77, 3, 6)
-    request.addfinalizer(lambda: (C.force_contract_variant(None), C.balanced_schedule_state(slot_cap=0)))
-    C.force_contract_variant("pair")
-    y_uniform = run_fwd(C, a, mu_w, rho_w, mu_b, rho_b, None, None, S, 0, rng_w=rw, rng_b=rb, sample_begin=2)
-    C.force_contract_variant("balanced")
-    C.balanced_schedule_state(slot_cap=6)
-    y_balanced = run_fwd(C, a, mu_w, rho_w, mu_b, rho_b, None, None, S, 0, rng_w=rw, rng_b=rb, sample_begin=2)
-    assert bool(torch.equal(y_balanced, y_uniform))
-
-
 def test_wgrad_philox_equals_injected(C):
     g = torch.Generator().manual_seed(9)
     M, N, K, S = 96, 72, 136, 5
