@@ -146,24 +146,20 @@ int tma_conv_fwd(const float* x, int64_t x_sample_stride, const float* mu_w, con
                  const float* sigma_b, const float* eps_w, const float* eps_b, bnn_view y, int64_t y_sample_stride,
                  const bnn_conv2d_nhwc* g, int S, uint32_t sample_begin, const bnn_rng* rng_w, const bnn_rng* rng_b,
                  cudaStream_t st);
-int tma_conv_dgrad(const float* dy, const float* mu_w, const float* sigma_w, const float* eps_w, float* dx,
-                   int64_t x_sample_stride, const bnn_conv2d_nhwc* g, int S, uint32_t sample_begin, const bnn_rng* rng_w,
-                   cudaStream_t st);
-int tma_conv_wgrad(const float* dy, const float* x, int64_t x_sample_stride, const float* rho_w, const float* eps_w,
+// the weight gradient of a conv layer takes (dy, x), that of a transposed conv its conv view's operands (x, dy)
+int tma_conv_wgrad(const float* dy, bool shared_dy, const float* a, bool shared_a, const float* rho_w, const float* eps_w,
                    float* dmu_w, float* drho_w, const bnn_conv2d_nhwc* g, int S, uint32_t sample_begin,
                    const bnn_rng* rng_w, cudaStream_t st);
-// transposed convolution, geometry of its conv view (see bnn_b200.h): forward as the strided transposed-filter gather
-// (one launch per output phase), input gradient as the conv view's forward, weight gradient as the conv view's
-int tma_conv_transpose_fwd(const float* x, int64_t x_sample_stride, const float* mu_w, const float* sigma_w,
-                           const float* mu_b, const float* sigma_b, const float* eps_w, const float* eps_b, float* y,
-                           const bnn_conv2d_nhwc* g, int S, uint32_t sample_begin, const bnn_rng* rng_w,
-                           const bnn_rng* rng_b, cudaStream_t st);
+// transposed-filter gather: the stride-1 conv input gradient (x = dy, sum_samples for a shared input) and the forward of a
+// transposed convolution in its conv view's geometry (see bnn_b200.h; one launch per output phase); input gradient of a
+// transposed convolution = the conv view's forward
+int tma_conv_gather(const float* x, bool shared_x, const float* mu_w, const float* sigma_w, const float* mu_b,
+                    const float* sigma_b, const float* eps_w, const float* eps_b, float* y, int64_t y_sample_stride,
+                    bool sum_samples, const bnn_conv2d_nhwc* g, int S, uint32_t sample_begin, const bnn_rng* rng_w,
+                    const bnn_rng* rng_b, cudaStream_t st);
 int tma_conv_transpose_dgrad(const float* dy, const float* mu_w, const float* sigma_w, const float* eps_w, float* dx,
                              int64_t x_sample_stride, const bnn_conv2d_nhwc* g, int S, uint32_t sample_begin,
                              const bnn_rng* rng_w, cudaStream_t st);
-int tma_conv_transpose_wgrad(const float* dy, const float* x, int64_t x_sample_stride, const float* rho_w,
-                             const float* eps_w, float* dmu_w, float* drho_w, const bnn_conv2d_nhwc* g, int S,
-                             uint32_t sample_begin, const bnn_rng* rng_w, cudaStream_t st);
 int conv_transpose_phases(const bnn_conv2d_nhwc* g, int32_t* out, int max_phases);   // host: the phase plan, 8 ints each
 int tma_selftest(float* max_err_dev, cudaStream_t st);
 int tma_pair_tile_plan(int m_blocks, int S, int slots, int32_t* out7);   // test aid: TilePlan fields {on, n_a, s1, a1, b1, a2, b2}

@@ -489,8 +489,12 @@ int bnn_sampled_conv2d_dgrad(const float* dy, const float* mu_w, const float* si
               "bnn_sampled_conv2d_dgrad: NULL pointer or bad sample count");
   rc = check_device();
   if (rc != BNN_OK) return rc;
-  rc = contract::tma_conv_dgrad(dy, mu_w, sigma_w, eps_w, dx, x_sample_stride, g, S, sample_begin, rng_w,
-                                static_cast<cudaStream_t>(stream));
+  // strided layers keep the explicit lowering (col2im of the column gradients)
+  rc = g->sh != 1 || g->sw != 1
+           ? contract::kNotEligible
+           : contract::tma_conv_gather(dy, false, mu_w, sigma_w, nullptr, nullptr, eps_w, nullptr, dx, x_sample_stride,
+                                       x_sample_stride == 0, g, S, sample_begin, rng_w, nullptr,
+                                       static_cast<cudaStream_t>(stream));
   if (rc == contract::kNotEligible)
     return fail(BNN_ERR_UNSUPPORTED, "bnn_sampled_conv2d_dgrad: needs stride 1, Cout %% 32 == 0, C %% 4 == 0 and 16-byte "
                                      "aligned tensors (use bnn_sampled_gemm_dgrad + bnn_col2im_nhwc)");
@@ -506,7 +510,7 @@ int bnn_sampled_conv2d_wgrad(const float* dy, const float* x, int64_t x_sample_s
               "bnn_sampled_conv2d_wgrad: NULL pointer or bad sample count");
   rc = check_device();
   if (rc != BNN_OK) return rc;
-  rc = contract::tma_conv_wgrad(dy, x, x_sample_stride, rho_w, eps_w, dmu_w, drho_w, g, S, sample_begin, rng_w,
+  rc = contract::tma_conv_wgrad(dy, false, x, x_sample_stride == 0, rho_w, eps_w, dmu_w, drho_w, g, S, sample_begin, rng_w,
                                 static_cast<cudaStream_t>(stream));
   if (rc == contract::kNotEligible)
     return fail(BNN_ERR_UNSUPPORTED, "bnn_sampled_conv2d_wgrad: needs C %% 32 == 0, Cout %% 4 == 0 and 16-byte aligned "
@@ -527,8 +531,9 @@ int bnn_sampled_conv_transpose2d_fwd(const float* x, int64_t x_sample_stride, co
               "bnn_sampled_conv_transpose2d_fwd: bias needs mu_b, sigma_b and rng_b");
   rc = check_device();
   if (rc != BNN_OK) return rc;
-  rc = contract::tma_conv_transpose_fwd(x, x_sample_stride, mu_w, sigma_w, mu_b, sigma_b, eps_w, eps_b, y, g, S,
-                                        sample_begin, rng_w, rng_b, static_cast<cudaStream_t>(stream));
+  rc = contract::tma_conv_gather(x, x_sample_stride == 0, mu_w, sigma_w, mu_b, sigma_b, eps_w, eps_b, y,
+                                 static_cast<int64_t>(g->B) * g->H * g->W * g->C, false, g, S, sample_begin, rng_w, rng_b,
+                                 static_cast<cudaStream_t>(stream));
   if (rc == contract::kNotEligible)
     return fail(BNN_ERR_UNSUPPORTED, "bnn_sampled_conv_transpose2d_fwd: needs Cout %% 32 == 0, C %% 4 == 0, stride <= 8, "
                                      "16-byte aligned tensors and phase corners within the im2col descriptor's limits "
@@ -563,8 +568,9 @@ int bnn_sampled_conv_transpose2d_wgrad(const float* dy, const float* x, int64_t 
               "bnn_sampled_conv_transpose2d_wgrad: NULL pointer or bad sample count");
   rc = check_device();
   if (rc != BNN_OK) return rc;
-  rc = contract::tma_conv_transpose_wgrad(dy, x, x_sample_stride, rho_w, eps_w, dmu_w, drho_w, g, S, sample_begin, rng_w,
-                                          static_cast<cudaStream_t>(stream));
+  // conv view: the "dY" operand is the transposed input x (shared by the samples when x_sample_stride == 0), A = dy
+  rc = contract::tma_conv_wgrad(x, x_sample_stride == 0, dy, false, rho_w, eps_w, dmu_w, drho_w, g, S, sample_begin, rng_w,
+                                static_cast<cudaStream_t>(stream));
   if (rc == contract::kNotEligible)
     return fail(BNN_ERR_UNSUPPORTED, "bnn_sampled_conv_transpose2d_wgrad: needs C %% 32 == 0, Cout %% 4 == 0 and 16-byte "
                                      "aligned tensors (use bnn_im2col_nhwc + bnn_sampled_gemm_wgrad)");

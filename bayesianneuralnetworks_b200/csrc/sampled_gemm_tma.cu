@@ -213,7 +213,8 @@ struct TmaContractParams {
   int z_per;                // sum_samples: samples per CTA (grid.z = sample groups); more than one group -> the partial
   int atomic_out;           //   sums are ADDED to the (zeroed) output
   int vec_out;
-  int exp_flags;            // profiling builds: 1 = skip weight generation, 2 = skip TMA loads, 4 = skip MMA issue
+  int exp_flags;            // profiling builds: 1 = skip weight generation, 2 = eps read from memory; single CTA only:
+                            //   4 = skip TMA loads, 8 = skip MMA issue
 };
 
 struct TmaPipe {
@@ -416,566 +417,52 @@ __device__ __forceinline__ void drain_tile_shared(uint32_t tmem, uint32_t stage_
   }
 }
 
-template <int MB, bool kDgrad, int kMode>      // kMode: 0 plain, 1 conv (im2col maps), 2 rank-one sign noise (Flipout)
+// Forward / data gradient.  kPair: the same contraction over a cluster of two CTAs (cta_group::2): the pair computes
+// 2 x MB x 128 output rows against ONE 128-column weight tile of which each CTA generates only its half (64 n-rows forward
+// / 64 k-columns dgrad) — half the Philox work per SM and per MMA cycle.  Each CTA loads its own activation tiles by TMA
+// (transaction bytes land on the LEADER's barrier), the generator warps of the peer arrive on the leader's barrier through
+// the cluster address space, the leader's single MMA thread issues tcgen05.mma.cta_group::2 (M = 256) and frees the slots
+// of BOTH CTAs with multicast commits.  Epilogue: every CTA drains its own TMEM.
+// The pair's weight ring holds kWSlots 8 KiB half tiles.  Eight slots were measured: the generators wait less (19 k
+// instead of 26 k cycles per C3 tile), the MMA thread's 8.8 k cycles of waiting for weights do not move — they are the
+// cold start of a tile (first mu / sigma loads, instruction cache), not a lack of slack in the ring.
+constexpr int kHalfTileBytes = kTileBytes / 2;
+
+// One body, contract_body.inc (see there why it is included rather than called)
+template <int MB, bool kDgrad, int kMode>
 __global__ void __launch_bounds__(kThreadsTma, 1) contract_tma_kernel(const __grid_constant__ TmaContractParams p) {
-  constexpr bool kConv = kMode == 1;
-  constexpr int kSigns = kMode == 2 ? 1 : 0;
-  extern __shared__ __align__(16) uint8_t smem_raw[];
-  long long w_kernel = 0, w_mma_w = 0, w_mma_a = 0, w_gen = 0, w_tma = 0;
-  (void)w_kernel; (void)w_mma_w; (void)w_mma_a; (void)w_gen; (void)w_tma;
-#ifdef BNN_PROFILE_WAITS
-  const long long t_kernel0 = clock64();
-#endif
-  constexpr uint32_t kTmemCols = tmem_cols_pow2(MB * 128);
-  const TmaPipe pipe = carve_tma(smem_raw);
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  if (threadIdx.x == 0) {
-    // full_a[g]: the MB activation tiles of k-block group g (two groups of MB slots); full_w[j]: generated weight
-    // tile j (one arrival per generator warp); empty_w[j] = "k-block consumed": ONE tcgen05.commit per k-block frees
-    // weight slot j for the generators and, two k-blocks later, activation group j & 1 for the TMA thread
-    for (int i = 0; i < 2; ++i) mbar_init(pipe.full_a + i, 1);
-    for (int i = 0; i < kWSlots; ++i) { mbar_init(pipe.full_w + i, kGroupWarps); mbar_init(pipe.empty_w + i, 1); }
-    mbar_init(pipe.accum_full, 1);
-    fence_mbar_init();
-  }
-  if (warp == kTmaWarp && lane == 0) tma_prefetch_desc(&p.map_l);
-  if (warp == kMmaWarpT) tmem_alloc(pipe.tmem_slot, kTmemCols);
-  tc_fence_before_sync();
-  __syncthreads();
-  tc_fence_after_sync();
-  const uint32_t tmem = *reinterpret_cast<volatile uint32_t*>(pipe.tmem_slot);
-
-  const int col0 = blockIdx.x * 128;                   // output columns (n for fwd, k for dgrad)
-  const int row0 = blockIdx.y * (MB * 128);            // output rows (m)
-  const int n_cols = kDgrad ? p.K : p.N;
-  const int n_red = kDgrad ? p.N : p.K;
-  const int s_begin = p.sum_samples ? static_cast<int>(blockIdx.z) * p.z_per : blockIdx.z;
-  const int s_end = p.sum_samples ? (s_begin + p.z_per < p.S ? s_begin + p.z_per : p.S) : blockIdx.z + 1;
-  const int red_blocks = (n_red + kBK - 1) / kBK;
-  int mb_used = (p.M - row0 + 127) / 128;
-  if (mb_used > MB) mb_used = MB;
-
-  // the accumulator is drained by the epilogue warps AND, once their loop has ended, three generator warps per TMEM lane
-  // quarter (staged, coalesced write-out through the operand rings, which are dead by then); uniform per CTA
-  View out_tile = p.out;
-  out_tile.base += (p.sum_samples ? 0 : static_cast<int64_t>(blockIdx.z) * p.out_sample_stride);
-  const int cols_tile = n_cols - col0 < 128 ? n_cols - col0 : 128;
-  const bool staged = stage_eligible(out_tile, p.vec_out != 0, cols_tile) && (out_tile.P == 1 || (p.M & 3) == 0);
-  // sampled bias row in the epilogue: the forward pass, and the conv data gradient of a transposed convolution's forward
-  const bool bias = !kDgrad || (kConv && p.mu_b != nullptr);
-
-  if (warp < kGenWarps) {
-    // ------------------------------------------------------------------ weight generators (four groups, slot = group)
-    const int group = warp / kGroupWarps, tid = threadIdx.x - group * kGroupThreads;
-    const RngKey key = resolve_rng(p.rng_w);
-    const int total = red_blocks * (s_end - s_begin);
-    for (int it = group; it < total; it += kGenGroups) {
-      const int s = s_begin + it / red_blocks, rb = it - (it / red_blocks) * red_blocks;
-      EpsSrc eps;
-      eps.inj = p.eps_w ? p.eps_w + static_cast<int64_t>(s) * p.w_numel : nullptr;
-      eps.key = key;
-      eps.sample = p.sample_begin + s;
-      { BNN_T0(); mbar_wait(pipe.empty_w + group, ((it >> 2) & 1) ^ 1); BNN_ACC(w_gen); }
-      const uint32_t tile = pipe.ring_w + group * kTileBytes;
-#ifdef BNN_PROFILE_WAITS
-      if (p.exp_flags & 1) { /* skip */ } else
-#endif
-      if (!kDgrad)
-        gen_w_tile<128, false, kSigns>(tile, p.mu_w, p.sigma_w, eps, col0, p.N, rb * kBK, p.K, tid, p.K, 0);
-      else if (!kConv)
-        gen_w_tile<128, true, kSigns>(tile, p.mu_w, p.sigma_w, eps, rb * kBK, p.N, col0, p.K, tid, p.K, 0);
-      else {          // conv data gradient: k-block = (flipped tap, 32 output channels o0 ..)
-        const int tapf = rb / p.conv.cblocks, o0 = (rb - tapf * p.conv.cblocks) * kBK;
-        gen_w_tile<128, true, kSigns>(tile, p.mu_w, p.sigma_w, eps, o0, p.conv.w_rows, col0, p.K, tid,
-                              static_cast<int64_t>(p.conv.wtaps) * p.K, conv_dgrad_tap(p.conv, tapf) * p.K);
-      }
-      fence_proxy_async_smem();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(pipe.full_w + group);
-    }
-    if (staged && (warp >> 2) < kDrainPerQuad - 1) {     // join the drain (TMEM lane quarter = warp % 4)
-      if (bias) named_bar_sync(kDrainBarrier, kDrainThreads);             // the bias row is in shared memory
-      mbar_wait(pipe.accum_full, 0);
-      tc_fence_after_sync();
-      if (bias)
-        drain_tile_shared<true, kDgrad && kConv>(tmem, pipe.ring_a, pipe.aux, out_tile, row0, p.M, mb_used, col0, cols_tile, warp & 3,
-                                1 + (warp >> 2), lane, p.atomic_out != 0);
-      else
-        drain_tile_shared<false, kDgrad && kConv>(tmem, pipe.ring_a, pipe.aux, out_tile, row0, p.M, mb_used, col0, cols_tile, warp & 3,
-                                 1 + (warp >> 2), lane, p.atomic_out != 0);
-    }
-  } else if (warp == kTmaWarp) {
-    // ------------------------------------------------------------------ TMA issuer
-    if (lane == 0) {
-      int it = 0;
-      for (int s = s_begin; s < s_end; ++s) {
-        const int smp = p.shared_l ? 0 : s;
-        int cw[MB], ch[MB], cn[MB];                // conv: first pixel of each row block (fixed over the k-blocks)
-        if (kConv) {
-#pragma unroll
-          for (int mb = 0; mb < MB; ++mb) conv_pixel(p.conv, row0 + mb * 128, smp, &cw[mb], &ch[mb], &cn[mb]);
-        }
-        int tap = 0, cb = 0;                       // conv: k-block rb = (tap, 32-channel block cb), walked incrementally
-        for (int rb = 0; rb < red_blocks; ++rb, ++it) {
-          const int g = it & 1;
-          if (it >= 2) { BNN_T0(); mbar_wait(pipe.empty_w + ((it - 2) & 3), ((it - 2) >> 2) & 1); BNN_ACC(w_tma); }
-#ifdef BNN_PROFILE_WAITS
-          if (p.exp_flags & 2) { mbar_arrive(pipe.full_a + g); continue; }
-#endif
-          mbar_arrive_expect_tx(pipe.full_a + g, mb_used * kTileBytes);
-          if (!kConv) {
-            for (int mb = 0; mb < mb_used; ++mb)
-              tma_load_3d(pipe.ring_a + (g * MB + mb) * kTileBytes, &p.map_l, rb * kBK, row0 + mb * 128, smp, pipe.full_a + g);
-          } else {
-            const int kh = tap / p.conv.KW, kw = tap - kh * p.conv.KW;
-#pragma unroll
-            for (int mb = 0; mb < MB; ++mb)
-              if (mb < mb_used)
-                tma_load_im2col_4d(pipe.ring_a + (g * MB + mb) * kTileBytes, &p.map_l, cb * kBK, cw[mb], ch[mb], cn[mb],
-                                   static_cast<uint16_t>(kw * p.conv.dw), static_cast<uint16_t>(kh * p.conv.dh), pipe.full_a + g);
-            if (++cb == p.conv.cblocks) { cb = 0; ++tap; }
-          }
-        }
-      }
-    }
-    __syncwarp();
-  } else if (warp == kMmaWarpT) {
-    // ------------------------------------------------------------------ MMA issuer
-    if (lane == 0) {
-      const uint32_t idesc = make_idesc_tf32(128, mma_n(n_cols - col0), false, kDgrad);
-      const uint64_t desc_a0 = make_smem_desc(pipe.ring_a);
-      const uint64_t desc_w0 = kDgrad ? make_smem_desc_mn(pipe.ring_w, kMnLbo, kMnSbo) : make_smem_desc(pipe.ring_w);
-      int it = 0;
-      for (int s = s_begin; s < s_end; ++s) {
-        for (int rb = 0; rb < red_blocks; ++rb, ++it) {
-          const int wslot = it & 3, g = it & 1;
-          { BNN_T0(); mbar_wait(pipe.full_w + wslot, (it >> 2) & 1); BNN_ACC(w_mma_w); }
-          { BNN_T0(); mbar_wait(pipe.full_a + g, (it >> 1) & 1); BNN_ACC(w_mma_a); }
-          tc_fence_after_sync();
-          const uint64_t da0 = desc_advance(desc_a0, static_cast<uint32_t>(g * MB) * (kTileBytes >> 4));
-          const uint64_t db0 = desc_advance(desc_w0, static_cast<uint32_t>(wslot) * (kTileBytes >> 4));
-#ifdef BNN_PROFILE_WAITS
-          if (!(p.exp_flags & 4))
-#endif
-          for (int mb = 0; mb < mb_used; ++mb) {
-#pragma unroll
-            for (int ks = 0; ks < kBK / 8; ++ks)
-              mma_tf32(tmem + mb * 128, desc_advance(da0, mb * (kTileBytes >> 4) + ks * 2),
-                       desc_advance(db0, ks * ((kDgrad ? kMnKStep : 32u) >> 4)), idesc, it > 0 || ks > 0);
-          }
-          mma_commit(pipe.empty_w + wslot);           // the one commit of this k-block
-        }
-      }
-      mma_commit(pipe.accum_full);
-    }
-    __syncwarp();
-  } else {
-    // ------------------------------------------------------------------ epilogue
-    const int et = threadIdx.x - kEpiWarp0T * 32;   // 0..127
-    const int quad = warp & 3;
-    if (bias) {
-      float b = 0.f;
-      const int n = col0 + et;
-      if (p.mu_b != nullptr && n < n_cols) {
-        const int s = blockIdx.z;
-        const float e = p.eps_b ? __ldg(p.eps_b + static_cast<int64_t>(s) * n_cols + n)
-                                : eps1(resolve_rng(p.rng_b), p.sample_begin + s, static_cast<uint64_t>(n));
-        b = fmaf(__ldg(p.sigma_b + n), e, __ldg(p.mu_b + n));
-      }
-      pipe.aux[et] = b;
-      named_bar_sync(kEpiBarrier, kEpiThreads);
-      if (staged) named_bar_sync(kDrainBarrier, kDrainThreads);
-    }
-    mbar_wait(pipe.accum_full, 0);
-    tc_fence_after_sync();
-    if (staged) {
-      if (bias)
-        drain_tile_shared<true, kDgrad && kConv>(tmem, pipe.ring_a, pipe.aux, out_tile, row0, p.M, mb_used, col0, cols_tile, quad, 0, lane,
-                                p.atomic_out != 0);
-      else
-        drain_tile_shared<false, kDgrad && kConv>(tmem, pipe.ring_a, pipe.aux, out_tile, row0, p.M, mb_used, col0, cols_tile, quad, 0, lane,
-                                 p.atomic_out != 0);
-    } else {
-      const View& out = out_tile;
-      const int cols_here = cols_tile;
-      for (int mb = 0; mb < mb_used; ++mb) {
-        const int m = row0 + mb * 128 + quad * 32 + lane;
-        for (int c = 0; c * 16 < cols_here; ++c) {
-          float v[16];
-          tmem_ld16(tmem + (static_cast<uint32_t>(quad * 32) << 16) + mb * 128 + c * 16, v);
-          if (bias) {
-#pragma unroll
-            for (int j = 0; j < 16; ++j) v[j] += pipe.aux[c * 16 + j];
-          }
-          if (m < p.M) {
-            if (p.atomic_out) add_chunk(out, m, col0 + c * 16, n_cols, v, p.vec_out != 0);
-            else store_chunk(out, m, col0 + c * 16, n_cols, v, p.vec_out != 0);
-          }
-        }
-      }
-    }
-  }
-#ifdef BNN_PROFILE_WAITS
-  {
-    const int w_ = threadIdx.x >> 5, l_ = threadIdx.x & 31;
-    if (l_ == 0) {
-      if (w_ == 0) { atomicAdd(&g_wait_cycles[3], (unsigned long long)w_gen); atomicAdd(&g_wait_cycles[0], (unsigned long long)(clock64() - t_kernel0)); atomicAdd(&g_wait_cycles[5], 1ull); }
-      if (w_mma_w | w_mma_a) { atomicAdd(&g_wait_cycles[1], (unsigned long long)w_mma_w); atomicAdd(&g_wait_cycles[2], (unsigned long long)w_mma_a); }
-      if (w_tma) atomicAdd(&g_wait_cycles[4], (unsigned long long)w_tma);
-    }
-  }
-#endif
-  tc_fence_before_sync();
-  __syncthreads();
-  if (warp == kMmaWarpT) {
-    tc_fence_after_sync();
-    tmem_dealloc(tmem, kTmemCols);
-  }
+  constexpr bool kPair = false;
+#include "contract_body.inc"
 }
-
-constexpr size_t kContractSmem = kSmemAux + 1024 + static_cast<size_t>(kASlots + kWSlots) * kTileBytes;
+template <int MB, bool kDgrad, int kMode>
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreadsTma, 1)
+contract_pair_kernel(const __grid_constant__ TmaContractParams p) {
+  constexpr bool kPair = true;
+#include "contract_body.inc"
+}
 
 // The conv variants (im2col tensor maps, tap-major weight rows) are separate instantiations: folded into one kernel, the
 // conv state kept live across the generator loop pushed every input-gradient variant over its register budget (116-152
 // bytes of spill stores in the hot loop: C4 input gradient 2.33 -> 2.86 ms).
-template <int MB, bool kDgrad, int kMode>
-int launch_tma_contract_v(const TmaContractParams& p, dim3 grid, cudaStream_t st) {
+template <bool kPair, int MB, bool kDgrad, int kMode>
+int launch_contract_v(const TmaContractParams& p, dim3 grid, cudaStream_t st) {
+  constexpr size_t kSmem = kSmemAux + 1024 + static_cast<size_t>(kASlots) * kTileBytes +
+                           static_cast<size_t>(kWSlots) * (kPair ? kHalfTileBytes : kTileBytes);
+  void (*kernel)(TmaContractParams);
+  if constexpr (kPair) kernel = contract_pair_kernel<MB, kDgrad, kMode>;
+  else kernel = contract_tma_kernel<MB, kDgrad, kMode>;
   static SmemOptIn opt_in;
-  const int rc = allow_dynamic_smem(contract_tma_kernel<MB, kDgrad, kMode>, kContractSmem, &opt_in);
+  const int rc = allow_dynamic_smem(kernel, kSmem, &opt_in);
   if (rc != BNN_OK) return rc;
-  contract_tma_kernel<MB, kDgrad, kMode><<<grid, kThreadsTma, kContractSmem, st>>>(p);
+  kernel<<<grid, kThreadsTma, kSmem, st>>>(p);
   BNN_CUDA_OK(cudaGetLastError());
   return BNN_OK;
 }
-template <int MB, bool kDgrad>
-int launch_tma_contract(const TmaContractParams& p, dim3 grid, cudaStream_t st) {
-  if (p.conv.on) return launch_tma_contract_v<MB, kDgrad, 1>(p, grid, st);
-  if (p.rng_w.row_sign != nullptr) return launch_tma_contract_v<MB, kDgrad, 2>(p, grid, st);
-  return launch_tma_contract_v<MB, kDgrad, 0>(p, grid, st);
-}
-
-// ---------------------------------------------------------------------------------------------- CTA-pair forward / dgrad
-// Same contraction, two SMs per tile (cta_group::2): the pair computes 2 x MB x 128 output rows against ONE 128-column
-// weight tile of which each CTA generates only its half (64 n-rows forward / 64 k-columns dgrad) — half the Philox work
-// per SM and per MMA cycle.  Each CTA loads its own activation tiles by TMA (transaction bytes land on the LEADER's
-// barrier), the generator warps of the peer arrive on the leader's barrier through the cluster address space, the
-// leader's single MMA thread issues tcgen05.mma.cta_group::2 (M = 256) and frees the slots of BOTH CTAs with
-// multicast commits.  Epilogue: every CTA drains its own TMEM.
-constexpr int kPairWSlots = 4;               // 8 KiB half-tiles: slot = k-block % kPairWSlots (a power of two, a multiple of
-constexpr int kPairWShift = 2;               // the four generator groups).  Eight slots were measured: the generators wait
-                                             // less (19 k instead of 26 k cycles per C3 tile), the MMA thread's 8.8 k cycles of
-                                             // waiting for weights do not move — they are the cold start of a tile (first
-                                             // mu / sigma loads, instruction cache), not a lack of slack in the ring
-constexpr int kHalfTileBytes = kTileBytes / 2;
-constexpr size_t kPairSmem = kSmemAux + 1024 + static_cast<size_t>(kASlots) * kTileBytes + kPairWSlots * kHalfTileBytes;
-
-struct PairPipe {
-  uint64_t* full_a;      // [2]  leader: 1 arrival (expect_tx) + the bytes of both CTAs' tiles of one k-block group
-  uint64_t* full_w;      // [kPairWSlots]  leader: one arrival per warp of the owning generator group of both CTAs
-  uint64_t* empty_w;     // [kPairWSlots]  both CTAs: "k-block consumed", one multicast tcgen05.commit per k-block
-  uint64_t* accum_full;  // both CTAs
-  uint32_t* tmem_slot;
-  float* aux;
-  uint32_t ring_a, ring_w;
-};
-
-__device__ __forceinline__ PairPipe carve_pair(uint8_t* smem_raw) {
-  PairPipe p;
-  p.full_a = reinterpret_cast<uint64_t*>(smem_raw);
-  p.full_w = p.full_a + 2;
-  p.empty_w = p.full_w + kPairWSlots;
-  p.accum_full = p.empty_w + kPairWSlots;
-  p.tmem_slot = reinterpret_cast<uint32_t*>(p.accum_full + 1);
-  p.aux = reinterpret_cast<float*>(smem_raw + 512);
-  const uint32_t base = smem_u32(smem_raw) + kSmemAux;
-  p.ring_a = (base + 1023u) & ~1023u;
-  p.ring_w = p.ring_a + kASlots * kTileBytes;
-  return p;
-}
-
-template <int MB, bool kDgrad, int kMode>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreadsTma, 1)
-contract_pair_kernel(const __grid_constant__ TmaContractParams p) {
-  constexpr bool kConv = kMode == 1;
-  constexpr int kSigns = kMode == 2 ? 1 : 0;
-  extern __shared__ __align__(16) uint8_t smem_raw[];
-  long long w_kernel = 0, w_mma_w = 0, w_mma_a = 0, w_gen = 0, w_tma = 0;
-  (void)w_kernel; (void)w_mma_w; (void)w_mma_a; (void)w_gen; (void)w_tma;
-#ifdef BNN_PROFILE_WAITS
-  const long long t_kernel0 = clock64();
-  if (threadIdx.x == 0) {
-    unsigned long long g;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(g));
-    atomicMin(&g_stage_cycles[6], g);
-  }
-#endif
-  constexpr uint32_t kTmemCols = tmem_cols_pow2(MB * 128);
-  const PairPipe pipe = carve_pair(smem_raw);
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const uint32_t rank = cluster_ctarank();          // 0 = leader
-  if (threadIdx.x == 0) {
-    // leader: full_a[g] = activation tiles of k-block group g of BOTH CTAs (1 arrival + bytes), full_w[j] = both halves of
-    // weight tile j (one arrival per generator warp of both CTAs); both CTAs: empty_w[j] = "k-block consumed", ONE
-    // multicast tcgen05.commit per k-block (frees weight slot j, and activation group j & 1 two k-blocks later)
-    for (int i = 0; i < 2; ++i) mbar_init(pipe.full_a + i, 1);
-    for (int i = 0; i < kPairWSlots; ++i) { mbar_init(pipe.full_w + i, 2 * kGroupWarps); mbar_init(pipe.empty_w + i, 1); }
-    mbar_init(pipe.accum_full, 1);
-    fence_mbar_init();
-  }
-  if (warp == kTmaWarp && lane == 0) tma_prefetch_desc(&p.map_l);
-  if (warp == kMmaWarpT) tmem_alloc_pair(pipe.tmem_slot, kTmemCols);
-  tc_fence_before_sync();
-  cluster_sync_all();                                // barriers of both CTAs initialised before any remote arrive
-  tc_fence_after_sync();
-  const uint32_t tmem = *reinterpret_cast<volatile uint32_t*>(pipe.tmem_slot);
-#ifdef BNN_PROFILE_WAITS
-  if (threadIdx.x == 0) { BNN_STAGE(0, t_kernel0); atomicAdd(&g_stage_cycles[5], 1ull); }
-#endif
-
-  const int col0 = blockIdx.y * 128;                   // output columns of the PAIR (n for fwd, k for dgrad)
-  // the pair's tile: sample, first row of the leader, row blocks per CTA (uniform grid: MB; tile plan: 4 or 3)
-  int tile_s = blockIdx.z, lead_row0 = (blockIdx.x & ~1u) * (MB * 128), mb_cap = MB;
-  if (MB == 4 && p.plan.on) {
-    const TilePlan& pl = p.plan;
-    const int t = blockIdx.x >> 1;
-    if (t < pl.n_a) {
-      const int first = pl.s1 * pl.a1;
-      int j;
-      if (t < first) { tile_s = t / pl.a1; j = t - tile_s * pl.a1; }
-      else { const int u = t - first; tile_s = pl.s1 + u / pl.a2; j = u - (u / pl.a2) * pl.a2; }
-      lead_row0 = j * (8 * 128);
-    } else {
-      const int v = t - pl.n_a, first = pl.s1 * pl.b1;
-      int j, a;
-      if (v < first) { tile_s = v / pl.b1; j = v - tile_s * pl.b1; a = pl.a1; }
-      else { const int u = v - first; tile_s = pl.s1 + u / pl.b2; j = u - (u / pl.b2) * pl.b2; a = pl.a2; }
-      lead_row0 = (a * 8 + j * 6) * 128;
-      mb_cap = 3;
-    }
-  }
-  const int row0 = lead_row0 + static_cast<int>(blockIdx.x & 1u) * (mb_cap * 128);      // output rows of THIS CTA
-  const int n_cols = kDgrad ? p.K : p.N;
-  const int n_red = kDgrad ? p.N : p.K;
-  const int s_begin = p.sum_samples ? static_cast<int>(blockIdx.z) * p.z_per : tile_s;
-  const int s_end = p.sum_samples ? (s_begin + p.z_per < p.S ? s_begin + p.z_per : p.S) : tile_s + 1;
-  const int red_blocks = (n_red + kBK - 1) / kBK;
-  // both CTAs walk the same number of M-blocks (the leader holds the lower rows, so its count is the larger one);
-  // tiles beyond M are zero-filled by TMA and never stored
-  int mb_pair = (p.M - lead_row0 + 127) / 128;
-  if (mb_pair > mb_cap) mb_pair = mb_cap;
-
-  // the accumulator is drained by the epilogue warps AND, once their loop has ended, three generator warps per TMEM lane
-  // quarter (staged, coalesced write-out through the operand rings, which are dead by then); uniform per CTA
-  View out_tile = p.out;
-  out_tile.base += (p.sum_samples ? 0 : static_cast<int64_t>(tile_s) * p.out_sample_stride);
-  const int cols_tile = n_cols - col0 < 128 ? n_cols - col0 : 128;
-  const bool staged = stage_eligible(out_tile, p.vec_out != 0, cols_tile) && (out_tile.P == 1 || (p.M & 3) == 0);
-  // sampled bias row in the epilogue: the forward pass, and the conv data gradient of a transposed convolution's forward
-  const bool bias = !kDgrad || (kConv && p.mu_b != nullptr);
-
-  if (warp < kGenWarps) {
-    // ------------------------------------------------------------------ weight generators (half tile per CTA, four groups)
-    const int group = warp / kGroupWarps, tid = threadIdx.x - group * kGroupThreads;
-    const RngKey key = resolve_rng(p.rng_w);
-    const int half0 = col0 + static_cast<int>(rank) * 64;
-    const int total = red_blocks * (s_end - s_begin);
-    const uint32_t lead_full_w0 = mapa_u32(smem_u32(pipe.full_w), 0);
-    for (int it = group; it < total; it += kGenGroups) {
-      const int wslot = it & (kPairWSlots - 1);
-      const int s = s_begin + it / red_blocks, rb = it - (it / red_blocks) * red_blocks;
-      EpsSrc eps;
-      eps.inj = p.eps_w ? p.eps_w + static_cast<int64_t>(s) * p.w_numel : nullptr;
-      eps.key = key;
-      eps.sample = p.sample_begin + s;
-      { BNN_T0(); mbar_wait(pipe.empty_w + wslot, ((it >> kPairWShift) & 1) ^ 1); BNN_ACC(w_gen); }
-      const uint32_t tile = pipe.ring_w + wslot * kHalfTileBytes;
-#ifdef BNN_PROFILE_WAITS
-      if (p.exp_flags & 2) eps.inj = p.sigma_w;   // elimination run: eps read from memory (any valid array): loads and stores, no Philox
-      if (p.exp_flags & 1) { /* elimination run: barrier traffic only, no generation */ } else
-#endif
-      if (!kDgrad)
-        gen_w_tile<64, false, kSigns>(tile, p.mu_w, p.sigma_w, eps, half0, p.N, rb * kBK, p.K, tid, p.K, 0);
-      else if (!kConv)
-        gen_w_tile<64, true, kSigns>(tile, p.mu_w, p.sigma_w, eps, rb * kBK, p.N, half0, p.K, tid, p.K, 0);
-      else {
-        const int tapf = rb / p.conv.cblocks, o0 = (rb - tapf * p.conv.cblocks) * kBK;
-        gen_w_tile<64, true, kSigns>(tile, p.mu_w, p.sigma_w, eps, o0, p.conv.w_rows, half0, p.K, tid,
-                             static_cast<int64_t>(p.conv.wtaps) * p.K, conv_dgrad_tap(p.conv, tapf) * p.K);
-      }
-      fence_proxy_async_smem();
-      __syncwarp();
-      if (lane == 0) mbar_arrive_cluster(lead_full_w0 + wslot * 8);
-    }
-    if (staged && (warp >> 2) < kDrainPerQuad - 1) {     // join the drain (TMEM lane quarter = warp % 4)
-      if (bias) named_bar_sync(kDrainBarrier, kDrainThreads);             // the bias row is in shared memory
-      mbar_wait(pipe.accum_full, 0);
-      tc_fence_after_sync();
-      if (bias)
-        drain_tile_shared<true, kDgrad && kConv>(tmem, pipe.ring_a, pipe.aux, out_tile, row0, p.M, mb_pair, col0, cols_tile, warp & 3,
-                                1 + (warp >> 2), lane, p.atomic_out != 0);
-      else
-        drain_tile_shared<false, kDgrad && kConv>(tmem, pipe.ring_a, pipe.aux, out_tile, row0, p.M, mb_pair, col0, cols_tile, warp & 3,
-                                 1 + (warp >> 2), lane, p.atomic_out != 0);
-    }
-  } else if (warp == kTmaWarp) {
-    // ------------------------------------------------------------------ TMA issuer (own rows; bytes counted by the leader)
-    if (lane == 0) {
-      int it = 0;
-      const uint32_t lead_full_a = mapa_u32(smem_u32(pipe.full_a), 0);
-      for (int s = s_begin; s < s_end; ++s) {
-        const int smp = p.shared_l ? 0 : s;
-        int cw[MB], ch[MB], cn[MB];
-        if (kConv) {
-#pragma unroll
-          for (int mb = 0; mb < MB; ++mb) conv_pixel(p.conv, row0 + mb * 128, smp, &cw[mb], &ch[mb], &cn[mb]);
-        }
-        int tap = 0, cb = 0;
-        for (int rb = 0; rb < red_blocks; ++rb, ++it) {
-          const int g = it & 1;
-          if (it >= 2) { BNN_T0(); mbar_wait(pipe.empty_w + ((it - 2) & (kPairWSlots - 1)), ((it - 2) >> kPairWShift) & 1); BNN_ACC(w_tma); }
-          if (rank == 0) mbar_arrive_expect_tx(pipe.full_a + g, 2 * mb_pair * kTileBytes);
-          if (!kConv) {
-            for (int mb = 0; mb < mb_pair; ++mb)
-              tma_load_3d_pair(pipe.ring_a + (g * MB + mb) * kTileBytes, &p.map_l, rb * kBK, row0 + mb * 128, smp,
-                               lead_full_a + g * 8);
-          } else {
-            const int kh = tap / p.conv.KW, kw = tap - kh * p.conv.KW;
-#pragma unroll
-            for (int mb = 0; mb < MB; ++mb)
-              if (mb < mb_pair)
-                tma_load_im2col_4d_pair(pipe.ring_a + (g * MB + mb) * kTileBytes, &p.map_l, cb * kBK, cw[mb], ch[mb], cn[mb],
-                                        static_cast<uint16_t>(kw * p.conv.dw), static_cast<uint16_t>(kh * p.conv.dh),
-                                        lead_full_a + g * 8);
-            if (++cb == p.conv.cblocks) { cb = 0; ++tap; }
-          }
-        }
-      }
-    }
-    __syncwarp();
-  } else if (warp == kMmaWarpT) {
-    // ------------------------------------------------------------------ MMA issuer (leader only)
-    if (rank == 0 && lane == 0) {
-      // N = 128 always: each CTA contributes its 64-row half of the weight tile (zero rows beyond the matrix edge)
-      const uint32_t idesc = make_idesc_tf32(256, 128, false, kDgrad);
-      const uint64_t desc_a0 = make_smem_desc(pipe.ring_a);
-      const uint64_t desc_w0 = kDgrad ? make_smem_desc_mn(pipe.ring_w, kMnLbo, kMnSbo) : make_smem_desc(pipe.ring_w);
-      int it = 0;
-      for (int s = s_begin; s < s_end; ++s) {
-        for (int rb = 0; rb < red_blocks; ++rb, ++it) {
-          const int wslot = it & (kPairWSlots - 1), g = it & 1;
-          { BNN_T0(); mbar_wait_cluster(pipe.full_w + wslot, (it >> kPairWShift) & 1); BNN_ACC(w_mma_w); }
-#ifdef BNN_PROFILE_WAITS
-          if (it == 0) atomicAdd(&g_wait_cycles[6], (unsigned long long)(clock64() - t_kernel0));    // first weight tile ready
-          if (it == 4) atomicAdd(&g_wait_cycles[7], (unsigned long long)w_mma_w);                    // weight waits of k-blocks 0..4
-#endif
-          { BNN_T0(); mbar_wait_cluster(pipe.full_a + g, (it >> 1) & 1); BNN_ACC(w_mma_a); }
-          tc_fence_after_sync();
-          const uint64_t da0 = desc_advance(desc_a0, static_cast<uint32_t>(g * MB) * (kTileBytes >> 4));
-          const uint64_t db0 = desc_advance(desc_w0, static_cast<uint32_t>(wslot) * (kHalfTileBytes >> 4));
-          for (int mb = 0; mb < mb_pair; ++mb) {
-#pragma unroll
-            for (int ks = 0; ks < kBK / 8; ++ks)
-              mma_tf32_pair(tmem + mb * 128, desc_advance(da0, mb * (kTileBytes >> 4) + ks * 2),
-                            desc_advance(db0, ks * ((kDgrad ? kMnKStep : 32u) >> 4)), idesc, it > 0 || ks > 0);
-          }
-          mma_commit_pair(pipe.empty_w + wslot, 3);   // the one (multicast) commit of this k-block
-        }
-      }
-      mma_commit_pair(pipe.accum_full, 3);
-    }
-    __syncwarp();
-  } else {
-    // ------------------------------------------------------------------ epilogue (own TMEM, own rows)
-    const int et = threadIdx.x - kEpiWarp0T * 32;   // 0..127
-    const int quad = warp & 3;
-    if (bias) {
-      float b = 0.f;
-      const int n = col0 + et;
-      if (p.mu_b != nullptr && n < n_cols) {
-        const int s = tile_s;
-        const float e = p.eps_b ? __ldg(p.eps_b + static_cast<int64_t>(s) * n_cols + n)
-                                : eps1(resolve_rng(p.rng_b), p.sample_begin + s, static_cast<uint64_t>(n));
-        b = fmaf(__ldg(p.sigma_b + n), e, __ldg(p.mu_b + n));
-      }
-      pipe.aux[et] = b;
-      named_bar_sync(kEpiBarrier, kEpiThreads);
-      if (staged) named_bar_sync(kDrainBarrier, kDrainThreads);
-    }
-    mbar_wait(pipe.accum_full, 0);
-    tc_fence_after_sync();
-#ifdef BNN_PROFILE_WAITS
-    if (threadIdx.x == kEpiWarp0T * 32) BNN_STAGE(2, t_kernel0);
-#endif
-    if (staged) {
-      if (bias)
-        drain_tile_shared<true, kDgrad && kConv>(tmem, pipe.ring_a, pipe.aux, out_tile, row0, p.M, mb_pair, col0, cols_tile, quad, 0, lane,
-                                p.atomic_out != 0);
-      else
-        drain_tile_shared<false, kDgrad && kConv>(tmem, pipe.ring_a, pipe.aux, out_tile, row0, p.M, mb_pair, col0, cols_tile, quad, 0, lane,
-                                 p.atomic_out != 0);
-    } else {
-      const View& out = out_tile;
-      const int cols_here = cols_tile;
-      for (int mb = 0; mb < mb_pair; ++mb) {
-        const int m = row0 + mb * 128 + quad * 32 + lane;
-        if (row0 + mb * 128 >= p.M) break;               // uniform per CTA
-        for (int c = 0; c * 16 < cols_here; ++c) {
-          float v[16];
-          tmem_ld16(tmem + (static_cast<uint32_t>(quad * 32) << 16) + mb * 128 + c * 16, v);
-          if (bias) {
-#pragma unroll
-            for (int j = 0; j < 16; ++j) v[j] += pipe.aux[c * 16 + j];
-          }
-          if (m < p.M) {
-            if (p.atomic_out) add_chunk(out, m, col0 + c * 16, n_cols, v, p.vec_out != 0);
-            else store_chunk(out, m, col0 + c * 16, n_cols, v, p.vec_out != 0);
-          }
-        }
-      }
-    }
-  }
-#ifdef BNN_PROFILE_WAITS
-  if (threadIdx.x == kEpiWarp0T * 32) BNN_STAGE(3, t_kernel0);
-  if (threadIdx.x == 0) BNN_STAGE(1, t_kernel0);
-  {
-    const int w_ = threadIdx.x >> 5, l_ = threadIdx.x & 31;
-    if (l_ == 0) {
-      if (w_ == 0) { atomicAdd(&g_wait_cycles[3], (unsigned long long)w_gen); atomicAdd(&g_wait_cycles[0], (unsigned long long)(clock64() - t_kernel0)); atomicAdd(&g_wait_cycles[5], 1ull); }
-      if (w_mma_w | w_mma_a) { atomicAdd(&g_wait_cycles[1], (unsigned long long)w_mma_w); atomicAdd(&g_wait_cycles[2], (unsigned long long)w_mma_a); }
-      if (w_tma) atomicAdd(&g_wait_cycles[4], (unsigned long long)w_tma);
-    }
-  }
-#endif
-  tc_fence_before_sync();
-  cluster_sync_all();                                // nobody leaves while the partner may still signal or read
-  if (warp == kMmaWarpT) {
-    tc_fence_after_sync();
-    tmem_dealloc_pair(tmem, kTmemCols);
-  }
-#ifdef BNN_PROFILE_WAITS
-  if (threadIdx.x == 0) {
-    BNN_STAGE(4, t_kernel0);
-    unsigned long long g;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(g));
-    atomicMax(&g_stage_cycles[7], g);
-  }
-#endif
-}
-
-template <int MB, bool kDgrad, int kMode>
-int launch_pair_contract_v(const TmaContractParams& p, dim3 grid, cudaStream_t st) {
-  static SmemOptIn opt_in;
-  const int rc = allow_dynamic_smem(contract_pair_kernel<MB, kDgrad, kMode>, kPairSmem, &opt_in);
-  if (rc != BNN_OK) return rc;
-  contract_pair_kernel<MB, kDgrad, kMode><<<grid, kThreadsTma, kPairSmem, st>>>(p);
-  BNN_CUDA_OK(cudaGetLastError());
-  return BNN_OK;
-}
-template <int MB, bool kDgrad>
-int launch_pair_contract(const TmaContractParams& p, dim3 grid, cudaStream_t st) {
-  if (p.conv.on) return launch_pair_contract_v<MB, kDgrad, 1>(p, grid, st);
-  if (p.rng_w.row_sign != nullptr) return launch_pair_contract_v<MB, kDgrad, 2>(p, grid, st);
-  return launch_pair_contract_v<MB, kDgrad, 0>(p, grid, st);
+template <bool kPair, int MB, bool kDgrad>
+int launch_contract(const TmaContractParams& p, dim3 grid, cudaStream_t st) {
+  if (p.conv.on) return launch_contract_v<kPair, MB, kDgrad, 1>(p, grid, st);
+  if (p.rng_w.row_sign != nullptr) return launch_contract_v<kPair, MB, kDgrad, 2>(p, grid, st);
+  return launch_contract_v<kPair, MB, kDgrad, 0>(p, grid, st);
 }
 
 // Test aid: force one kernel variant (0 = pair, 1 / 2 / 4 = rows blocks per CTA, -1 = cost model) so that small test
@@ -1093,12 +580,12 @@ int dispatch_tma_contract(TmaContractParams& p, int n_cols, cudaStream_t st) {
   if (best == 0) {                                                // two CTAs (one cluster) per 1024 rows
     const int pairs = (m_blocks + 7) / 8;
     if (plan_pair_tiles(&p.plan, m_blocks, p.S, gx, gz, p.sum_samples != 0, sms / 2))
-      return launch_pair_contract<4, kDgrad>(p, dim3(2 * (p.plan.n_a + p.plan.s1 * p.plan.b1 + (p.S - p.plan.s1) * p.plan.b2), 1, 1), st);
-    return launch_pair_contract<4, kDgrad>(p, dim3(2 * pairs, gx, gz), st);
+      return launch_contract<true, 4, kDgrad>(p, dim3(2 * (p.plan.n_a + p.plan.s1 * p.plan.b1 + (p.S - p.plan.s1) * p.plan.b2), 1, 1), st);
+    return launch_contract<true, 4, kDgrad>(p, dim3(2 * pairs, gx, gz), st);
   }
-  if (best == 4) return launch_tma_contract<4, kDgrad>(p, dim3(gx, (m_blocks + 3) / 4, gz), st);
-  if (best == 2) return launch_tma_contract<2, kDgrad>(p, dim3(gx, (m_blocks + 1) / 2, gz), st);
-  return launch_tma_contract<1, kDgrad>(p, dim3(gx, m_blocks, gz), st);
+  if (best == 4) return launch_contract<false, 4, kDgrad>(p, dim3(gx, (m_blocks + 3) / 4, gz), st);
+  if (best == 2) return launch_contract<false, 2, kDgrad>(p, dim3(gx, (m_blocks + 1) / 2, gz), st);
+  return launch_contract<false, 1, kDgrad>(p, dim3(gx, m_blocks, gz), st);
 }
 
 // ---------------------------------------------------------------------------------------------- weight gradient
@@ -1608,64 +1095,35 @@ int tma_conv_fwd(const float* x, int64_t x_sample_stride, const float* mu_w, con
                          sample_begin, rng_w, rng_b, false, st);
 }
 
-// dX[n][h][w][c] = sum_{kh, kw, o} dY[n][h + ph - kh dh][w + pw - kw dw][o] W[o][kh][kw][c]   (stride 1): the transposed-
-// filter form — an im2col load of dY with lower corner p - (K - 1) d, taps walked in flipped order — so the input gradient
-// is a gather like the forward pass: no column matrix, no scatter.
-int tma_conv_dgrad(const float* dy, const float* mu_w, const float* sigma_w, const float* eps_w, float* dx,
-                   int64_t x_sample_stride, const bnn_conv2d_nhwc* g, int S, uint32_t sample_begin, const bnn_rng* rng_w,
-                   cudaStream_t st) {
-  if (g->sh != 1 || g->sw != 1 || g->Cout % kBK != 0 || g->C % 4 != 0 || !aligned16(dy) || !aligned16(dx) ||
-      rng_w->elem_offset % 4 != 0 || !aligned16(mu_w) || !aligned16(sigma_w) || (eps_w != nullptr && !aligned16(eps_w)))
-    return kNotEligible;
-  const int lo_w = g->pw - (g->KW - 1) * g->dw, lo_h = g->ph - (g->KH - 1) * g->dh;
-  const int up_w = lo_w + g->W - g->OW, up_h = lo_h + g->H - g->OH;
-  if (lo_w < -128 || lo_h < -128 || lo_w > 127 || lo_h > 127 || up_w < -128 || up_h < -128 || up_w > 127 || up_h > 127 ||
-      (g->KH - 1) * g->dh >= 256 || (g->KW - 1) * g->dw >= 256)
-    return kNotEligible;
-  TmaContractParams p{};
-  int rc = make_im2col_map(&p.map_l, dy, g->Cout, g->OW, g->OH, static_cast<int64_t>(S) * g->B, lo_w, lo_h, up_w, up_h, 1,
-                           1, 128, false);
-  if (rc != BNN_OK) return rc;
-  ConvCoords c{};
-  c.on = 1; c.P = g->H * g->W; c.OW = g->W; c.imgs = g->B; c.sh = 1; c.sw = 1; c.lh = lo_h; c.lw = lo_w;
-  c.dh = g->dh; c.dw = g->dw; c.KW = g->KW; c.taps = g->KH * g->KW; c.cblocks = g->Cout / kBK; c.w_rows = g->Cout;
-  c.chans = g->Cout;
-  c.wtaps = c.taps; c.wKW = g->KW; c.tkh = g->KH - 1; c.tkw = g->KW - 1; c.tdh = 1; c.tdw = 1;
-  p.conv = c;
-  p.out.base = dx; p.out.bs = g->C; p.out.P = 1; p.out_sample_stride = x_sample_stride;
-  p.mu_w = mu_w; p.sigma_w = sigma_w; p.eps_w = eps_w;
-  p.M = g->B * g->H * g->W; p.N = c.taps * g->Cout; p.K = g->C; p.S = S; p.sample_begin = sample_begin;
-  p.w_numel = static_cast<int64_t>(g->Cout) * c.taps * g->C;
-  p.rng_w = *rng_w; p.rng_b = *rng_w;
-  p.shared_l = 0;
-  p.sum_samples = (x_sample_stride == 0) ? 1 : 0;
-  p.vec_out = (x_sample_stride % 4 == 0);
-  return dispatch_tma_contract<true>(p, p.K, st);
-}
-
-int tma_conv_wgrad(const float* dy, const float* x, int64_t x_sample_stride, const float* rho_w, const float* eps_w,
+// Weight gradient of the implicit GEMM: G = dY^T A with dY [S or 1][B*OH*OW][Cout] (map_dy) and A the NHWC tensor
+// [S or 1][B][H][W][C] seen through the im2col map (map_a).  A convolution passes (dy, x), shared_a when all samples
+// share x; a transposed convolution passes its conv view's operands (x, dy), shared_dy when all samples share x.
+int tma_conv_wgrad(const float* dy, bool shared_dy, const float* a, bool shared_a, const float* rho_w, const float* eps_w,
                    float* dmu_w, float* drho_w, const bnn_conv2d_nhwc* g, int S, uint32_t sample_begin,
                    const bnn_rng* rng_w, cudaStream_t st) {
-  const bool shared = x_sample_stride == 0;
   const int M = g->B * g->OH * g->OW, N = g->Cout, K = g->KH * g->KW * g->C;
-  if (!conv_ok(*g) || N % 4 != 0 || !aligned16(dy) || !aligned16(x) || rng_w->elem_offset % 4 != 0 || !aligned16(rho_w) ||
+  if (!conv_ok(*g) || N % 4 != 0 || !aligned16(dy) || !aligned16(a) || rng_w->elem_offset % 4 != 0 || !aligned16(rho_w) ||
       !aligned16(dmu_w) || !aligned16(drho_w) || (eps_w != nullptr && !aligned16(eps_w)))
     return kNotEligible;
   TmaWgradParams p{};
-  int rc = make_map(&p.map_dy, dy, N, M, S, N, static_cast<int64_t>(M) * N, kWgRows, true);
+  int rc = make_map(&p.map_dy, dy, N, M, shared_dy ? 1 : S, N, static_cast<int64_t>(M) * N, kWgRows, true);
   if (rc != BNN_OK) return rc;
-  rc = make_im2col_map(&p.map_a, x, g->C, g->W, g->H, static_cast<int64_t>(shared ? 1 : S) * g->B, -g->pw, -g->ph,
+  rc = make_im2col_map(&p.map_a, a, g->C, g->W, g->H, static_cast<int64_t>(shared_a ? 1 : S) * g->B, -g->pw, -g->ph,
                        g->pw - (g->KW - 1) * g->dw, g->ph - (g->KH - 1) * g->dh, g->sw, g->sh, kWgRows, true);
   if (rc != BNN_OK) return rc;
   p.conv = conv_coords_fwd(*g);
   p.rho_w = rho_w; p.eps_w = eps_w; p.dmu_w = dmu_w; p.drho_w = drho_w;
   p.M = M; p.N = N; p.K = K; p.S = S; p.sample_begin = sample_begin;
   p.rng_w = *rng_w;
-  p.shared_a = shared ? 1 : 0;
+  p.shared_a = shared_a ? 1 : 0;
+  p.shared_dy = shared_dy ? 1 : 0;
   return wgrad_plan_and_launch(p, M, N, K, S, st);
 }
 
-// ---------------------------------------------------------------------------------------------- transposed convolution
+// ---------------------------------------------------------------------------------------------- transposed-filter gather
+// The input gradient of a stride-1 convolution is a gather like the forward pass, no column matrix and no scatter:
+//   dX[n][h][w][c] = sum_{kh, kw, o} dY[n][h + ph - kh dh][w + pw - kw dw][o] W[o][kh][kw][c]
+// an im2col load of dY with lower corner p - (K - 1) d, taps walked in flipped order.
 // A transposed convolution with weight W [Cin][Cout][KH][KW] is the adjoint of its CONV VIEW, the convolution from the
 // transposed output (C = Cout channels, H x W) to the transposed input (Cout_view = Cin channels, OH x OW) with the same W
 // read as OIHW.  Its forward is therefore the conv view's data gradient plus a bias:
@@ -1674,7 +1132,8 @@ int tma_conv_wgrad(const float* dy, const float* x, int64_t x_sample_stride, con
 // and then from input row i + (r + ph - kh dh) / sh for output row r + sh i: every phase is a STRIDE-1 gather over x with
 // its own taps (tdh = sh / gcd(sh, dh) apart, dh / gcd(sh, dh) input rows apart) and its own im2col corner.  One launch of
 // the data-gradient kernel per phase walks exactly that phase's taps x 32-channel blocks (no MMA on inserted zeros) and
-// writes its rows through a phase view; phases without a tap get the bias alone.
+// writes its rows through a phase view; phases without a tap get the bias alone.  At stride 1 there is one phase with
+// every tap: the conv input gradient above, written through the plain row view.
 namespace {
 struct PhaseDim {
   int r, rows;              // phase offset, output rows of the phase
@@ -1736,12 +1195,13 @@ int conv_transpose_phases(const bnn_conv2d_nhwc* g, int32_t* out, int max_phases
   return n;
 }
 
-int tma_conv_transpose_fwd(const float* x, int64_t x_sample_stride, const float* mu_w, const float* sigma_w,
-                           const float* mu_b, const float* sigma_b, const float* eps_w, const float* eps_b, float* y,
-                           const bnn_conv2d_nhwc* g, int S, uint32_t sample_begin, const bnn_rng* rng_w,
-                           const bnn_rng* rng_b, cudaStream_t st) {
-  // conv view: C = transposed output channels (the drained columns), Cout = transposed input channels (reduction)
-  const bool shared = x_sample_stride == 0;
+// x: the gathered NHWC tensor [S or 1][B][OH][OW][Cout] (conv view), shared_x: all samples read sample 0 of x; y: the
+// NHWC output [S][B][H][W][C] with the optional sampled bias, or with sum_samples one output summed over the samples
+int tma_conv_gather(const float* x, bool shared_x, const float* mu_w, const float* sigma_w, const float* mu_b,
+                    const float* sigma_b, const float* eps_w, const float* eps_b, float* y, int64_t y_sample_stride,
+                    bool sum_samples, const bnn_conv2d_nhwc* g, int S, uint32_t sample_begin, const bnn_rng* rng_w,
+                    const bnn_rng* rng_b, cudaStream_t st) {
+  // conv view: C = gathered output channels (the drained columns), Cout = channels of x (reduction)
   if (g->Cout % kBK != 0 || g->C % 4 != 0 || g->sh > 8 || g->sw > 8 || !aligned16(x) || !aligned16(y) ||
       rng_w->elem_offset % 4 != 0 || !aligned16(mu_w) || !aligned16(sigma_w) || (eps_w != nullptr && !aligned16(eps_w)))
     return kNotEligible;
@@ -1757,7 +1217,8 @@ int tma_conv_transpose_fwd(const float* x, int64_t x_sample_stride, const float*
           up_w > 127 || (a.taps - 1) * a.dstep >= 256 || (b.taps - 1) * b.dstep >= 256)
         return kNotEligible;
     }
-  const int64_t C = g->C, img_y = static_cast<int64_t>(g->H) * g->W * C, y_ss = g->B * img_y;
+  const bool phased = g->sh != 1 || g->sw != 1;
+  const int64_t C = g->C, img_y = static_cast<int64_t>(g->H) * g->W * C;
   for (int rh = 0; rh < ph_h; ++rh)
     for (int rw = 0; rw < ph_w; ++rw) {
       const PhaseDim a = phase_dim(rh, g->H, g->sh, g->ph, g->dh, g->KH);
@@ -1766,15 +1227,16 @@ int tma_conv_transpose_fwd(const float* x, int64_t x_sample_stride, const float*
       if (a.taps == 0 || b.taps == 0) {
         const int64_t total = static_cast<int64_t>(S) * g->B * a.rows * b.rows * C;
         const int blocks = static_cast<int>(std::min<int64_t>((total + 255) / 256, 4 * sm_count()));
-        phase_bias_kernel<<<blocks, 256, 0, st>>>(base, y_ss, img_y, g->sh * g->W * C, g->sw * C, S, g->B, a.rows, b.rows,
-                                                  g->C, mu_b, sigma_b, eps_b, sample_begin, rng_b ? *rng_b : *rng_w);
+        phase_bias_kernel<<<blocks, 256, 0, st>>>(base, y_sample_stride, img_y, g->sh * g->W * C, g->sw * C, S, g->B,
+                                                  a.rows, b.rows, g->C, mu_b, sigma_b, eps_b, sample_begin,
+                                                  rng_b ? *rng_b : *rng_w);
         BNN_CUDA_OK(cudaGetLastError());
         continue;
       }
       TmaContractParams p{};
       const int up_h = a.lo + a.rows - g->OH, up_w = b.lo + b.rows - g->OW;
-      int rc = make_im2col_map(&p.map_l, x, g->Cout, g->OW, g->OH, static_cast<int64_t>(shared ? 1 : S) * g->B, b.lo, a.lo,
-                               up_w, up_h, 1, 1, 128, false);
+      int rc = make_im2col_map(&p.map_l, x, g->Cout, g->OW, g->OH, static_cast<int64_t>(shared_x ? 1 : S) * g->B, b.lo,
+                               a.lo, up_w, up_h, 1, 1, 128, false);
       if (rc != BNN_OK) return rc;
       ConvCoords c{};
       c.on = 1; c.P = a.rows * b.rows; c.OW = b.rows; c.imgs = g->B; c.sh = 1; c.sw = 1; c.lh = a.lo; c.lw = b.lo;
@@ -1783,15 +1245,16 @@ int tma_conv_transpose_fwd(const float* x, int64_t x_sample_stride, const float*
       c.wtaps = g->KH * g->KW; c.wKW = g->KW; c.tkh = a.tlast; c.tkw = b.tlast; c.tdh = a.tstep; c.tdw = b.tstep;
       p.conv = c;
       p.out.base = base; p.out.bs = g->sw * C; p.out.P = 1;
-      p.out.pw = b.rows; p.out.pimg = a.rows * b.rows; p.out.s_i = g->sh * g->W * C; p.out.s_img = img_y;
-      p.out_sample_stride = y_ss;
+      if (phased) { p.out.pw = b.rows; p.out.pimg = a.rows * b.rows; p.out.s_i = g->sh * g->W * C; p.out.s_img = img_y; }
+      p.out_sample_stride = y_sample_stride;
       p.mu_w = mu_w; p.sigma_w = sigma_w; p.eps_w = eps_w; p.mu_b = mu_b; p.sigma_b = sigma_b; p.eps_b = eps_b;
       p.M = g->B * a.rows * b.rows; p.N = c.taps * g->Cout; p.K = g->C; p.S = S; p.sample_begin = sample_begin;
       p.w_numel = static_cast<int64_t>(g->Cout) * c.wtaps * g->C;
       p.rng_w = *rng_w; p.rng_b = rng_b ? *rng_b : *rng_w;
-      p.shared_l = shared ? 1 : 0;
-      p.sum_samples = 0;
-      p.vec_out = 1;            // C % 4 == 0: every CTA takes the staged drain, the only one with the phase view
+      p.shared_l = shared_x ? 1 : 0;
+      p.sum_samples = sum_samples ? 1 : 0;
+      // C % 4 == 0: with a 4-aligned sample stride every CTA takes the staged drain, the only one with the phase view
+      p.vec_out = (y_sample_stride % 4 == 0);
       rc = dispatch_tma_contract<true>(p, p.K, st);
       if (rc != BNN_OK) return rc;
     }
@@ -1808,30 +1271,6 @@ int tma_conv_transpose_dgrad(const float* dy, const float* mu_w, const float* si
   v.base = dx; v.batch_stride = g->Cout; v.P = 1;
   return conv_fwd_launch(dy, static_cast<int64_t>(g->B) * g->H * g->W * g->C, mu_w, sigma_w, nullptr, nullptr, eps_w,
                          nullptr, v, x_sample_stride, g, S, sample_begin, rng_w, nullptr, x_sample_stride == 0, st);
-}
-
-int tma_conv_transpose_wgrad(const float* dy, const float* x, int64_t x_sample_stride, const float* rho_w,
-                             const float* eps_w, float* dmu_w, float* drho_w, const bnn_conv2d_nhwc* g, int S,
-                             uint32_t sample_begin, const bnn_rng* rng_w, cudaStream_t st) {
-  // conv view: "dY" operand = the transposed input x [S or 1][B*OH*OW][Cout], A = im2col(dy) over [S][B][H][W][C]
-  const int M = g->B * g->OH * g->OW, N = g->Cout, K = g->KH * g->KW * g->C;
-  if (!conv_ok(*g) || N % 4 != 0 || !aligned16(dy) || !aligned16(x) || rng_w->elem_offset % 4 != 0 || !aligned16(rho_w) ||
-      !aligned16(dmu_w) || !aligned16(drho_w) || (eps_w != nullptr && !aligned16(eps_w)))
-    return kNotEligible;
-  const bool shared = x_sample_stride == 0;
-  TmaWgradParams p{};
-  int rc = make_map(&p.map_dy, x, N, M, shared ? 1 : S, N, static_cast<int64_t>(M) * N, kWgRows, true);
-  if (rc != BNN_OK) return rc;
-  rc = make_im2col_map(&p.map_a, dy, g->C, g->W, g->H, static_cast<int64_t>(S) * g->B, -g->pw, -g->ph,
-                       g->pw - (g->KW - 1) * g->dw, g->ph - (g->KH - 1) * g->dh, g->sw, g->sh, kWgRows, true);
-  if (rc != BNN_OK) return rc;
-  p.conv = conv_coords_fwd(*g);
-  p.rho_w = rho_w; p.eps_w = eps_w; p.dmu_w = dmu_w; p.drho_w = drho_w;
-  p.M = M; p.N = N; p.K = K; p.S = S; p.sample_begin = sample_begin;
-  p.rng_w = *rng_w;
-  p.shared_a = 0;
-  p.shared_dy = shared ? 1 : 0;
-  return wgrad_plan_and_launch(p, M, N, K, S, st);
 }
 
 int tma_wait_counters(unsigned long long* out8, int reset) {

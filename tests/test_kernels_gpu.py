@@ -592,6 +592,68 @@ def test_pair_kernel_tile_plan_covers_every_row_once(C, request, M, N, K, S):
     assert rel_err(da, torch.bmm(dy.double(), w)) < TOL[0]
 
 
+@pytest.mark.parametrize("variant", ["pair", "mb4", "mb2", "mb1"])
+@pytest.mark.parametrize("shared", [True, False])
+def test_every_tma_contraction_variant_in_the_conv_and_sign_noise_modes(C, request, variant, shared):
+    """The single-CTA and CTA-pair kernels share one body in all three modes; force each variant through (a) the
+    implicit-GEMM conv mode: stride-1 NormalConv2d forward and input gradient on injected eps against torch fp64, and (b)
+    the rank-one sign-noise mode: the fused FlipoutNormalLinear forward and input gradient against the two-contraction
+    formula.  765 and 700 rows per sample: more than 4 row blocks, which the forced pair variant needs.  NaN-filled
+    outputs: every row must be written."""
+    C.force_contract_variant(variant)
+    request.addfinalizer(lambda: C.force_contract_variant(None))
+    g = torch.Generator().manual_seed(14)
+    # (a) conv, 3x3, padding 1: weights in (o, kh, kw, c) order, NHWC activations
+    S, B, Cin, H, W, Cout = 2, 3, 32, 15, 17, 64
+    M = B * H * W
+    x = torch.randn(1 if shared else S, B, Cin, H, W, generator=g)
+    mu_w, rho_w = init_params((Cout, Cin, 3, 3), g)
+    mu_b, rho_b = init_params((Cout,), g, fan_in=Cin * 9)
+    eps_w = torch.randn(S, Cout, Cin, 3, 3, generator=g)
+    eps_b = torch.randn(S, Cout, generator=g)
+    w = mu_w.double() + orc.stddev(rho_w.double()) * eps_w.double()                  # [S, Cout, Cin, 3, 3]
+    b = mu_b.double() + orc.stddev(rho_b.double()) * eps_b.double()
+    geom = C.conv_geom(B, H, W, Cin, H, W, Cout, 3, 3, (1, 1), (1, 1), (1, 1))
+    mu_o, sig_o = mu_w.permute(0, 2, 3, 1).contiguous().cuda(), C.stddev(rho_w.permute(0, 2, 3, 1).contiguous().cuda())
+    eps_o = eps_w.permute(0, 1, 3, 4, 2).contiguous().cuda()
+    y = torch.full((S, M, Cout), float("nan"), device="cuda")
+    C.sampled_conv2d_fwd(x.permute(0, 1, 3, 4, 2).contiguous().cuda(), 0 if shared else M * Cin, mu_o, sig_o, mu_b.cuda(),
+                         C.stddev(rho_b.cuda()), eps_o, eps_b.cuda(), C.make_view(y.data_ptr(), Cout, 1), M * Cout, geom, S, 0,
+                         C.make_rng(0, 0, 0), C.make_rng(0, 0, 1))
+    dy = torch.randn(S, B, Cout, H, W, generator=g)
+    dx = torch.full((1 if shared else S, B, H, W, Cin), float("nan"), device="cuda")
+    C.sampled_conv2d_dgrad(dy.permute(0, 1, 3, 4, 2).contiguous().cuda(), mu_o, sig_o, eps_o, dx, 0 if shared else M * Cin,
+                           geom, S, 0, C.make_rng(0, 0, 0))
+    torch.cuda.synchronize()
+    dx_ref = torch.zeros(dx.shape, dtype=torch.float64)
+    for s in range(S):
+        ref = F.conv2d(x[0 if shared else s].double(), w[s], b[s], padding=1)
+        assert rel_err(y[s], ref.permute(0, 2, 3, 1).reshape(M, Cout)) < TOL[0], f"conv forward, sample {s}"
+        dx_ref[0 if shared else s] += F.conv_transpose2d(dy[s].double(), w[s], padding=1).permute(0, 2, 3, 1)
+    assert rel_err(dx, dx_ref) < TOL[0]
+    # (b) rank-one sign noise eps_s = R_s Sg_s^T, no bias
+    M, N, K, S = 700, 136, 96, 3
+    a, mu_w, rho_w, _, _, _, _ = gemm_inputs(M, N, K, S, shared, g, bias=False)
+    R = (torch.randint(0, 2, (S, N), generator=g) * 2 - 1).float()
+    Sg = (torch.randint(0, 2, (S, K), generator=g) * 2 - 1).float()
+    rng = C.make_rng(0, 0, 0, signs=(R.cuda(), Sg.cuda()))
+    y = run_fwd(C, a, mu_w, rho_w, None, None, None, None, S, 0, rng_w=rng)
+    dy = torch.randn(S, M, N, generator=g)
+    da = torch.full(tuple(a.shape), float("nan"), device="cuda")
+    sig = orc.stddev(rho_w.double())
+    ddy = dy.cuda()
+    C.sampled_gemm_dgrad(C.make_view(ddy.data_ptr(), N, 1), M * N, mu_w.cuda(), C.stddev(rho_w.cuda()), None, da, K,
+                         0 if shared else M * K, M, N, K, S, 0, rng, 0)
+    torch.cuda.synchronize()
+    da_ref = torch.zeros(a.shape, dtype=torch.float64)
+    for s in range(S):
+        x_s, r, c = a[0 if shared else s].double(), R[s].double(), Sg[s].double()
+        ref = x_s @ mu_w.double().t() + ((x_s * c) @ sig.t()) * r
+        assert rel_err(y[s], ref) < TOL[0], f"sign-noise forward, sample {s}"
+        da_ref[0 if shared else s] += dy[s].double() @ mu_w.double() + ((dy[s].double() * r) @ sig) * c
+    assert rel_err(da, da_ref) < TOL[0]
+
+
 def test_wgrad_philox_equals_injected(C):
     g = torch.Generator().manual_seed(9)
     M, N, K, S = 96, 72, 136, 5
