@@ -49,6 +49,12 @@ class bnn_conv2d_nhwc(ctypes.Structure):
                 ("B", "H", "W", "C", "OH", "OW", "Cout", "KH", "KW", "sh", "sw", "ph", "pw", "dh", "dw", "reserved")]
 
 
+class bnn_conv3d_nhwc(ctypes.Structure):
+    _fields_ = [(n, ctypes.c_int32) for n in
+                ("B", "D", "H", "W", "C", "OD", "OH", "OW", "Cout", "KD", "KH", "KW", "sd", "sh", "sw", "pd", "ph", "pw",
+                 "dd", "dh", "dw", "reserved")]
+
+
 class bnn_kl_tensor(ctypes.Structure):
     _fields_ = [("mu", ctypes.c_void_p), ("rho", ctypes.c_void_p), ("grad_mu", ctypes.c_void_p),
                 ("grad_rho", ctypes.c_void_p), ("numel", ctypes.c_int64),
@@ -136,6 +142,18 @@ _SIGNATURES = {
                                                           ctypes.c_uint32, ctypes.POINTER(bnn_rng), ctypes.c_void_p]),
     "bnn_debug_conv_transpose_phases": (ctypes.c_int, [ctypes.POINTER(bnn_conv2d_nhwc), ctypes.POINTER(ctypes.c_int32),
                                                        ctypes.c_int32]),
+    "bnn_sampled_conv_transpose3d_fwd": (ctypes.c_int, [_c_f32p, ctypes.c_int64, _c_f32p, _c_f32p, _c_f32p, _c_f32p, _c_f32p,
+                                                        _c_f32p, _c_f32p, ctypes.POINTER(bnn_conv3d_nhwc), ctypes.c_int32,
+                                                        ctypes.c_uint32, ctypes.POINTER(bnn_rng), ctypes.POINTER(bnn_rng),
+                                                        ctypes.c_void_p]),
+    "bnn_sampled_conv_transpose3d_dgrad": (ctypes.c_int, [_c_f32p, _c_f32p, _c_f32p, _c_f32p, _c_f32p, ctypes.c_int64,
+                                                          ctypes.POINTER(bnn_conv3d_nhwc), ctypes.c_int32, ctypes.c_uint32,
+                                                          ctypes.POINTER(bnn_rng), ctypes.c_void_p]),
+    "bnn_sampled_conv_transpose3d_wgrad": (ctypes.c_int, [_c_f32p, _c_f32p, ctypes.c_int64, _c_f32p, _c_f32p, _c_f32p,
+                                                          _c_f32p, ctypes.POINTER(bnn_conv3d_nhwc), ctypes.c_int32,
+                                                          ctypes.c_uint32, ctypes.POINTER(bnn_rng), ctypes.c_void_p]),
+    "bnn_debug_conv_transpose3d_phases": (ctypes.c_int, [ctypes.POINTER(bnn_conv3d_nhwc), ctypes.POINTER(ctypes.c_int32),
+                                                         ctypes.c_int32]),
     "bnn_conv2d_weight_layout": (ctypes.c_int, [_c_f32p, _c_f32p, _c_f32p, _c_f32p, _c_f32p, ctypes.c_int32, ctypes.c_int32,
                                                 ctypes.c_int32, ctypes.c_void_p]),
     "bnn_conv2d_weight_unlayout": (ctypes.c_int, [_c_f32p, _c_f32p, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32,
@@ -838,3 +856,42 @@ def conv_transpose_phases(geom):
             "first_h", "first_w", "in_step_h", "in_step_w")
     return [dict(zip(keys, buf[14 * i:14 * i + 14])) for i in range(min(n, cap))]
 
+
+# ---- 3-d transposed convolution (NDHWC; geometry = the conv view, see bnn_b200.h) -------------------------------------
+def conv3d_geom(B, D, H, W, C, OD, OH, OW, Cout, kernel, stride, padding, dilation):
+    return bnn_conv3d_nhwc(B, D, H, W, C, OD, OH, OW, Cout, *kernel, *stride, *padding, *dilation, 0)
+
+
+def try_sampled_conv_transpose3d_fwd(x, x_sample_stride, mu_w, sigma_w, mu_b, sigma_b, eps_w, eps_b, y, geom, S,
+                                     sample_begin, rng_w, rng_b):
+    """The phase-decomposed gather; False (nothing launched) when the request is outside the kernels' limits."""
+    return _try_call("bnn_sampled_conv_transpose3d_fwd", y.device, _ptr(x), x_sample_stride, _ptr(mu_w), _ptr(sigma_w),
+                     _ptr(mu_b), _ptr(sigma_b), _ptr(eps_w), _ptr(eps_b), _ptr(y), ctypes.byref(geom), S, sample_begin,
+                     ctypes.byref(rng_w), ctypes.byref(rng_b) if rng_b is not None else None, _stream())
+
+
+def sampled_conv_transpose3d_dgrad(dy, mu_w, sigma_w, eps_w, dx, x_sample_stride, geom, S, sample_begin, rng_w):
+    """Raises on refusal: the forward that accepted the request checked the same predicate."""
+    with torch.cuda.device(dx.device):
+        _call("bnn_sampled_conv_transpose3d_dgrad", _ptr(dy), _ptr(mu_w), _ptr(sigma_w), _ptr(eps_w), _ptr(dx),
+              x_sample_stride, ctypes.byref(geom), S, sample_begin, ctypes.byref(rng_w), _stream())
+    _count()
+
+
+def sampled_conv_transpose3d_wgrad(dy, x, x_sample_stride, rho_w, eps_w, dmu_w, drho_w, geom, S, sample_begin, rng_w):
+    with torch.cuda.device(x.device):
+        _call("bnn_sampled_conv_transpose3d_wgrad", _ptr(dy), _ptr(x), x_sample_stride, _ptr(rho_w), _ptr(eps_w),
+              _ptr(dmu_w), _ptr(drho_w), ctypes.byref(geom), S, sample_begin, ctypes.byref(rng_w), _stream())
+    _count()
+
+
+def conv_transpose3d_phases(geom):
+    """Host-side phase plan of bnn_sampled_conv_transpose3d_fwd: one dict per output phase (no device needed)."""
+    cap = 512
+    buf = (ctypes.c_int32 * (21 * cap))()
+    n = lib().bnn_debug_conv_transpose3d_phases(ctypes.byref(geom), buf, cap)
+    if n < 0:
+        _check(-n, "bnn_debug_conv_transpose3d_phases")
+    fields = ("r", "rows", "taps", "last", "tap_step", "first", "in_step")
+    keys = tuple(f"{f}_{a}" for f in fields for a in "dhw")
+    return [dict(zip(keys, buf[21 * i:21 * i + 21])) for i in range(min(n, cap))]

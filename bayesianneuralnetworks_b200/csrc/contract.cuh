@@ -31,10 +31,21 @@ struct View {
   // grid lands at base + img * s_img + i * s_i + j * bs — one output phase of a strided transposed convolution
   int pw = 0, pimg = 0;
   int64_t s_i = 0, s_img = 0;
+  // depth level of the phase view (3-d data-gradient drain only): row m = (img, a, i, j) of an img x (pimg / pplane) x
+  // (pplane / pw) x pw grid lands at base + img * s_img + a * s_a + i * s_i + j * bs
+  int pplane = 0;
+  int64_t s_a = 0;
 };
 __device__ __forceinline__ float* phase_row(const View& v, int m) {
   const int img = m / v.pimg, r = m - img * v.pimg, i = r / v.pw, j = r - i * v.pw;
   return v.base + static_cast<int64_t>(img) * v.s_img + static_cast<int64_t>(i) * v.s_i + static_cast<int64_t>(j) * v.bs;
+}
+// the offset within an image in 32 bits (an image below 2^31 floats, checked by the host)
+__device__ __forceinline__ float* phase_row3(const View& v, int m) {
+  const int img = m / v.pimg, r = m - img * v.pimg, a = r / v.pplane, r2 = r - a * v.pplane, i = r2 / v.pw,
+            j = r2 - i * v.pw;
+  return v.base + static_cast<int64_t>(img) * v.s_img +
+         (a * static_cast<int>(v.s_a) + i * static_cast<int>(v.s_i) + j * static_cast<int>(v.bs));
 }
 __device__ __forceinline__ int64_t view_off(const View& v, int m, int n) {
   if (v.P == 1) return static_cast<int64_t>(m) * v.bs + n;
@@ -141,26 +152,36 @@ int tma_dgrad(bnn_view dy, int64_t dy_sample_stride, const float* mu_w, const fl
 int tma_wgrad(bnn_view dy, int64_t dy_sample_stride, const float* a, int64_t lda, int64_t a_sample_stride,
               const float* rho_w, const float* eps_w, float* dmu_w, float* drho_w, int M, int N, int K, int S,
               uint32_t sample_begin, const bnn_rng* rng_w, cudaStream_t st);
-// implicit-GEMM convolution (NHWC activations through an im2col tensor map, weights [Cout][KH][KW][C])
+// implicit-GEMM convolution (NHWC activations through an im2col tensor map, weights [Cout][KH][KW][C]).  Geometry of
+// the launchers: a 3-d convolution (vol: NDHWC tensors, rank-5 maps, the kMode 3 kernels) or a 2-d one as depth 1
+// (D = OD = KD = sd = dd = 1, pd = 0: rank-4 maps, the kMode 1 kernels)
+struct ConvGeom {
+  bnn_conv3d_nhwc g;
+  bool vol;
+};
+ConvGeom conv_geom_2d(const bnn_conv2d_nhwc& g);
 int tma_conv_fwd(const float* x, int64_t x_sample_stride, const float* mu_w, const float* sigma_w, const float* mu_b,
                  const float* sigma_b, const float* eps_w, const float* eps_b, bnn_view y, int64_t y_sample_stride,
-                 const bnn_conv2d_nhwc* g, int S, uint32_t sample_begin, const bnn_rng* rng_w, const bnn_rng* rng_b,
+                 const ConvGeom& g, int S, uint32_t sample_begin, const bnn_rng* rng_w, const bnn_rng* rng_b,
                  cudaStream_t st);
 // the weight gradient of a conv layer takes (dy, x), that of a transposed conv its conv view's operands (x, dy)
 int tma_conv_wgrad(const float* dy, bool shared_dy, const float* a, bool shared_a, const float* rho_w, const float* eps_w,
-                   float* dmu_w, float* drho_w, const bnn_conv2d_nhwc* g, int S, uint32_t sample_begin,
+                   float* dmu_w, float* drho_w, const ConvGeom& g, int S, uint32_t sample_begin,
                    const bnn_rng* rng_w, cudaStream_t st);
 // transposed-filter gather: the stride-1 conv input gradient (x = dy, sum_samples for a shared input) and the forward of a
 // transposed convolution in its conv view's geometry (see bnn_b200.h; one launch per output phase); input gradient of a
 // transposed convolution = the conv view's forward
 int tma_conv_gather(const float* x, bool shared_x, const float* mu_w, const float* sigma_w, const float* mu_b,
                     const float* sigma_b, const float* eps_w, const float* eps_b, float* y, int64_t y_sample_stride,
-                    bool sum_samples, const bnn_conv2d_nhwc* g, int S, uint32_t sample_begin, const bnn_rng* rng_w,
+                    bool sum_samples, const ConvGeom& g, int S, uint32_t sample_begin, const bnn_rng* rng_w,
                     const bnn_rng* rng_b, cudaStream_t st);
 int tma_conv_transpose_dgrad(const float* dy, const float* mu_w, const float* sigma_w, const float* eps_w, float* dx,
-                             int64_t x_sample_stride, const bnn_conv2d_nhwc* g, int S, uint32_t sample_begin,
+                             int64_t x_sample_stride, const ConvGeom& g, int S, uint32_t sample_begin,
                              const bnn_rng* rng_w, cudaStream_t st);
-int conv_transpose_phases(const bnn_conv2d_nhwc* g, int32_t* out, int max_phases);   // host: the phase plan, 8 ints each
+// host: the phase plan, 7 ints per phase dimension (14 per phase in 2-d, 21 in 3-d)
+int conv_transpose_phases(const ConvGeom& g, int32_t* out, int max_phases);
+// host: geometry part of the 3-d transposed convolution's eligibility (channels, strides, every conv-view and phase corner)
+bool conv_transpose_ok(const ConvGeom& g);
 int tma_selftest(float* max_err_dev, cudaStream_t st);
 int tma_pair_tile_plan(int m_blocks, int S, int slots, int32_t* out7);   // test aid: TilePlan fields {on, n_a, s1, a1, b1, a2, b2}
 int tma_force_variant(int variant);   // test aid: 0 = CTA pair, 1 / 2 / 4 = row blocks per CTA, -1 = cost model (default)

@@ -9,6 +9,9 @@
 //
 // bnn_im2col_nhwc / bnn_col2im_nhwc are the explicit lowering in the same (kh, kw, c) column order, for the requests
 // the TMA path does not take: fp32 (3xTF32) mode and the input gradient of strided layers.
+//
+// The transposed layers (NormalConvTranspose1d / 2d / 3d) run on the same kernels through their conv view; the 3-d entry
+// points (NDHWC tensors, rank-5 im2col maps) check one eligibility predicate for their three passes.
 #include "contract.cuh"
 
 namespace bnn {
@@ -472,7 +475,8 @@ int bnn_sampled_conv2d_fwd(const float* x, int64_t x_sample_stride, const float*
   BNN_REQUIRE(y.P >= 1, BNN_ERR_BAD_ARGUMENT, "bnn_sampled_conv2d_fwd: bad output view");
   rc = check_device();
   if (rc != BNN_OK) return rc;
-  rc = contract::tma_conv_fwd(x, x_sample_stride, mu_w, sigma_w, mu_b, sigma_b, eps_w, eps_b, y, y_sample_stride, g, S,
+  rc = contract::tma_conv_fwd(x, x_sample_stride, mu_w, sigma_w, mu_b, sigma_b, eps_w, eps_b, y, y_sample_stride,
+                              contract::conv_geom_2d(*g), S,
                               sample_begin, rng_w, rng_b, static_cast<cudaStream_t>(stream));
   if (rc == contract::kNotEligible)
     return fail(BNN_ERR_UNSUPPORTED, "bnn_sampled_conv2d_fwd: needs C %% 32 == 0, 16-byte aligned tensors and a filter "
@@ -493,7 +497,7 @@ int bnn_sampled_conv2d_dgrad(const float* dy, const float* mu_w, const float* si
   rc = g->sh != 1 || g->sw != 1
            ? contract::kNotEligible
            : contract::tma_conv_gather(dy, false, mu_w, sigma_w, nullptr, nullptr, eps_w, nullptr, dx, x_sample_stride,
-                                       x_sample_stride == 0, g, S, sample_begin, rng_w, nullptr,
+                                       x_sample_stride == 0, contract::conv_geom_2d(*g), S, sample_begin, rng_w, nullptr,
                                        static_cast<cudaStream_t>(stream));
   if (rc == contract::kNotEligible)
     return fail(BNN_ERR_UNSUPPORTED, "bnn_sampled_conv2d_dgrad: needs stride 1, Cout %% 32 == 0, C %% 4 == 0 and 16-byte "
@@ -510,7 +514,8 @@ int bnn_sampled_conv2d_wgrad(const float* dy, const float* x, int64_t x_sample_s
               "bnn_sampled_conv2d_wgrad: NULL pointer or bad sample count");
   rc = check_device();
   if (rc != BNN_OK) return rc;
-  rc = contract::tma_conv_wgrad(dy, false, x, x_sample_stride == 0, rho_w, eps_w, dmu_w, drho_w, g, S, sample_begin, rng_w,
+  rc = contract::tma_conv_wgrad(dy, false, x, x_sample_stride == 0, rho_w, eps_w, dmu_w, drho_w, contract::conv_geom_2d(*g),
+                                S, sample_begin, rng_w,
                                 static_cast<cudaStream_t>(stream));
   if (rc == contract::kNotEligible)
     return fail(BNN_ERR_UNSUPPORTED, "bnn_sampled_conv2d_wgrad: needs C %% 32 == 0, Cout %% 4 == 0 and 16-byte aligned "
@@ -532,7 +537,8 @@ int bnn_sampled_conv_transpose2d_fwd(const float* x, int64_t x_sample_stride, co
   rc = check_device();
   if (rc != BNN_OK) return rc;
   rc = contract::tma_conv_gather(x, x_sample_stride == 0, mu_w, sigma_w, mu_b, sigma_b, eps_w, eps_b, y,
-                                 static_cast<int64_t>(g->B) * g->H * g->W * g->C, false, g, S, sample_begin, rng_w, rng_b,
+                                 static_cast<int64_t>(g->B) * g->H * g->W * g->C, false, contract::conv_geom_2d(*g), S,
+                                 sample_begin, rng_w, rng_b,
                                  static_cast<cudaStream_t>(stream));
   if (rc == contract::kNotEligible)
     return fail(BNN_ERR_UNSUPPORTED, "bnn_sampled_conv_transpose2d_fwd: needs Cout %% 32 == 0, C %% 4 == 0, stride <= 8, "
@@ -550,7 +556,8 @@ int bnn_sampled_conv_transpose2d_dgrad(const float* dy, const float* mu_w, const
               "bnn_sampled_conv_transpose2d_dgrad: NULL pointer or bad sample count");
   rc = check_device();
   if (rc != BNN_OK) return rc;
-  rc = contract::tma_conv_transpose_dgrad(dy, mu_w, sigma_w, eps_w, dx, x_sample_stride, g, S, sample_begin, rng_w,
+  rc = contract::tma_conv_transpose_dgrad(dy, mu_w, sigma_w, eps_w, dx, x_sample_stride, contract::conv_geom_2d(*g), S,
+                                          sample_begin, rng_w,
                                           static_cast<cudaStream_t>(stream));
   if (rc == contract::kNotEligible)
     return fail(BNN_ERR_UNSUPPORTED, "bnn_sampled_conv_transpose2d_dgrad: needs C %% 32 == 0, Cout %% 4 == 0, 16-byte "
@@ -569,7 +576,8 @@ int bnn_sampled_conv_transpose2d_wgrad(const float* dy, const float* x, int64_t 
   rc = check_device();
   if (rc != BNN_OK) return rc;
   // conv view: the "dY" operand is the transposed input x (shared by the samples when x_sample_stride == 0), A = dy
-  rc = contract::tma_conv_wgrad(x, x_sample_stride == 0, dy, false, rho_w, eps_w, dmu_w, drho_w, g, S, sample_begin, rng_w,
+  rc = contract::tma_conv_wgrad(x, x_sample_stride == 0, dy, false, rho_w, eps_w, dmu_w, drho_w, contract::conv_geom_2d(*g),
+                                S, sample_begin, rng_w,
                                 static_cast<cudaStream_t>(stream));
   if (rc == contract::kNotEligible)
     return fail(BNN_ERR_UNSUPPORTED, "bnn_sampled_conv_transpose2d_wgrad: needs C %% 32 == 0, Cout %% 4 == 0 and 16-byte "
@@ -581,7 +589,102 @@ int bnn_debug_conv_transpose_phases(const bnn_conv2d_nhwc* g, int32_t* out, int3
   const int rc = check_geom(g, "bnn_debug_conv_transpose_phases");
   if (rc != BNN_OK) return -rc;
   if (out == nullptr && max_phases > 0) return -fail(BNN_ERR_BAD_ARGUMENT, "bnn_debug_conv_transpose_phases: NULL output");
-  return contract::conv_transpose_phases(g, out, max_phases);
+  return contract::conv_transpose_phases(contract::conv_geom_2d(*g), out, max_phases);
+}
+
+// ---- 3-d transposed convolution: one eligibility predicate for the three passes (bnn_b200.h)
+namespace {
+int check_geom3d(const bnn_conv3d_nhwc* g, const char* who) {
+  BNN_REQUIRE(g != nullptr, BNN_ERR_BAD_ARGUMENT, "%s: geometry is NULL", who);
+  BNN_REQUIRE(g->B > 0 && g->D > 0 && g->H > 0 && g->W > 0 && g->C > 0 && g->Cout > 0 && g->KD > 0 && g->KH > 0 &&
+                  g->KW > 0 && g->OD > 0 && g->OH > 0 && g->OW > 0 && g->sd > 0 && g->sh > 0 && g->sw > 0 && g->dd > 0 &&
+                  g->dh > 0 && g->dw > 0 && g->pd >= 0 && g->ph >= 0 && g->pw >= 0,
+              BNN_ERR_BAD_ARGUMENT, "%s: bad geometry", who);
+  BNN_REQUIRE(g->OD == (g->D + 2 * g->pd - g->dd * (g->KD - 1) - 1) / g->sd + 1 &&
+                  g->OH == (g->H + 2 * g->ph - g->dh * (g->KH - 1) - 1) / g->sh + 1 &&
+                  g->OW == (g->W + 2 * g->pw - g->dw * (g->KW - 1) - 1) / g->sw + 1,
+              BNN_ERR_BAD_ARGUMENT, "%s: OD / OH / OW do not match the geometry", who);
+  return BNN_OK;
+}
+contract::ConvGeom geom3d(const bnn_conv3d_nhwc* g) {
+  contract::ConvGeom cg{};
+  cg.g = *g;
+  cg.vol = true;
+  return cg;
+}
+// the predicate: channels, strides, every conv-view and phase corner (contract::conv_transpose_ok), alignment
+bool transpose3d_ok(const bnn_conv3d_nhwc* g, std::initializer_list<const void*> tensors, const bnn_rng* rng_w) {
+  for (const void* t : tensors)
+    if (t != nullptr && !aligned16(t)) return false;
+  return g->C % 32 == 0 && rng_w->elem_offset % 4 == 0 && contract::conv_transpose_ok(geom3d(g));
+}
+constexpr const char* kT3dLimits = "needs Cin %% 32 == 0, Cout %% 32 == 0, stride <= 8, 16-byte aligned tensors and every "
+                                   "phase and conv-view corner within the rank-5 im2col descriptor's limits";
+}  // namespace
+
+int bnn_sampled_conv_transpose3d_fwd(const float* x, int64_t x_sample_stride, const float* mu_w, const float* sigma_w,
+                                     const float* mu_b, const float* sigma_b, const float* eps_w, const float* eps_b, float* y,
+                                     const bnn_conv3d_nhwc* g, int32_t S, uint32_t sample_begin, const bnn_rng* rng_w,
+                                     const bnn_rng* rng_b, void* stream) {
+  int rc = check_geom3d(g, "bnn_sampled_conv_transpose3d_fwd");
+  if (rc != BNN_OK) return rc;
+  BNN_REQUIRE(x && mu_w && sigma_w && y && rng_w && S > 0 && S <= 65535, BNN_ERR_BAD_ARGUMENT,
+              "bnn_sampled_conv_transpose3d_fwd: NULL pointer or bad sample count");
+  BNN_REQUIRE((mu_b == nullptr) == (sigma_b == nullptr) && (mu_b == nullptr || rng_b != nullptr), BNN_ERR_BAD_ARGUMENT,
+              "bnn_sampled_conv_transpose3d_fwd: bias needs mu_b, sigma_b and rng_b");
+  if (!transpose3d_ok(g, {x, mu_w, sigma_w, eps_w, y}, rng_w))
+    return fail(BNN_ERR_UNSUPPORTED, "bnn_sampled_conv_transpose3d_fwd: %s", kT3dLimits);
+  rc = check_device();
+  if (rc != BNN_OK) return rc;
+  rc = contract::tma_conv_gather(x, x_sample_stride == 0, mu_w, sigma_w, mu_b, sigma_b, eps_w, eps_b, y,
+                                 static_cast<int64_t>(g->B) * g->D * g->H * g->W * g->C, false, geom3d(g), S, sample_begin,
+                                 rng_w, rng_b, static_cast<cudaStream_t>(stream));
+  if (rc == contract::kNotEligible)
+    return fail(BNN_ERR_UNSUPPORTED, "bnn_sampled_conv_transpose3d_fwd: %s", kT3dLimits);
+  return rc;
+}
+
+int bnn_sampled_conv_transpose3d_dgrad(const float* dy, const float* mu_w, const float* sigma_w, const float* eps_w,
+                                       float* dx, int64_t x_sample_stride, const bnn_conv3d_nhwc* g, int32_t S,
+                                       uint32_t sample_begin, const bnn_rng* rng_w, void* stream) {
+  int rc = check_geom3d(g, "bnn_sampled_conv_transpose3d_dgrad");
+  if (rc != BNN_OK) return rc;
+  BNN_REQUIRE(dy && mu_w && sigma_w && dx && rng_w && S > 0 && S <= 65535, BNN_ERR_BAD_ARGUMENT,
+              "bnn_sampled_conv_transpose3d_dgrad: NULL pointer or bad sample count");
+  if (!transpose3d_ok(g, {dy, mu_w, sigma_w, eps_w, dx}, rng_w))
+    return fail(BNN_ERR_UNSUPPORTED, "bnn_sampled_conv_transpose3d_dgrad: %s", kT3dLimits);
+  rc = check_device();
+  if (rc != BNN_OK) return rc;
+  rc = contract::tma_conv_transpose_dgrad(dy, mu_w, sigma_w, eps_w, dx, x_sample_stride, geom3d(g), S, sample_begin, rng_w,
+                                          static_cast<cudaStream_t>(stream));
+  if (rc == contract::kNotEligible)
+    return fail(BNN_ERR_UNSUPPORTED, "bnn_sampled_conv_transpose3d_dgrad: %s", kT3dLimits);
+  return rc;
+}
+
+int bnn_sampled_conv_transpose3d_wgrad(const float* dy, const float* x, int64_t x_sample_stride, const float* rho_w,
+                                       const float* eps_w, float* dmu_w, float* drho_w, const bnn_conv3d_nhwc* g, int32_t S,
+                                       uint32_t sample_begin, const bnn_rng* rng_w, void* stream) {
+  int rc = check_geom3d(g, "bnn_sampled_conv_transpose3d_wgrad");
+  if (rc != BNN_OK) return rc;
+  BNN_REQUIRE(dy && x && rho_w && dmu_w && drho_w && rng_w && S > 0 && S <= 65535, BNN_ERR_BAD_ARGUMENT,
+              "bnn_sampled_conv_transpose3d_wgrad: NULL pointer or bad sample count");
+  if (!transpose3d_ok(g, {dy, x, rho_w, eps_w, dmu_w, drho_w}, rng_w))
+    return fail(BNN_ERR_UNSUPPORTED, "bnn_sampled_conv_transpose3d_wgrad: %s", kT3dLimits);
+  rc = check_device();
+  if (rc != BNN_OK) return rc;
+  rc = contract::tma_conv_wgrad(x, x_sample_stride == 0, dy, false, rho_w, eps_w, dmu_w, drho_w, geom3d(g), S, sample_begin,
+                                rng_w, static_cast<cudaStream_t>(stream));
+  if (rc == contract::kNotEligible)
+    return fail(BNN_ERR_UNSUPPORTED, "bnn_sampled_conv_transpose3d_wgrad: %s", kT3dLimits);
+  return rc;
+}
+
+int bnn_debug_conv_transpose3d_phases(const bnn_conv3d_nhwc* g, int32_t* out, int32_t max_phases) {
+  const int rc = check_geom3d(g, "bnn_debug_conv_transpose3d_phases");
+  if (rc != BNN_OK) return -rc;
+  if (out == nullptr && max_phases > 0) return -fail(BNN_ERR_BAD_ARGUMENT, "bnn_debug_conv_transpose3d_phases: NULL output");
+  return contract::conv_transpose_phases(geom3d(g), out, max_phases);
 }
 
 }  // extern "C"

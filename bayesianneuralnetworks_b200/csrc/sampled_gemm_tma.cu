@@ -121,26 +121,36 @@ EncodeIm2colFn encode_im2col_fn() {
   return fn;
 }
 
+// Depth: the rank-5 map of an NDHWC tensor [n_imgs][D][H][W][C] (3-d convolutions, vol); without it the rank-4 map.
+struct Im2colDepth {
+  bool vol;
+  int64_t D;
+  int lower, upper, stride;
+};
 int make_im2col_map(CUtensorMap* map, const float* base, int64_t C, int64_t W, int64_t H, int64_t n_imgs, int lower_w,
-                    int lower_h, int upper_w, int upper_h, int stride_w, int stride_h, int box_pixels, bool mn_major) {
+                    int lower_h, int upper_w, int upper_h, int stride_w, int stride_h, int box_pixels, bool mn_major,
+                    const Im2colDepth& dep = Im2colDepth{false, 1, 0, 0, 1}) {
   EncodeIm2colFn fn = encode_im2col_fn();
   if (fn == nullptr) return kNotEligible;
-  const cuuint64_t dims[4] = {static_cast<cuuint64_t>(C), static_cast<cuuint64_t>(W), static_cast<cuuint64_t>(H),
-                              static_cast<cuuint64_t>(n_imgs)};
-  const cuuint64_t strides[3] = {static_cast<cuuint64_t>(C) * 4u, static_cast<cuuint64_t>(W * C) * 4u,
-                                 static_cast<cuuint64_t>(H * W * C) * 4u};
-  const int lower[2] = {lower_w, lower_h}, upper[2] = {upper_w, upper_h};
-  const cuuint32_t estr[4] = {1u, static_cast<cuuint32_t>(stride_w), static_cast<cuuint32_t>(stride_h), 1u};
-  const CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_TFLOAT32, 4, const_cast<float*>(base), dims, strides, lower, upper,
+  const int64_t D = dep.vol ? dep.D : 1;
+  const cuuint32_t rank = dep.vol ? 5u : 4u;
+  const cuuint64_t dims[5] = {static_cast<cuuint64_t>(C), static_cast<cuuint64_t>(W), static_cast<cuuint64_t>(H),
+                              static_cast<cuuint64_t>(dep.vol ? D : n_imgs), static_cast<cuuint64_t>(n_imgs)};
+  const cuuint64_t strides[4] = {static_cast<cuuint64_t>(C) * 4u, static_cast<cuuint64_t>(W * C) * 4u,
+                                 static_cast<cuuint64_t>(H * W * C) * 4u, static_cast<cuuint64_t>(D * H * W * C) * 4u};
+  const int lower[3] = {lower_w, lower_h, dep.lower}, upper[3] = {upper_w, upper_h, dep.upper};
+  const cuuint32_t estr[5] = {1u, static_cast<cuuint32_t>(stride_w), static_cast<cuuint32_t>(stride_h),
+                              dep.vol ? static_cast<cuuint32_t>(dep.stride) : 1u, 1u};
+  const CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_TFLOAT32, rank, const_cast<float*>(base), dims, strides, lower, upper,
                         32u, static_cast<cuuint32_t>(box_pixels), estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                         mn_major ? CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B : CU_TENSOR_MAP_SWIZZLE_128B,
                         CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) return kNotEligible;
   // Known driver issue (CUDA <= 13.1, the workaround CUTLASS applies in cute/atom/copy_traits_sm90_im2col.hpp): for tensors
   // smaller than 128 KiB the encoder sets bit 21 of the descriptor's second word, which makes the copy engine misread the
-  // extent; clear it.
+  // extent; clear it (rank 4 and rank 5 alike).
   int driver = 0;
-  if (cudaDriverGetVersion(&driver) == cudaSuccess && driver <= 13010 && n_imgs * H * W * C * 4 < 131072)
+  if (cudaDriverGetVersion(&driver) == cudaSuccess && driver <= 13010 && n_imgs * D * H * W * C * 4 < 131072)
     reinterpret_cast<uint64_t*>(map)[1] &= ~(1ull << 21);
   return BNN_OK;
 }
@@ -153,7 +163,7 @@ bool tma_ok(const void* base, int64_t ld, int64_t ss) {
 // Implicit-GEMM addressing of the TMA-loaded operand (conv layers): the operand is never an im2col MATRIX, it is the NHWC
 // tensor itself seen through an im2col tensor map; row m of the GEMM is the pixel (img, p, q) of a P = rows x OW grid
 // (output pixels for forward / weight gradient, input pixels for the data gradient), k-block rb is (filter tap, 32
-// channels).  on == 0: plain row-major matrix.
+// channels).  on == 0: plain row-major matrix; 1: 2-d (rank-4 map), 2: 3-d (rank-5 map, kMode 3 kernels).
 struct ConvCoords {
   int on;
   int P, OW;                // pixel grid of the GEMM rows
@@ -169,16 +179,33 @@ struct ConvCoords {
   // wtaps = KH x wKW filter.  Stride 1: every tap (tkh = KH - 1, tdh = 1, ...); one phase of a strided transposed
   // convolution: the taps of that phase only, tdh = sh / gcd(sh, dh) apart
   int wtaps, wKW, tkh, tkw, tdh, tdw;
+  // 3-d convolutions (kMode 3, rank-5 map): row m = (img, d, h, w), HW pixels per depth plane; depth stride, lower corner
+  // and dilation; KH x KW = KHW walked taps per depth plane; data gradient: walked tap (jd, jh, jw) is the weight's tap
+  // (tkd - jd tdd, tkh - jh tdh, tkw - jw tdw) of a filter wKH high
+  int HW, sd, ld, dd, KH, KHW, tkd, tdd, wKH;
 };
 __device__ __forceinline__ int64_t conv_dgrad_tap(const ConvCoords& c, int tapf) {
   const int jh = tapf / c.KW, jw = tapf - jh * c.KW;
   return static_cast<int64_t>((c.tkh - jh * c.tdh) * c.wKW + c.tkw - jw * c.tdw);
+}
+__device__ __forceinline__ int64_t conv_dgrad_tap3d(const ConvCoords& c, int tapf) {
+  const int jd = tapf / c.KHW, r = tapf - jd * c.KHW, jh = r / c.KW, jw = r - jh * c.KW;
+  return static_cast<int64_t>(((c.tkd - jd * c.tdd) * c.wKH + c.tkh - jh * c.tdh) * c.wKW + c.tkw - jw * c.tdw);
 }
 __device__ __forceinline__ void conv_pixel(const ConvCoords& c, int m, int smp, int* w, int* h, int* n) {
   const int img = m / c.P, rem = m - img * c.P;
   const int ph = rem / c.OW, q = rem - ph * c.OW;
   *w = q * c.sw + c.lw;
   *h = ph * c.sh + c.lh;
+  *n = smp * c.imgs + img;
+}
+__device__ __forceinline__ void conv_pixel3d(const ConvCoords& c, int m, int smp, int* w, int* h, int* d, int* n) {
+  const int img = m / c.P, rem = m - img * c.P;
+  const int pd = rem / c.HW, r2 = rem - pd * c.HW;
+  const int ph = r2 / c.OW, q = r2 - ph * c.OW;
+  *w = q * c.sw + c.lw;
+  *h = ph * c.sh + c.lh;
+  *d = pd * c.sd + c.ld;
   *n = smp * c.imgs + img;
 }
 
@@ -315,8 +342,8 @@ __device__ __forceinline__ bool stage_eligible(const View& out, bool vec_out, in
 // m0 .. m0 + 31 of the output, columns col0 .. col0 + cols_here): two tcgen05.ld per round trip, then (+ bias) ->
 // staging -> coalesced stores / adds.
 // kPhase: the output may be a phase view (View::pw; conv data-gradient instantiations only — the others keep the plain
-// row addressing)
-template <bool kBias, bool kPhase = false>
+// row addressing); 2: with the depth level (3-d conv data gradient)
+template <bool kBias, int kPhase = 0>
 __device__ __forceinline__ void drain_block_staged(uint32_t taddr, uint32_t stage, const float* aux, const View& out,
                                                    int m0, int M, int col0, int cols_here, int lane, bool add,
                                                    int h_begin = 0, int h_end = 2) {
@@ -376,7 +403,8 @@ __device__ __forceinline__ void drain_block_staged(uint32_t taddr, uint32_t stag
         if (c4 * 4 < cols_half && m0 + row < M) {
           const float4 q = lds128(stage + row * 272 + c4 * 16);
           float* d = (!kPhase || out.pw == 0) ? dst + static_cast<int64_t>(2 * i) * out.bs + h * 64
-                                              : phase_row(out, m0 + row) + col0 + (c4 << 2) + h * 64;
+                                              : (kPhase == 2 ? phase_row3(out, m0 + row) : phase_row(out, m0 + row)) +
+                                                    col0 + (c4 << 2) + h * 64;
           if (add) red_add4(d, q.x, q.y, q.z, q.w);
           else *reinterpret_cast<float4*>(d) = q;
         }
@@ -403,7 +431,7 @@ __device__ __forceinline__ void drain_block_staged(uint32_t taddr, uint32_t stag
 constexpr int kDrainPerQuad = 4;
 constexpr int kDrainThreads = 4 * kDrainPerQuad * 32;
 constexpr int kDrainBarrier = 2;
-template <bool kBias, bool kPhase = false>
+template <bool kBias, int kPhase = 0>
 __device__ __forceinline__ void drain_tile_shared(uint32_t tmem, uint32_t stage_base, const float* aux, const View& out,
                                                   int row0, int M, int mb_count, int col0, int cols_here, int quad,
                                                   int idx, int lane, bool add) {
@@ -460,6 +488,7 @@ int launch_contract_v(const TmaContractParams& p, dim3 grid, cudaStream_t st) {
 }
 template <bool kPair, int MB, bool kDgrad>
 int launch_contract(const TmaContractParams& p, dim3 grid, cudaStream_t st) {
+  if (p.conv.on == 2) return launch_contract_v<kPair, MB, kDgrad, 3>(p, grid, st);
   if (p.conv.on) return launch_contract_v<kPair, MB, kDgrad, 1>(p, grid, st);
   if (p.rng_w.row_sign != nullptr) return launch_contract_v<kPair, MB, kDgrad, 2>(p, grid, st);
   return launch_contract_v<kPair, MB, kDgrad, 0>(p, grid, st);
@@ -621,7 +650,8 @@ struct TmaWgradParams {
 // n-tiles and ONE k-tile, tcgen05.mma.cta_group::2 computes 256 (n) x 128 (k) per instruction, and each CTA loads its own
 // dY^T tile but only HALF of the shared A^T tile (48 instead of 64 KiB per stage and CTA: the kernel is paced by operand
 // delivery).  TMA bytes and the epilogue's buffer releases land on the leader's barriers; commits are multicast.
-template <bool kPair, bool kSignNoise>
+// kVol: 3-d convolutions (rank-5 im2col map of A)
+template <bool kPair, bool kSignNoise, bool kVol = false>
 __global__ void __launch_bounds__(kWgThreads, 1) wgrad_tma_kernel(const __grid_constant__ TmaWgradParams p) {
   extern __shared__ __align__(16) uint8_t smem_raw[];
   constexpr uint32_t kTmemCols = 512;
@@ -670,13 +700,19 @@ __global__ void __launch_bounds__(kWgThreads, 1) wgrad_tma_kernel(const __grid_c
         // CTA; groups beyond K read channel `chans` (outside the tensor: zeros, the transaction still completes)
         int g_c0[4] = {0, 0, 0, 0};
         uint16_t g_ow[4] = {0, 0, 0, 0}, g_oh[4] = {0, 0, 0, 0};
+        uint16_t g_od[kVol ? 4 : 1] = {0};
         if (p.conv.on) {
 #pragma unroll
           for (int g = 0; g < 4; ++g) {
             const int kc = k0 + g * 32;
             if (kc >= p.K) { g_c0[g] = p.conv.chans; continue; }
-            const int tap = kc / p.conv.chans;
+            int tap = kc / p.conv.chans;
             g_c0[g] = kc - tap * p.conv.chans;
+            if constexpr (kVol) {
+              const int kd = tap / p.conv.KHW;
+              g_od[g] = static_cast<uint16_t>(kd * p.conv.dd);
+              tap -= kd * p.conv.KHW;
+            }
             const int kh = tap / p.conv.KW, kw = tap - kh * p.conv.KW;
             g_ow[g] = static_cast<uint16_t>(kw * p.conv.dw);
             g_oh[g] = static_cast<uint16_t>(kh * p.conv.dh);
@@ -691,14 +727,19 @@ __global__ void __launch_bounds__(kWgThreads, 1) wgrad_tma_kernel(const __grid_c
             const int stage = it % kWgStages;
             mbar_wait(empty + stage, ((it / kWgStages) & 1) ^ 1);
             const uint32_t base = ring + stage * 2 * kWgOperandBytes;
-            int cw = 0, ch = 0, cn = 0;
-            if (p.conv.on) conv_pixel(p.conv, mb * kWgRows, sa, &cw, &ch, &cn);
+            int cw = 0, ch = 0, cn = 0, cd = 0;
+            if constexpr (kVol) conv_pixel3d(p.conv, mb * kWgRows, sa, &cw, &ch, &cd, &cn);
+            else if (p.conv.on) conv_pixel(p.conv, mb * kWgRows, sa, &cw, &ch, &cn);
+            (void)cd;
             if (!kPair) {
               mbar_arrive_expect_tx(full + stage, 2 * kWgOperandBytes);
 #pragma unroll
               for (int g = 0; g < 4; ++g) {
                 tma_load_3d(base + g * kWgLbo, &p.map_dy, n0 + g * 32, mb * kWgRows, sd, full + stage);
-                if (!p.conv.on) {
+                if constexpr (kVol) {
+                  tma_load_im2col_5d(base + kWgOperandBytes + g * kWgLbo, &p.map_a, g_c0[g], cw, ch, cd, cn, g_ow[g], g_oh[g],
+                                     g_od[g], full + stage);
+                } else if (!p.conv.on) {
                   tma_load_3d(base + kWgOperandBytes + g * kWgLbo, &p.map_a, k0 + g * 32, mb * kWgRows, sa, full + stage);
                 } else {
                   tma_load_im2col_4d(base + kWgOperandBytes + g * kWgLbo, &p.map_a, g_c0[g], cw, ch, cn, g_ow[g], g_oh[g],
@@ -714,7 +755,11 @@ __global__ void __launch_bounds__(kWgThreads, 1) wgrad_tma_kernel(const __grid_c
 #pragma unroll
               for (int g = 0; g < 2; ++g) {     // this CTA's half (64 columns) of the shared A^T tile
                 const int kc = k0 + static_cast<int>(rank) * 64 + g * 32;
-                if (!p.conv.on) {
+                if constexpr (kVol) {
+                  const int gi = static_cast<int>(rank) * 2 + g;
+                  tma_load_im2col_5d_pair(base + kWgOperandBytes + g * kWgLbo, &p.map_a, g_c0[gi], cw, ch, cd, cn, g_ow[gi],
+                                          g_oh[gi], g_od[gi], lead_full);
+                } else if (!p.conv.on) {
                   tma_load_3d_pair(base + kWgOperandBytes + g * kWgLbo, &p.map_a, kc, mb * kWgRows, sa, lead_full);
                 } else {
                   const int gi = static_cast<int>(rank) * 2 + g;
@@ -986,12 +1031,14 @@ int wgrad_plan_and_launch(TmaWgradParams& p, int M, int N, int K, int S, cudaStr
   p.chunk_blocks = best_cb;
   p.n_chunks = best_n;
   const int groups = static_cast<int>((static_cast<int64_t>(S) * best_n + best_per - 1) / best_per);
-  static SmemOptIn opt_in[4];
-  const bool signs = p.rng_w.row_sign != nullptr;
+  static SmemOptIn opt_in[6];
+  const bool signs = p.rng_w.row_sign != nullptr, vol = p.conv.on == 2;
   rc = allow_dynamic_smem(wgrad_tma_kernel<false, false>, kWgradSmem, &opt_in[0]);
   if (rc == BNN_OK) rc = allow_dynamic_smem(wgrad_tma_kernel<true, false>, kWgradSmem, &opt_in[1]);
   if (rc == BNN_OK) rc = allow_dynamic_smem(wgrad_tma_kernel<false, true>, kWgradSmem, &opt_in[2]);
   if (rc == BNN_OK) rc = allow_dynamic_smem(wgrad_tma_kernel<true, true>, kWgradSmem, &opt_in[3]);
+  if (rc == BNN_OK) rc = allow_dynamic_smem(wgrad_tma_kernel<false, false, true>, kWgradSmem, &opt_in[4]);
+  if (rc == BNN_OK) rc = allow_dynamic_smem(wgrad_tma_kernel<true, false, true>, kWgradSmem, &opt_in[5]);
   if (rc != BNN_OK) return rc;
   const int n_tiles = (N + 127) / 128, k_tiles = (K + 127) / 128;
   if (n_tiles >= 2 && static_cast<int64_t>(tiles) * groups >= 2 * sm_count()) {
@@ -1006,10 +1053,12 @@ int wgrad_plan_and_launch(TmaWgradParams& p, int M, int N, int K, int S, cudaStr
     attr.val.clusterDim.x = 2; attr.val.clusterDim.y = 1; attr.val.clusterDim.z = 1;
     cfg.attrs = &attr;
     cfg.numAttrs = 1;
-    if (signs) BNN_CUDA_OK(cudaLaunchKernelEx(&cfg, wgrad_tma_kernel<true, true>, p));
+    if (vol) BNN_CUDA_OK(cudaLaunchKernelEx(&cfg, wgrad_tma_kernel<true, false, true>, p));
+    else if (signs) BNN_CUDA_OK(cudaLaunchKernelEx(&cfg, wgrad_tma_kernel<true, true>, p));
     else BNN_CUDA_OK(cudaLaunchKernelEx(&cfg, wgrad_tma_kernel<true, false>, p));
   } else {
-    if (signs) wgrad_tma_kernel<false, true><<<dim3(n_tiles, k_tiles, groups), kWgThreads, kWgradSmem, st>>>(p);
+    if (vol) wgrad_tma_kernel<false, false, true><<<dim3(n_tiles, k_tiles, groups), kWgThreads, kWgradSmem, st>>>(p);
+    else if (signs) wgrad_tma_kernel<false, true><<<dim3(n_tiles, k_tiles, groups), kWgThreads, kWgradSmem, st>>>(p);
     else wgrad_tma_kernel<false, false><<<dim3(n_tiles, k_tiles, groups), kWgThreads, kWgradSmem, st>>>(p);
   }
   BNN_CUDA_OK(cudaGetLastError());
@@ -1040,41 +1089,68 @@ int tma_wgrad(bnn_view dy, int64_t dy_sample_stride, const float* a, int64_t lda
 // ---------------------------------------------------------------------------------------------- implicit-GEMM convolution
 // The same kernels with the activation operand addressed through an im2col tensor map over the NHWC tensor: no im2col
 // matrix exists.  Weights are [Cout][KH][KW][C] (k = (kh, kw, c), c fastest), so a 32-wide k-block is one filter tap and
-// 32 consecutive channels — C % 32 == 0 is the eligibility condition.
+// 32 consecutive channels — C % 32 == 0 is the eligibility condition.  3-d convolutions (ConvGeom::vol) take the same
+// path with NDHWC tensors, [Cout][KD][KH][KW][C] weights, rank-5 maps and the kMode 3 kernels.
 namespace {
-ConvCoords conv_coords_fwd(const bnn_conv2d_nhwc& g) {
+// im2col descriptor limits (cuTensorMapEncodeIm2col): box corners within [-128, 127] at rank 4 and [-16, 15] at rank 5;
+// the copy's tap offsets address the box, so a filter extent (k - 1) d must stay below its span (256 / 32)
+bool corner_ok(int v, bool vol) { return vol ? (v >= -16 && v <= 15) : (v >= -128 && v <= 127); }
+bool extent_ok(int e, bool vol) { return e < (vol ? 32 : 256); }
+
+ConvCoords conv_coords_fwd(const ConvGeom& cg) {
+  const bnn_conv3d_nhwc& g = cg.g;
   ConvCoords c{};
-  c.on = 1; c.P = g.OH * g.OW; c.OW = g.OW; c.imgs = g.B;
+  c.on = cg.vol ? 2 : 1; c.P = g.OD * g.OH * g.OW; c.OW = g.OW; c.imgs = g.B;
   c.sh = g.sh; c.sw = g.sw; c.lh = -g.ph; c.lw = -g.pw; c.dh = g.dh; c.dw = g.dw;
-  c.KW = g.KW; c.taps = g.KH * g.KW; c.cblocks = g.C / kBK; c.w_rows = g.Cout; c.chans = g.C;
+  c.KW = g.KW; c.taps = g.KD * g.KH * g.KW; c.cblocks = g.C / kBK; c.w_rows = g.Cout; c.chans = g.C;
+  c.HW = g.OH * g.OW; c.sd = g.sd; c.ld = -g.pd; c.dd = g.dd; c.KH = g.KH; c.KHW = g.KH * g.KW;
   return c;
 }
-bool conv_ok(const bnn_conv2d_nhwc& g) {
-  const int lo_h = -g.ph, lo_w = -g.pw, up_h = g.ph - (g.KH - 1) * g.dh, up_w = g.pw - (g.KW - 1) * g.dw;
-  return g.C % kBK == 0 && lo_h >= -128 && lo_w >= -128 && up_h >= -128 && up_w >= -128 && up_h <= 127 && up_w <= 127 &&
-         (g.KH - 1) * g.dh < 256 && (g.KW - 1) * g.dw < 256 && g.sh >= 1 && g.sw >= 1 && g.sh <= 8 && g.sw <= 8;
+bool conv_ok(const ConvGeom& cg) {
+  const bnn_conv3d_nhwc& g = cg.g;
+  auto dim_ok = [&](int pad, int k, int d, int s) {
+    return corner_ok(-pad, cg.vol) && corner_ok(pad - (k - 1) * d, cg.vol) && extent_ok((k - 1) * d, cg.vol) && s >= 1 &&
+           s <= 8;
+  };
+  return g.C % kBK == 0 && dim_ok(g.ph, g.KH, g.dh, g.sh) && dim_ok(g.pw, g.KW, g.dw, g.sw) &&
+         (!cg.vol || dim_ok(g.pd, g.KD, g.dd, g.sd));
+}
+Im2colDepth depth_fwd(const ConvGeom& cg) {
+  const bnn_conv3d_nhwc& g = cg.g;
+  return Im2colDepth{cg.vol, g.D, -g.pd, g.pd - (g.KD - 1) * g.dd, g.sd};
 }
 }  // namespace
+
+ConvGeom conv_geom_2d(const bnn_conv2d_nhwc& g) {
+  ConvGeom cg{};
+  cg.vol = false;
+  cg.g = bnn_conv3d_nhwc{g.B, 1, g.H, g.W, g.C, 1, g.OH, g.OW, g.Cout, 1, g.KH, g.KW, 1, g.sh, g.sw, 0, g.ph, g.pw,
+                         1, g.dh, g.dw, 0};
+  return cg;
+}
 
 namespace {
 // sum_samples: every sample reads its own x and the S results are summed into one y (the input gradient of a transposed
 // convolution with shared input); else x_sample_stride == 0 means all samples share x
 int conv_fwd_launch(const float* x, int64_t x_sample_stride, const float* mu_w, const float* sigma_w, const float* mu_b,
                     const float* sigma_b, const float* eps_w, const float* eps_b, bnn_view y, int64_t y_sample_stride,
-                    const bnn_conv2d_nhwc* g, int S, uint32_t sample_begin, const bnn_rng* rng_w, const bnn_rng* rng_b,
+                    const ConvGeom& cg, int S, uint32_t sample_begin, const bnn_rng* rng_w, const bnn_rng* rng_b,
                     bool sum_samples, cudaStream_t st) {
+  const bnn_conv3d_nhwc* g = &cg.g;
   const bool shared = x_sample_stride == 0 && !sum_samples;
-  if (!conv_ok(*g) || !aligned16(x) || rng_w->elem_offset % 4 != 0 || !aligned16(mu_w) || !aligned16(sigma_w) ||
+  if (!conv_ok(cg) || !aligned16(x) || rng_w->elem_offset % 4 != 0 || !aligned16(mu_w) || !aligned16(sigma_w) ||
       (eps_w != nullptr && !aligned16(eps_w)))
     return kNotEligible;
   TmaContractParams p{};
   int rc = make_im2col_map(&p.map_l, x, g->C, g->W, g->H, static_cast<int64_t>(shared ? 1 : S) * g->B, -g->pw, -g->ph,
-                           g->pw - (g->KW - 1) * g->dw, g->ph - (g->KH - 1) * g->dh, g->sw, g->sh, 128, false);
+                           g->pw - (g->KW - 1) * g->dw, g->ph - (g->KH - 1) * g->dh, g->sw, g->sh, 128, false,
+                           depth_fwd(cg));
   if (rc != BNN_OK) return rc;
-  p.conv = conv_coords_fwd(*g);
+  p.conv = conv_coords_fwd(cg);
   p.out.base = y.base; p.out.bs = y.batch_stride; p.out.P = y.P; p.out_sample_stride = y_sample_stride;
   p.mu_w = mu_w; p.sigma_w = sigma_w; p.eps_w = eps_w; p.mu_b = mu_b; p.sigma_b = sigma_b; p.eps_b = eps_b;
-  p.M = g->B * g->OH * g->OW; p.N = g->Cout; p.K = g->KH * g->KW * g->C; p.S = S; p.sample_begin = sample_begin;
+  p.M = g->B * g->OD * g->OH * g->OW; p.N = g->Cout; p.K = g->KD * g->KH * g->KW * g->C; p.S = S;
+  p.sample_begin = sample_begin;
   p.w_numel = static_cast<int64_t>(p.N) * p.K;
   p.rng_w = *rng_w; p.rng_b = rng_b ? *rng_b : *rng_w;
   p.shared_l = shared ? 1 : 0;
@@ -1089,7 +1165,7 @@ int conv_fwd_launch(const float* x, int64_t x_sample_stride, const float* mu_w, 
 
 int tma_conv_fwd(const float* x, int64_t x_sample_stride, const float* mu_w, const float* sigma_w, const float* mu_b,
                  const float* sigma_b, const float* eps_w, const float* eps_b, bnn_view y, int64_t y_sample_stride,
-                 const bnn_conv2d_nhwc* g, int S, uint32_t sample_begin, const bnn_rng* rng_w, const bnn_rng* rng_b,
+                 const ConvGeom& g, int S, uint32_t sample_begin, const bnn_rng* rng_w, const bnn_rng* rng_b,
                  cudaStream_t st) {
   return conv_fwd_launch(x, x_sample_stride, mu_w, sigma_w, mu_b, sigma_b, eps_w, eps_b, y, y_sample_stride, g, S,
                          sample_begin, rng_w, rng_b, false, st);
@@ -1099,19 +1175,21 @@ int tma_conv_fwd(const float* x, int64_t x_sample_stride, const float* mu_w, con
 // [S or 1][B][H][W][C] seen through the im2col map (map_a).  A convolution passes (dy, x), shared_a when all samples
 // share x; a transposed convolution passes its conv view's operands (x, dy), shared_dy when all samples share x.
 int tma_conv_wgrad(const float* dy, bool shared_dy, const float* a, bool shared_a, const float* rho_w, const float* eps_w,
-                   float* dmu_w, float* drho_w, const bnn_conv2d_nhwc* g, int S, uint32_t sample_begin,
+                   float* dmu_w, float* drho_w, const ConvGeom& cg, int S, uint32_t sample_begin,
                    const bnn_rng* rng_w, cudaStream_t st) {
-  const int M = g->B * g->OH * g->OW, N = g->Cout, K = g->KH * g->KW * g->C;
-  if (!conv_ok(*g) || N % 4 != 0 || !aligned16(dy) || !aligned16(a) || rng_w->elem_offset % 4 != 0 || !aligned16(rho_w) ||
+  const bnn_conv3d_nhwc* g = &cg.g;
+  const int M = g->B * g->OD * g->OH * g->OW, N = g->Cout, K = g->KD * g->KH * g->KW * g->C;
+  if (!conv_ok(cg) || N % 4 != 0 || !aligned16(dy) || !aligned16(a) || rng_w->elem_offset % 4 != 0 || !aligned16(rho_w) ||
       !aligned16(dmu_w) || !aligned16(drho_w) || (eps_w != nullptr && !aligned16(eps_w)))
     return kNotEligible;
   TmaWgradParams p{};
   int rc = make_map(&p.map_dy, dy, N, M, shared_dy ? 1 : S, N, static_cast<int64_t>(M) * N, kWgRows, true);
   if (rc != BNN_OK) return rc;
   rc = make_im2col_map(&p.map_a, a, g->C, g->W, g->H, static_cast<int64_t>(shared_a ? 1 : S) * g->B, -g->pw, -g->ph,
-                       g->pw - (g->KW - 1) * g->dw, g->ph - (g->KH - 1) * g->dh, g->sw, g->sh, kWgRows, true);
+                       g->pw - (g->KW - 1) * g->dw, g->ph - (g->KH - 1) * g->dh, g->sw, g->sh, kWgRows, true,
+                       depth_fwd(cg));
   if (rc != BNN_OK) return rc;
-  p.conv = conv_coords_fwd(*g);
+  p.conv = conv_coords_fwd(cg);
   p.rho_w = rho_w; p.eps_w = eps_w; p.dmu_w = dmu_w; p.drho_w = drho_w;
   p.M = M; p.N = N; p.K = K; p.S = S; p.sample_begin = sample_begin;
   p.rng_w = *rng_w;
@@ -1133,7 +1211,8 @@ int tma_conv_wgrad(const float* dy, bool shared_dy, const float* a, bool shared_
 // its own taps (tdh = sh / gcd(sh, dh) apart, dh / gcd(sh, dh) input rows apart) and its own im2col corner.  One launch of
 // the data-gradient kernel per phase walks exactly that phase's taps x 32-channel blocks (no MMA on inserted zeros) and
 // writes its rows through a phase view; phases without a tap get the bias alone.  At stride 1 there is one phase with
-// every tap: the conv input gradient above, written through the plain row view.
+// every tap: the conv input gradient above, written through the plain row view.  A 3-d transposed convolution adds the
+// depth as a third phase dimension (sd x sh x sw phases) and a depth level to the phase view.
 namespace {
 struct PhaseDim {
   int r, rows;              // phase offset, output rows of the phase
@@ -1157,16 +1236,45 @@ PhaseDim phase_dim(int r, int n_out, int s, int pad, int d, int k) {
   return pd;
 }
 
-__global__ void phase_bias_kernel(float* y, int64_t ss, int64_t s_img, int64_t s_i, int64_t s_j, int S, int B, int rows,
-                                  int cols, int C, const float* mu_b, const float* sigma_b, const float* eps_b,
-                                  uint32_t sample_begin, bnn_rng rng_b) {
-  const int64_t total = static_cast<int64_t>(S) * B * rows * cols * C;
+// the phases of a request, depth-major: (d, h, w) phase dimensions; a 2-d request has one depth phase of one row
+struct Phase {
+  PhaseDim d, h, w;
+};
+template <class F>
+void for_each_phase(const ConvGeom& cg, F&& f) {
+  const bnn_conv3d_nhwc& g = cg.g;
+  const int ph_d = g.sd < g.D ? g.sd : g.D, ph_h = g.sh < g.H ? g.sh : g.H, ph_w = g.sw < g.W ? g.sw : g.W;
+  for (int rd = 0; rd < ph_d; ++rd)
+    for (int rh = 0; rh < ph_h; ++rh)
+      for (int rw = 0; rw < ph_w; ++rw)
+        f(Phase{phase_dim(rd, g.D, g.sd, g.pd, g.dd, g.KD), phase_dim(rh, g.H, g.sh, g.ph, g.dh, g.KH),
+                phase_dim(rw, g.W, g.sw, g.pw, g.dw, g.KW)});
+}
+// every phase's corners and tap offsets within the im2col descriptor's range
+bool phases_ok(const ConvGeom& cg) {
+  const bnn_conv3d_nhwc& g = cg.g;
+  bool ok = true;
+  auto dim_ok = [&](const PhaseDim& a, int n_in) {
+    return corner_ok(a.lo, cg.vol) && corner_ok(a.lo + a.rows - n_in, cg.vol) && extent_ok((a.taps - 1) * a.dstep, cg.vol);
+  };
+  for_each_phase(cg, [&](const Phase& ph) {
+    if (ph.d.taps == 0 || ph.h.taps == 0 || ph.w.taps == 0) return;
+    ok = ok && dim_ok(ph.h, g.OH) && dim_ok(ph.w, g.OW) && (!cg.vol || dim_ok(ph.d, g.OD));
+  });
+  return ok;
+}
+
+__global__ void phase_bias_kernel(float* y, int64_t ss, int64_t s_img, int64_t s_a, int64_t s_i, int64_t s_j, int S, int B,
+                                  int planes, int rows, int cols, int C, const float* mu_b, const float* sigma_b,
+                                  const float* eps_b, uint32_t sample_begin, bnn_rng rng_b) {
+  const int64_t total = static_cast<int64_t>(S) * B * planes * rows * cols * C;
   for (int64_t t = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; t < total;
        t += static_cast<int64_t>(gridDim.x) * blockDim.x) {
     int64_t q = t;
     const int c = static_cast<int>(q % C); q /= C;
     const int j = static_cast<int>(q % cols); q /= cols;
     const int i = static_cast<int>(q % rows); q /= rows;
+    const int a = static_cast<int>(q % planes); q /= planes;
     const int img = static_cast<int>(q % B);
     const int s = static_cast<int>(q / B);
     float b = 0.f;
@@ -1175,102 +1283,110 @@ __global__ void phase_bias_kernel(float* y, int64_t ss, int64_t s_img, int64_t s
                             : eps1(resolve_rng(rng_b), sample_begin + s, static_cast<uint64_t>(c));
       b = fmaf(__ldg(sigma_b + c), e, __ldg(mu_b + c));
     }
-    y[s * ss + img * s_img + i * s_i + j * s_j + c] = b;
+    y[s * ss + img * s_img + a * s_a + i * s_i + j * s_j + c] = b;
   }
 }
 }  // namespace
 
-int conv_transpose_phases(const bnn_conv2d_nhwc* g, int32_t* out, int max_phases) {
-  const int ph_h = g->sh < g->H ? g->sh : g->H, ph_w = g->sw < g->W ? g->sw : g->W;
+int conv_transpose_phases(const ConvGeom& cg, int32_t* out, int max_phases) {
+  const int per = cg.vol ? 21 : 14;
   int n = 0;
-  for (int rh = 0; rh < ph_h; ++rh)
-    for (int rw = 0; rw < ph_w; ++rw, ++n) {
-      if (n >= max_phases) continue;
-      const PhaseDim a = phase_dim(rh, g->H, g->sh, g->ph, g->dh, g->KH);
-      const PhaseDim b = phase_dim(rw, g->W, g->sw, g->pw, g->dw, g->KW);
-      const int32_t v[14] = {a.r, b.r, a.rows, b.rows, a.taps, b.taps, a.tlast, b.tlast, a.tstep, b.tstep, a.lo, b.lo,
-                             a.dstep, b.dstep};
-      for (int i = 0; i < 14; ++i) out[14 * n + i] = v[i];
+  for_each_phase(cg, [&](const Phase& ph) {
+    if (n < max_phases) {
+      int32_t* o = out + per * n;
+      const PhaseDim* dims[3] = {&ph.d, &ph.h, &ph.w};
+      const int first = cg.vol ? 0 : 1, nd = 3 - first;
+      for (int k = 0; k < nd; ++k) {
+        const PhaseDim& a = *dims[first + k];
+        const int32_t v[7] = {a.r, a.rows, a.taps, a.tlast, a.tstep, a.lo, a.dstep};
+        for (int f = 0; f < 7; ++f) o[f * nd + k] = v[f];
+      }
     }
+    ++n;
+  });
   return n;
+}
+
+bool conv_transpose_ok(const ConvGeom& cg) {
+  const bnn_conv3d_nhwc& g = cg.g;
+  // the 3-d phase view addresses within an output image in 32 bits
+  return g.Cout % kBK == 0 && static_cast<int64_t>(g.D) * g.H * g.W * g.C < (int64_t(1) << 31) && conv_ok(cg) &&
+         phases_ok(cg);
 }
 
 // x: the gathered NHWC tensor [S or 1][B][OH][OW][Cout] (conv view), shared_x: all samples read sample 0 of x; y: the
 // NHWC output [S][B][H][W][C] with the optional sampled bias, or with sum_samples one output summed over the samples
 int tma_conv_gather(const float* x, bool shared_x, const float* mu_w, const float* sigma_w, const float* mu_b,
                     const float* sigma_b, const float* eps_w, const float* eps_b, float* y, int64_t y_sample_stride,
-                    bool sum_samples, const bnn_conv2d_nhwc* g, int S, uint32_t sample_begin, const bnn_rng* rng_w,
+                    bool sum_samples, const ConvGeom& cg, int S, uint32_t sample_begin, const bnn_rng* rng_w,
                     const bnn_rng* rng_b, cudaStream_t st) {
+  const bnn_conv3d_nhwc* g = &cg.g;
   // conv view: C = gathered output channels (the drained columns), Cout = channels of x (reduction)
-  if (g->Cout % kBK != 0 || g->C % 4 != 0 || g->sh > 8 || g->sw > 8 || !aligned16(x) || !aligned16(y) ||
+  if (g->Cout % kBK != 0 || g->C % 4 != 0 || g->sh > 8 || g->sw > 8 || g->sd > 8 || !aligned16(x) || !aligned16(y) ||
       rng_w->elem_offset % 4 != 0 || !aligned16(mu_w) || !aligned16(sigma_w) || (eps_w != nullptr && !aligned16(eps_w)))
     return kNotEligible;
-  const int ph_h = g->sh < g->H ? g->sh : g->H, ph_w = g->sw < g->W ? g->sw : g->W;
-  // every phase's corners and tap offsets within the im2col descriptor's range, checked before anything is launched
-  for (int rh = 0; rh < ph_h; ++rh)
-    for (int rw = 0; rw < ph_w; ++rw) {
-      const PhaseDim a = phase_dim(rh, g->H, g->sh, g->ph, g->dh, g->KH);
-      const PhaseDim b = phase_dim(rw, g->W, g->sw, g->pw, g->dw, g->KW);
-      if (a.taps == 0 || b.taps == 0) continue;
-      const int up_h = a.lo + a.rows - g->OH, up_w = b.lo + b.rows - g->OW;
-      if (a.lo < -128 || a.lo > 127 || b.lo < -128 || b.lo > 127 || up_h < -128 || up_h > 127 || up_w < -128 ||
-          up_w > 127 || (a.taps - 1) * a.dstep >= 256 || (b.taps - 1) * b.dstep >= 256)
-        return kNotEligible;
+  // checked for every phase before anything is launched
+  if (!phases_ok(cg)) return kNotEligible;
+  const bool phased = g->sh != 1 || g->sw != 1 || g->sd != 1;
+  const int64_t C = g->C, img_y = static_cast<int64_t>(g->D) * g->H * g->W * C;
+  int rc = BNN_OK;
+  for_each_phase(cg, [&](const Phase& ph) {
+    if (rc != BNN_OK) return;
+    const PhaseDim &e = ph.d, &a = ph.h, &b = ph.w;
+    float* base = y + ((static_cast<int64_t>(e.r) * g->H + a.r) * g->W + b.r) * C;
+    if (e.taps == 0 || a.taps == 0 || b.taps == 0) {
+      const int64_t total = static_cast<int64_t>(S) * g->B * e.rows * a.rows * b.rows * C;
+      const int blocks = static_cast<int>(std::min<int64_t>((total + 255) / 256, 4 * sm_count()));
+      phase_bias_kernel<<<blocks, 256, 0, st>>>(base, y_sample_stride, img_y, g->sd * g->H * g->W * C, g->sh * g->W * C,
+                                                g->sw * C, S, g->B, e.rows, a.rows, b.rows, g->C, mu_b, sigma_b, eps_b,
+                                                sample_begin, rng_b ? *rng_b : *rng_w);
+      const cudaError_t err = cudaGetLastError();
+      if (err != cudaSuccess) rc = fail(BNN_ERR_CUDA, "phase_bias_kernel: %s", cudaGetErrorString(err));
+      return;
     }
-  const bool phased = g->sh != 1 || g->sw != 1;
-  const int64_t C = g->C, img_y = static_cast<int64_t>(g->H) * g->W * C;
-  for (int rh = 0; rh < ph_h; ++rh)
-    for (int rw = 0; rw < ph_w; ++rw) {
-      const PhaseDim a = phase_dim(rh, g->H, g->sh, g->ph, g->dh, g->KH);
-      const PhaseDim b = phase_dim(rw, g->W, g->sw, g->pw, g->dw, g->KW);
-      float* base = y + (static_cast<int64_t>(rh) * g->W + rw) * C;
-      if (a.taps == 0 || b.taps == 0) {
-        const int64_t total = static_cast<int64_t>(S) * g->B * a.rows * b.rows * C;
-        const int blocks = static_cast<int>(std::min<int64_t>((total + 255) / 256, 4 * sm_count()));
-        phase_bias_kernel<<<blocks, 256, 0, st>>>(base, y_sample_stride, img_y, g->sh * g->W * C, g->sw * C, S, g->B,
-                                                  a.rows, b.rows, g->C, mu_b, sigma_b, eps_b, sample_begin,
-                                                  rng_b ? *rng_b : *rng_w);
-        BNN_CUDA_OK(cudaGetLastError());
-        continue;
-      }
-      TmaContractParams p{};
-      const int up_h = a.lo + a.rows - g->OH, up_w = b.lo + b.rows - g->OW;
-      int rc = make_im2col_map(&p.map_l, x, g->Cout, g->OW, g->OH, static_cast<int64_t>(shared_x ? 1 : S) * g->B, b.lo,
-                               a.lo, up_w, up_h, 1, 1, 128, false);
-      if (rc != BNN_OK) return rc;
-      ConvCoords c{};
-      c.on = 1; c.P = a.rows * b.rows; c.OW = b.rows; c.imgs = g->B; c.sh = 1; c.sw = 1; c.lh = a.lo; c.lw = b.lo;
-      c.dh = a.dstep; c.dw = b.dstep; c.KW = b.taps; c.taps = a.taps * b.taps; c.cblocks = g->Cout / kBK;
-      c.w_rows = g->Cout; c.chans = g->Cout;
-      c.wtaps = g->KH * g->KW; c.wKW = g->KW; c.tkh = a.tlast; c.tkw = b.tlast; c.tdh = a.tstep; c.tdw = b.tstep;
-      p.conv = c;
-      p.out.base = base; p.out.bs = g->sw * C; p.out.P = 1;
-      if (phased) { p.out.pw = b.rows; p.out.pimg = a.rows * b.rows; p.out.s_i = g->sh * g->W * C; p.out.s_img = img_y; }
-      p.out_sample_stride = y_sample_stride;
-      p.mu_w = mu_w; p.sigma_w = sigma_w; p.eps_w = eps_w; p.mu_b = mu_b; p.sigma_b = sigma_b; p.eps_b = eps_b;
-      p.M = g->B * a.rows * b.rows; p.N = c.taps * g->Cout; p.K = g->C; p.S = S; p.sample_begin = sample_begin;
-      p.w_numel = static_cast<int64_t>(g->Cout) * c.wtaps * g->C;
-      p.rng_w = *rng_w; p.rng_b = rng_b ? *rng_b : *rng_w;
-      p.shared_l = shared_x ? 1 : 0;
-      p.sum_samples = sum_samples ? 1 : 0;
-      // C % 4 == 0: with a 4-aligned sample stride every CTA takes the staged drain, the only one with the phase view
-      p.vec_out = (y_sample_stride % 4 == 0);
-      rc = dispatch_tma_contract<true>(p, p.K, st);
-      if (rc != BNN_OK) return rc;
+    TmaContractParams p{};
+    const int up_h = a.lo + a.rows - g->OH, up_w = b.lo + b.rows - g->OW;
+    rc = make_im2col_map(&p.map_l, x, g->Cout, g->OW, g->OH, static_cast<int64_t>(shared_x ? 1 : S) * g->B, b.lo, a.lo,
+                         up_w, up_h, 1, 1, 128, false, Im2colDepth{cg.vol, g->OD, e.lo, e.lo + e.rows - g->OD, 1});
+    if (rc != BNN_OK) return;
+    ConvCoords c{};
+    c.on = cg.vol ? 2 : 1; c.P = e.rows * a.rows * b.rows; c.OW = b.rows; c.imgs = g->B; c.sh = 1; c.sw = 1;
+    c.lh = a.lo; c.lw = b.lo; c.dh = a.dstep; c.dw = b.dstep; c.KW = b.taps; c.taps = e.taps * a.taps * b.taps;
+    c.cblocks = g->Cout / kBK; c.w_rows = g->Cout; c.chans = g->Cout;
+    c.wtaps = g->KD * g->KH * g->KW; c.wKW = g->KW; c.tkh = a.tlast; c.tkw = b.tlast; c.tdh = a.tstep; c.tdw = b.tstep;
+    c.HW = a.rows * b.rows; c.sd = 1; c.ld = e.lo; c.dd = e.dstep; c.KH = a.taps; c.KHW = a.taps * b.taps;
+    c.tkd = e.tlast; c.tdd = e.tstep; c.wKH = g->KH;
+    p.conv = c;
+    p.out.base = base; p.out.bs = g->sw * C; p.out.P = 1;
+    if (phased) {
+      p.out.pw = b.rows; p.out.pimg = c.P; p.out.s_i = g->sh * g->W * C; p.out.s_img = img_y;
+      p.out.pplane = a.rows * b.rows; p.out.s_a = static_cast<int64_t>(g->sd) * g->H * g->W * C;
     }
-  return BNN_OK;
+    p.out_sample_stride = y_sample_stride;
+    p.mu_w = mu_w; p.sigma_w = sigma_w; p.eps_w = eps_w; p.mu_b = mu_b; p.sigma_b = sigma_b; p.eps_b = eps_b;
+    p.M = g->B * c.P; p.N = c.taps * g->Cout; p.K = g->C; p.S = S; p.sample_begin = sample_begin;
+    p.w_numel = static_cast<int64_t>(g->Cout) * c.wtaps * g->C;
+    p.rng_w = *rng_w; p.rng_b = rng_b ? *rng_b : *rng_w;
+    p.shared_l = shared_x ? 1 : 0;
+    p.sum_samples = sum_samples ? 1 : 0;
+    // C % 4 == 0: with a 4-aligned sample stride every CTA takes the staged drain, the only one with the phase view
+    p.vec_out = (y_sample_stride % 4 == 0);
+    rc = dispatch_tma_contract<true>(p, p.K, st);
+  });
+  return rc;
 }
 
 int tma_conv_transpose_dgrad(const float* dy, const float* mu_w, const float* sigma_w, const float* eps_w, float* dx,
-                             int64_t x_sample_stride, const bnn_conv2d_nhwc* g, int S, uint32_t sample_begin,
+                             int64_t x_sample_stride, const ConvGeom& cg, int S, uint32_t sample_begin,
                              const bnn_rng* rng_w, cudaStream_t st) {
-  if (!conv_ok(*g) || g->Cout % 4 != 0 || !aligned16(dy) || !aligned16(dx) || rng_w->elem_offset % 4 != 0 ||
+  const bnn_conv3d_nhwc* g = &cg.g;
+  if (!conv_ok(cg) || g->Cout % 4 != 0 || !aligned16(dy) || !aligned16(dx) || rng_w->elem_offset % 4 != 0 ||
       !aligned16(mu_w) || !aligned16(sigma_w) || (eps_w != nullptr && !aligned16(eps_w)))
     return kNotEligible;
   bnn_view v{};
   v.base = dx; v.batch_stride = g->Cout; v.P = 1;
-  return conv_fwd_launch(dy, static_cast<int64_t>(g->B) * g->H * g->W * g->C, mu_w, sigma_w, nullptr, nullptr, eps_w,
-                         nullptr, v, x_sample_stride, g, S, sample_begin, rng_w, nullptr, x_sample_stride == 0, st);
+  return conv_fwd_launch(dy, static_cast<int64_t>(g->B) * g->D * g->H * g->W * g->C, mu_w, sigma_w, nullptr, nullptr, eps_w,
+                         nullptr, v, x_sample_stride, cg, S, sample_begin, rng_w, nullptr, x_sample_stride == 0, st);
 }
 
 int tma_wait_counters(unsigned long long* out8, int reset) {

@@ -306,6 +306,28 @@ __device__ __forceinline__ void tma_load_im2col_4d_pair(uint32_t smem_dst, const
         "h"(off_w), "h"(off_h)
       : "memory");
 }
+// 3-d convolutions: NDHWC tensor {c, w, h, d, n} through a rank-5 im2col map, tap offsets {w, h, d}
+__device__ __forceinline__ void tma_load_im2col_5d(uint32_t smem_dst, const void* tmap, int c, int w, int h, int d, int n,
+                                                   uint16_t off_w, uint16_t off_h, uint16_t off_d, uint64_t* bar) {
+  asm volatile(
+      "cp.async.bulk.tensor.5d.shared::cluster.global.im2col.mbarrier::complete_tx::bytes [%0], "
+      "[%1, {%3, %4, %5, %6, %7}], [%2], {%8, %9, %10};"
+      :
+      : "r"(smem_dst), "l"(reinterpret_cast<uint64_t>(tmap)), "r"(smem_u32(bar)), "r"(c), "r"(w), "r"(h), "r"(d), "r"(n),
+        "h"(off_w), "h"(off_h), "h"(off_d)
+      : "memory");
+}
+__device__ __forceinline__ void tma_load_im2col_5d_pair(uint32_t smem_dst, const void* tmap, int c, int w, int h, int d,
+                                                        int n, uint16_t off_w, uint16_t off_h, uint16_t off_d,
+                                                        uint32_t mbar_cluster_addr) {
+  asm volatile(
+      "cp.async.bulk.tensor.5d.im2col.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], "
+      "[%1, {%3, %4, %5, %6, %7}], [%2], {%8, %9, %10};"
+      :
+      : "r"(smem_dst), "l"(reinterpret_cast<uint64_t>(tmap)), "r"(mbar_cluster_addr), "r"(c), "r"(w), "r"(h), "r"(d),
+        "r"(n), "h"(off_w), "h"(off_h), "h"(off_d)
+      : "memory");
+}
 
 __host__ __device__ constexpr uint32_t tmem_cols_pow2(uint32_t need) {
   return need <= 32 ? 32u : need <= 64 ? 64u : need <= 128 ? 128u : need <= 256 ? 256u : 512u;

@@ -266,6 +266,12 @@ def set_conv_output_format(fmt):
     _CONV_OUTPUT["format"] = fmt
 
 
+def conv_output_nchw(x):
+    """Whether a conv layer's output is NC(D)HW-contiguous (set_conv_output_format): always under 'contiguous', and under
+    'preserve' for an input that is."""
+    return _CONV_OUTPUT["format"] == "contiguous" or x.is_contiguous()
+
+
 def _nhwc(t):
     """(tensor whose memory is NHWC-contiguous, copied?) for a logical NCHW tensor."""
     if t.permute(0, 2, 3, 1).is_contiguous():
@@ -623,6 +629,149 @@ class SampledConvTranspose2d(torch.autograd.Function):
             dx = dxs.view(S, B, Cin, H, W).sum(0) if shared and S > 1 else dxs
         return (dx, grads[0] if need_w else None, grads[1] if need_w else None,
                 bg[0] if need_b else None, bg[1] if need_b else None) + (None,) * 10
+
+
+class ConvTranspose3dRefused(Exception):
+    """The 3-d implicit-GEMM kernels do not take this request; raised by SampledConvTranspose3dImplicit before anything
+    is launched, so that the layer can contract materialised samples instead."""
+
+
+def _ndhwc(t):
+    """(tensor whose memory is NDHWC-contiguous, copied?) for a logical NCDHW tensor."""
+    if t.permute(0, 2, 3, 4, 1).is_contiguous():
+        return t
+    return t.contiguous(memory_format=torch.channels_last_3d)
+
+
+class SampledConvTranspose3dImplicit(torch.autograd.Function):
+    """y[s] = conv_transpose3d(x[s], W_s, b_s) for S samples, W [Cin, Cout, KD, KH, KW], TF32, on the 3-d implicit-GEMM
+    kernels (rank-5 im2col tensor maps): the forward is the conv view's input gradient, cut into sd x sh x sw phases (one
+    stride-1 gather per phase, the bias in its epilogue); the input gradient is the conv view's forward and the weight
+    gradient its weight gradient.  The C library checks one predicate for the three passes (Cin % 32 == 0,
+    Cout % 32 == 0, stride <= 8, alignment, every corner within the rank-5 descriptor's limits); a request outside it
+    raises ConvTranspose3dRefused from the forward, and once the forward has run, the backward cannot be refused.
+
+    x: logical [S*B, Cin, D, H, W] (sample-major) or, when `shared`, [B, Cin, D, H, W]; any memory format.  The kernels
+    write channels_last_3d; the result is converted once to NCDHW-contiguous unless set_conv_output_format('preserve') and
+    x is channels_last_3d."""
+
+    @staticmethod
+    def forward(ctx, x, mu_w, rho_w, mu_b, rho_b, S, shared, spec_w, spec_b, stride, padding, output_padding, dilation):
+        for n, t in (("input", x), ("weight.mean", mu_w), ("weight.scale", rho_w), ("bias.mean", mu_b),
+                     ("bias.scale", rho_b)):
+            _check_f32_cuda(n, t)
+        Cin, Cout, KD, KH, KW = mu_w.shape
+        if x.dim() != 5 or x.shape[1] != Cin:
+            raise RuntimeError(f"sampled conv_transpose3d: input {tuple(x.shape)} does not match weight {tuple(mu_w.shape)}")
+        rows, _, D, H, W = x.shape
+        B = rows if shared else rows // S
+        if not shared and B * S != rows:
+            raise RuntimeError(f"sampled conv_transpose3d: batch {rows} is not divisible by {S} Monte-Carlo samples")
+        OD, OH, OW = (conv_transpose_out(n, k, s, p, op, d) for n, k, s, p, op, d in
+                      zip((D, H, W), (KD, KH, KW), stride, padding, output_padding, dilation))
+        if OD <= 0 or OH <= 0 or OW <= 0:
+            raise RuntimeError("sampled conv_transpose3d: empty output")
+        nchw_out = conv_output_nchw(x)
+        x_cl = _ndhwc(x)
+        geom = _C.conv3d_geom(B, OD, OH, OW, Cout, D, H, W, Cin, (KD, KH, KW), stride, padding, dilation)   # the conv view
+        wl = _C.conv_weight_layout(mu_w.contiguous(), rho_w.contiguous())      # (o = Cin, kd, kh, kw, c = Cout) order
+        has_bias = mu_b is not None
+        sigma_b = _C.stddev(rho_b.contiguous()) if has_bias else None
+        y = torch.empty((S * B, Cout, OD, OH, OW), device=x.device, dtype=torch.float32,
+                        memory_format=torch.channels_last_3d)
+        if not _C.try_sampled_conv_transpose3d_fwd(
+                x_cl, 0 if shared else B * D * H * W * Cin, wl[0], wl[1], mu_b.contiguous() if has_bias else None,
+                sigma_b, _eps_slice(spec_w, S, mu_w.numel()), _eps_slice(spec_b, S, Cout) if has_bias else None, y,
+                geom, S, spec_w.sample_begin, spec_w.rng(), spec_b.rng() if has_bias else None):
+            raise ConvTranspose3dRefused()
+        ctx.save_for_backward(x_cl, wl, rho_b)
+        ctx.meta = (S, shared, spec_w, spec_b, geom, tuple(mu_w.shape))
+        return y.contiguous() if nchw_out else y
+
+    @staticmethod
+    def backward(ctx, dy):
+        x_cl, wl, rho_b = ctx.saved_tensors
+        S, shared, spec_w, spec_b, geom, w_shape = ctx.meta
+        Cin, Cout = w_shape[0], w_shape[1]
+        B, OD, OH, OW = geom.B, geom.D, geom.H, geom.W                        # transposed output OD x OH x OW
+        M = B * geom.OD * geom.OH * geom.OW
+        eps_w = _eps_slice(spec_w, S, math.prod(w_shape))
+        x_ss = 0 if shared else M * Cin
+        need_x = ctx.needs_input_grad[0]
+        need_w = ctx.needs_input_grad[1] or ctx.needs_input_grad[2]
+        need_b = rho_b is not None and (ctx.needs_input_grad[3] or ctx.needs_input_grad[4])
+        # the kernels read dY as NDHWC rows; an NCDHW-contiguous gradient goes through ONE transposing pass (P = D*H*W)
+        # that forms the bias gradient on the way
+        bias_done, bg_fused = False, None
+        if dy.permute(0, 2, 3, 4, 1).is_contiguous():
+            dy_cl = dy
+        else:
+            dy_cl = None
+            if dy.is_contiguous():
+                if need_b:
+                    bg_fused = torch.zeros((2, Cout), device=dy.device, dtype=torch.float32)
+                t = _C.nchw_to_nhwc_bias_grad(dy.view(dy.shape[0], Cout, OD, OH * OW), B,
+                                              rho_b.contiguous() if need_b else None,
+                                              _eps_slice(spec_b, S, Cout) if need_b else None,
+                                              bg_fused[0] if need_b else None, bg_fused[1] if need_b else None,
+                                              spec_b.sample_begin if need_b else 0, spec_b.rng() if need_b else None)
+                if t is not None:
+                    dy_cl = t.permute(0, 2, 3, 1).view(dy.shape[0], OD, OH, OW, Cout).permute(0, 4, 1, 2, 3)
+                    bias_done = need_b
+            if dy_cl is None:
+                dy_cl = dy.contiguous(memory_format=torch.channels_last_3d)
+        dx = None
+        if need_x:
+            dx = torch.empty(x_cl.shape, device=dy.device, dtype=torch.float32, memory_format=torch.channels_last_3d)
+            _C.sampled_conv_transpose3d_dgrad(dy_cl, wl[0], wl[1], eps_w, dx, x_ss, geom, S, spec_w.sample_begin,
+                                              spec_w.rng())
+        grads_p, bg = _zero_grads((math.prod(w_shape),) if need_w else None, Cout if (need_b and not bias_done) else None,
+                                  dy.device)
+        if bias_done:
+            bg = bg_fused
+        dmu = drho = None
+        if need_w:
+            _C.sampled_conv_transpose3d_wgrad(dy_cl, x_cl, x_ss, wl[2], eps_w, grads_p[0], grads_p[1], geom, S,
+                                              spec_w.sample_begin, spec_w.rng())
+            g = _C.conv_weight_unlayout(grads_p, w_shape)
+            dmu, drho = g[0], g[1]
+        if need_b and not bias_done:
+            rows_y = B * OD * OH * OW
+            _C.bias_grad(_C.make_view(dy_cl.data_ptr(), Cout, 1), rows_y * Cout, rho_b.contiguous(),
+                         _eps_slice(spec_b, S, Cout), bg[0], bg[1], rows_y, Cout, S, spec_b.sample_begin, spec_b.rng())
+        return (dx, dmu, drho, bg[0] if need_b else None, bg[1] if need_b else None) + (None,) * 8
+
+
+class CudnnConvTranspose3d(torch.autograd.Function):
+    """F.conv_transpose3d(x, w, b, ...) with cuDNN's TF32 switched to `tf32` in the forward AND the backward pass (autograd
+    runs the backward outside any context the forward was called in): the materialised-sample form of
+    NormalConvTranspose3d, which in fp32 mode must not round its operands to TF32."""
+
+    @staticmethod
+    def _tf32(flag, fn):
+        prev = torch.backends.cudnn.allow_tf32
+        torch.backends.cudnn.allow_tf32 = flag
+        try:
+            return fn()
+        finally:
+            torch.backends.cudnn.allow_tf32 = prev
+
+    @staticmethod
+    def forward(ctx, x, w, b, stride, padding, output_padding, groups, dilation, tf32):
+        ctx.save_for_backward(x, w)
+        ctx.meta = (b is not None, stride, padding, output_padding, groups, dilation, tf32)
+        return CudnnConvTranspose3d._tf32(tf32, lambda: torch.nn.functional.conv_transpose3d(
+            x, w, b, stride, padding, output_padding, groups, dilation))
+
+    @staticmethod
+    def backward(ctx, gy):
+        x, w = ctx.saved_tensors
+        has_b, stride, padding, output_padding, groups, dilation, tf32 = ctx.meta
+        mask = [ctx.needs_input_grad[0], ctx.needs_input_grad[1], has_b and ctx.needs_input_grad[2]]
+        gx, gw, gb = CudnnConvTranspose3d._tf32(tf32, lambda: torch.ops.aten.convolution_backward(
+            gy, x, w, [w.shape[1] * groups] if has_b else None, list(stride), list(padding), list(dilation), True,
+            list(output_padding), groups, mask))
+        return (gx, gw, gb if has_b else None) + (None,) * 6
 
 
 # ------------------------------------------------------------------------------------------------

@@ -5,7 +5,8 @@ scope (MC-dropout, evidential regression) are plain torch (nn/other.py)."""
 from .container import BayesianModule, BayesianNetworkModule, register_rowwise_module
 from .variational import WeightNormal
 from .layers import (BayesianLinear, NormalLinear, BayesianConvNd, NormalConvNd, NormalConv1d, NormalConv2d,
-                     NormalConv3d, NormalConvTransposeNd, NormalConvTranspose1d, NormalConvTranspose2d)
+                     NormalConv3d, NormalConvTransposeNd, NormalConvTranspose1d, NormalConvTranspose2d,
+                     NormalConvTranspose3d)
 from .flipout import (FlipoutNormalLinear, FlipOutNormalConvNd, FlipOutNormalConv1d, FlipOutNormalConv2d,
                       FlipOutNormalConv3d)
 from .mvn import WeightMultivariateNormal, MultivariateNormalLinear
@@ -21,5 +22,5 @@ __all__ = [
     'MultivariateNormalLinear', 'KLDivergence', 'Entropy', 'MCSamples', 'mc_mean_loss',
     'NormalInverseGaussianLinear', 'MCDropoutLinear', 'MCDropoutConvNd', 'MCDropoutConv1d', 'MCDropoutConv2d',
     'MCDropoutConv3d', 'NormalInverseGaussianLoss', 'NormalInverseGaussianUncertainty',
-    'NormalConvTransposeNd', 'NormalConvTranspose1d', 'NormalConvTranspose2d',
+    'NormalConvTransposeNd', 'NormalConvTranspose1d', 'NormalConvTranspose2d', 'NormalConvTranspose3d',
 ]

@@ -2,7 +2,7 @@
 
 Constructor signatures, attributes (`weight`, `bias`, `sampled`, `sample()`, priors, conv geometry)
 and `forward(x, sample=True)` follow the reference; the arithmetic runs in libbnn_b200.so:
-NormalLinear, NormalConv1d/2d and NormalConvTranspose1d/2d call the fused sample-and-contract kernels (no sampled
+NormalLinear, NormalConv1d/2d and NormalConvTranspose1d/2d/3d call the fused sample-and-contract kernels (no sampled
 weight in memory), NormalConv3d contracts materialised samples with torch's conv3d.
 """
 import math
@@ -11,9 +11,10 @@ import torch
 from torch.distributions.normal import Normal
 from torch.nn import init
 
-from .. import runtime
-from ..functional import (SampledConv2d, SampledConv2dImplicit, SampledConvTranspose2d, SampledConvTranspose2dImplicit,
-                          SampledLinear, conv_implicit_eligible)
+from .. import _C, runtime
+from ..functional import (ConvTranspose3dRefused, CudnnConvTranspose3d, SampledConv2d, SampledConv2dImplicit,
+                          SampledConvTranspose2d, SampledConvTranspose2dImplicit, SampledConvTranspose3dImplicit,
+                          SampledLinear, conv_implicit_eligible, conv_output_nchw)
 from ..utils.traversal import _pair, _single, _triple
 from .container import BayesianModule
 from .variational import WeightNormal
@@ -249,6 +250,27 @@ class NormalConvTransposeNd(NormalConvNd):
         self.output_padding = output_padding
         _mark_implicit(self)
 
+    def _output_padding(self, x, output_size):
+        """output_padding of this call: the layer's own, or the one that gives `output_size` (torch's
+        _ConvTransposeNd._output_padding: the same accepted sizes, [min, min + stride - 1] per dimension, and errors)."""
+        if output_size is None:
+            return tuple(self.output_padding)
+        n = len(self.kernel_size)
+        non_spatial = 2 if x.dim() == n + 2 else 1
+        if len(output_size) == non_spatial + n:
+            output_size = output_size[non_spatial:]
+        if len(output_size) != n:
+            raise ValueError(f"ConvTranspose{n}D: for {x.dim()}D input, output_size must have {n} or {non_spatial + n} "
+                             f"elements (got {len(output_size)})")
+        min_sizes = [(x.size(d + non_spatial) - 1) * self.stride[d] - 2 * self.padding[d] +
+                     self.dilation[d] * (self.kernel_size[d] - 1) + 1 for d in range(n)]
+        max_sizes = [m + s - 1 for m, s in zip(min_sizes, self.stride)]
+        for size, lo, hi in zip(output_size, min_sizes, max_sizes):
+            if size < lo or size > hi:
+                raise ValueError(f"requested an output size of {output_size}, but valid sizes range from {min_sizes} "
+                                 f"to {max_sizes} (for an input of {x.size()[2:]})")
+        return tuple(size - lo for size, lo in zip(output_size, min_sizes))
+
     def _conv_transpose2d(self, x, w_shape, S, shared, spec_w, spec_b, stride, padding, output_padding, dilation):
         # output_padding >= stride (possible when dilation > stride): the rows beyond the conv view are reached by
         # appending zero input rows, which leaves output_padding % stride
@@ -274,11 +296,12 @@ class NormalConvTranspose2d(_FusedBayesianLayer, NormalConvTransposeNd):
                                                     _pair(padding), _pair(output_padding), groups, bias,
                                                     _pair(dilation), prior)
 
-    def forward(self, x, sample=True):
+    def forward(self, x, sample=True, output_size=None):
+        output_padding = self._output_padding(x, output_size)
         S, shared, offset, total, ctx = self._mc_shape(x)
         spec_w, spec_b = self._draws(sample, S, offset, total)
         y = self._conv_transpose2d(x, tuple(self.weight.mean.shape), S, shared, spec_w, spec_b, tuple(self.stride),
-                                   tuple(self.padding), tuple(self.output_padding), tuple(self.dilation))
+                                   tuple(self.padding), output_padding, tuple(self.dilation))
         if ctx is not None:
             ctx.expanded = True
         return y
@@ -293,16 +316,75 @@ class NormalConvTranspose1d(_FusedBayesianLayer, NormalConvTransposeNd):
                                                     _single(padding), _single(output_padding), groups, bias,
                                                     _single(dilation), prior)
 
-    def forward(self, x, sample=True):
+    def forward(self, x, sample=True, output_size=None):
+        output_padding = self._output_padding(x, output_size)
         S, shared, offset, total, ctx = self._mc_shape(x)
         spec_w, spec_b = self._draws(sample, S, offset, total)
         w = self.weight.mean.shape
         y = self._conv_transpose2d(x.unsqueeze(2), (w[0], w[1], 1, w[2]), S, shared, spec_w, spec_b,
                                    (1, tuple(self.stride)[0]), (0, tuple(self.padding)[0]),
-                                   (0, tuple(self.output_padding)[0]), (1, tuple(self.dilation)[0]))
+                                   (0, output_padding[0]), (1, tuple(self.dilation)[0]))
         if ctx is not None:
             ctx.expanded = True
         return y.squeeze(2)
+
+
+class NormalConvTranspose3d(_FusedBayesianLayer, NormalConvTransposeNd):
+    """torch.nn.ConvTranspose3d's constructor order with a Normal variational posterior on weight and bias — the
+    upsampling layer of Bayesian volumetric decoders (3-D U-Nets, V-Nets).  CUDA, TF32, groups == 1 with in_ and
+    out_channels multiples of 32 and a geometry within the rank-5 im2col descriptor's limits: the 3-d implicit-GEMM kernels
+    (SampledConvTranspose3dImplicit, all Monte-Carlo samples in one call per output phase).  Everything else — fp32 mode,
+    other channel counts (e.g. a 1-channel output), groups > 1, geometry outside those limits — contracts the S
+    materialised draws (the same draws: WeightNormal.materialize applies the layer's eps order) with one
+    F.conv_transpose3d per sample, with cuDNN's TF32 off in fp32 mode."""
+
+    def __init__(self, in_channels, out_channels, kernel_size, stride=1, padding=0, output_padding=0, groups=1,
+                 bias=True, dilation=1, prior=Normal(0, .1)):
+        super(NormalConvTranspose3d, self).__init__(in_channels, out_channels, _triple(kernel_size), _triple(stride),
+                                                    _triple(padding), _triple(output_padding), groups, bias,
+                                                    _triple(dilation), prior)
+
+    def _materialized(self, x, S, shared, spec_w, spec_b, stride, padding, output_padding, dilation):
+        """The reference's form: W_s (autograd-tracked) and one cuDNN transposed convolution per sample."""
+        def begin(spec):
+            return (spec.step << 32) | spec.sample_begin
+        # contiguous: the draws of a layer with the (o, kd, kh, kw, c) eps order come back as a strided view
+        w = self.weight.materialize(begin(spec_w), S).contiguous()
+        b = self.bias.materialize(begin(spec_b), S) if self.bias is not None else None
+        xs = x if shared else x.reshape((S, x.shape[0] // S) + tuple(x.shape[1:]))
+        tf32 = runtime.precision() == _C.PREC_TF32
+        y = torch.cat([CudnnConvTranspose3d.apply(x if shared else xs[s], w[s], b[s] if b is not None else None, stride,
+                                                  padding, output_padding, self.groups, dilation, tf32)
+                       for s in range(S)], 0)
+        return y.contiguous() if conv_output_nchw(x) else y
+
+    def _conv_transpose3d(self, x, S, shared, spec_w, spec_b, output_padding):
+        stride, padding, dilation = tuple(self.stride), tuple(self.padding), tuple(self.dilation)
+        if self._implicit and runtime.precision() == _C.PREC_TF32:
+            # output_padding >= stride (dilation > stride): zero input rows appended, as in _conv_transpose2d
+            extra = [op // s for op, s in zip(output_padding, stride)]
+            xi, opi = x, output_padding
+            if any(extra):
+                xi = torch.nn.functional.pad(x, (0, extra[2], 0, extra[1], 0, extra[0]))
+                opi = tuple(op % s for op, s in zip(output_padding, stride))
+            bias = self.bias
+            try:
+                return SampledConvTranspose3dImplicit.apply(xi, self.weight.mean, self.weight.scale,
+                                                            bias.mean if bias is not None else None,
+                                                            bias.scale if bias is not None else None, S, shared, spec_w,
+                                                            spec_b, stride, padding, opi, dilation)
+            except ConvTranspose3dRefused:
+                pass
+        return self._materialized(x, S, shared, spec_w, spec_b, stride, padding, output_padding, dilation)
+
+    def forward(self, x, sample=True, output_size=None):
+        output_padding = self._output_padding(x, output_size)
+        S, shared, offset, total, ctx = self._mc_shape(x)
+        spec_w, spec_b = self._draws(sample, S, offset, total)
+        y = self._conv_transpose3d(x, S, shared, spec_w, spec_b, output_padding)
+        if ctx is not None:
+            ctx.expanded = True
+        return y
 
 
 _UNFOLD_LIMIT_BYTES = 1 << 30      # NormalConv3d: largest lowered activation matrix the fused path builds

@@ -226,6 +226,37 @@ int bnn_sampled_conv_transpose2d_wgrad(const float* dy, const float* x, int64_t 
  * the phase is kh = last - j * tap step, read at input row i + first + j * input step for output row rh + sh * i.  Returns
  * the number of phases (may exceed max_phases; only max_phases are written) or a negative bnn_status. */
 int bnn_debug_conv_transpose_phases(const bnn_conv2d_nhwc* g, int32_t* out, int32_t max_phases);
+/* ---- 3-d transposed convolution (NormalConvTranspose3d) ----
+ * The same three passes with a depth: activations NDHWC (torch.channels_last_3d memory), W [Cin][Cout][KD][KH][KW] and
+ * `g` the conv view with the 2-d convention above (g->C = Cout, g->D, g->H, g->W = output size; g->Cout = Cin, g->OD,
+ * g->OH, g->OW = input size).  Weights, sigma, rho, eps and gradients in (o, kd, kh, kw, c) order = [Cin][KD][KH][KW][Cout]
+ * (bnn_conv2d_weight_layout with Cout = Cin, taps = KD*KH*KW).  The activation operand reaches the tensor cores through a
+ * rank-5 im2col tensor map; GEMM row m = (img, d, h, w).  The forward cuts the outputs into sd x sh x sw phases.
+ * One predicate for all three passes: Cin % 32 == 0, Cout % 32 == 0, stride <= 8, 16-byte aligned tensors, and every
+ * phase corner and conv-view corner within [-16, 15] with every filter extent (k - 1) d below 32 (the rank-5 im2col
+ * descriptor).  BNN_ERR_UNSUPPORTED when it does not hold; callers then contract materialised samples. */
+typedef struct bnn_conv3d_nhwc {
+  int32_t B;                 /* images per Monte-Carlo sample */
+  int32_t D, H, W, C;        /* input depth, height, width, channels */
+  int32_t OD, OH, OW, Cout;
+  int32_t KD, KH, KW;
+  int32_t sd, sh, sw, pd, ph, pw, dd, dh, dw;
+  int32_t reserved;
+} bnn_conv3d_nhwc;
+int bnn_sampled_conv_transpose3d_fwd(const float* x, int64_t x_sample_stride, const float* mu_w, const float* sigma_w,
+                                     const float* mu_b, const float* sigma_b, const float* eps_w, const float* eps_b, float* y,
+                                     const bnn_conv3d_nhwc* g, int32_t S, uint32_t sample_begin, const bnn_rng* rng_w,
+                                     const bnn_rng* rng_b, void* stream);
+int bnn_sampled_conv_transpose3d_dgrad(const float* dy, const float* mu_w, const float* sigma_w, const float* eps_w,
+                                       float* dx, int64_t x_sample_stride, const bnn_conv3d_nhwc* g, int32_t S,
+                                       uint32_t sample_begin, const bnn_rng* rng_w, void* stream);
+int bnn_sampled_conv_transpose3d_wgrad(const float* dy, const float* x, int64_t x_sample_stride, const float* rho_w,
+                                       const float* eps_w, float* dmu_w, float* drho_w, const bnn_conv3d_nhwc* g, int32_t S,
+                                       uint32_t sample_begin, const bnn_rng* rng_w, void* stream);
+/* Host only (test aid): the phase plan of bnn_sampled_conv_transpose3d_fwd, 21 ints per phase: the seven fields of
+ * bnn_debug_conv_transpose_phases, each for d, h, w {rd, rh, rw, rows_d, rows_h, rows_w, taps_d, ...}.  Returns the
+ * number of phases (may exceed max_phases) or a negative bnn_status. */
+int bnn_debug_conv_transpose3d_phases(const bnn_conv3d_nhwc* g, int32_t* out, int32_t max_phases);
 /* OIHW parameters [Cout][Cg][taps] -> (o, kh, kw, c) order: mu_p, and optionally sigma_p = 1e-10 + softplus(rho) and
  * rho_p (NULL to skip); the inverse for `n_arrays` arrays stored back to back (gradients of mean and scale). */
 int bnn_conv2d_weight_layout(const float* mu, const float* rho, float* mu_p, float* sigma_p, float* rho_p, int32_t Cout,
