@@ -96,7 +96,7 @@ __device__ __forceinline__ float grad1(const AdamTable& tab, const float* g) {
   const int64_t off = g - tab.peer[tab.rank];
   float acc = ld_peer1(tab.peer[0] + off);
   for (int r = 1; r < tab.world; ++r) acc += ld_peer1(tab.peer[r] + off);
-  return acc / static_cast<float>(tab.world);
+  return acc * (1.0f / static_cast<float>(tab.world));     // as grad4 and bnn_peer_average: alignment changes no bit
 }
 
 template <bool kPeers>
@@ -187,7 +187,8 @@ int adam_launch(const bnn_adam_tensor* tensors, int32_t n_tensors, float lr, flo
                 "%s: tensor %d has a NULL parameter or moment pointer", who, i);
     BNN_REQUIRE(t.numel == 0 || t.rho == nullptr || (t.m_rho && t.v_rho), BNN_ERR_BAD_ARGUMENT,
                 "%s: tensor %d has rho but no moment buffers for it", who, i);
-    BNN_REQUIRE(t.rho != nullptr || (t.kl_coeff == 0.f && t.g_rho == nullptr), BNN_ERR_BAD_ARGUMENT,
+    // an empty tensor has NULL pointers (torch's data_ptr() of zero elements): it is skipped, whatever its kind
+    BNN_REQUIRE(t.numel == 0 || t.rho != nullptr || (t.kl_coeff == 0.f && t.g_rho == nullptr), BNN_ERR_BAD_ARGUMENT,
                 "%s: tensor %d is a plain parameter (rho NULL): kl_coeff must be 0 and g_rho NULL", who, i);
     BNN_REQUIRE(t.kl_coeff == 0.f || t.prior_scale > 0.f, BNN_ERR_BAD_ARGUMENT, "%s: tensor %d needs prior scale > 0", who, i);
     if (use_peers) {
