@@ -193,7 +193,10 @@ _SIGNATURES = {
     "bnn_debug_force_contract_variant": (ctypes.c_int, [ctypes.c_int32]),
     "bnn_debug_pair_tile_plan": (ctypes.c_int, [ctypes.c_int32, ctypes.c_int32, ctypes.c_int32,
                                                 ctypes.POINTER(ctypes.c_int32)]),
-    "bnn_selftest_umma": (ctypes.c_int, [_c_f32p, ctypes.c_void_p]),
+    "bnn_debug_wgrad_plan": (ctypes.c_int, [ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32,
+                                            ctypes.POINTER(ctypes.c_int32)]),
+    "bnn_debug_force_wgrad_plan": (ctypes.c_int, [ctypes.c_int32, ctypes.c_int32, ctypes.c_int32]),
+    "bnn_selftest_umma":(ctypes.c_int, [_c_f32p, ctypes.c_void_p]),
     "bnn_selftest_umma_mn": (ctypes.c_int, [_c_f32p, ctypes.c_void_p]),
 }
 
@@ -804,6 +807,23 @@ def force_contract_variant(variant):
     """Test aid: 'pair' | 'mb4' | 'mb2' | 'mb1' | None (cost model) for the TMA-fed forward / data-gradient kernels."""
     code = {None: -1, "pair": 0, "mb1": 1, "mb2": 2, "mb4": 4}[variant]
     _check(lib().bnn_debug_force_contract_variant(code), "bnn_debug_force_contract_variant")
+
+
+def wgrad_plan(M, N, K, S, sms=None):
+    """Host-side plan of the TMA weight gradient (no device needed): dict of pair, n_chunks, chunk_blocks, units_per_cta
+    and groups on `sms` SMs (default: those of the current device), including a forced override."""
+    if sms is None:
+        sms = torch.cuda.get_device_properties(torch.cuda.current_device()).multi_processor_count
+    out = (ctypes.c_int32 * 5)()
+    _check(lib().bnn_debug_wgrad_plan(M, N, K, S, sms, out), "bnn_debug_wgrad_plan")
+    return dict(zip(("pair", "n_chunks", "chunk_blocks", "units_per_cta", "groups"), list(out)))
+
+
+def force_wgrad_plan(pair=None, n_chunks=None, units_per_cta=None):
+    """Test aid: force parts of the TMA weight-gradient plan (None = the cost model's choice; all None resets).  A forced
+    value the shape cannot take makes the launch raise instead of running another plan."""
+    code = lambda v: -1 if v is None else int(v)
+    _check(lib().bnn_debug_force_wgrad_plan(code(pair), code(n_chunks), code(units_per_cta)), "bnn_debug_force_wgrad_plan")
 
 
 def selftest_umma(device="cuda", mn_major=False):

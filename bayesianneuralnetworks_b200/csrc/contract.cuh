@@ -185,6 +185,16 @@ bool conv_transpose_ok(const ConvGeom& g);
 int tma_selftest(float* max_err_dev, cudaStream_t st);
 int tma_pair_tile_plan(int m_blocks, int S, int slots, int32_t* out7);   // test aid: TilePlan fields {on, n_a, s1, a1, b1, a2, b2}
 int tma_force_variant(int variant);   // test aid: 0 = CTA pair, 1 / 2 / 4 = row blocks per CTA, -1 = cost model (default)
+// host: the weight-gradient launch plan on `sms` SMs (including a forced override); the launcher runs exactly this plan
+struct WgradPlan {
+  int pair;           // CTA pairs over adjacent n-tiles
+  int n_chunks;       // M-chunks per sample; a work unit = (sample, chunk)
+  int chunk_blocks;   // 64-row stages per chunk (the last chunk may be shorter)
+  int per;            // work units per CTA: ceil(S * n_chunks / groups), as the kernel derives it
+  int groups;         // gridDim.z
+};
+int wgrad_plan(int M, int N, int K, int S, int sms, WgradPlan* plan);
+int tma_force_wgrad_plan(int pair, int n_chunks, int units_per_cta);   // test aid: -1 = the cost model's choice
 int tma_stage_counters(unsigned long long* out8, int reset);  // profiling builds only: CTA timeline of the pair kernels
 int tma_wait_counters(unsigned long long* out8, int reset);   // profiling builds (-DBNN_PROFILE_WAITS) only
 

@@ -996,30 +996,47 @@ int tma_dgrad(bnn_view dy, int64_t dy_sample_stride, const float* mu_w, const fl
   return dispatch_tma_contract<true>(p, K, st);
 }
 
-// Work-unit plan + launch shared by the matrix and the implicit-GEMM (conv) weight gradient
-int wgrad_plan_and_launch(TmaWgradParams& p, int M, int N, int K, int S, cudaStream_t st) {
-  int rc = BNN_OK;
+namespace {
+// Test aid (bnn_debug_force_wgrad_plan): forced {pair, n_chunks, units per CTA}, -1 = the cost model's choice.  Unlike
+// the contraction variant, a forced value the shape cannot take is an error, never a silent fall-back to another plan.
+std::atomic<int> g_forced_wgrad[3] = {-1, -1, -1};
+}  // namespace
+
+// Work-unit plan of the weight gradient (host arithmetic) on `sms` SMs.  Work units = (sample, M-chunk); a CTA =
+// (tile, group) walks `per` consecutive units, the epilogue of one unit (TMEM drain + eps regeneration for 128 x 128
+// weights, ~6 stage times) overlapping the MMAs of the next.  The plan minimises  waves x (per x (stages per unit + 0.5)
+// + 6)  over the number of M-chunks and units per CTA: small layers get ONE wave of CTAs with long units instead of
+// several waves of short ones (every extra unit costs an epilogue), and no CTA is launched without work.  The cost
+// model cuts the m_total 64-row stages of a sample into at most min(ceil(m_total / 4), 64) chunks, i.e. no more chunks
+// than 256-row pieces; every chunk holds chunk_blocks = ceil(m_total / n_chunks) stages except the last, which holds
+// what is left and may be shorter (m_total = 5: 3 + 2 stages; m_total = 13: 4 + 4 + 4 + 1).
+int wgrad_plan(int M, int N, int K, int S, int sms, WgradPlan* out) {
   const int tiles = ((N + 127) / 128) * ((K + 127) / 128);
   const int m_total = (M + kWgRows - 1) / kWgRows;         // 64-row stages
-  // Work units = (sample, M-chunk); a CTA = (tile, group) walks `per` consecutive units, the epilogue of one unit
-  // (TMEM drain + eps regeneration for 128 x 128 weights, ~6 stage times) overlapping the MMAs of the next.  The plan
-  // minimises  waves x (per x (stages per unit + 0.5) + 6)  over the number of M-chunks and units per CTA: small layers
-  // get ONE wave of CTAs with long units instead of several waves of short ones (every extra unit costs an epilogue),
-  // and no CTA is launched without work.  Units keep >= 4 stages (256 rows).
-  const int sms = sm_count();
+  const int f_pair = g_forced_wgrad[0].load(std::memory_order_relaxed);
+  const int f_chunks = g_forced_wgrad[1].load(std::memory_order_relaxed);
+  const int f_per = g_forced_wgrad[2].load(std::memory_order_relaxed);
+  if (f_chunks > 0) {
+    const int cb = (m_total + f_chunks - 1) / f_chunks;
+    BNN_REQUIRE((m_total + cb - 1) / cb == f_chunks, BNN_ERR_BAD_ARGUMENT,
+                "forced weight-gradient plan: n_chunks = %d does not cut %d stages of 64 rows into %d non-empty chunks",
+                f_chunks, m_total, f_chunks);
+  }
   const int max_chunks = (m_total + 3) / 4 < 64 ? (m_total + 3) / 4 : 64;
   double best_cost = 0.0;
   int best_cb = m_total, best_n = 1, best_per = S;
   bool have = false;
-  for (int n = 1; n <= (max_chunks < 1 ? 1 : max_chunks); ++n) {
+  const int n_first = f_chunks > 0 ? f_chunks : 1, n_last = f_chunks > 0 ? f_chunks : (max_chunks < 1 ? 1 : max_chunks);
+  for (int n = n_first; n <= n_last; ++n) {
     const int cb = (m_total + n - 1) / n, n_eff = (m_total + cb - 1) / cb;
     if (n_eff != n) continue;
     const int64_t units = static_cast<int64_t>(S) * n;
-    for (int c = 0; c < 32; ++c) {
-      const int64_t per = c < 16 ? c + 1 : (units + (c - 16)) / (c - 15);        // 1..16, then units / (1..16) rounded up
+    for (int c = 0; c < (f_per > 0 ? 1 : 32); ++c) {
+      const int64_t per = f_per > 0 ? f_per : c < 16 ? c + 1 : (units + (c - 16)) / (c - 15);   // 1..16, then units / (1..16) rounded up
       if (per < 1 || per > units) continue;
       const int64_t groups = (units + per - 1) / per;
       if (groups > 65535) continue;
+      if (f_per > 0 && (units + groups - 1) / groups != per) continue;       // the kernel would walk fewer units per CTA
       const int64_t ctas = static_cast<int64_t>(tiles) * groups;
       const double waves = static_cast<double>((ctas + sms - 1) / sms);
       const double cost = waves * (static_cast<double>(per) * (cb + 0.5) + 6.0);
@@ -1028,9 +1045,43 @@ int wgrad_plan_and_launch(TmaWgradParams& p, int M, int N, int K, int S, cudaStr
       }
     }
   }
-  p.chunk_blocks = best_cb;
-  p.n_chunks = best_n;
-  const int groups = static_cast<int>((static_cast<int64_t>(S) * best_n + best_per - 1) / best_per);
+  BNN_REQUIRE(have || f_per <= 0, BNN_ERR_BAD_ARGUMENT,
+              "forced weight-gradient plan: units_per_cta = %d fits no plan of %d samples (more than S x n_chunks units, "
+              "more than 65535 groups, or the last group would be short enough to shrink every CTA's share)", f_per, S);
+  const int64_t units = static_cast<int64_t>(S) * best_n;
+  const int groups = static_cast<int>((units + best_per - 1) / best_per);
+  const int n_tiles = (N + 127) / 128;
+  bool pair = n_tiles >= 2 && static_cast<int64_t>(tiles) * groups >= 2 * sms;
+  if (f_pair >= 0) {
+    BNN_REQUIRE(f_pair == 0 || n_tiles >= 2, BNN_ERR_BAD_ARGUMENT,
+                "forced weight-gradient plan: pair = 1 needs at least two 128-row n-tiles, N = %d has one", N);
+    pair = f_pair == 1;
+  }
+  out->pair = pair ? 1 : 0;
+  out->n_chunks = best_n;
+  out->chunk_blocks = best_cb;
+  out->per = static_cast<int>((units + groups - 1) / groups);           // what the kernel derives from gridDim.z
+  out->groups = groups;
+  return BNN_OK;
+}
+
+int tma_force_wgrad_plan(int pair, int n_chunks, int units_per_cta) {
+  BNN_REQUIRE(pair >= -1 && pair <= 1 && (n_chunks == -1 || n_chunks >= 1) && (units_per_cta == -1 || units_per_cta >= 1),
+              BNN_ERR_BAD_ARGUMENT, "bnn_debug_force_wgrad_plan: pair in {-1, 0, 1}, n_chunks and units_per_cta -1 or >= 1");
+  g_forced_wgrad[0].store(pair, std::memory_order_relaxed);
+  g_forced_wgrad[1].store(n_chunks, std::memory_order_relaxed);
+  g_forced_wgrad[2].store(units_per_cta, std::memory_order_relaxed);
+  return BNN_OK;
+}
+
+// Plan + launch shared by the matrix and the implicit-GEMM (conv) weight gradient
+int wgrad_plan_and_launch(TmaWgradParams& p, int M, int N, int K, int S, cudaStream_t st) {
+  WgradPlan plan{};
+  int rc = wgrad_plan(M, N, K, S, sm_count(), &plan);
+  if (rc != BNN_OK) return rc;
+  p.chunk_blocks = plan.chunk_blocks;
+  p.n_chunks = plan.n_chunks;
+  const int groups = plan.groups;
   static SmemOptIn opt_in[6];
   const bool signs = p.rng_w.row_sign != nullptr, vol = p.conv.on == 2;
   rc = allow_dynamic_smem(wgrad_tma_kernel<false, false>, kWgradSmem, &opt_in[0]);
@@ -1041,7 +1092,7 @@ int wgrad_plan_and_launch(TmaWgradParams& p, int M, int N, int K, int S, cudaStr
   if (rc == BNN_OK) rc = allow_dynamic_smem(wgrad_tma_kernel<true, false, true>, kWgradSmem, &opt_in[5]);
   if (rc != BNN_OK) return rc;
   const int n_tiles = (N + 127) / 128, k_tiles = (K + 127) / 128;
-  if (n_tiles >= 2 && static_cast<int64_t>(tiles) * groups >= 2 * sm_count()) {
+  if (plan.pair) {
     // CTA pairs over adjacent n-tiles (large problems: the kernel is paced by operand delivery, a pair halves the A^T traffic)
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((n_tiles + 1) / 2 * 2, k_tiles, groups);

@@ -470,6 +470,20 @@ int bnn_debug_force_contract_variant(int32_t variant);
  * [0, s1) are cut into a1 tiles of 8 row blocks followed by b1 tiles of 6, the others into a2 / b2; n_a = number of
  * 8-block tiles; on = 0: the uniform grid is kept. */
 int bnn_debug_pair_tile_plan(int32_t m_blocks, int32_t samples, int32_t pair_slots, int32_t* out7);
+/* test aid, host arithmetic only: the plan of the TMA-fed TF32 weight gradient (dmu / drho of an M x N x K contraction
+ * over S samples) on `sms` SMs, including a forced override.  out5 = {pair, n_chunks, chunk_blocks, units_per_cta,
+ * groups}: each sample's M rows are cut into n_chunks chunks of chunk_blocks 64-row stages (the last one may be shorter),
+ * a work unit is (sample, chunk) numbered u = sample * n_chunks + chunk, and CTA group z (gridDim.z = groups) walks
+ * units [z * units_per_cta, min((z + 1) * units_per_cta, S * n_chunks)); pair = 1: CTA pairs over adjacent 128-row
+ * n-tiles.  BNN_ERR_BAD_ARGUMENT when a forced value does not fit the shape. */
+int bnn_debug_wgrad_plan(int32_t M, int32_t N, int32_t K, int32_t S, int32_t sms, int32_t* out5);
+/* test aid: force parts of that plan for every later weight-gradient launch: pair (0 / 1), n_chunks, units_per_cta;
+ * -1 each = the cost model's choice (default).  A forced value the shape cannot take (pair with one n-tile, an n_chunks
+ * that does not give exactly that many non-empty chunks, more units per CTA than S * n_chunks, more than 65535 groups,
+ * a units_per_cta whose ceil(S * n_chunks / groups) is smaller)
+ * makes the launch fail with BNN_ERR_BAD_ARGUMENT instead of running another plan.  Process-wide; not for production
+ * use. */
+int bnn_debug_force_wgrad_plan(int32_t pair, int32_t n_chunks, int32_t units_per_cta);
 
 #ifdef __cplusplus
 }

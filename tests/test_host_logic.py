@@ -429,3 +429,103 @@ def test_pair_kernel_tile_plans_cover_every_row_block_exactly_once():
     out = (ctypes.c_int32 * 7)()
     lib.bnn_debug_pair_tile_plan(64, 16, 74, out)           # C3 conv forward: 74 + 72 tiles on 74 pair slots
     assert out[0] == 1 and out[1] + out[2] * out[4] + (16 - out[2]) * out[6] <= 148
+
+
+def _wgrad_plan(M, N, K, S, sms=148):
+    out = (ctypes.c_int32 * 5)()
+    rc = _C.lib().bnn_debug_wgrad_plan(M, N, K, S, sms, out)
+    return rc, list(out)
+
+
+def _assert_wgrad_plan_covers(M, N, K, S, plan, sms=148, forced_pair=None):
+    """Decodes a weight-gradient plan exactly as wgrad_tma_kernel does (per from gridDim.z, units [z per, (z + 1) per),
+    unit u = chunk u % n_chunks of sample u / n_chunks, chunk c = stages [c chunk_blocks, + chunk_blocks) clipped to
+    m_total): every (sample, 64-row stage) is reduced exactly once, and no CTA is launched without work."""
+    import numpy as np
+    pair, n_chunks, cb, per, groups = plan
+    m_total = (M + 63) // 64
+    units = S * n_chunks
+    n_tiles = (N + 127) // 128
+    tiles = n_tiles * ((K + 127) // 128)
+    assert 1 <= groups <= 65535 and n_chunks >= 1 and cb >= 1
+    assert per == (units + groups - 1) // groups                     # what the kernel derives from gridDim.z
+    z = np.arange(groups)
+    s_begin, s_end = z * per, np.minimum(z * per + per, units)
+    assert (s_begin < s_end).all(), "a CTA group without work"
+    assert s_begin[0] == 0 and s_end[-1] == units and (s_begin[1:] == s_end[:-1]).all()
+    u = np.arange(units)
+    s, mb0 = u // n_chunks, (u % n_chunks) * cb
+    nb = np.minimum(cb, m_total - mb0)
+    assert (nb >= 1).all(), "an empty chunk"
+    diff = np.zeros((S, m_total + 1), dtype=np.int64)
+    np.add.at(diff, (s, mb0), 1)
+    np.add.at(diff, (s, mb0 + nb), -1)
+    assert (np.cumsum(diff, axis=1)[:, :m_total] == 1).all(), "a stage reduced twice or never"
+    rule = n_tiles >= 2 and tiles * groups >= 2 * sms
+    if forced_pair is None:
+        assert pair == int(rule)
+    else:
+        assert pair == forced_pair and (not pair or n_tiles >= 2)
+
+
+def test_wgrad_plans_reduce_every_stage_exactly_once():
+    """sampled_gemm_tma.cu: wgrad_plan, the plan wgrad_plan_and_launch runs (bnn_debug_wgrad_plan, host arithmetic).  Over
+    a sweep of M (ragged, 1 to 5 stages, thousands of rows), N and K on both sides of 128 and 256, and S from 1 to 64 on
+    148 SMs, and over forced plans: every (sample, stage) covered once, no empty CTA, groups <= 65535, CTA pairs only
+    under their rule.  Forced values the shape cannot take are refused, and the figures DESIGN states are pinned."""
+    try:
+        n_plans = n_pair = n_multi = 0
+        chunk_stats = set()
+        for M in (1, 63, 64, 100, 150, 250, 300, 777, 1000, 2100, 2304, 4100, 8192):
+            for N in (4, 100, 128, 132, 256, 260, 512):
+                for K in (4, 128, 132, 256, 288, 1152):
+                    for S in (1, 2, 5, 16, 64):
+                        rc, plan = _wgrad_plan(M, N, K, S)
+                        assert rc == 0
+                        _assert_wgrad_plan_covers(M, N, K, S, plan)
+                        m_total, n_chunks, cb = (M + 63) // 64, plan[1], plan[2]
+                        assert n_chunks <= max(1, min((m_total + 3) // 4, 64))   # the cost model's chunk limit
+                        chunk_stats.add((m_total, n_chunks, cb, m_total - (n_chunks - 1) * cb))
+                        n_plans, n_pair, n_multi = n_plans + 1, n_pair + plan[0], n_multi + (plan[3] > 1)
+        assert n_plans > 2000 and n_pair >= 10 and n_multi > 100
+        assert (5, 2, 3, 2) in chunk_stats                        # m_total = 5 is cut 3 + 2: units may be < 4 stages
+        # forced plans, including ones the cost model never picks (every sample's stages a chunk of their own, one CTA
+        # group walking every unit, units that cross sample boundaries)
+        forced = [((1000, 260, 100, 5), (1, 4, 3)), ((1000, 260, 100, 5), (0, 4, 3)), ((1000, 260, 100, 5), (1, 1, 5)),
+                  ((1000, 260, 100, 5), (0, 16, 1)), ((2100, 136, 96, 7), (1, 4, 3)), ((2100, 136, 96, 7), (0, 33, 2)),
+                  ((300, 128, 64, 3), (0, 2, 6)), ((4100, 512, 32, 64), (1, 65, 8)), ((700, 260, 96, 3), (1, 2, 3))]
+        for (M, N, K, S), (pair, n_chunks, per) in forced:
+            assert _C.lib().bnn_debug_force_wgrad_plan(pair, n_chunks, per) == 0
+            rc, plan = _wgrad_plan(M, N, K, S)
+            assert rc == 0, _C.lib().bnn_last_error_string()
+            assert (plan[0], plan[1], plan[3]) == (pair, n_chunks, per), ((M, N, K, S), plan)
+            _assert_wgrad_plan_covers(M, N, K, S, plan, forced_pair=pair)
+        assert _C.lib().bnn_debug_force_wgrad_plan(-1, 3, -1) == 0       # one value forced, the others chosen
+        rc, plan = _wgrad_plan(2304, 64, 576, 8)
+        assert rc == 0 and plan[1] == 3
+        _assert_wgrad_plan_covers(2304, 64, 576, 8, plan)
+        # values the shape cannot take: refused with a message naming them, never another plan
+        for (M, N, K, S), (pair, n_chunks, per), word in [
+                ((1000, 128, 100, 5), (1, -1, -1), "pair"),              # one n-tile
+                ((300, 256, 64, 3), (-1, 4, -1), "n_chunks"),            # 5 stages in chunks of 2: 3 chunks, not 4
+                ((300, 256, 64, 3), (-1, 6, -1), "n_chunks"),            # more chunks than stages
+                ((300, 256, 64, 3), (-1, 2, 7), "units_per_cta"),        # more than S x n_chunks = 6 units
+                ((300, 256, 64, 12), (-1, 1, 5), "units_per_cta"),       # 3 groups of 5 units: the kernel would walk 4
+                ((64, 256, 64, 70000), (-1, 1, 1), "units_per_cta")]:    # 70000 groups
+            assert _C.lib().bnn_debug_force_wgrad_plan(pair, n_chunks, per) == 0
+            rc, _ = _wgrad_plan(M, N, K, S)
+            assert rc == 1 and word in _C.lib().bnn_last_error_string().decode(), ((M, N, K, S), rc)
+        for bad in [(2, -1, -1), (-1, 0, -1), (-1, -1, 0), (-2, -1, -1)]:
+            assert _C.lib().bnn_debug_force_wgrad_plan(*bad) == 1
+    finally:
+        _C.lib().bnn_debug_force_wgrad_plan(-1, -1, -1)
+    # the override is gone: the figures DESIGN states
+    tiles_ctas = lambda M, N, K, S: (_wgrad_plan(M, N, K, S)[1], ((N + 127) // 128) * ((K + 127) // 128))
+    plan, tiles = tiles_ctas(2304, 64, 576, 8)                   # C2 conv weight gradient
+    assert plan[0] == 0 and tiles * plan[4] == 120
+    plan, tiles = tiles_ctas(8192, 128, 1152, 16)                # C3 conv weight gradient
+    assert plan[0] == 0 and tiles * plan[4] == 144 and plan[3] == 1
+    plan, _ = tiles_ctas(1024, 4096, 4096, 2)                    # C4
+    assert plan[0] == 1
+    plan, _ = tiles_ctas(1024, 512, 1024, 16)                    # one CTA walks several samples
+    assert plan[0] == 0 and plan[3] > 1
