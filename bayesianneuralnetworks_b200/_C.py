@@ -154,6 +154,8 @@ _SIGNATURES = {
                                                           ctypes.c_uint32, ctypes.POINTER(bnn_rng), ctypes.c_void_p]),
     "bnn_debug_conv_transpose3d_phases": (ctypes.c_int, [ctypes.POINTER(bnn_conv3d_nhwc), ctypes.POINTER(ctypes.c_int32),
                                                          ctypes.c_int32]),
+    "bnn_conv_transpose2d_supported": (ctypes.c_int, [ctypes.POINTER(bnn_conv2d_nhwc)]),
+    "bnn_conv_transpose3d_supported": (ctypes.c_int, [ctypes.POINTER(bnn_conv3d_nhwc)]),
     "bnn_conv2d_weight_layout": (ctypes.c_int, [_c_f32p, _c_f32p, _c_f32p, _c_f32p, _c_f32p, ctypes.c_int32, ctypes.c_int32,
                                                 ctypes.c_int32, ctypes.c_void_p]),
     "bnn_conv2d_weight_unlayout": (ctypes.c_int, [_c_f32p, _c_f32p, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32,
@@ -163,6 +165,10 @@ _SIGNATURES = {
                                                   ctypes.POINTER(bnn_rng), ctypes.c_void_p]),
     "bnn_im2col_nhwc": (ctypes.c_int, [_c_f32p, _c_f32p, ctypes.POINTER(bnn_conv2d_nhwc), ctypes.c_int64, ctypes.c_void_p]),
     "bnn_col2im_nhwc": (ctypes.c_int, [_c_f32p, _c_f32p, ctypes.POINTER(bnn_conv2d_nhwc), ctypes.c_int64, ctypes.c_void_p]),
+    "bnn_flipout_split": (ctypes.c_int, [_c_f32p, ctypes.c_int32, _c_f32p, _c_f32p, _c_f32p, ctypes.c_int64, ctypes.c_int32,
+                                         ctypes.c_int64, ctypes.c_void_p]),
+    "bnn_flipout_combine": (ctypes.c_int, [_c_f32p, _c_f32p, _c_f32p, _c_f32p, ctypes.c_int32, ctypes.c_int64, ctypes.c_int32,
+                                           ctypes.c_int64, ctypes.c_void_p]),
     "bnn_kl_workspace_size": (ctypes.c_size_t, [ctypes.c_int32]),
     "bnn_kl": (ctypes.c_int, [ctypes.POINTER(bnn_kl_tensor), ctypes.c_int32, ctypes.c_void_p, _c_f32p, _c_f32p,
                               ctypes.c_void_p, ctypes.c_size_t, ctypes.c_void_p]),
@@ -462,6 +468,61 @@ def nchw_to_nhwc_bias_grad(dy, B, rho_b=None, eps_b=None, dmu_b=None, drho_b=Non
     with torch.cuda.device(dy.device):
         _call("bnn_nchw_to_nhwc_bias_grad", _ptr(dy), _ptr(out), R, B, N, P, _ptr(rho_b), _ptr(eps_b), _ptr(dmu_b),
               _ptr(drho_b), sample_begin, ctypes.byref(rng_b) if rng_b is not None else None, _stream())
+    _count()
+    return out
+
+
+def _channels_last(t):
+    """Whether a logical [n, C, *spatial] tensor's memory is channels-last ([n][spatial][C]) without gaps."""
+    return t.permute(0, *range(2, t.dim()), 1).is_contiguous()
+
+
+def _signs_for(a, sign):
+    require_cuda(a, sign)
+    if a.dim() < 3 or a.dtype != torch.float32 or not (a.is_contiguous() or _channels_last(a)):
+        raise ValueError("a must be a float32 [n, C, *spatial] tensor, NC(D)HW-contiguous or channels-last")
+    sign = _f32c(sign, "sign")
+    if sign.numel() != a.shape[0] * a.shape[1] or sign.device != a.device:
+        raise ValueError(f"sign must hold n x C = {a.shape[0]} x {a.shape[1]} values on {a.device}")
+    return sign
+
+
+def flipout_split(a, sign):
+    """(a in channels-last memory, sign[n][c] * a in channels-last memory) for a logical [n, C, *spatial] tensor `a` that
+    is NC(D)HW-contiguous or channels-last; the first is `a` itself when it already is channels-last.  One read of a."""
+    sign = _signs_for(a, sign)
+    n, C = a.shape[0], a.shape[1]
+    P = a.numel() // (n * C)
+    cl = _channels_last(a)
+    fmt = torch.channels_last if a.dim() == 4 else torch.channels_last_3d if a.dim() == 5 else None
+    def empty():
+        if fmt is not None:
+            return torch.empty(a.shape, device=a.device, dtype=torch.float32, memory_format=fmt)
+        return torch.empty((n,) + tuple(a.shape[2:]) + (C,), device=a.device, dtype=torch.float32).movedim(-1, 1)
+    a_cl = a if cl else empty()
+    sa_cl = empty()
+    with torch.cuda.device(a.device):
+        _call("bnn_flipout_split", _ptr(a), int(cl), _ptr(sign), None if cl else _ptr(a_cl), _ptr(sa_cl), n, C, P,
+              _stream())
+    _count()
+    return a_cl, sa_cl
+
+
+def flipout_combine(a, b, sign, channels_last):
+    """a + sign[n][c] * b for two channels-last logical [n, C, *spatial] tensors, written channels-last or
+    NC(D)HW-contiguous; bit-identical to torch's `a + b * sign`."""
+    sign = _signs_for(a, sign)
+    if b.shape != a.shape or not (_channels_last(a) and _channels_last(b)) or b.dtype != torch.float32:
+        raise ValueError("flipout_combine: a and b must be float32 channels-last tensors of one shape")
+    require_cuda(b)
+    n, C = a.shape[0], a.shape[1]
+    P = a.numel() // (n * C)
+    if channels_last:
+        out = torch.empty_like(a)
+    else:
+        out = torch.empty(a.shape, device=a.device, dtype=torch.float32)
+    with torch.cuda.device(a.device):
+        _call("bnn_flipout_combine", _ptr(a), _ptr(b), _ptr(sign), _ptr(out), int(channels_last), n, C, P, _stream())
     _count()
     return out
 
@@ -862,6 +923,17 @@ def _try_call(name, device, *args):
         return False
     _check(rc, name)
     _count()
+    return True
+
+
+def conv_transpose_supported(geom):
+    """Whether the transposed-convolution kernels take all three passes of this conv-view geometry (bnn_conv2d_nhwc or
+    bnn_conv3d_nhwc); host only, nothing is launched.  Raises for an inconsistent geometry."""
+    name = "bnn_conv_transpose3d_supported" if isinstance(geom, bnn_conv3d_nhwc) else "bnn_conv_transpose2d_supported"
+    rc = getattr(lib(), name)(ctypes.byref(geom))
+    if rc == _ERR_UNSUPPORTED:
+        return False
+    _check(rc, name)
     return True
 
 

@@ -10,7 +10,7 @@ import sys
 _HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(_HERE, "csrc")
 LIB_PATH = os.path.join(_HERE, "libbnn_b200.so")
-SOURCES = ["api.cu", "adam.cu", "ce.cu", "conv.cu", "elementwise.cu", "kl.cu", "prune.cu", "sampled_gemm.cu", "sampled_gemm_tma.cu"]
+SOURCES = ["api.cu", "adam.cu", "ce.cu", "conv.cu", "elementwise.cu", "flipout.cu", "kl.cu", "prune.cu", "sampled_gemm.cu", "sampled_gemm_tma.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-O3", "-lineinfo", "-std=c++17",

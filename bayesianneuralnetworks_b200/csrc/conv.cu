@@ -680,6 +680,24 @@ int bnn_sampled_conv_transpose3d_wgrad(const float* dy, const float* x, int64_t 
   return rc;
 }
 
+int bnn_conv_transpose2d_supported(const bnn_conv2d_nhwc* g) {
+  const int rc = check_geom(g, "bnn_conv_transpose2d_supported");
+  if (rc != BNN_OK) return rc;
+  // the forward's phase corners and the input / weight gradients' conv-view corners (conv_ok) in one predicate
+  if (!contract::conv_transpose_ok(contract::conv_geom_2d(*g)))
+    return fail(BNN_ERR_UNSUPPORTED, "bnn_conv_transpose2d_supported: needs Cin %% 32 == 0, Cout %% 32 == 0, stride <= 8 and "
+                                     "every phase and conv-view corner within the im2col descriptor's limits");
+  return BNN_OK;
+}
+
+int bnn_conv_transpose3d_supported(const bnn_conv3d_nhwc* g) {
+  const int rc = check_geom3d(g, "bnn_conv_transpose3d_supported");
+  if (rc != BNN_OK) return rc;
+  if (g->C % 32 != 0 || !contract::conv_transpose_ok(geom3d(g)))
+    return fail(BNN_ERR_UNSUPPORTED, "bnn_conv_transpose3d_supported: %s", kT3dLimits);
+  return BNN_OK;
+}
+
 int bnn_debug_conv_transpose3d_phases(const bnn_conv3d_nhwc* g, int32_t* out, int32_t max_phases) {
   const int rc = check_geom3d(g, "bnn_debug_conv_transpose3d_phases");
   if (rc != BNN_OK) return -rc;

@@ -742,10 +742,117 @@ class SampledConvTranspose3dImplicit(torch.autograd.Function):
         return (dx, dmu, drho, bg[0] if need_b else None, bg[1] if need_b else None) + (None,) * 8
 
 
-class CudnnConvTranspose3d(torch.autograd.Function):
-    """F.conv_transpose3d(x, w, b, ...) with cuDNN's TF32 switched to `tf32` in the forward AND the backward pass (autograd
-    runs the backward outside any context the forward was called in): the materialised-sample form of
-    NormalConvTranspose3d, which in fp32 mode must not round its operands to TF32."""
+class FlipoutContractionRefused(Exception):
+    """The transposed-convolution kernels do not take every pass of a Flipout call's geometry; raised by
+    FlipoutConvTransposeImplicit before anything has launched, so that the layer evaluates its composite instead."""
+
+
+class FlipoutConvTransposeImplicit(torch.autograd.Function):
+    """The Flipout transposed convolution with per-example signs R [n, Cout] and S [n, Cin] (nn.flipout):
+
+        y  = convT(x, mu) + R o convT(x o S, sigma),             sigma = 1e-10 + softplus(rho)
+        dx = convT^T(g, mu) + S o convT^T(R o g, sigma),  d mu = wgrad(g, x),  d sigma = wgrad(R o g, x o S),
+        d rho = d sigma * sigmoid(rho).
+
+    x: logical [n, Cin, H, W] (the 1-d layers: H = 1) or [n, Cin, D, H, W], NC(D)HW-contiguous or channels-last; weights
+    [Cin, Cout, *k].  Every contraction is one call of the transposed-convolution kernels with one sample and injected
+    eps = 0 (`zero`, [1, numel]), so the kernels' weight mu + sigma * eps is the given operand exactly: mu, or sigma
+    (computed once by the layout kernel) in the mean slot; the d mean slot of the sigma contraction's weight gradient is
+    d sigma.  The sign products and the layout changes around the contractions are two bandwidth passes,
+    bnn_flipout_split ((x, S) forward, (g, R) backward) and bnn_flipout_combine ((y_mu, y_sigma, R) forward,
+    (dx_mu, dx_sigma, S) backward), which also writes the NC(D)HW output.  TF32 only.  Whether the kernels take all
+    three passes of the geometry is asked once (bnn_conv_transpose{2,3}d_supported) before anything launches:
+    FlipoutContractionRefused when they do not, so that the layer evaluates its composite; a refusal after that is an
+    error."""
+
+    @staticmethod
+    def _passes(x, w_shape, stride, padding, output_padding, dilation):
+        """(geometry of the conv view, fwd, dgrad, wgrad, memory format) of this call's rank; fwd / dgrad / wgrad return
+        False when refused."""
+        rows, Cin, Cout, k = x.shape[0], w_shape[0], w_shape[1], tuple(w_shape[2:])
+        out = tuple(conv_transpose_out(n, kk, s, p, op, d) for n, kk, s, p, op, d in
+                    zip(x.shape[2:], k, stride, padding, output_padding, dilation))
+        if min(out) <= 0:
+            raise RuntimeError("flipout conv_transpose: empty output")
+        if x.dim() == 4:
+            geom = _C.conv_geom(rows, *out, Cout, *x.shape[2:], Cin, *k, stride, padding, dilation)
+            return (geom, _C.try_sampled_conv_transpose2d_fwd, _C.try_sampled_conv_transpose2d_dgrad,
+                    _C.try_sampled_conv_transpose2d_wgrad, torch.channels_last, out)
+        geom = _C.conv3d_geom(rows, *out, Cout, *x.shape[2:], Cin, k, stride, padding, dilation)
+
+        def dgrad(*args):                  # the 3-d predicate is one for the three passes: the forward has checked it
+            _C.sampled_conv_transpose3d_dgrad(*args)
+            return True
+
+        def wgrad(*args):
+            _C.sampled_conv_transpose3d_wgrad(*args)
+            return True
+        return geom, _C.try_sampled_conv_transpose3d_fwd, dgrad, wgrad, torch.channels_last_3d, out
+
+    @staticmethod
+    def forward(ctx, x, mu, rho, R, S, zero, stride, padding, output_padding, dilation, nchw_out):
+        for n, t in (("input", x), ("weight.mean", mu), ("weight.scale", rho), ("R", R), ("S", S)):
+            _check_f32_cuda(n, t)
+        if x.dim() not in (4, 5) or x.shape[1] != mu.shape[0] or mu.dim() != x.dim():
+            raise RuntimeError(f"flipout conv_transpose: input {tuple(x.shape)} does not match weight {tuple(mu.shape)}")
+        geom, fwd, _, _, fmt, out = FlipoutConvTransposeImplicit._passes(x, tuple(mu.shape), stride, padding,
+                                                                         output_padding, dilation)
+        # one predicate for the forward, input-gradient and weight-gradient kernels, asked before anything launches: in
+        # 2-d the forward's phase corners (divided by the stride) admit geometries whose conv view the gradients refuse
+        if not _C.conv_transpose_supported(geom):
+            raise FlipoutContractionRefused()
+        if x.data_ptr() % 16:                      # the kernels read 16-byte aligned tensors: a fresh copy is
+            x = x.clone()
+        spec = DrawSpec(0, 0, 0, eps=zero)
+        rng = spec.rng()
+        wl = _C.conv_weight_layout(mu.contiguous(), rho.contiguous())          # mean, sigma, scale in (o, taps, c) order
+        x_cl, xs_cl = _C.flipout_split(x, S)
+        shape = (x.shape[0], mu.shape[1]) + out
+        y_mu = torch.empty(shape, device=x.device, dtype=torch.float32, memory_format=fmt)
+        y_sigma = torch.empty(shape, device=x.device, dtype=torch.float32, memory_format=fmt)
+        if not (fwd(x_cl, 0, wl[0], wl[1], None, None, zero, None, y_mu, geom, 1, 0, rng, None) and
+                fwd(xs_cl, 0, wl[1], wl[1], None, None, zero, None, y_sigma, geom, 1, 0, rng, None)):
+            raise RuntimeError("flipout conv_transpose: the kernels refused a forward contraction of a geometry they accept")
+        ctx.save_for_backward(x_cl, xs_cl, wl, rho, R, S, zero)
+        ctx.meta = (geom, tuple(mu.shape), stride, padding, output_padding, dilation, not x.is_contiguous())
+        return _C.flipout_combine(y_mu, y_sigma, R, channels_last=not nchw_out)
+
+    @staticmethod
+    def backward(ctx, g):
+        x_cl, xs_cl, wl, rho, R, S, zero = ctx.saved_tensors
+        geom, w_shape, stride, padding, output_padding, dilation, x_channels_last = ctx.meta
+        _, _, dgrad, wgrad, fmt, _ = FlipoutConvTransposeImplicit._passes(x_cl, w_shape, stride, padding, output_padding,
+                                                                          dilation)
+        rng = DrawSpec(0, 0, 0, eps=zero).rng()
+        if g.data_ptr() % 16 or not (g.is_contiguous() or g.permute(0, *range(2, g.dim()), 1).is_contiguous()):
+            g = g.clone(memory_format=torch.contiguous_format)
+        g_cl, gr_cl = _C.flipout_split(g, R)
+        dx = dmu = drho = None
+        if ctx.needs_input_grad[0]:
+            dx_mu = torch.empty(x_cl.shape, device=g.device, dtype=torch.float32, memory_format=fmt)
+            dx_sigma = torch.empty(x_cl.shape, device=g.device, dtype=torch.float32, memory_format=fmt)
+            if not (dgrad(g_cl, wl[0], wl[1], zero, dx_mu, 0, geom, 1, 0, rng) and
+                    dgrad(gr_cl, wl[1], wl[1], zero, dx_sigma, 0, geom, 1, 0, rng)):
+                raise RuntimeError("flipout conv_transpose: the kernels refused the input gradient of a call whose forward "
+                                   "they ran")
+            dx = _C.flipout_combine(dx_mu, dx_sigma, S, channels_last=x_channels_last)
+        if ctx.needs_input_grad[1] or ctx.needs_input_grad[2]:
+            # d mean, d sigma and the (zero) d scale slot both calls accumulate into
+            acc = torch.zeros((3, wl.shape[1]), device=g.device, dtype=torch.float32)
+            if not (wgrad(g_cl, x_cl, 0, wl[2], zero, acc[0], acc[2], geom, 1, 0, rng) and
+                    wgrad(gr_cl, xs_cl, 0, wl[2], zero, acc[1], acc[2], geom, 1, 0, rng)):
+                raise RuntimeError("flipout conv_transpose: the kernels refused the weight gradient of a call whose "
+                                   "forward they ran")
+            grads = _C.conv_weight_unlayout(acc[:2], w_shape)
+            dmu, drho = grads[0], grads[1] * torch.sigmoid(rho)
+        return (dx, dmu, drho) + (None,) * 8
+
+
+class CudnnConvTranspose(torch.autograd.Function):
+    """F.conv_transposeNd(x, w, b, ...) (N from the rank of x) with cuDNN's TF32 switched to `tf32` in the forward AND the
+    backward pass (autograd runs the backward outside any context the forward was called in): the materialised-sample
+    form of NormalConvTranspose3d and the composite of the Flipout transposed layers, which in fp32 mode must not round
+    their operands to TF32."""
 
     @staticmethod
     def _tf32(flag, fn):
@@ -760,18 +867,21 @@ class CudnnConvTranspose3d(torch.autograd.Function):
     def forward(ctx, x, w, b, stride, padding, output_padding, groups, dilation, tf32):
         ctx.save_for_backward(x, w)
         ctx.meta = (b is not None, stride, padding, output_padding, groups, dilation, tf32)
-        return CudnnConvTranspose3d._tf32(tf32, lambda: torch.nn.functional.conv_transpose3d(
-            x, w, b, stride, padding, output_padding, groups, dilation))
+        op = getattr(torch.nn.functional, f"conv_transpose{x.dim() - 2}d")
+        return CudnnConvTranspose._tf32(tf32, lambda: op(x, w, b, stride, padding, output_padding, groups, dilation))
 
     @staticmethod
     def backward(ctx, gy):
         x, w = ctx.saved_tensors
         has_b, stride, padding, output_padding, groups, dilation, tf32 = ctx.meta
         mask = [ctx.needs_input_grad[0], ctx.needs_input_grad[1], has_b and ctx.needs_input_grad[2]]
-        gx, gw, gb = CudnnConvTranspose3d._tf32(tf32, lambda: torch.ops.aten.convolution_backward(
+        gx, gw, gb = CudnnConvTranspose._tf32(tf32, lambda: torch.ops.aten.convolution_backward(
             gy, x, w, [w.shape[1] * groups] if has_b else None, list(stride), list(padding), list(dilation), True,
             list(output_padding), groups, mask))
         return (gx, gw, gb if has_b else None) + (None,) * 6
+
+
+CudnnConvTranspose3d = CudnnConvTranspose      # the name NormalConvTranspose3d's materialised-sample path was written with
 
 
 # ------------------------------------------------------------------------------------------------

@@ -8,7 +8,8 @@ from .layers import (BayesianLinear, NormalLinear, BayesianConvNd, NormalConvNd,
                      NormalConv3d, NormalConvTransposeNd, NormalConvTranspose1d, NormalConvTranspose2d,
                      NormalConvTranspose3d)
 from .flipout import (FlipoutNormalLinear, FlipOutNormalConvNd, FlipOutNormalConv1d, FlipOutNormalConv2d,
-                      FlipOutNormalConv3d)
+                      FlipOutNormalConv3d, FlipOutNormalConvTransposeNd, FlipOutNormalConvTranspose1d,
+                      FlipOutNormalConvTranspose2d, FlipOutNormalConvTranspose3d)
 from .mvn import WeightMultivariateNormal, MultivariateNormalLinear
 from .loss import KLDivergence, Entropy
 from .elbo import MCSamples, mc_mean_loss
@@ -23,4 +24,6 @@ __all__ = [
     'NormalInverseGaussianLinear', 'MCDropoutLinear', 'MCDropoutConvNd', 'MCDropoutConv1d', 'MCDropoutConv2d',
     'MCDropoutConv3d', 'NormalInverseGaussianLoss', 'NormalInverseGaussianUncertainty',
     'NormalConvTransposeNd', 'NormalConvTranspose1d', 'NormalConvTranspose2d', 'NormalConvTranspose3d',
+    'FlipOutNormalConvTransposeNd', 'FlipOutNormalConvTranspose1d', 'FlipOutNormalConvTranspose2d',
+    'FlipOutNormalConvTranspose3d',
 ]

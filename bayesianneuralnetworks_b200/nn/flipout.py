@@ -18,6 +18,9 @@ signs are per example (conv.py:154-161).
   operand, tcgen05 MMAs; forward, input gradient and weight gradients), with the sign products and d stddev / d scale
   left to torch element-wise ops; everything else (3-d, grouped, odd channel counts, CPU tensors) evaluates the
   reference's composite with torch's convolutions.
+* FlipOutNormalConvTranspose1d / 2d / 3d: the transposed form the reference prepared (`transposed=True`) but never built,
+  on the transposed-convolution kernels, with the sign products and layout changes in two bandwidth kernels
+  (bnn_flipout_split / bnn_flipout_combine, functional.FlipoutConvTransposeImplicit).
 Their variational tensor is a WeightNormal, hence KLDivergence and PruneNormal treat them like every other Bayesian layer
 (the fused KL / prune kernels).
 """
@@ -25,10 +28,11 @@ import torch
 import torch.nn.functional as F
 from torch.distributions.normal import Normal
 
-from .. import runtime
-from ..functional import conv_implicit_eligible
+from .. import _C, runtime
+from ..functional import (CudnnConvTranspose, FlipoutContractionRefused, FlipoutConvTransposeImplicit,
+                          conv_implicit_eligible, conv_output_nchw)
 from ..utils.traversal import _pair, _single, _triple
-from .layers import NormalConvNd, NormalLinear
+from .layers import NormalConvNd, NormalConvTransposeNd, NormalLinear
 
 
 def _signs(*shape, device):
@@ -45,7 +49,8 @@ def set_fused_flipout_linear(flag=True):
 
 
 def set_flipout_conv_kernels(flag=True):
-    """False: FlipOutNormalConv1d / 2d evaluate the reference's composite with torch's convolutions on CUDA too."""
+    """False: FlipOutNormalConv1d / 2d and FlipOutNormalConvTranspose1d / 2d / 3d evaluate the reference's composite with
+    torch's convolutions on CUDA too."""
     _KERNEL_CONV["on"] = bool(flag)
 
 
@@ -205,3 +210,144 @@ class FlipOutNormalConv3d(FlipOutNormalConvNd):
 
     def forward(self, x, sample=True):
         return self._flipout(x, 3, sample)
+
+
+class FlipOutNormalConvTransposeNd(NormalConvTransposeNd):
+    """Flipout transposed convolution: the reference's FlipOutNormalConvNd takes `transposed` like BayesianConvNd but
+    never built the transposed forward; this one is
+
+        y = conv_transposeNd(x, mean) + R o conv_transposeNd(x o S, stddev),
+
+    with per-example signs (conv.py:154-161) R [B, out_channels, 1, ...] and S [B, in_channels, 1, ...], no bias, and the
+    geometry, validation and `output_size` of NormalConvTransposeNd.  CUDA, TF32, groups == 1, in_ and out_channels
+    multiples of 32 and a geometry the transposed-convolution kernels take: two contractions of those kernels per pass,
+    with the sign products and layout changes in two bandwidth kernels (functional.FlipoutConvTransposeImplicit).
+    Everything else — CPU tensors, fp32 mode (cuDNN's TF32 off in both passes), groups > 1, other channel counts,
+    geometry the kernels refuse, set_flipout_conv_kernels(False) — evaluates the composite with torch's
+    conv_transposeNd."""
+    _fused = False
+    _mc_composite = True  # per-example signs: S*B rows of the batched Monte-Carlo forward draw S*B sign sets
+
+    def __init__(self, in_channels, out_channels, kernel_size, stride, padding, output_padding, groups, dilation, prior):
+        super(FlipOutNormalConvTransposeNd, self).__init__(in_channels, out_channels, kernel_size, stride, padding,
+                                                           output_padding, groups, False, dilation, prior)
+
+    def sample(self, batch_size=1, additional_dims=()):
+        """R over the out_channels, then S over the in_channels.  FlipOutNormalConvNd.sample reads the two counts from
+        weight.size(0) and weight.size(1), which for a transposed weight [in_channels, out_channels // groups, *k] are
+        the in_channels and out_channels // groups: the wrong channels, and too few of them for groups > 1."""
+        self.R = _signs(batch_size, self.out_channels, *additional_dims, device=self.weight.device)
+        self.S = _signs(batch_size, self.in_channels, *additional_dims, device=self.weight.device)
+
+    @property
+    def sampled(self):
+        return (self.R, self.S)
+
+    def _kernel_path(self, x):
+        w = self.weight.mean
+        return (_KERNEL_CONV["on"] and x.is_cuda and x.dtype == torch.float32 and w.is_cuda and w.dtype == torch.float32
+                and runtime.precision() == _C.PREC_TF32 and self.groups == 1 and self.in_channels % 32 == 0
+                and self.out_channels % 32 == 0)
+
+    def _kernels(self, x, nd, output_padding):
+        """The kernel path; FlipoutContractionRefused when the kernels do not take the geometry."""
+        stride, padding, dilation = tuple(self.stride), tuple(self.padding), tuple(self.dilation)
+        mean, scale = self.weight.mean, self.weight.scale
+        if nd == 1:               # a 2-d transposed convolution with a height of one
+            x = x.unsqueeze(2)
+            shape4 = (mean.shape[0], mean.shape[1], 1, mean.shape[2])
+            mean, scale = mean.view(shape4), scale.view(shape4)
+            stride, padding, output_padding, dilation = ((1, stride[0]), (0, padding[0]), (0, output_padding[0]),
+                                                         (1, dilation[0]))
+        nchw_out = conv_output_nchw(x)
+        # output_padding >= stride (dilation > stride): zero input rows appended, as in NormalConvTransposeNd
+        extra = [op // s for op, s in zip(output_padding, stride)]
+        if any(extra):
+            pad = []
+            for e in reversed(extra):
+                pad += [0, e]
+            x = F.pad(x, pad)
+            output_padding = tuple(op % s for op, s in zip(output_padding, stride))
+        if not (x.is_contiguous() or x.permute(0, *range(2, x.dim()), 1).is_contiguous()):
+            x = x.contiguous()
+        zero = getattr(self, "_zero_eps", None)
+        if zero is None or zero.device != mean.device or zero.numel() != mean.numel():
+            zero = torch.zeros(1, mean.numel(), device=mean.device, dtype=torch.float32)
+            self._zero_eps = zero
+        n = x.shape[0]
+        R = self.R.reshape(n, -1).to(x.device, torch.float32).contiguous()
+        S = self.S.reshape(n, -1).to(x.device, torch.float32).contiguous()
+        y = FlipoutConvTransposeImplicit.apply(x, mean, scale, R, S, zero, stride, padding, output_padding, dilation,
+                                               nchw_out)
+        return y.squeeze(2) if nd == 1 else y
+
+    def _composite(self, x, output_padding):
+        """The reference's form with torch's conv_transposeNd; cuDNN's TF32 follows the precision mode."""
+        tf32 = runtime.precision() == _C.PREC_TF32
+        args = (tuple(self.stride), tuple(self.padding), tuple(output_padding), self.groups, tuple(self.dilation), tf32)
+        R, S = self.R.to(x.device), self.S.to(x.device)
+        out = CudnnConvTranspose.apply(x, self.weight.mean, None, *args)
+        y = out + CudnnConvTranspose.apply(x * S.expand_as(x), self.weight.stddev, None, *args) * R.expand_as(out)
+        return y.contiguous() if conv_output_nchw(x) else y
+
+    def _flipout(self, x, nd, sample, output_size):
+        output_padding = self._output_padding(x, output_size)
+        _, x, _ = runtime.mc_expand_rows(x)
+        if sample:
+            self.sample(x.size(0), (1,) * nd)
+        else:
+            # the signs of an earlier forward (or sample(B, (1,) * nd)); the draw at construction has no spatial dims
+            n, ones = x.size(0), (1,) * nd
+            R, S = getattr(self, "R", None), getattr(self, "S", None)
+            if (R is None or S is None or tuple(R.shape) != (n, self.out_channels) + ones
+                    or tuple(S.shape) != (n, self.in_channels) + ones):
+                have = "no signs" if R is None or S is None else f"R {tuple(R.shape)} and S {tuple(S.shape)}"
+                raise RuntimeError(f"forward(sample=False) reuses the signs of an earlier forward, which must be "
+                                   f"R {(n, self.out_channels) + ones} and S {(n, self.in_channels) + ones} for this "
+                                   f"batch of {n} examples; the layer holds {have}")
+        if self._kernel_path(x):
+            try:
+                return self._kernels(x, nd, output_padding)
+            except FlipoutContractionRefused:
+                pass
+        return self._composite(x, output_padding)
+
+
+class FlipOutNormalConvTranspose1d(FlipOutNormalConvTransposeNd):
+    """torch.nn.ConvTranspose1d's constructor order without `bias` — evaluated as a 2-d transposed convolution with a
+    height of one on the kernel path."""
+
+    def __init__(self, in_channels, out_channels, kernel_size, stride=1, padding=0, output_padding=0, groups=1,
+                 dilation=1, prior=Normal(0, .1)):
+        super(FlipOutNormalConvTranspose1d, self).__init__(in_channels, out_channels, _single(kernel_size),
+                                                           _single(stride), _single(padding), _single(output_padding),
+                                                           groups, _single(dilation), prior)
+
+    def forward(self, x, sample=True, output_size=None):
+        return self._flipout(x, 1, sample, output_size)
+
+
+class FlipOutNormalConvTranspose2d(FlipOutNormalConvTransposeNd):
+    """torch.nn.ConvTranspose2d's constructor order without `bias`."""
+
+    def __init__(self, in_channels, out_channels, kernel_size, stride=1, padding=0, output_padding=0, groups=1,
+                 dilation=1, prior=Normal(0, .1)):
+        super(FlipOutNormalConvTranspose2d, self).__init__(in_channels, out_channels, _pair(kernel_size), _pair(stride),
+                                                           _pair(padding), _pair(output_padding), groups, _pair(dilation),
+                                                           prior)
+
+    def forward(self, x, sample=True, output_size=None):
+        return self._flipout(x, 2, sample, output_size)
+
+
+class FlipOutNormalConvTranspose3d(FlipOutNormalConvTransposeNd):
+    """torch.nn.ConvTranspose3d's constructor order without `bias`."""
+
+    def __init__(self, in_channels, out_channels, kernel_size, stride=1, padding=0, output_padding=0, groups=1,
+                 dilation=1, prior=Normal(0, .1)):
+        super(FlipOutNormalConvTranspose3d, self).__init__(in_channels, out_channels, _triple(kernel_size),
+                                                           _triple(stride), _triple(padding), _triple(output_padding),
+                                                           groups, _triple(dilation), prior)
+
+    def forward(self, x, sample=True, output_size=None):
+        return self._flipout(x, 3, sample, output_size)

@@ -12,7 +12,7 @@ from torch.distributions.normal import Normal
 from torch.nn import init
 
 from .. import _C, runtime
-from ..functional import (ConvTranspose3dRefused, CudnnConvTranspose3d, SampledConv2d, SampledConv2dImplicit,
+from ..functional import (ConvTranspose3dRefused, CudnnConvTranspose, SampledConv2d, SampledConv2dImplicit,
                           SampledConvTranspose2d, SampledConvTranspose2dImplicit, SampledConvTranspose3dImplicit,
                           SampledLinear, conv_implicit_eligible, conv_output_nchw)
 from ..utils.traversal import _pair, _single, _triple
@@ -353,7 +353,7 @@ class NormalConvTranspose3d(_FusedBayesianLayer, NormalConvTransposeNd):
         b = self.bias.materialize(begin(spec_b), S) if self.bias is not None else None
         xs = x if shared else x.reshape((S, x.shape[0] // S) + tuple(x.shape[1:]))
         tf32 = runtime.precision() == _C.PREC_TF32
-        y = torch.cat([CudnnConvTranspose3d.apply(x if shared else xs[s], w[s], b[s] if b is not None else None, stride,
+        y = torch.cat([CudnnConvTranspose.apply(x if shared else xs[s], w[s], b[s] if b is not None else None, stride,
                                                   padding, output_padding, self.groups, dilation, tf32)
                        for s in range(S)], 0)
         return y.contiguous() if conv_output_nchw(x) else y

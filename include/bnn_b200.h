@@ -257,6 +257,14 @@ int bnn_sampled_conv_transpose3d_wgrad(const float* dy, const float* x, int64_t 
  * bnn_debug_conv_transpose_phases, each for d, h, w {rd, rh, rw, rows_d, rows_h, rows_w, taps_d, ...}.  Returns the
  * number of phases (may exceed max_phases) or a negative bnn_status. */
 int bnn_debug_conv_transpose3d_phases(const bnn_conv3d_nhwc* g, int32_t* out, int32_t max_phases);
+/* Host only: whether the transposed-convolution kernels take ALL THREE passes (fwd, dgrad, wgrad) of the conv-view
+ * geometry `g` — channel counts, strides, every phase corner of the forward and every conv-view corner of the gradients.
+ * In 2-d the entry points check these one pass at a time, and with stride >= 2 the forward's phase corners (divided by
+ * the stride) admit geometries whose conv view the gradients refuse; a caller that must not mix paths within one call
+ * asks here before launching anything.  Tensor alignment is the caller's (16-byte bases).  BNN_OK when taken,
+ * BNN_ERR_UNSUPPORTED when not, BNN_ERR_BAD_ARGUMENT for a NULL or inconsistent geometry.  No device needed. */
+int bnn_conv_transpose2d_supported(const bnn_conv2d_nhwc* g);
+int bnn_conv_transpose3d_supported(const bnn_conv3d_nhwc* g);
 /* OIHW parameters [Cout][Cg][taps] -> (o, kh, kw, c) order: mu_p, and optionally sigma_p = 1e-10 + softplus(rho) and
  * rho_p (NULL to skip); the inverse for `n_arrays` arrays stored back to back (gradients of mean and scale). */
 int bnn_conv2d_weight_layout(const float* mu, const float* rho, float* mu_p, float* sigma_p, float* rho_p, int32_t Cout,
@@ -275,6 +283,21 @@ int bnn_nchw_to_nhwc_bias_grad(const float* dy, float* dy_nhwc, int64_t n_imgs, 
  *   dx[n][h][w][c] = sum of the dcol entries that read (n, h, w, c)  (gather form, overwrites dx) */
 int bnn_im2col_nhwc(const float* x, float* col, const bnn_conv2d_nhwc* g, int64_t n_imgs, void* stream);
 int bnn_col2im_nhwc(const float* dcol, float* dx, const bnn_conv2d_nhwc* g, int64_t n_imgs, void* stream);
+/* ---- Flipout sign passes (FlipOutNormalConvTranspose1d / 2d / 3d) ----
+ * Tensors of n images with C channels and P pixels per image (P = L, H*W or D*H*W); sign [n][C] of +-1.  "Channels-last"
+ * is [n][P][C], "NC(D)HW" is [n][C][P].  The arithmetic is torch's: the sign product is exact, then one fp32 add, so the
+ * outputs are bit-identical to `a * sign` and `a + b * sign`.  No size limit per image; 64-bit indexing.
+ *   split    reads a once ([n][C][P], or channels-last when a_channels_last != 0) and writes sa_cl = sign * a in
+ *            channels-last and, unless a already is channels-last (a_cl is then ignored and may be NULL), a_cl = a in
+ *            channels-last.
+ *   combine  reads channels-last a and b and writes out = a + sign * b, channels-last when out_channels_last != 0,
+ *            else NC(D)HW-contiguous.
+ * No allocation, no stream synchronisation.  BNN_ERR_BAD_ARGUMENT for NULL pointers, non-positive sizes or n*C*P beyond
+ * 64 bits. */
+int bnn_flipout_split(const float* a, int32_t a_channels_last, const float* sign, float* a_cl, float* sa_cl, int64_t n,
+                      int32_t C, int64_t P, void* stream);
+int bnn_flipout_combine(const float* a, const float* b, const float* sign, float* out, int32_t out_channels_last,
+                        int64_t n, int32_t C, int64_t P, void* stream);
 
 /* ---- KL divergence, closed form, many tensors per launch ----
  * For tensor t with posterior N(mu, sigma = 1e-10 + softplus(rho)) and scalar prior N(loc, scale):
